@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark: marching-tetrahedra extraction of a 512^3 fp32 volume on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n 512]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n 512] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one synthetic 512^3 volume per GPU (BASELINE.json configs[2]:
 CT-like fp32 volume, single isovalue, indexed mesh with normals).  N > 1 (torchrun, one rank per GPU):
@@ -9,6 +9,9 @@ weak scaling, each rank owns a 512-plane z-slab (+halo) of a (512*N) x 512 x 512
 independently and joins an NCCL all-gather of (n_verts, n_tris) -> global vertex offsets.
 
 Prints ONE JSON line (rank 0).  See DESIGN.md section 6 for what each key means.
+
+--dump-outputs DIR (rank 0): after the timed steps, the mesh of the last timed step as DIR/<name>.npy (see
+dump_outputs), so that two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -196,6 +199,28 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------ our arm
+DUMP_ROWS = 1 << 20     # vertex and triangle rows kept by --dump-outputs: 12.6 + 12.6 + 25.2 MB at most
+
+
+def dump_outputs(out_dir, counts, mesh):
+    """--dump-outputs: what a caller of the timed path receives -- the counts and the mesh mt3d_fetch() returns -- as
+    DIR/{counts,verts,normals,tris}.npy (float32 geometry, float64 counts and triangle vertex ids).  Above DUMP_ROWS
+    rows, verts / normals keep the same fixed sample of vertex rows and tris a fixed sample of triangle rows (seed 0,
+    in row order): two builds with the same counts are compared on the same rows."""
+    rng = np.random.default_rng(0)
+
+    def rows(n):
+        return np.arange(n) if n <= DUMP_ROWS else np.sort(rng.choice(n, DUMP_ROWS, replace=False))
+    vi, ti = rows(len(mesh["verts"])), rows(len(mesh["tris"]))
+    arrays = {"counts": np.array([counts.n_verts, counts.n_tris], dtype=np.float64),
+              "verts": mesh["verts"][vi], "tris": mesh["tris"][ti].astype(np.float64)}
+    if mesh["normals"] is not None:
+        arrays["normals"] = mesh["normals"][vi]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def c5_strong(eng, world, rank, dev, stream, n=2048, chunk=256, steps=2, warmup=1):
     """BASELINE configs[4]: the 2048^3 fp32 turbulence field (isovalue 0), STRONG scaling: the volume is fixed and rank r
     takes 1/N of the owner planes, walking them in chunks of `chunk` planes (the 32 GiB field is generated chunk by
@@ -395,6 +420,8 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     if clocks is not None:
         clocks["window"] = "%d untimed steps of the same loop directly before the timed region, and the timed region" % PRELOAD
+    if args.dump_outputs and rank == 0:                  # the context of the last timed step still holds its mesh
+        dump_outputs(args.dump_outputs, c, engines[(n_step[0] - 1) & 1].mt3d_fetch())
     tmax = torch.tensor([dev_ms], dtype=torch.float64, device=dev)
     tot = torch.tensor([c.n_tris, c.n_verts], dtype=torch.int64, device=dev)
     if world > 1:
@@ -582,7 +609,12 @@ def main():
     ap.add_argument("--e2e-slabs", type=int, default=8, help="slabs of the pipelined host-array call (1 = run + fetch)")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer leg and the CPU baseline (profiling runs)")
     ap.add_argument("--no-c5", action="store_true", help="skip the 2048^3 strong-scaling leg (c5_strong)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the mesh of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -236,9 +236,16 @@ def main():
                 g[k] = g[k].astype(np.int16)
             g["tris"] = g["tris"].astype(np.int32)
             g["final_tris"] = g["final_tris"].astype(np.int32)
+            # every final point is one of the raw interpolations: stored as its row in key_pos, which keeps the
+            # files under 1 MB (the tests' load() maps the rows back to positions)
+            first = {}
+            for i, p in enumerate(map(tuple, g["key_pos"])):
+                first.setdefault(p, i)
+            final_points = g.pop("final_points")
+            g["final_idx"] = np.array([first[tuple(p)] for p in final_points], dtype=np.int32)
             np.savez_compressed(os.path.join(HERE, "post3d_%s.npz" % name), **g)
             print(name, arr.shape, "raw", len(g["key_pos"]), len(g["tris"]), "after quantize", int(g["n_after_quantize"]),
-                  "after tiny", int(g["n_after_tiny"]), "final", g["final_points"].shape, g["final_tris"].shape)
+                  "after tiny", int(g["n_after_tiny"]), "final", final_points.shape, g["final_tris"].shape)
     if "seeded" in which:
         for name, (arr, value, seeds) in fields_seeded().items():
             g = run_seeded(arr, value, seeds)

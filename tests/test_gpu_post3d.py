@@ -17,6 +17,8 @@ FILES = sorted(glob.glob(os.path.join(GOLDEN, "post3d_*.npz")))
 
 def load(path):
     g = dict(np.load(path))
+    if "final_idx" in g:                       # final points stored as rows of the raw interpolations
+        g["final_points"] = g["key_pos"][g.pop("final_idx")]
     if "field" not in g:
         g["field"] = c1_golden()["field"]
     g["value"] = float(g["value"]) if "value" in g else 0.5

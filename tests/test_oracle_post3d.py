@@ -34,6 +34,8 @@ RESIDUE = {
 
 def load(path):
     g = dict(np.load(path))
+    if "final_idx" in g:                       # final points stored as rows of the raw interpolations
+        g["final_points"] = g["key_pos"][g.pop("final_idx")]
     if "field" not in g:
         g["field"] = c1_golden()["field"]
     for k in ("key_low", "key_high", "tris", "final_tris"):
