@@ -6,6 +6,9 @@
 #include <string.h>
 
 #include <algorithm>
+#include <climits>
+#include <limits>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -40,6 +43,8 @@ __device__ __forceinline__ unsigned long long order_key(double x) {
 //   k_bitplane_tma     : same stream staged through shared memory by TMA bulk copies (cp.async.bulk +
 //                        mbarrier full/empty ring): one producer lane + 8 consumer warps per CTA; consumers
 //                        read the staged samples bank-conflict-free and ballot straight into bit words.
+//   k_bitplane_generic_int / k_bitplane_tma_int : the same for uint8 / int16 / uint16 samples (integer thresholds; the
+//                        TMA consumers compare 4 / 2 samples per register and assemble words from lane bit groups).
 // ------------------------------------------------------------------------------------------------
 struct RowGeom {
   uint8_t* rowflag;
@@ -376,6 +381,255 @@ __global__ void __launch_bounds__((TMA_CONSUMER_WARPS + 1) * 32) k_bitplane_tma(
   minmax_commit(mn, mx, anynear, ctr);
 }
 
+// ---- integer samples (uint8 / int16 / uint16) ----------------------------------------------------
+// An integer sample f meets the fp64 predicates on its widened value exactly when it meets integer ones (IntThr, from
+// thresholds_int on the host):   f < v  <=>  f < thr;   v - r <= f <= v + r  <=>  nlo <= f <= nhi.
+struct IntThr {
+  int thr;            // ceil(v) clamped to [min(T), max(T) + 1]
+  int nlo, nhi;       // near samples, clipped to T's range; nlo > nhi: none
+};
+
+__device__ __forceinline__ void minmax_commit_int(int mn, int mx, MinMaxKeys* ctr) {
+  mn = __reduce_min_sync(0xffffffffu, mn);
+  mx = __reduce_max_sync(0xffffffffu, mx);
+  if (lane_id() == 0 && mn <= mx) {
+    atomicMin(&ctr->min_key, order_key((double)mn));
+    atomicMax(&ctr->max_key, order_key((double)mx));
+  }
+}
+
+// any shape: one warp converts 32 samples per step (the integer twin of k_bitplane_generic, also used for
+// CTR_BITPLANE=vec)
+template <typename T, int UNROLL, bool MINMAX>
+__global__ void __launch_bounds__(256) k_bitplane_generic_int(const T* __restrict__ f, unsigned nrows, int n2, int W,
+                                                              IntThr th, uint32_t* __restrict__ bits,
+                                                              uint32_t* __restrict__ nbits, RowGeom rg, MinMaxKeys* ctr) {
+  ctr_pdl_enter();
+  const unsigned lane = lane_id();
+  const unsigned nwords = nrows * (unsigned)W;
+  const unsigned warps = gridDim.x * (blockDim.x >> 5);
+  unsigned g = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  int mn = INT_MAX, mx = INT_MIN;
+  for (; g < nwords; g += warps * UNROLL) {
+    int val[UNROLL];
+    bool ok[UNROLL];
+#pragma unroll
+    for (int u = 0; u < UNROLL; ++u) {
+      unsigned gu = g + (unsigned)u * warps;
+      ok[u] = false;
+      val[u] = 0;
+      if (gu < nwords) {
+        unsigned row = gu / (unsigned)W;
+        int k = (int)(gu - row * (unsigned)W) * 32 + (int)lane;
+        if (k < n2) {
+          ok[u] = true;
+          val[u] = (int)__ldg(f + (size_t)row * n2 + k);
+        }
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < UNROLL; ++u) {
+      unsigned gu = g + (unsigned)u * warps;
+      if (gu < nwords) {                       // warp-uniform
+        unsigned wl = __ballot_sync(0xffffffffu, ok[u] && (val[u] < th.thr));
+        unsigned wn = __ballot_sync(0xffffffffu, ok[u] && (val[u] >= th.nlo) && (val[u] <= th.nhi));
+        if (lane == 0) {
+          bits[gu] = wl;
+          nbits[gu] = wn;
+          if (wn) flag_rows(rg, gu);
+        }
+        if (MINMAX && ok[u]) {
+          mn = min(mn, val[u]);
+          mx = max(mx, val[u]);
+        }
+      }
+    }
+  }
+  minmax_commit_int(mn, mx, ctr);
+}
+
+// SIMD view of one 32-bit register holding N = 4 (uint8) or 2 (int16 / uint16) samples.  Compares give 0 / all-ones
+// per sample; pack() turns that into N bits, sample q at bit q; zeros() is non-zero iff some sample of t is 0 (the
+// borrow can mark more samples than the zero ones, never a register without one).
+template <typename T>
+struct Simd;
+template <>
+struct Simd<uint8_t> {
+  static constexpr int N = 4, MIN = 0, MAX = 255;
+  __host__ __device__ static unsigned rep(int x) { return ((unsigned)x & 0xffu) * 0x01010101u; }
+  __device__ static __forceinline__ unsigned lt(unsigned a, unsigned b) { return __vcmpltu4(a, b); }
+  __device__ static __forceinline__ unsigned eq(unsigned a, unsigned b) { return __vcmpeq4(a, b); }
+  __device__ static __forceinline__ unsigned mn(unsigned a, unsigned b) { return __vminu4(a, b); }
+  __device__ static __forceinline__ unsigned mx(unsigned a, unsigned b) { return __vmaxu4(a, b); }
+  __device__ static __forceinline__ unsigned pack(unsigned m) { return ((m & 0x08040201u) * 0x01010101u) >> 24; }
+  __device__ static __forceinline__ unsigned zeros(unsigned t) { return (t - 0x01010101u) & ~t & 0x80808080u; }
+  __device__ static __forceinline__ int hmin(unsigned m) {
+    return (int)min(min(m & 0xffu, (m >> 8) & 0xffu), min((m >> 16) & 0xffu, m >> 24));
+  }
+  __device__ static __forceinline__ int hmax(unsigned m) {
+    return (int)max(max(m & 0xffu, (m >> 8) & 0xffu), max((m >> 16) & 0xffu, m >> 24));
+  }
+};
+template <>
+struct Simd<uint16_t> {
+  static constexpr int N = 2, MIN = 0, MAX = 65535;
+  __host__ __device__ static unsigned rep(int x) { return ((unsigned)x & 0xffffu) * 0x00010001u; }
+  // unsigned order = signed order with the sign bits flipped: one LOP3 in front of __vcmplts2 is shorter than __vcmpltu2
+  __device__ static __forceinline__ unsigned lt(unsigned a, unsigned b) { return __vcmplts2(a ^ 0x80008000u, b ^ 0x80008000u); }
+  __device__ static __forceinline__ unsigned eq(unsigned a, unsigned b) { return __vcmpeq2(a, b); }
+  __device__ static __forceinline__ unsigned mn(unsigned a, unsigned b) { return __vminu2(a, b); }
+  __device__ static __forceinline__ unsigned mx(unsigned a, unsigned b) { return __vmaxu2(a, b); }
+  __device__ static __forceinline__ unsigned pack(unsigned m) { return ((m & 0x00020001u) * 0x00010001u) >> 16; }
+  __device__ static __forceinline__ unsigned zeros(unsigned t) { return (t - 0x00010001u) & ~t & 0x80008000u; }
+  __device__ static __forceinline__ int hmin(unsigned m) { return (int)min(m & 0xffffu, m >> 16); }
+  __device__ static __forceinline__ int hmax(unsigned m) { return (int)max(m & 0xffffu, m >> 16); }
+};
+template <>
+struct Simd<int16_t> : Simd<uint16_t> {
+  static constexpr int MIN = -32768, MAX = 32767;
+  __device__ static __forceinline__ unsigned lt(unsigned a, unsigned b) { return __vcmplts2(a, b); }
+  __device__ static __forceinline__ unsigned mn(unsigned a, unsigned b) { return __vmins2(a, b); }
+  __device__ static __forceinline__ unsigned mx(unsigned a, unsigned b) { return __vmaxs2(a, b); }
+  __device__ static __forceinline__ int hmin(unsigned m) { return min((int)(short)(m & 0xffffu), (int)(short)(m >> 16)); }
+  __device__ static __forceinline__ int hmax(unsigned m) { return max((int)(short)(m & 0xffffu), (int)(short)(m >> 16)); }
+};
+
+// Stage-1 thresholds of the TMA kernel for 1- and 2-byte samples, replicated into every sample slot of a register.
+struct IntThrRep {
+  unsigned thr;       // f < thr per sample (thr clamped to max(T)) ...
+  unsigned lowall;    // ... or every sample is low (ceil(v) > max(T)): all ones
+  unsigned near0, near1;  // the (at most two) near values
+  int nnear;          // 0, 1 or 2
+};
+
+// The same ring, producer and PDL placement as k_bitplane_tma; the consumers read 16 bytes (16 / 8 samples) per lane and
+// load, compare 4 / 2 samples per instruction sequence (Simd<T>) and assemble each 32-bit word from the bit groups of
+// 2 / 4 neighbouring lanes.  A warp's 2 KiB of a stage is 4 passes of 512 bytes: pass q, lane l has the samples of word
+// q * WPP + l / GROUP, bits (l % GROUP) * S ...
+template <typename T, bool MINMAX>
+__global__ void __launch_bounds__((TMA_CONSUMER_WARPS + 1) * 32) k_bitplane_tma_int(const T* __restrict__ f, size_t nbytes,
+                                                                                      IntThrRep th, uint32_t* __restrict__ bits,
+                                                                                      uint32_t* __restrict__ nbits, RowGeom rg,
+                                                                                      MinMaxKeys* ctr, int TMA_STAGES, int l2_hint) {
+  typedef Simd<T> V;
+  constexpr int S = 16 / (int)sizeof(T);                        // samples per lane and pass
+  constexpr int GROUP = 32 / S;                                 // lanes per bit word
+  constexpr int WPP = 32 / GROUP;                               // words per warp and pass
+  constexpr int WARP_BYTES = TMA_CHUNK / TMA_CONSUMER_WARPS;
+  constexpr int PASSES = WARP_BYTES / 512;
+  constexpr int WPW = PASSES * WPP;                             // words per warp per stage
+  static_assert(PASSES * 512 == WARP_BYTES && WPW * 32 * (int)sizeof(T) == WARP_BYTES, "stage geometry");
+  extern __shared__ __align__(128) unsigned char smem[];
+  uint64_t* full = reinterpret_cast<uint64_t*>(smem + (size_t)TMA_STAGES * TMA_CHUNK);
+  uint64_t* empty = full + TMA_STAGES;
+  const unsigned warp = threadIdx.x >> 5, lane = lane_id();
+  if (threadIdx.x == 0) {
+    for (int s = 0; s < TMA_STAGES; ++s) {
+      mbar_init(&full[s], 1);
+      mbar_init(&empty[s], TMA_CONSUMER_WARPS);
+    }
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  __syncthreads();
+  const size_t nchunks = (nbytes + TMA_CHUNK - 1) / TMA_CHUNK;
+  const unsigned char* src = reinterpret_cast<const unsigned char*>(f);
+  if (warp == TMA_CONSUMER_WARPS) {
+    if (lane == 0) {
+      unsigned it = 0;
+      const uint64_t pol = l2_evict_first_policy();
+      for (size_t c = blockIdx.x; c < nchunks; c += gridDim.x, ++it) {
+        const int s = it % TMA_STAGES;
+        const unsigned ph = (it / TMA_STAGES) & 1u;
+        mbar_wait(&empty[s], ph ^ 1u);
+        size_t off = c * (size_t)TMA_CHUNK;
+        unsigned bytes = (unsigned)((nbytes - off) < (size_t)TMA_CHUNK ? (nbytes - off) : (size_t)TMA_CHUNK);
+        mbar_expect_tx(&full[s], bytes);
+        if (l2_hint) tma_bulk_g2s_hint(smem + (size_t)s * TMA_CHUNK, src + off, bytes, &full[s], pol);
+        else tma_bulk_g2s(smem + (size_t)s * TMA_CHUNK, src + off, bytes, &full[s]);
+      }
+    }
+    return;
+  }
+  const unsigned sub = lane % GROUP;
+  unsigned vmn = V::rep(V::MAX), vmx = V::rep(V::MIN);        // identities of V::mn / V::mx
+  unsigned it = 0;
+  ctr_pdl_enter();                                              // see k_bitplane_tma
+  for (size_t c = blockIdx.x; c < nchunks; c += gridDim.x, ++it) {
+    const int s = it % TMA_STAGES;
+    const unsigned ph = (it / TMA_STAGES) & 1u;
+    const size_t off = c * (size_t)TMA_CHUNK;
+    const unsigned bytes = (unsigned)((nbytes - off) < (size_t)TMA_CHUNK ? (nbytes - off) : (size_t)TMA_CHUNK);
+    const unsigned words_here = bytes / (32u * (unsigned)sizeof(T));
+    const uint4* sv = reinterpret_cast<const uint4*>(smem + (size_t)s * TMA_CHUNK + (size_t)warp * WARP_BYTES);
+    mbar_wait(&full[s], ph);
+    uint4 v[PASSES];
+#pragma unroll
+    for (int q = 0; q < PASSES; ++q) v[q] = sv[q * 32 + lane];   // 16 bytes per lane: conflict-free
+    __syncwarp();
+    if (lane == 0) mbar_arrive(&empty[s]);
+    const unsigned wbase = warp * WPW;
+    const size_t word0 = off / (32 * sizeof(T)) + wbase;
+    unsigned lo[PASSES], zacc = 0;
+    bool ok[PASSES];
+#pragma unroll
+    for (int q = 0; q < PASSES; ++q) {
+      // a partial last chunk: the words past its end are stale shared memory; their lanes contribute nothing
+      ok[q] = wbase + q * WPP + lane / GROUP < words_here;
+      const unsigned x[4] = {v[q].x, v[q].y, v[q].z, v[q].w};
+      unsigned b = 0, z = 0;
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        b |= V::pack(V::lt(x[e], th.thr) | th.lowall) << (e * V::N);
+        if (th.nnear > 0) z |= V::zeros(x[e] ^ th.near0);
+        if (th.nnear > 1) z |= V::zeros(x[e] ^ th.near1);
+        if (MINMAX && ok[q]) {
+          vmn = V::mn(vmn, x[e]);
+          vmx = V::mx(vmx, x[e]);
+        }
+      }
+      lo[q] = ok[q] ? b : 0u;
+      if (ok[q]) zacc |= z;
+    }
+#pragma unroll
+    for (int q = 0; q < PASSES; ++q) {
+      unsigned wl = lo[q] << (S * sub);
+#pragma unroll
+      for (int o = 1; o < GROUP; o <<= 1) wl |= __shfl_xor_sync(0xffffffffu, wl, o);
+      if (sub == 0 && ok[q]) bits[word0 + q * WPP + lane / GROUP] = wl;
+    }
+    unsigned nr[PASSES];
+#pragma unroll
+    for (int q = 0; q < PASSES; ++q) nr[q] = 0;
+    if (__any_sync(0xffffffffu, zacc != 0)) {                   // some sample of this warp is near: materialise the words
+#pragma unroll
+      for (int q = 0; q < PASSES; ++q) {
+        const unsigned x[4] = {v[q].x, v[q].y, v[q].z, v[q].w};
+        unsigned b = 0;
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+          unsigned m = V::eq(x[e], th.near0);
+          if (th.nnear > 1) m |= V::eq(x[e], th.near1);
+          b |= V::pack(m) << (e * V::N);
+        }
+        unsigned wn = ok[q] ? b << (S * sub) : 0u;
+#pragma unroll
+        for (int o = 1; o < GROUP; o <<= 1) wn |= __shfl_xor_sync(0xffffffffu, wn, o);
+        nr[q] = wn;
+        if (sub == 0 && ok[q] && wn) flag_rows(rg, (unsigned)(word0 + q * WPP + lane / GROUP));
+      }
+    }
+#pragma unroll
+    for (int q = 0; q < PASSES; ++q)
+      if (sub == 0 && ok[q]) nbits[word0 + q * WPP + lane / GROUP] = nr[q];
+  }
+  int mn = INT_MAX, mx = INT_MIN;
+  if (MINMAX) {
+    mn = V::hmin(vmn);
+    mx = V::hmax(vmx);
+  }
+  minmax_commit_int(mn, mx, ctr);
+}
+
 
 double key_to_double(unsigned long long k) {
   unsigned long long u = (k >> 63) ? (k & 0x7fffffffffffffffull) : ~k;
@@ -405,6 +659,26 @@ void thresholds<float>(double v, float& thr, float& nlo, float& nhi) {
   if ((double)nhi < v + r) nhi = nextafterf(nhi, INFINITY);
 }
 
+// Integer samples: the same predicates as thresholds<double> on the widened sample, as integer bounds (IntThr).
+template <typename T>
+IntThr thresholds_int(double v) {
+  const double tmin = (double)std::numeric_limits<T>::min(), tmax = (double)std::numeric_limits<T>::max();
+  IntThr t;
+  const double c = ceil(v);                     // f < v  <=>  f < ceil(v) for integer f (v = +-inf included)
+  t.thr = c > tmax ? (int)tmax + 1 : c < tmin ? (int)tmin : (int)c;
+  const double r = (1e-8 + 1e-5 * fabs(v)) * 1.0001;
+  const double a = ceil(std::max(v - r, tmin)), b = floor(std::min(v + r, tmax));
+  // v - r or v + r is NaN for v = +-inf (inf - inf): no sample is near, as in the fp64 compare
+  if (a <= b) {
+    t.nlo = (int)a;
+    t.nhi = (int)b;
+  } else {
+    t.nlo = 1;
+    t.nhi = 0;
+  }
+  return t;
+}
+
 enum BitplaneKind { BP_AUTO = 0, BP_GENERIC = 1, BP_VEC = 2, BP_TMA = 3 };
 
 BitplaneKind bitplane_choice() {
@@ -416,19 +690,8 @@ BitplaneKind bitplane_choice() {
   return BP_AUTO;
 }
 
-template <typename T, bool MINMAX>
-int launch_bitplane(ctr_ctx* ctx, const T* dfield, unsigned nrows, int n2, int W, int rb, int rc, double iso,
-                    uint32_t* bits, uint32_t* nbits, uint8_t* rowflag, MinMaxKeys* dctr, bool clear_rowflag = true,
-                    uint32_t* wordflag = nullptr) {
-  cudaStream_t st = ctx->stream;
-  T thr, nlo, nhi;
-  thresholds<T>(iso, thr, nlo, nhi);
-  const size_t nsamp = (size_t)nrows * n2;
-  const size_t nwords = (size_t)nrows * W;
-  const bool linear_ok = (n2 % 32 == 0) && (((uintptr_t)dfield) % 16 == 0);
-  BitplaneKind kind = bitplane_choice();
-  if (kind == BP_AUTO) kind = linear_ok ? BP_TMA : BP_GENERIC;
-  if (!linear_ok) kind = BP_GENERIC;
+// host-side pieces shared by the float and the integer launchers
+RowGeom row_geom(uint8_t* rowflag, uint32_t* wordflag, int W, int rb, int rc) {
   RowGeom rg;
   rg.rowflag = rowflag;
   rg.wordflag = wordflag;
@@ -440,11 +703,43 @@ int launch_bitplane(ctr_ctx* ctx, const T* dfield, unsigned nrows, int n2, int W
   rg.divRb.init((unsigned)rb);
   rg.rb = rb;
   rg.rc = rc;
+  return rg;
+}
+
+struct TmaKnobs {
+  int stages, ctas_per_sm, l2_hint;
+};
+const TmaKnobs& tma_knobs() {
+  static const TmaKnobs k = {getenv("CTR_BP_STAGES") ? atoi(getenv("CTR_BP_STAGES")) : TMA_STAGES_DEFAULT,
+                             getenv("CTR_BP_CTAS") ? atoi(getenv("CTR_BP_CTAS")) : 3,
+                             getenv("CTR_BP_L2HINT") ? atoi(getenv("CTR_BP_L2HINT")) : 1};   // L2 hint: 0.428 -> 0.418 ms per 512^3 step
+  return k;
+}
+
+// grid of the generic kernels: 256 threads, 4 words per warp and round, at most 8 blocks per SM
+int generic_blocks(const ctr_ctx* ctx, size_t nwords) {
+  const size_t need = (nwords + 8 * 4 - 1) / (8 * 4);
+  return (int)std::min<size_t>(std::max<size_t>(need, 1), (size_t)ctx->sm_count * 8);
+}
+
+template <typename T, bool MINMAX>
+std::enable_if_t<std::is_floating_point<T>::value, int> launch_bitplane(ctr_ctx* ctx, const T* dfield, unsigned nrows, int n2, int W, int rb, int rc, double iso,
+                    uint32_t* bits, uint32_t* nbits, uint8_t* rowflag, MinMaxKeys* dctr, bool clear_rowflag = true,
+                    uint32_t* wordflag = nullptr) {
+  cudaStream_t st = ctx->stream;
+  T thr, nlo, nhi;
+  thresholds<T>(iso, thr, nlo, nhi);
+  const size_t nsamp = (size_t)nrows * n2;
+  const size_t nwords = (size_t)nrows * W;
+  const bool linear_ok = (n2 % 32 == 0) && (((uintptr_t)dfield) % 16 == 0);
+  BitplaneKind kind = bitplane_choice();
+  if (kind == BP_AUTO) kind = linear_ok ? BP_TMA : BP_GENERIC;
+  if (!linear_ok) kind = BP_GENERIC;
+  const RowGeom rg = row_geom(rowflag, wordflag, W, rb, rc);
   if (clear_rowflag) CTR_CUDA(ctx, cudaMemsetAsync(rg.rowflag, 0, (size_t)nrows, st));
   if (kind == BP_TMA) {
-    static const int TMA_STAGES = getenv("CTR_BP_STAGES") ? atoi(getenv("CTR_BP_STAGES")) : TMA_STAGES_DEFAULT;
-    static const int ctas_per_sm = getenv("CTR_BP_CTAS") ? atoi(getenv("CTR_BP_CTAS")) : 3;
-    static const int l2_hint = getenv("CTR_BP_L2HINT") ? atoi(getenv("CTR_BP_L2HINT")) : 1;   // 0.428 -> 0.418 ms per 512^3 step
+    const TmaKnobs& kn = tma_knobs();
+    const int TMA_STAGES = kn.stages, ctas_per_sm = kn.ctas_per_sm, l2_hint = kn.l2_hint;
     const int smem = TMA_STAGES * TMA_CHUNK + 2 * TMA_STAGES * 8 + TMA_CONSUMER_WARPS * 32 * 4 + 64;
     // this header is compiled into two translation units (anonymous namespaces): each has its own kernel instances
     const int ti = CTR_BP_ATTR_BASE + (sizeof(T) == 4 ? 0 : 1) + (MINMAX ? 2 : 0);
@@ -463,8 +758,7 @@ int launch_bitplane(ctr_ctx* ctx, const T* dfield, unsigned nrows, int n2, int W
     int blocks = (int)std::min<size_t>(std::max<size_t>(need, 1), (size_t)ctx->sm_count * 8);
     k_bitplane_vec<T, 4, MINMAX><<<blocks, 256, 0, st>>>(dfield, nsamp, thr, nlo, nhi, bits, nbits, rg, dctr);
   } else {
-    size_t need = (nwords + 8 * 4 - 1) / (8 * 4);
-    int blocks = (int)std::min<size_t>(std::max<size_t>(need, 1), (size_t)ctx->sm_count * 8);
+    const int blocks = generic_blocks(ctx, nwords);
     k_bitplane_generic<T, 4, MINMAX><<<blocks, 256, 0, st>>>(dfield, nrows, n2, W, thr, nlo, nhi, bits, nbits, rg, dctr);
   }
   ctx->launches++;
@@ -472,5 +766,57 @@ int launch_bitplane(ctr_ctx* ctx, const T* dfield, unsigned nrows, int n2, int W
   return 0;
 }
 
+#ifdef CTR_BP_ATTR_INT_BASE
+// uint8 / int16 / uint16 samples, for translation units that define the attribute bits of these instances:
+// CTR_BP_ATTR_INT_BASE + 2 * (0 uint8, 1 int16, 2 uint16) + MINMAX.
+template <typename T, bool MINMAX>
+std::enable_if_t<std::is_integral<T>::value, int> launch_bitplane(ctr_ctx* ctx, const T* dfield, unsigned nrows, int n2, int W,
+                                                                   int rb, int rc, double iso, uint32_t* bits, uint32_t* nbits,
+                                                                   uint8_t* rowflag, MinMaxKeys* dctr, bool clear_rowflag = true,
+                                                                   uint32_t* wordflag = nullptr) {
+  static_assert(std::is_same<T, uint8_t>::value || std::is_same<T, int16_t>::value || std::is_same<T, uint16_t>::value,
+                "integer samples: uint8, int16, uint16");
+  cudaStream_t st = ctx->stream;
+  const IntThr th = thresholds_int<T>(iso);
+  const size_t nsamp = (size_t)nrows * n2;
+  const size_t nwords = (size_t)nrows * W;
+  // the TMA consumers compare against at most two near values: always so for these types (r < 0.66 inside their range)
+  const bool linear_ok = (n2 % 32 == 0) && (((uintptr_t)dfield) % 16 == 0) && (th.nlo > th.nhi || th.nhi - th.nlo <= 1);
+  BitplaneKind kind = bitplane_choice();
+  if (kind == BP_AUTO) kind = linear_ok ? BP_TMA : BP_GENERIC;
+  if (!linear_ok || kind == BP_VEC) kind = BP_GENERIC;
+  const RowGeom rg = row_geom(rowflag, wordflag, W, rb, rc);
+  if (clear_rowflag) CTR_CUDA(ctx, cudaMemsetAsync(rg.rowflag, 0, (size_t)nrows, st));
+  if (kind == BP_TMA) {
+    const TmaKnobs& kn = tma_knobs();
+    const int TMA_STAGES = kn.stages, ctas_per_sm = kn.ctas_per_sm, l2_hint = kn.l2_hint;
+    const int smem = TMA_STAGES * TMA_CHUNK + 2 * TMA_STAGES * 8 + 64;
+    const int ti = CTR_BP_ATTR_INT_BASE + 2 * (sizeof(T) == 1 ? 0 : std::is_signed<T>::value ? 1 : 2) + (MINMAX ? 1 : 0);
+    if (!(ctx->attr_mask & (1u << ti))) {
+      CTR_CUDA(ctx, cudaFuncSetAttribute(k_bitplane_tma_int<T, MINMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, 8 * TMA_CHUNK + 1024));
+      ctx->attr_mask |= 1u << ti;
+    }
+    typedef Simd<T> V;
+    const int tmax = (int)std::numeric_limits<T>::max();
+    IntThrRep tr;
+    tr.thr = V::rep(std::min(th.thr, tmax));
+    tr.lowall = th.thr > tmax ? 0xffffffffu : 0u;
+    tr.nnear = th.nlo > th.nhi ? 0 : th.nhi - th.nlo + 1;
+    tr.near0 = V::rep(th.nlo);
+    tr.near1 = V::rep(th.nhi);
+    const size_t nbytes = nsamp * sizeof(T);
+    const size_t nchunks = (nbytes + TMA_CHUNK - 1) / TMA_CHUNK;
+    int blocks = (int)std::min<size_t>(nchunks, (size_t)ctx->sm_count * ctas_per_sm);
+    ctr_launch_dep(k_bitplane_tma_int<T, MINMAX>, blocks, (TMA_CONSUMER_WARPS + 1) * 32, smem, st, dfield, nbytes, tr, bits, nbits,
+                   rg, dctr, (int)TMA_STAGES, (int)l2_hint);
+  } else {
+    const int blocks = generic_blocks(ctx, nwords);
+    k_bitplane_generic_int<T, 4, MINMAX><<<blocks, 256, 0, st>>>(dfield, nrows, n2, W, th, bits, nbits, rg, dctr);
+  }
+  ctx->launches++;
+  CTR_CUDA(ctx, cudaGetLastError());
+  return 0;
+}
+#endif
 
 }  // namespace

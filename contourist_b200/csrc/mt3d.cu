@@ -29,6 +29,7 @@
 #include <vector>
 
 #define CTR_BP_ATTR_BASE 0   // bits of ctr_ctx::attr_mask used by this file's bitplane kernels
+#define CTR_BP_ATTR_INT_BASE 9   // bits 9-14: its integer-sample bitplane kernels
 #include "bitplane.cuh"
 #include "tables.h"
 #include "uf_hash.cuh"
@@ -1669,7 +1670,8 @@ static int mt3d_check(ctr_ctx* ctx, const ctr_mt3d_params* p) {
   if (!(p->isovalue == p->isovalue)) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "isovalue is NaN");
   for (int a = 0; a < 3; ++a)
     if (p->delta[a] == 0.0) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "delta must be non-zero");
-  if (p->dtype != CTR_F32 && p->dtype != CTR_F64) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "dtype must be CTR_F32 or CTR_F64");
+  if (p->dtype != CTR_F32 && p->dtype != CTR_F64 && p->dtype != CTR_U8 && p->dtype != CTR_I16 && p->dtype != CTR_U16)
+    return ctr_fail(ctx, CTR_ERR_BAD_ARG, "dtype must be CTR_F32, CTR_F64, CTR_U8, CTR_I16 or CTR_U16");
   return 0;
 }
 
@@ -1677,8 +1679,14 @@ static int mt3d_dispatch(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
   if (out) memset(out, 0, sizeof *out);
   ctx->last_kind = 0;
-  if (p->dtype == CTR_F32) return run_typed<float>(ctx, p, out, phase);
-  return run_typed<double>(ctx, p, out, phase);
+  switch (p->dtype) {
+    case CTR_F32: return run_typed<float>(ctx, p, out, phase);
+    case CTR_F64: return run_typed<double>(ctx, p, out, phase);
+    case CTR_U8: return run_typed<uint8_t>(ctx, p, out, phase);
+    case CTR_I16: return run_typed<int16_t>(ctx, p, out, phase);
+    case CTR_U16: return run_typed<uint16_t>(ctx, p, out, phase);
+  }
+  return ctr_fail(ctx, CTR_ERR_BAD_ARG, "unknown dtype");
 }
 
 extern "C" int ctr_mt3d_run(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts* out) {
@@ -1789,8 +1797,14 @@ extern "C" int ctr_mt3d_select_seeded(ctr_ctx* ctx, const int32_t* seed_voxels, 
   if (ctx->last3_edited)
     return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has already been selected from or cleaned; run ctr_mt3d_run again");
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
-  if (p->dtype == CTR_F32) return select_typed<float>(ctx, p, seed_voxels, n_seeds, n_verts, n_tris, n_voxels);
-  return select_typed<double>(ctx, p, seed_voxels, n_seeds, n_verts, n_tris, n_voxels);
+  switch (p->dtype) {
+    case CTR_F32: return select_typed<float>(ctx, p, seed_voxels, n_seeds, n_verts, n_tris, n_voxels);
+    case CTR_F64: return select_typed<double>(ctx, p, seed_voxels, n_seeds, n_verts, n_tris, n_voxels);
+    case CTR_U8: return select_typed<uint8_t>(ctx, p, seed_voxels, n_seeds, n_verts, n_tris, n_voxels);
+    case CTR_I16: return select_typed<int16_t>(ctx, p, seed_voxels, n_seeds, n_verts, n_tris, n_voxels);
+    case CTR_U16: return select_typed<uint16_t>(ctx, p, seed_voxels, n_seeds, n_verts, n_tris, n_voxels);
+  }
+  return ctr_fail(ctx, CTR_ERR_BAD_ARG, "unknown dtype");
 }
 
 extern "C" int ctr_mt3d_clean(ctr_ctx* ctx, const ctr_clean_params* cp, ctr_clean_counts* out) {

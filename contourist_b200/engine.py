@@ -11,7 +11,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CTR_LIB") or os.path.join(_HERE, "libcontourist_b200.so")   # CTR_LIB: experiment builds
 
-F32, F64 = 0, 1
+F32, F64, U8, I16, U16 = 0, 1, 2, 3, 4
 FIELD_ON_DEVICE = 1
 GEOM_F64 = 2
 WANT_NORMALS = 4
@@ -24,6 +24,36 @@ MORPH = 128
 
 class EngineError(RuntimeError):
     pass
+
+
+# sample type codes (ctr_dtype) of the native sample types; the 2D and 4D runs take the float types only
+DTYPE_CODES = {np.dtype(np.float32): F32, np.dtype(np.float64): F64, np.dtype(np.uint8): U8, np.dtype(np.int16): I16,
+               np.dtype(np.uint16): U16}
+FLOAT_CODES = (F32, F64)
+
+
+def dtype_code(dtype, accepted=tuple(DTYPE_CODES.values())):
+    """ctr_dtype code of a native sample type (None -> float64), or None when the entry point does not read it."""
+    code = DTYPE_CODES.get(np.dtype(dtype))
+    return code if code in accepted else None
+
+
+def _host_field(field, ndim, accepted):
+    """C-contiguous array of a type the entry point reads natively; any other type is widened to float64."""
+    if dtype_code(field.dtype, accepted) is None:
+        field = field.astype(np.float64)
+    field = np.ascontiguousarray(field)
+    if field.ndim != ndim:
+        raise ValueError("%dD field expected" % ndim)
+    return field
+
+
+def _device_code(dtype, accepted):
+    code = dtype_code(dtype, accepted)
+    if code is None:
+        raise ValueError("device field of dtype %s: this entry point reads %s" % (
+            np.dtype(dtype), ", ".join(str(d) for d, c in DTYPE_CODES.items() if c in accepted)))
+    return code
 
 
 class Mt3dParams(ctypes.Structure):
@@ -232,19 +262,15 @@ class Engine(object):
     def _mt3d_params(self, field, value, origin, delta, flags, i_lo, i_hi, plane_offset, shape, dtype, vert_id_base):
         p = Mt3dParams()
         if isinstance(field, np.ndarray):
-            if field.dtype not in (np.float32, np.float64):
-                field = field.astype(np.float64)
-            field = np.ascontiguousarray(field)
-            if field.ndim != 3:
-                raise ValueError("3D field expected")
+            field = _host_field(field, 3, tuple(DTYPE_CODES.values()))
             self._keep = field
             p.field = field.ctypes.data
-            p.dtype = F32 if field.dtype == np.float32 else F64
+            p.dtype = dtype_code(field.dtype)
             shape = field.shape
             flags &= ~FIELD_ON_DEVICE
         else:
             p.field = int(field)
-            p.dtype = F32 if np.dtype(dtype) == np.float32 else F64
+            p.dtype = _device_code(dtype, tuple(DTYPE_CODES.values()))
             flags |= FIELD_ON_DEVICE
         p.flags = flags
         p.n0, p.n1, p.n2 = (int(s) for s in shape)
@@ -260,8 +286,10 @@ class Engine(object):
 
     def mt3d_run(self, field, value, origin=(0.0, 0.0, 0.0), delta=(1.0, 1.0, 1.0), flags=0,
                  i_lo=0, i_hi=None, plane_offset=0, shape=None, dtype=None, vert_id_base=0):
-        """field: C-contiguous numpy array [n0,n1,n2] float32/float64, or an integer device pointer
-        (then pass shape, dtype and FIELD_ON_DEVICE).  Returns Mt3dCounts."""
+        """field: C-contiguous numpy array [n0,n1,n2], or an integer device pointer (then pass shape, dtype and
+        FIELD_ON_DEVICE).  float32, float64, uint8, int16 and uint16 samples are read as they are (an integer field gives
+        exactly the result of its float64 copy); host arrays of any other type are widened to float64, device fields
+        of any other type raise ValueError.  Returns Mt3dCounts."""
         p, flags = self._mt3d_params(field, value, origin, delta, flags, i_lo, i_hi, plane_offset, shape, dtype, vert_id_base)
         c = Mt3dCounts()
         self.run_serial += 1
@@ -427,8 +455,8 @@ class Engine(object):
         from . import sharding
         if not (isinstance(field, np.ndarray) and field.ndim == 3 and field.flags["C_CONTIGUOUS"]):
             raise ValueError("mt3d_extract_host needs a C-contiguous 3D numpy array")
-        if field.dtype not in (np.float32, np.float64):
-            raise ValueError("float32 / float64 samples expected")
+        if dtype_code(field.dtype) is None:
+            raise ValueError("float32 / float64 / uint8 / int16 / uint16 samples expected")
         flags &= ~(FIELD_ON_DEVICE | WANT_CODES | NO_GEOMETRY)
         n0 = field.shape[0]
         own_a, own_b = (0, n0) if own is None else (int(own[0]), int(own[1]))
@@ -535,19 +563,15 @@ class Engine(object):
         from ._bindings import Mt2dParams, Mt2dCounts
         p = Mt2dParams()
         if isinstance(field, np.ndarray):
-            if field.dtype not in (np.float32, np.float64):
-                field = field.astype(np.float64)
-            field = np.ascontiguousarray(field)
-            if field.ndim != 2:
-                raise ValueError("2D field expected")
+            field = _host_field(field, 2, FLOAT_CODES)
             self._keep = field
             p.field = field.ctypes.data
-            p.dtype = F32 if field.dtype == np.float32 else F64
+            p.dtype = dtype_code(field.dtype)
             shape = field.shape
             flags &= ~FIELD_ON_DEVICE
         else:
             p.field = int(field)
-            p.dtype = F32 if np.dtype(dtype) == np.float32 else F64
+            p.dtype = _device_code(dtype, FLOAT_CODES)
             flags |= FIELD_ON_DEVICE
         lv = np.ascontiguousarray(np.asarray(levels, dtype=np.float64))
         self._keep_levels = lv
@@ -609,19 +633,15 @@ class Engine(object):
         from ._bindings import Mp4dParams, Mp4dCounts
         p = Mp4dParams()
         if isinstance(field, np.ndarray):
-            if field.dtype not in (np.float32, np.float64):
-                field = field.astype(np.float64)
-            field = np.ascontiguousarray(field)
-            if field.ndim != 4:
-                raise ValueError("4D field expected")
+            field = _host_field(field, 4, FLOAT_CODES)
             self._keep = field
             p.field = field.ctypes.data
-            p.dtype = F32 if field.dtype == np.float32 else F64
+            p.dtype = dtype_code(field.dtype)
             shape = field.shape
             flags &= ~FIELD_ON_DEVICE
         else:
             p.field = int(field)
-            p.dtype = F32 if np.dtype(dtype) == np.float32 else F64
+            p.dtype = _device_code(dtype, FLOAT_CODES)
             flags |= FIELD_ON_DEVICE
         p.flags = flags
         p.n0, p.n1, p.n2, p.n3 = (int(s) for s in shape)

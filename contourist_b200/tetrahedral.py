@@ -97,7 +97,10 @@ def initial_voxels(samples, value, end_points):
 
 
 class GridContour3d(object):
-    """Grid-coordinate engine front end (reference: GridContour + GridContour3d, tetrahedral.py:109-621)."""
+    """Grid-coordinate engine front end (reference: GridContour + GridContour3d, tetrahedral.py:109-621).
+
+    `function` may be an array of samples; uint8 / int16 / uint16 arrays reach the engine as they are (the result is
+    that of their float64 copy), other non-float types are widened to float64."""
 
     flatten = False
     smooth = None

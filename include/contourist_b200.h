@@ -48,7 +48,15 @@ typedef enum {
   CTR_ERR_OVERFLOW = -6
 } ctr_status;
 
-typedef enum { CTR_F32 = 0, CTR_F64 = 1 } ctr_dtype;
+/* Sample types.  Every entry point takes CTR_F32 and CTR_F64.  The integer types are accepted by the 3D extraction
+ * only (ctr_mt3d_run, ctr_mt3d_enqueue and, through the run it selects from, ctr_mt3d_select_seeded); the 2D and 4D
+ * runs reject them with CTR_ERR_BAD_ARG.  An integer field gives exactly the result of the same field widened to
+ * float64 (every uint8 / int16 / uint16 is exact in fp32 and fp64), so with fp32 geometry it also equals the float32
+ * run; stage 1 reads 1 or 2 bytes a sample instead of 4 or 8.  One known exception, in the float path: with
+ * CTR_WANT_MINMAX, a float32 / float64 field whose size in bytes is not a multiple of 16 KiB and that takes the TMA
+ * stage-1 kernel reports fmax = +inf (the padding of its partial last chunk enters the max); an integer field reports
+ * its true maximum. */
+typedef enum { CTR_F32 = 0, CTR_F64 = 1, CTR_U8 = 2, CTR_I16 = 3, CTR_U16 = 4 } ctr_dtype;
 
 /* flags */
 #define CTR_FIELD_ON_DEVICE 1u /* `field` is a device pointer (no H2D copy)                          */
@@ -103,7 +111,7 @@ CTR_API int ctr_wait_for(ctr_ctx* ctx, ctr_ctx* other);
  */
 typedef struct {
   const void* field;    /* n0*n1*n2 samples, host or device (CTR_FIELD_ON_DEVICE)                     */
-  int32_t dtype;        /* ctr_dtype of field                                                        */
+  int32_t dtype;        /* ctr_dtype of field (all five types)                                       */
   uint32_t flags;
   int64_t n0, n1, n2;   /* SAMPLES per axis; voxels have origins in [0, n-2]                          */
   double isovalue;
@@ -230,7 +238,7 @@ CTR_API int ctr_mt3d_clean(ctr_ctx* ctx, const ctr_clean_params* params, ctr_cle
  * lowmin = 1, (q, p) has lowmin = 0 (both exist when f(p) == f(q) == level).                        */
 typedef struct {
   const void* field;
-  int32_t dtype;
+  int32_t dtype;        /* CTR_F32 or CTR_F64 */
   uint32_t flags;          /* CTR_FIELD_ON_DEVICE, CTR_GEOM_F64, CTR_NO_GEOMETRY, CTR_WANT_MINMAX            */
   int64_t n0, n1;
   const double* levels;    /* host array, strictly increasing                                                */
@@ -282,7 +290,7 @@ CTR_API int ctr_mt2d_polylines_fetch(ctr_ctx* ctx, int32_t* level, uint8_t* clos
  *   pentatopes.py:336-348           removal of triangles with a zero-duration segment                    */
 typedef struct {
   const void* field;
-  int32_t dtype;
+  int32_t dtype;        /* CTR_F32 or CTR_F64 */
   uint32_t flags;
   int64_t n0, n1, n2, n3;
   double isovalue;
