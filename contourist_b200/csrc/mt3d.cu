@@ -629,6 +629,7 @@ __global__ void __launch_bounds__(CB_THREADS, CTR_CB_MINB) k_count_b(Grid<T> gin
   uint32_t any = 0, em = 0;
   uint2 slot = make_uint2(0u, 0u);
   bool flagged = false;
+  uint32_t r = 0;
   if (have) {
     gw = wlist[idx];
     slot = wslot[idx];
@@ -680,9 +681,25 @@ __global__ void __launch_bounds__(CB_THREADS, CTR_CB_MINB) k_count_b(Grid<T> gin
       t = we.ntri;
       em = we.emitting;
     }
-    const uint32_t r = v | (t << 8);
+    r = v | (t << 8);
     recc[idx] = r;                                        // record of list entry idx (k_scan walks the list, not the words)
-    if (r) atomicAdd(&tile_vt[(gw - word0) / CS_TILE], rec_vt(r));
+  }
+  // The tile aggregate, one atomic per tile and warp: a tile's entries are one contiguous chunk of the list, so the
+  // entries of a warp's tiles are runs of consecutive lanes (the lanes without an entry form the last run).  One atomic
+  // per word put ~100 atomics on the address of every tile: 0.322 against 0.312 ms per 512^3 step (B200, 1000 W).
+  {
+    const unsigned tix = have ? (gw - word0) / CS_TILE : 0xffffffffu;
+    const unsigned peers = __match_any_sync(0xffffffffu, tix);
+    unsigned long long sum = rec_vt(r);
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {                   // suffix sums inside the run
+      const unsigned long long u = __shfl_down_sync(0xffffffffu, sum, o);
+      if (lane + o < 32u && ((peers >> (lane + o)) & 1u)) sum += u;
+    }
+    if (have && (int)lane == __ffs(peers) - 1 && sum) atomicAdd(&tile_vt[tix], sum);
+  }
+  if (have) {
+    const unsigned v = r & 255u;
     if (v) {
       const uint2 dp = dir_pack(x);
       *reinterpret_cast<uint2*>(&wrec[gw].z) = dp;        // (.x, .y) = (vbase, tbase): k_scan
