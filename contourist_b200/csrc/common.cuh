@@ -64,9 +64,13 @@ struct ctr_ctx {
   size_t spec_v = 0, spec_t = 0, spec_own = 0, spec_cell = 0, last_own = 0, last_cell = 0, cover_own = 0, cover_cell = 0;
   size_t spec_w = 0, last_w = 0, cover_w = 0;   // interesting-word list of the split stage 2
   DevBuf wlist;
+  // 3D vertex values (ctr_mt3d_interpolate): rows and components of aux[43]; 0 = none since the last 3D run
+  size_t attr_rows = 0;
+  int attr_ncomp = 0;
 
   // 2D / 4D extra outputs are declared in their own translation units via these generic slots
-  DevBuf aux[48];            // 0-4, 32-35: 3D; 5-10: 2D; 12-26: 4D; 27-31: mesh passes
+  DevBuf aux[48];            // 0-4, 32-35, 41: 3D; 5-10: 2D; 12-26: 4D; 27-31: mesh passes; 36-40: 2D polylines;
+                             // 42-43: 3D vertex values (staged attribute field, values)
 };
 
 static inline int ctr_fail(ctr_ctx* ctx, int code, const char* what, const char* detail = "") {

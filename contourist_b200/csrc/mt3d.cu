@@ -1673,6 +1673,7 @@ int run_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts* out, int 
 
 #include "mt3d_select.cuh"
 #include "mt3d_clean.cuh"
+#include "attr3d.cuh"
 
 }  // namespace
 
@@ -1696,6 +1697,7 @@ static int mt3d_dispatch(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
   if (out) memset(out, 0, sizeof *out);
   ctx->last_kind = 0;
+  ctx->attr_ncomp = 0;                                 // vertex values of the previous run are gone
   switch (p->dtype) {
     case CTR_F32: return run_typed<float>(ctx, p, out, phase);
     case CTR_F64: return run_typed<double>(ctx, p, out, phase);
@@ -1845,4 +1847,52 @@ extern "C" int ctr_mt3d_clean(ctr_ctx* ctx, const ctr_clean_params* cp, ctr_clea
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
   if (ctx->last_flags & CTR_GEOM_F64) return clean_typed<double>(ctx, cp, out);
   return clean_typed<float>(ctx, cp, out);
+}
+
+extern "C" int ctr_mt3d_interpolate(ctr_ctx* ctx, const ctr_attr_params* a, int64_t* n_verts) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (!a || !a->field) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  if (a->ncomp < 1 || a->ncomp > 4) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "ncomp must be 1..4");
+  if (a->dtype != CTR_F32 && a->dtype != CTR_F64 && a->dtype != CTR_U8 && a->dtype != CTR_I16 && a->dtype != CTR_U16)
+    return ctr_fail(ctx, CTR_ERR_BAD_ARG, "dtype must be CTR_F32, CTR_F64, CTR_U8, CTR_I16 or CTR_U16");
+  if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
+    return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to interpolate on");
+  if (!(ctx->last_flags & CTR_WANT_KEYS)) return ctr_fail(ctx, CTR_ERR_STATE, "the run did not keep its keys: run with CTR_WANT_KEYS");
+  ctx->attr_ncomp = 0;                                 // the buffer is rewritten: earlier values are gone
+  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
+  const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
+  switch (p->dtype) {
+    case CTR_F32: return interp_typed<float>(ctx, a, n_verts);
+    case CTR_F64: return interp_typed<double>(ctx, a, n_verts);
+    case CTR_U8: return interp_typed<uint8_t>(ctx, a, n_verts);
+    case CTR_I16: return interp_typed<int16_t>(ctx, a, n_verts);
+    case CTR_U16: return interp_typed<uint16_t>(ctx, a, n_verts);
+  }
+  return ctr_fail(ctx, CTR_ERR_BAD_ARG, "unknown dtype");
+}
+
+static int interp_check(ctr_ctx* ctx) {
+  if (ctx->last_kind != 3 || !ctx->attr_ncomp) return ctr_fail(ctx, CTR_ERR_STATE, "no ctr_mt3d_interpolate since the last 3D run");
+  return 0;
+}
+
+extern "C" int ctr_mt3d_interpolate_fetch(ctr_ctx* ctx, void* values) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (!values) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  int rc = interp_check(ctx);
+  if (rc) return rc;
+  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
+  const size_t bytes = ctx->attr_rows * (size_t)ctx->attr_ncomp * ((ctx->last_flags & CTR_GEOM_F64) ? 8 : 4);
+  if (bytes) CTR_CUDA(ctx, cudaMemcpyAsync(values, ctx->aux[43].p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  CTR_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return 0;
+}
+
+extern "C" int ctr_mt3d_interpolate_device_ptr(ctr_ctx* ctx, void** values) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (!values) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  int rc = interp_check(ctx);
+  if (rc) return rc;
+  *values = ctx->aux[43].p;
+  return 0;
 }

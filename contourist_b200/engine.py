@@ -64,6 +64,11 @@ class Mt3dParams(ctypes.Structure):
                 ("vert_id_base", ctypes.c_int64)]
 
 
+class AttrParams(ctypes.Structure):
+    _fields_ = [("field", ctypes.c_void_p), ("dtype", ctypes.c_int32), ("flags", ctypes.c_uint32),
+                ("ncomp", ctypes.c_int32), ("reserved", ctypes.c_int32)]
+
+
 class CleanParams(ctypes.Structure):
     _fields_ = [("corner", ctypes.c_int64 * 3), ("divisions", ctypes.c_int32), ("flags", ctypes.c_uint32),
                 ("epsilon", ctypes.c_double), ("origin", ctypes.c_double * 3), ("delta", ctypes.c_double * 3)]
@@ -133,6 +138,12 @@ def load_library():
     lib.ctr_mt3d_select_seeded.restype = i32
     lib.ctr_mt3d_clean.argtypes = [vp, ctypes.POINTER(CleanParams), ctypes.POINTER(CleanCounts)]
     lib.ctr_mt3d_clean.restype = i32
+    lib.ctr_mt3d_interpolate.argtypes = [vp, ctypes.POINTER(AttrParams), ctypes.POINTER(i64)]
+    lib.ctr_mt3d_interpolate.restype = i32
+    lib.ctr_mt3d_interpolate_fetch.argtypes = [vp, vp]
+    lib.ctr_mt3d_interpolate_fetch.restype = i32
+    lib.ctr_mt3d_interpolate_device_ptr.argtypes = [vp, ctypes.POINTER(vp)]
+    lib.ctr_mt3d_interpolate_device_ptr.restype = i32
     lib.ctr_comm_unique_id.argtypes = [vp]
     lib.ctr_comm_unique_id.restype = i32
     lib.ctr_comm_init.argtypes = [vp, vp, i32, i32]
@@ -274,6 +285,7 @@ class Engine(object):
             flags |= FIELD_ON_DEVICE
         p.flags = flags
         p.n0, p.n1, p.n2 = (int(s) for s in shape)
+        self._shape3 = (p.n0, p.n1, p.n2)                             # the array mt3d_interpolate's fields match
         p.isovalue = float(value)
         for a in range(3):
             p.origin[a] = float(origin[a])
@@ -407,6 +419,47 @@ class Engine(object):
         c3.n_verts, c3.n_tris = int(c.n_verts), int(c.n_tris)
         self._last3 = (flags, c3)
         return c
+
+    def mt3d_interpolate(self, field, shape=None, dtype=None):
+        """Values of another field at the vertices of the last 3D run's mesh as it stands now (after a selection or
+        clean-up too), row for row with mt3d_fetch()'s vertices: a_low + ratio * (a_high - a_low) along each vertex's
+        edge, with the ratio of its position (ctr_mt3d_interpolate; the run needs WANT_KEYS).  field: numpy array of
+        the run's array shape [n0, n1, n2] or [n0, n1, n2, c] (c = 1..4), or an integer device pointer with shape and
+        dtype.  Host arrays of float32 / float64 / uint8 / int16 / uint16 are read as they are, other types are widened
+        to float64.  Returns [V] (or [V, c]) in the run's geometry type.  Values are not compacted by a later selection
+        or clean-up: interpolate after the last one."""
+        p = AttrParams()
+        codes = tuple(DTYPE_CODES.values())
+        if isinstance(field, np.ndarray):
+            if field.ndim not in (3, 4):
+                raise ValueError("field of shape (n0, n1, n2) or (n0, n1, n2, c) expected")
+            field = _host_field(field, field.ndim, codes)
+            p.field = field.ctypes.data
+            p.dtype = dtype_code(field.dtype)
+            shape = field.shape
+            p.flags = 0
+        else:
+            if shape is None or dtype is None:
+                raise ValueError("a device field needs shape and dtype")
+            p.field = int(field)
+            p.dtype = _device_code(dtype, codes)
+            p.flags = FIELD_ON_DEVICE
+        shape = tuple(int(s) for s in shape)
+        if len(shape) not in (3, 4) or shape[:3] != getattr(self, "_shape3", None):
+            raise ValueError("field of shape %r: the last 3D run's array is %r" % (shape, getattr(self, "_shape3", None)))
+        p.ncomp = shape[3] if len(shape) == 4 else 1
+        n = ctypes.c_int64()
+        self._check(self.lib.ctr_mt3d_interpolate(self.h, ctypes.byref(p), ctypes.byref(n)), "ctr_mt3d_interpolate")
+        flags, _ = self._last3
+        out = np.empty((int(n.value), int(p.ncomp)), np.float64 if flags & GEOM_F64 else np.float32)
+        self._check(self.lib.ctr_mt3d_interpolate_fetch(self.h, _ptr(out)), "ctr_mt3d_interpolate_fetch")
+        return out if len(shape) == 4 else out[:, 0]
+
+    def mt3d_interpolate_device_ptr(self):
+        """Device address of the last mt3d_interpolate()'s values (valid until the next run or interpolation)."""
+        v = ctypes.c_void_p()
+        self._check(self.lib.ctr_mt3d_interpolate_device_ptr(self.h, ctypes.byref(v)), "ctr_mt3d_interpolate_device_ptr")
+        return v.value
 
     def mt3d_fetch(self, verts=True, normals=None, tris=True, keys=None, codes=None, pinned=False):
         """Copy the last run's outputs to host arrays.  pinned=True: the arrays live in the engine's page-locked pool

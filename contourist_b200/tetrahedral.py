@@ -114,6 +114,12 @@ class GridContour3d(object):
     quantize_divisions = 10000                         # tetrahedral.py:190
     tiny_epsilon = 1e-4                                # tetrahedral.py:353
     prefetched = None                                  # (engine, run_serial, flags, counts) of a run search_for_endpoints() made
+    # vertex_fields: an array or callable, or a list of them, sampled on the field's grid (arrays may carry a trailing
+    # axis of up to 4 components); get_points_and_triangles() then leaves their values at the returned points in
+    # vertex_values (one array, or a list for a list), row for row (ctr_mt3d_interpolate)
+    vertex_fields = None
+    vertex_values = None
+    field_grid = None                                  # world drivers: the FunctionGrid that callables are sampled on
 
     def __init__(self, corner, function, value, segment_endpoints, linear_interpolate=True, callback=None,
                  origin=(0.0, 0.0, 0.0), delta=(1.0, 1.0, 1.0)):
@@ -137,14 +143,21 @@ class GridContour3d(object):
         assert self.dimension == 3
 
     def _field(self):
-        if isinstance(self.f, np.ndarray):
-            want = tuple(int(c) + 1 for c in self.corner)
-            if tuple(self.f.shape) != want:
-                raise ValueError("sample array has shape %r, corner %r needs %r" % (self.f.shape, tuple(self.corner), want))
-            return self.f
-        n = [int(c) + 1 for c in self.corner]
-        g = grid_field.FunctionGrid([0, 0, 0], [c for c in self.corner], [1, 1, 1], self.f)
-        assert tuple(g.grid_dimensions) == tuple(n), (tuple(g.grid_dimensions), n)
+        return self._samples_of(self.f)
+
+    def _samples_of(self, f, components=False):
+        """Samples of `f` on the grid of the isosurface's field: an array as it is (components=True: a trailing axis of
+        components allowed), a callable sampled at the grid points (on field_grid for the world-coordinate drivers)."""
+        want = tuple(int(c) + 1 for c in self.corner)
+        if isinstance(f, np.ndarray):
+            if tuple(f.shape) != want and not (components and f.ndim == 4 and tuple(f.shape[:3]) == want):
+                raise ValueError("sample array has shape %r, corner %r needs %r" % (f.shape, tuple(self.corner), want))
+            return f
+        if self.field_grid is not None:
+            g = self.field_grid
+            return grid_field.FunctionGrid(g.mins, g.maxes, g.delta, f).samples(1)
+        g = grid_field.FunctionGrid([0, 0, 0], [c for c in self.corner], [1, 1, 1], f)
+        assert tuple(g.grid_dimensions) == want, (tuple(g.grid_dimensions), want)
         return g.samples(0)
 
     def get_points_and_triangles(self, clean=True):
@@ -152,6 +165,8 @@ class GridContour3d(object):
             raise NotImplementedError("flatten / smooth (LP-based decimation, tetrahedral.py:217-351) are out of scope")
         eng = E.default_engine()
         flags = (E.GEOM_F64 if np.dtype(self.geometry_dtype) == np.float64 else 0) | (E.WANT_NORMALS if self.want_normals else 0)
+        if self.vertex_fields is not None:
+            flags |= E.WANT_KEYS                          # the values are interpolated along the vertices' keys
         field = self._field()
         identity = tuple(float(x) for x in self.origin) == (0.0, 0.0, 0.0) and tuple(float(x) for x in self.delta) == (1.0, 1.0, 1.0)
         # with post-processing the run is made in grid coordinates and ctr_mt3d_clean applies the transform last, like
@@ -177,6 +192,12 @@ class GridContour3d(object):
         elif self.reference_orientation:
             # surface_geometry.py:52-140 on the device mesh: one keep / reverse decision per edge-connected component
             self.components, self.flipped = eng.mt3d_orient_reference()
+        if self.vertex_fields is not None:
+            # after every pass that edits the mesh: the values line up with the points fetched below
+            many = isinstance(self.vertex_fields, (list, tuple))
+            vals = [eng.mt3d_interpolate(self._samples_of(f, components=True))
+                    for f in (self.vertex_fields if many else [self.vertex_fields])]
+            self.vertex_values = vals if many else vals[0]
         out = eng.mt3d_fetch()
         self.normals = out["normals"]
         points, triangles = out["verts"], out["tris"]
@@ -231,9 +252,10 @@ class Delta3DContour(object):
     def _configure(self, maker):
         "options set on this driver (before or after the maker was built) reach the maker"
         for name in ("post_process", "geometry_dtype", "want_normals", "reference_orientation", "quantize_divisions",
-                     "tiny_epsilon"):
+                     "tiny_epsilon", "vertex_fields"):
             if hasattr(self, name):
                 setattr(maker, name, getattr(self, name))
+        maker.field_grid = self.grid
         return maker
 
     def search_for_endpoints(self, skip=1):
@@ -243,7 +265,10 @@ class Delta3DContour(object):
 
     def get_points_and_triangles(self):
         # the engine applies grid_field.from_grid_coordinates (x*delta + mins) on the device
-        return self._configure(self.contour_maker).get_points_and_triangles()
+        maker = self._configure(self.contour_maker)
+        result = maker.get_points_and_triangles()
+        self.vertex_values = maker.vertex_values       # values of vertex_fields (when set) at the returned points
+        return result
 
 
 class TriangulatedIsosurfaces(Delta3DContour):

@@ -180,6 +180,35 @@ CTR_API int ctr_mt3d_orient_reference(ctr_ctx* ctx, int64_t* n_components, int64
 CTR_API int ctr_mt3d_select_seeded(ctr_ctx* ctx, const int32_t* seed_voxels, int64_t n_seeds, int64_t* n_verts,
                                    int64_t* n_tris, int64_t* n_voxels);
 
+/* Per-vertex values of another field (engine extension; the reference has none -- oracle/mt3d_values.py:vertex_values
+ * is the definition): every vertex of the LAST 3D run, as its mesh stands now (after ctr_mt3d_select_seeded / ctr_mt3d_clean
+ * too) and in the order ctr_mt3d_fetch returns it, gets
+ *   value[id][c] = a_low[c] + ratio * (a_high[c] - a_low[c])      (IEEE multiply, then add; no fused multiply-add)
+ * where low / high are the ends of the vertex's edge as its `lowmin` orders them, a = the attribute field's samples
+ * widened to the run's geometry type, and ratio is the one the vertex's position was made with (the run's samples and
+ * isovalue in the geometry type; 0.5 where |f_high - f_low| <= 1e-8; __fdividef in fp32 mode).  The world transform is
+ * not applied to values.  In grid coordinates the field of point coordinates (component c = index along axis c, axis 0
+ * global) gives the vertex positions bit for bit.
+ * The pass is driven by the device keys: the run must have used CTR_WANT_KEYS (else CTR_ERR_STATE, as for no 3D run or
+ * a CTR_NO_GEOMETRY run).  The run's field must still be valid when it was on the device.  The pass does not edit the
+ * mesh and may be called any number of times per run, with different fields; values computed before a selection or
+ * clean-up are NOT compacted with the mesh (interpolate after the last edit).  A host field is staged in a buffer of
+ * its own (the run's staged samples stay).  Synchronous on return.
+ *   _interpolate      : *n_verts (may be NULL) receives the number of vertices = rows of values
+ *   _interpolate_fetch: values [n_verts][ncomp] in the run's geometry type (float / double with CTR_GEOM_F64)
+ *   _interpolate_device_ptr: the same array on the device, valid until the next run or interpolation on this context */
+typedef struct {
+  const void* field;   /* the run's grid, component-last: [n0][n1][n2][ncomp], host or device (CTR_FIELD_ON_DEVICE);
+                          n0..n2 those of the run's array (a slab's planes for a slab run)                          */
+  int32_t dtype;       /* any ctr_dtype (F32, F64, U8, I16, U16), independent of the run's dtype                     */
+  uint32_t flags;      /* CTR_FIELD_ON_DEVICE                                                                         */
+  int32_t ncomp;       /* 1..4                                                                                        */
+  int32_t reserved;
+} ctr_attr_params;
+CTR_API int ctr_mt3d_interpolate(ctr_ctx* ctx, const ctr_attr_params* p, int64_t* n_verts);
+CTR_API int ctr_mt3d_interpolate_fetch(ctr_ctx* ctx, void* values);
+CTR_API int ctr_mt3d_interpolate_device_ptr(ctr_ctx* ctx, void** values);
+
 /* ---- multi-GPU: one process per GPU, z-slabs (SURVEY.md 8(e)) -----------------------------------------------------
  * Every rank runs ctr_mt3d_run on its slab (i_lo / i_hi / plane_offset) independently; NCCL carries only the counts and,
  * optionally, the mesh.  NCCL is bound at run time (the libnccl.so.2 already in the process, else the loader path).
