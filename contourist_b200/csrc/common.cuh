@@ -67,10 +67,14 @@ struct ctr_ctx {
   // 3D vertex values (ctr_mt3d_interpolate): rows and components of aux[43]; 0 = none since the last 3D run
   size_t attr_rows = 0;
   int attr_ncomp = 0;
+  // 3D connected components (ctr_mt3d_components): triangles and components of aux[44] / aux[45]; -1 = none since the
+  // last 3D run
+  int64_t comp_tris = 0, comp_count = -1;
 
   // 2D / 4D extra outputs are declared in their own translation units via these generic slots
   DevBuf aux[48];            // 0-4, 32-35, 41: 3D; 5-10: 2D; 12-26: 4D; 27-31: mesh passes; 36-40: 2D polylines;
-                             // 42-43: 3D vertex values (staged attribute field, values)
+                             // 42-43: 3D vertex values (staged attribute field, values);
+                             // 44-45: 3D connected components (triangle labels, component table)
 };
 
 static inline int ctr_fail(ctr_ctx* ctx, int code, const char* what, const char* detail = "") {

@@ -11,6 +11,7 @@
 //   k_o_best / k_o_pick : per component the triangle at that x with the largest |cross.x| (ties: smallest index);
 //   k_o_decide / k_o_flip : reverse the triangles of components whose seed has cross.x < 0.
 // Components are joined through shared EDGES, as in the reference (two sheets touching in one vertex stay apart).
+// components3d.cuh (ctr_mt3d_components) reuses the edge table and k_o_union to number and measure the components.
 #include <math.h>
 #include <string.h>
 
@@ -218,6 +219,8 @@ int orient_typed(ctr_ctx* ctx, int64_t* n_components, int64_t* n_flipped) {
   return 0;
 }
 
+#include "components3d.cuh"
+
 }  // namespace
 
 extern "C" int ctr_mt3d_orient_reference(ctr_ctx* ctx, int64_t* n_components, int64_t* n_flipped) {
@@ -227,4 +230,32 @@ extern "C" int ctr_mt3d_orient_reference(ctr_ctx* ctx, int64_t* n_components, in
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
   if (ctx->last_flags & CTR_GEOM_F64) return orient_typed<double>(ctx, n_components, n_flipped);
   return orient_typed<float>(ctx, n_components, n_flipped);
+}
+
+extern "C" int ctr_mt3d_components(ctr_ctx* ctx, int64_t* n_components) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (n_components) *n_components = 0;
+  ctx->comp_count = -1;                               // the buffers are rewritten: earlier results are gone
+  if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
+    return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to measure");
+  const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
+  if (p->i_lo != 0 || p->i_hi != p->n0 || p->vert_id_base != 0)
+    return ctr_fail(ctx, CTR_ERR_STATE, "components need a full-volume run with vert_id_base 0 (components cross slab faces)");
+  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
+  if (ctx->last_flags & CTR_GEOM_F64) return components_typed<double>(ctx, n_components);
+  return components_typed<float>(ctx, n_components);
+}
+
+extern "C" int ctr_mt3d_components_fetch(ctr_ctx* ctx, int32_t* tri_component, ctr_mt3d_component* components) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (ctx->last_kind != 3 || ctx->comp_count < 0)
+    return ctr_fail(ctx, CTR_ERR_STATE, "no ctr_mt3d_components since the last 3D run");
+  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
+  if (tri_component && ctx->comp_tris)
+    CTR_CUDA(ctx, cudaMemcpyAsync(tri_component, ctx->aux[44].p, (size_t)ctx->comp_tris * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  if (components && ctx->comp_count)
+    CTR_CUDA(ctx, cudaMemcpyAsync(components, ctx->aux[45].p, (size_t)ctx->comp_count * sizeof(ctr_mt3d_component),
+                                  cudaMemcpyDeviceToHost, ctx->stream));
+  CTR_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return 0;
 }

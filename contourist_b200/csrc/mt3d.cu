@@ -1698,6 +1698,7 @@ static int mt3d_dispatch(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts
   if (out) memset(out, 0, sizeof *out);
   ctx->last_kind = 0;
   ctx->attr_ncomp = 0;                                 // vertex values of the previous run are gone
+  ctx->comp_count = -1;                                // ... and so are its components
   switch (p->dtype) {
     case CTR_F32: return run_typed<float>(ctx, p, out, phase);
     case CTR_F64: return run_typed<double>(ctx, p, out, phase);

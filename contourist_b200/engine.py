@@ -69,6 +69,12 @@ class AttrParams(ctypes.Structure):
                 ("ncomp", ctypes.c_int32), ("reserved", ctypes.c_int32)]
 
 
+# ctr_mt3d_component (include/contourist_b200.h), 112 bytes: one row of Engine.mt3d_components()'s table
+COMPONENT_DTYPE = np.dtype([("n_tris", "<i8"), ("n_verts", "<i8"), ("n_edges", "<i8"), ("n_boundary_edges", "<i8"),
+                            ("n_nonmanifold_edges", "<i8"), ("first_tri", "<i8"), ("area", "<f8"), ("volume", "<f8"),
+                            ("lo", "<f8", (3,)), ("hi", "<f8", (3,))])
+
+
 class CleanParams(ctypes.Structure):
     _fields_ = [("corner", ctypes.c_int64 * 3), ("divisions", ctypes.c_int32), ("flags", ctypes.c_uint32),
                 ("epsilon", ctypes.c_double), ("origin", ctypes.c_double * 3), ("delta", ctypes.c_double * 3)]
@@ -138,6 +144,10 @@ def load_library():
     lib.ctr_mt3d_select_seeded.restype = i32
     lib.ctr_mt3d_clean.argtypes = [vp, ctypes.POINTER(CleanParams), ctypes.POINTER(CleanCounts)]
     lib.ctr_mt3d_clean.restype = i32
+    lib.ctr_mt3d_components.argtypes = [vp, ctypes.POINTER(i64)]
+    lib.ctr_mt3d_components.restype = i32
+    lib.ctr_mt3d_components_fetch.argtypes = [vp, vp, vp]
+    lib.ctr_mt3d_components_fetch.restype = i32
     lib.ctr_mt3d_interpolate.argtypes = [vp, ctypes.POINTER(AttrParams), ctypes.POINTER(i64)]
     lib.ctr_mt3d_interpolate.restype = i32
     lib.ctr_mt3d_interpolate_fetch.argtypes = [vp, vp]
@@ -419,6 +429,22 @@ class Engine(object):
         c3.n_verts, c3.n_tris = int(c.n_verts), int(c.n_tris)
         self._last3 = (flags, c3)
         return c
+
+    def mt3d_components(self):
+        """Edge-connected components of the last 3D run's mesh as it stands now (after a selection, clean-up or
+        orientation too): (tri_component [T] int32, row for row with mt3d_fetch()'s triangles, and table [C]
+        COMPONENT_DTYPE), numbered by smallest triangle index (ctr_mt3d_components).  Per component: triangle, vertex
+        and edge counts (n_verts - n_edges + n_tris is the Euler characteristic), boundary and non-manifold edges, fp64
+        area, signed enclosed volume (> 0 around a region below the isovalue on the raw mesh, >= 0 for closed
+        components after orientation) and the box lo / hi.  Not updated by a later selection or clean-up."""
+        n = ctypes.c_int64()
+        self._check(self.lib.ctr_mt3d_components(self.h, ctypes.byref(n)), "ctr_mt3d_components")
+        _, c = self._last3
+        labels = np.empty(int(c.n_tris), np.int32)
+        table = np.empty(int(n.value), COMPONENT_DTYPE)
+        self._check(self.lib.ctr_mt3d_components_fetch(self.h, _ptr(labels) if len(labels) else None,
+                                                       _ptr(table) if len(table) else None), "ctr_mt3d_components_fetch")
+        return labels, table
 
     def mt3d_interpolate(self, field, shape=None, dtype=None):
         """Values of another field at the vertices of the last 3D run's mesh as it stands now (after a selection or

@@ -120,6 +120,12 @@ class GridContour3d(object):
     vertex_fields = None
     vertex_values = None
     field_grid = None                                  # world drivers: the FunctionGrid that callables are sampled on
+    # measure_components: get_points_and_triangles() then leaves the edge-connected components of the returned mesh in
+    # triangle_components ([T] int32, row for row with the returned triangles) and component_table (engine.COMPONENT_DTYPE:
+    # counts, area, signed volume, box per component; ctr_mt3d_components)
+    measure_components = False
+    triangle_components = None
+    component_table = None
 
     def __init__(self, corner, function, value, segment_endpoints, linear_interpolate=True, callback=None,
                  origin=(0.0, 0.0, 0.0), delta=(1.0, 1.0, 1.0)):
@@ -198,6 +204,9 @@ class GridContour3d(object):
             vals = [eng.mt3d_interpolate(self._samples_of(f, components=True))
                     for f in (self.vertex_fields if many else [self.vertex_fields])]
             self.vertex_values = vals if many else vals[0]
+        if self.measure_components:
+            # after every pass that edits the mesh, like the values above
+            self.triangle_components, self.component_table = eng.mt3d_components()
         out = eng.mt3d_fetch()
         self.normals = out["normals"]
         points, triangles = out["verts"], out["tris"]
@@ -252,7 +261,7 @@ class Delta3DContour(object):
     def _configure(self, maker):
         "options set on this driver (before or after the maker was built) reach the maker"
         for name in ("post_process", "geometry_dtype", "want_normals", "reference_orientation", "quantize_divisions",
-                     "tiny_epsilon", "vertex_fields"):
+                     "tiny_epsilon", "vertex_fields", "measure_components"):
             if hasattr(self, name):
                 setattr(maker, name, getattr(self, name))
         maker.field_grid = self.grid
@@ -268,6 +277,8 @@ class Delta3DContour(object):
         maker = self._configure(self.contour_maker)
         result = maker.get_points_and_triangles()
         self.vertex_values = maker.vertex_values       # values of vertex_fields (when set) at the returned points
+        self.triangle_components = maker.triangle_components   # with measure_components: aligned with the triangles
+        self.component_table = maker.component_table
         return result
 
 

@@ -168,6 +168,44 @@ CTR_API int ctr_mt3d_device_ptrs(ctr_ctx* ctx, void** verts, void** normals, int
  * keep / reverse decision per component.  Fetch afterwards to get the rewound triangles.                            */
 CTR_API int ctr_mt3d_orient_reference(ctr_ctx* ctx, int64_t* n_components, int64_t* n_flipped);
 
+/* Connected components of the mesh with their size and topology (engine extension; the reference has none --
+ * oracle/mt3d_components.py:components is the definition).  Works on the LAST 3D run's device mesh as it stands now
+ * (after ctr_mt3d_select_seeded, ctr_mt3d_clean or ctr_mt3d_orient_reference too); it does not edit the mesh and may be
+ * called any number of times.  Synchronous on return.
+ *   - Components are EDGE-connected: two triangles are joined when they share an undirected vertex-id edge (the rule of
+ *     ctr_mt3d_orient_reference, whose n_components is the same number on every mesh).  Two sheets touching in one
+ *     vertex stay apart.
+ *   - Numbering: 0..C-1 in ascending order of each component's smallest triangle index (first_tri); deterministic.
+ *   - A vertex shared by k components counts in each of their n_verts, so n_verts - n_edges + n_tris is the
+ *     component's Euler characteristic (2 for a sphere, 0 for a torus, 1 for a disc cut by the volume's edge).  A
+ *     component is closed when n_boundary_edges == 0.
+ *   - area and volume are fp64 sums over its triangles (positions widened from the geometry type first), volume
+ *     relative to the component's box corner lo.  On the raw engine mesh (triangles wound towards the high side) a
+ *     closed component has volume > 0 when the region it encloses is below the isovalue and < 0 when it is above (a
+ *     blob brighter than its surroundings: negative).  After ctr_mt3d_orient_reference, or ctr_mt3d_clean with
+ *     CTR_CLEAN_ORIENT, every closed component faces outward and its volume is >= 0.  For an open component the value
+ *     is reported but is not an enclosed volume.
+ *   - The integer fields, first_tri and the box are exact.  area and volume are sums whose order may change between
+ *     calls: their last bits may differ.
+ *   - CTR_ERR_STATE: no 3D run or a CTR_NO_GEOMETRY run; a slab run (i_lo != 0 or i_hi != n0) or vert_id_base != 0; a
+ *     triangle id outside [0, n_verts) (e.g. after ctr_mt3d_offset_ids); _fetch with no ctr_mt3d_components since the
+ *     last run.  An empty mesh has 0 components.
+ *   _components      : *n_components (may be NULL) receives C
+ *   _components_fetch: tri_component [n_tris] (the component of every triangle, row for row with ctr_mt3d_fetch's
+ *                      triangles) and components [C]; either may be NULL.  These are the results of the last call: a
+ *                      later selection or clean-up does not update them.                                             */
+typedef struct {
+  int64_t n_tris, n_verts, n_edges;          /* faces, distinct vertices, distinct undirected edges of the component  */
+  int64_t n_boundary_edges;                  /* edges used by exactly one triangle                                     */
+  int64_t n_nonmanifold_edges;               /* edges used by three or more triangles                                  */
+  int64_t first_tri;                         /* smallest triangle index in the component (the numbering key)           */
+  double area;                               /* sum of |cross(b-a, c-a)| / 2                                           */
+  double volume;                             /* sum of (a-p) . ((b-p) x (c-p)) / 6, p = lo                             */
+  double lo[3], hi[3];                       /* bounding box of its vertices                                           */
+} ctr_mt3d_component;                        /* 112 bytes */
+CTR_API int ctr_mt3d_components(ctr_ctx* ctx, int64_t* n_components);
+CTR_API int ctr_mt3d_components_fetch(ctr_ctx* ctx, int32_t* tri_component, ctr_mt3d_component* components);
+
 /* Seeded extraction (SURVEY.md 8(f3)): restricts the LAST full-volume run's mesh to what the reference's tracker
  *   tetrahedral.py:443-469  expand_voxels / in_range  (flood fill over the 26-neighbourhood of border voxels)
  * reaches from the given start voxels (the output of find_initial_voxels, tetrahedral.py:396-441, which the binding
