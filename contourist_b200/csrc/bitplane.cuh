@@ -2,7 +2,6 @@
 // Rows are runs of the contiguous (last) axis; a row index decomposes as ((a*rb + b)*rc + c).
 #pragma once
 #include <math.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <algorithm>
@@ -38,13 +37,14 @@ __device__ __forceinline__ unsigned long long order_key(double x) {
 // Stage 1: field -> low bitplane (the only pass over the whole field; HBM-bound), plus the "any sample
 // near the isovalue" flag and optional min/max.  Near words are written with the low words; a word
 // that has a near sample also raises the (dilated) row flags that switch later stages to their exact paths.
+//   k_bitplane_tma     : rows a multiple of 32 samples, field 16-byte aligned: the volume is one linear stream, staged
+//                        through shared memory by TMA bulk copies (cp.async.bulk + mbarrier full/empty ring): one
+//                        producer lane + 8 consumer warps per CTA.  float / double consumers read the staged samples
+//                        bank-conflict-free and ballot straight into bit words; uint8 / int16 / uint16 consumers compare
+//                        4 / 2 samples per register and assemble words from lane bit groups.
 //   k_bitplane_generic : any shape (rows padded to whole words), one warp converts 32 samples per step.
-//   k_bitplane_vec     : rows a multiple of 32 samples: the volume is one linear stream; 128-bit loads.
-//   k_bitplane_tma     : same stream staged through shared memory by TMA bulk copies (cp.async.bulk +
-//                        mbarrier full/empty ring): one producer lane + 8 consumer warps per CTA; consumers
-//                        read the staged samples bank-conflict-free and ballot straight into bit words.
-//   k_bitplane_generic_int / k_bitplane_tma_int : the same for uint8 / int16 / uint16 samples (integer thresholds; the
-//                        TMA consumers compare 4 / 2 samples per register and assemble words from lane bit groups).
+// Both take float, double, uint8, int16 and uint16 samples.  Floats compare in T against thresholds<T>; integer samples
+// compare in int against thresholds_int<T>, which give the fp64 predicates on the widened sample exactly.
 // ------------------------------------------------------------------------------------------------
 struct RowGeom {
   uint8_t* rowflag;
@@ -77,14 +77,46 @@ __device__ __noinline__ void flag_rows(const RowGeom& rg, unsigned word) {
         }
 }
 
+// Float samples: f < thr is low, nlo <= f <= nhi is near (thresholds<T>).
 template <typename T>
-__device__ __forceinline__ void minmax_commit(T mn, T mx, bool anynear, MinMaxKeys* ctr) {
+struct FloatThr {
+  T thr, nlo, nhi;
+};
+
+// An integer sample f meets the fp64 predicates on its widened value exactly when it meets integer ones (IntThr, from
+// thresholds_int on the host):   f < v  <=>  f < thr;   v - r <= f <= v + r  <=>  nlo <= f <= nhi.
+struct IntThr {
+  int thr;            // ceil(v) clamped to [min(T), max(T) + 1]
+  int nlo, nhi;       // near samples, clipped to T's range; nlo > nhi: none
+};
+
+// What k_bitplane_generic compares a sample of type T in, and against: floats in T (fmin / fmax ignore NaN), integer
+// samples in int.
+template <typename T, bool FLOAT = std::is_floating_point<T>::value>
+struct Stage1 {
+  typedef T C;
+  typedef FloatThr<T> Thr;
+  static constexpr T TOP = INFINITY, BOTTOM = -INFINITY;      // identities of lo / hi
+  __device__ static __forceinline__ T lo(T a, T b) { return fmin(a, b); }
+  __device__ static __forceinline__ T hi(T a, T b) { return fmax(a, b); }
+};
+template <typename T>
+struct Stage1<T, false> {
+  typedef int C;
+  typedef IntThr Thr;
+  static constexpr int TOP = INT_MAX, BOTTOM = INT_MIN;
+  __device__ static __forceinline__ int lo(int a, int b) { return min(a, b); }
+  __device__ static __forceinline__ int hi(int a, int b) { return max(a, b); }
+};
+
+// One warp's min / max into the run's keys; lanes that saw no sample hold the identities (mn > mx).
+template <typename T>
+__device__ __forceinline__ void minmax_commit(T mn, T mx, MinMaxKeys* ctr) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     mn = fmin(mn, __shfl_xor_sync(0xffffffffu, mn, o));
     mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
   }
-  (void)anynear;
   if (lane_id() == 0) {
     if (mn <= mx) {
       atomicMin(&ctr->min_key, order_key((double)mn));
@@ -92,32 +124,42 @@ __device__ __forceinline__ void minmax_commit(T mn, T mx, bool anynear, MinMaxKe
     }
   }
 }
+__device__ __forceinline__ void minmax_commit(int mn, int mx, MinMaxKeys* ctr) {
+  mn = __reduce_min_sync(0xffffffffu, mn);
+  mx = __reduce_max_sync(0xffffffffu, mx);
+  if (lane_id() == 0 && mn <= mx) {
+    atomicMin(&ctr->min_key, order_key((double)mn));
+    atomicMax(&ctr->max_key, order_key((double)mx));
+  }
+}
 
-template <typename T, int UNROLL, bool MINMAX>
+template <typename T, bool MINMAX>
 __global__ void __launch_bounds__(256) k_bitplane_generic(const T* __restrict__ f, unsigned nrows, int n2, int W,
-                                                          T thr, T near_lo, T near_hi, uint32_t* __restrict__ bits,
+                                                          typename Stage1<T>::Thr th, uint32_t* __restrict__ bits,
                                                           uint32_t* __restrict__ nbits, RowGeom rg, MinMaxKeys* ctr) {
+  typedef Stage1<T> S;
+  typedef typename S::C C;
+  constexpr int UNROLL = 4;
   ctr_pdl_enter();
   const unsigned lane = lane_id();
   const unsigned nwords = nrows * (unsigned)W;
   const unsigned warps = gridDim.x * (blockDim.x >> 5);
   unsigned g = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  T mn = INFINITY, mx = -INFINITY;
-  bool anynear = false;
+  C mn = S::TOP, mx = S::BOTTOM;
   for (; g < nwords; g += warps * UNROLL) {
-    T val[UNROLL];
+    C val[UNROLL];
     bool ok[UNROLL];
 #pragma unroll
     for (int u = 0; u < UNROLL; ++u) {
       unsigned gu = g + (unsigned)u * warps;
       ok[u] = false;
-      val[u] = (T)0;
+      val[u] = (C)0;
       if (gu < nwords) {
         unsigned row = gu / (unsigned)W;
         int k = (int)(gu - row * (unsigned)W) * 32 + (int)lane;
         if (k < n2) {
           ok[u] = true;
-          val[u] = __ldg(f + (size_t)row * n2 + k);
+          val[u] = (C)__ldg(f + (size_t)row * n2 + k);
         }
       }
     }
@@ -125,111 +167,24 @@ __global__ void __launch_bounds__(256) k_bitplane_generic(const T* __restrict__ 
     for (int u = 0; u < UNROLL; ++u) {
       unsigned gu = g + (unsigned)u * warps;
       if (gu < nwords) {                       // warp-uniform
-        unsigned wl = __ballot_sync(0xffffffffu, ok[u] && (val[u] < thr));
-        unsigned wn = __ballot_sync(0xffffffffu, ok[u] && (val[u] >= near_lo) && (val[u] <= near_hi));
+        unsigned wl = __ballot_sync(0xffffffffu, ok[u] && (val[u] < th.thr));
+        unsigned wn = __ballot_sync(0xffffffffu, ok[u] && (val[u] >= th.nlo) && (val[u] <= th.nhi));
         if (lane == 0) {
           bits[gu] = wl;
           nbits[gu] = wn;
           if (wn) flag_rows(rg, gu);
         }
-        if (ok[u]) {
-          if (MINMAX) {
-            mn = fmin(mn, val[u]);             // fmin/fmax ignore NaN
-            mx = fmax(mx, val[u]);
-          }
+        if (MINMAX && ok[u]) {
+          mn = S::lo(mn, val[u]);
+          mx = S::hi(mx, val[u]);
         }
       }
     }
   }
-  minmax_commit(mn, mx, anynear, ctr);
+  minmax_commit(mn, mx, ctr);
 }
 
-// 16 bytes = VEC samples per lane; one warp-wide 128-bit load covers 32*VEC samples = VEC bit words.
-template <typename T>
-struct Vec16;
-template <>
-struct Vec16<float> {
-  static constexpr int VEC = 4;
-  typedef float4 type;
-  __device__ static __forceinline__ void get(const float4& v, float out[4]) { out[0] = v.x; out[1] = v.y; out[2] = v.z; out[3] = v.w; }
-};
-template <>
-struct Vec16<double> {
-  static constexpr int VEC = 2;
-  typedef double2 type;
-  __device__ static __forceinline__ void get(const double2& v, double out[2]) { out[0] = v.x; out[1] = v.y; }
-};
-
-template <typename T, int UNROLL, bool MINMAX>
-__global__ void __launch_bounds__(256) k_bitplane_vec(const T* __restrict__ f, size_t nsamp, T thr, T near_lo, T near_hi,
-                                                      uint32_t* __restrict__ bits, uint32_t* __restrict__ nbits, RowGeom rg,
-                                                      MinMaxKeys* ctr) {
-  typedef typename Vec16<T>::type V;
-  constexpr int VEC = Vec16<T>::VEC;
-  constexpr int GROUP = 32 / VEC;               // lanes per output word
-  ctr_pdl_enter();
-  const unsigned lane = lane_id();
-  const size_t nchunks = (nsamp + 32 * VEC - 1) / (32 * VEC);
-  const size_t warps = (size_t)gridDim.x * (blockDim.x >> 5);
-  size_t c = (size_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  T mn = INFINITY, mx = -INFINITY;
-  bool anynear = false;
-  const V* fv = reinterpret_cast<const V*>(f);
-  for (; c < nchunks; c += warps * UNROLL) {
-    V v[UNROLL];
-    bool ok[UNROLL];
-#pragma unroll
-    for (int u = 0; u < UNROLL; ++u) {
-      size_t cu = c + (size_t)u * warps;
-      size_t s0 = (cu * 32 + lane) * VEC;
-      ok[u] = cu < nchunks && s0 < nsamp;
-      if (ok[u]) v[u] = __ldcs(fv + cu * 32 + lane);       // streaming load (evict-first)
-    }
-#pragma unroll
-    for (int u = 0; u < UNROLL; ++u) {
-      size_t cu = c + (size_t)u * warps;
-      if (cu >= nchunks) continue;                          // warp-uniform
-      T x[VEC];
-      Vec16<T>::get(v[u], x);
-      unsigned lo = 0, nr = 0;
-      if (ok[u]) {
-        T m4 = x[0], M4 = x[0];
-#pragma unroll
-        for (int q = 0; q < VEC; ++q) {
-          lo |= (x[q] < thr ? 1u : 0u) << q;
-          m4 = fmin(m4, x[q]);
-          M4 = fmax(M4, x[q]);
-        }
-        if (MINMAX) {
-          mn = fmin(mn, m4);
-          mx = fmax(mx, M4);
-        }
-        if (!(M4 < near_lo || m4 > near_hi)) {              // rarely taken: some sample may be in the hull
-#pragma unroll
-          for (int q = 0; q < VEC; ++q) nr |= ((x[q] >= near_lo) && (x[q] <= near_hi) ? 1u : 0u) << q;
-        }
-      }
-      unsigned wl = lo << (VEC * (lane & (GROUP - 1)));
-#pragma unroll
-      for (int o = 1; o < GROUP; o <<= 1) wl |= __shfl_xor_sync(0xffffffffu, wl, o);
-      unsigned wn = 0;
-      if (__any_sync(0xffffffffu, nr != 0)) {               // rare
-        wn = nr << (VEC * (lane & (GROUP - 1)));
-#pragma unroll
-        for (int o = 1; o < GROUP; o <<= 1) wn |= __shfl_xor_sync(0xffffffffu, wn, o);
-      }
-      if ((lane & (GROUP - 1)) == 0 && ok[u]) {
-        const size_t word = cu * VEC + lane / GROUP;
-        bits[word] = wl;
-        nbits[word] = wn;
-        if (wn) flag_rows(rg, (unsigned)word);
-      }
-    }
-  }
-  minmax_commit(mn, mx, anynear, ctr);
-}
-
-// ---- TMA (bulk async copy) variant ---------------------------------------------------------------
+// ---- TMA (bulk async copy) ring -------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t* bar, unsigned count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
@@ -253,12 +208,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, unsigned parity) {
       "r"(parity)
       : "memory");
 }
-__device__ __forceinline__ void tma_bulk_g2s(void* dst, const void* src, unsigned bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                   smem_u32(dst)),
-               "l"(src), "r"(bytes), "r"(smem_u32(bar))
-               : "memory");
-}
 // The field is read exactly once: its lines enter L2 marked evict-first, so that they do not push out the bitplanes this
 // kernel writes (32 MiB that stage 2 reads right away) nor the dirty lines of the previous extraction's mesh.
 __device__ __forceinline__ uint64_t l2_evict_first_policy() {
@@ -266,93 +215,61 @@ __device__ __forceinline__ uint64_t l2_evict_first_policy() {
   asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
   return pol;
 }
-__device__ __forceinline__ void tma_bulk_g2s_hint(void* dst, const void* src, unsigned bytes, uint64_t* bar, uint64_t pol) {
+__device__ __forceinline__ void tma_bulk_g2s(void* dst, const void* src, unsigned bytes, uint64_t* bar, uint64_t pol) {
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(
                    smem_u32(dst)),
                "l"(src), "r"(bytes), "r"(smem_u32(bar)), "l"(pol)
                : "memory");
 }
 
-constexpr int TMA_STAGES_DEFAULT = 3;              // x 16 KiB per CTA; 3 CTAs per SM (measured best of 1..6 x 2..6)
-constexpr int TMA_CHUNK = 16384;                 // bytes per stage
+constexpr int TMA_STAGES = 3;                      // x 16 KiB per CTA, 3 CTAs per SM: measured best of 1..6 x 2..6
+constexpr int TMA_CTAS_PER_SM = 3;
+constexpr int TMA_CHUNK = 16384;                   // bytes per stage
 constexpr int TMA_CONSUMER_WARPS = 8;
+constexpr int TMA_WARP_BYTES = TMA_CHUNK / TMA_CONSUMER_WARPS;   // a consumer warp's slice of a stage
 
-template <typename T, bool MINMAX>
-__global__ void __launch_bounds__((TMA_CONSUMER_WARPS + 1) * 32) k_bitplane_tma(const T* __restrict__ f, size_t nbytes,
-                                                                                  T thr, T near_lo, T near_hi,
-                                                                                  uint32_t* __restrict__ bits,
-                                                                                  uint32_t* __restrict__ nbits, RowGeom rg,
-                                                                                  MinMaxKeys* ctr, int TMA_STAGES, int l2_hint) {
-  extern __shared__ __align__(128) unsigned char smem[];
-  uint64_t* full = reinterpret_cast<uint64_t*>(smem + (size_t)TMA_STAGES * TMA_CHUNK);
-  uint64_t* empty = full + TMA_STAGES;
-  const unsigned warp = threadIdx.x >> 5, lane = lane_id();
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < TMA_STAGES; ++s) {
-      mbar_init(&full[s], 1);
-      mbar_init(&empty[s], TMA_CONSUMER_WARPS);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncthreads();
-  const size_t nchunks = (nbytes + TMA_CHUNK - 1) / TMA_CHUNK;
-  const unsigned char* src = reinterpret_cast<const unsigned char*>(f);
-  if (warp == TMA_CONSUMER_WARPS) {
-    if (lane == 0) {
-      unsigned it = 0;
-      const uint64_t pol = l2_evict_first_policy();
-      for (size_t c = blockIdx.x; c < nchunks; c += gridDim.x, ++it) {
-        const int s = it % TMA_STAGES;
-        const unsigned ph = (it / TMA_STAGES) & 1u;
-        mbar_wait(&empty[s], ph ^ 1u);                           // first round passes immediately
-        size_t off = c * (size_t)TMA_CHUNK;
-        unsigned bytes = (unsigned)((nbytes - off) < (size_t)TMA_CHUNK ? (nbytes - off) : (size_t)TMA_CHUNK);
-        mbar_expect_tx(&full[s], bytes);
-        if (l2_hint) tma_bulk_g2s_hint(smem + (size_t)s * TMA_CHUNK, src + off, bytes, &full[s], pol);
-        else tma_bulk_g2s(smem + (size_t)s * TMA_CHUNK, src + off, bytes, &full[s]);
-      }
-    }
-    return;
-  }
-  constexpr int NW = TMA_CHUNK / (32 * (int)sizeof(T));          // bit words per stage
-  constexpr int WPW = NW / TMA_CONSUMER_WARPS;                   // words per warp per stage (<= 32)
+// The consumer step of k_bitplane_tma, per sample type: load() copies the warp's slice of a stage into registers (the
+// kernel releases the stage right after), step() turns them into the words word0 + [0, WPW) of the bitplanes, of
+// which those below words_here (counted from the stage's first word) exist; commit() adds min / max to the run's.
+template <typename T, bool MINMAX, bool FLOAT = std::is_floating_point<T>::value>
+struct TmaConsumer {
+  typedef FloatThr<T> Thr;
+  static constexpr int NW = TMA_CHUNK / (32 * (int)sizeof(T));        // bit words per stage
+  static constexpr int WPW = NW / TMA_CONSUMER_WARPS;                 // words per warp per stage (<= 32)
   static_assert(WPW >= 1 && WPW <= 32, "stage geometry");
-  uint32_t* swords = reinterpret_cast<uint32_t*>(empty + TMA_STAGES) + warp * 32;   // per-warp word staging
-  // conservative centre / radius form of the hull test: |x - vc| <= vr  (superset of [near_lo, near_hi])
-  const T vc = (T)0.5 * near_lo + (T)0.5 * near_hi;
-  const T vr = (near_hi - near_lo) * (T)0.55 + fabs(vc) * (T)1e-6 + (T)1e-30;
+  static constexpr int SCRATCH = TMA_CONSUMER_WARPS * 32 * 4;         // per-warp word staging, behind the barriers
+  // registers for exactly TMA_CTAS_PER_SM CTAs per SM: with fewer, a fourth CTA fits, and CTAs that become resident
+  // early (behind the previous kernel) crowd onto the SMs that free first (B200, 1000 W: 0.312 -> 0.356 ms per 512^3 step)
+  static constexpr int MIN_CTAS = TMA_CTAS_PER_SM;
+  uint32_t* swords;
+  T vc, vr;
   T mn = INFINITY, mx = -INFINITY;
-  const bool anynear = false;
-  unsigned it = 0;
-  // The producer above starts fetching at once: the field is complete before the kernel in front of this one passed its
-  // own wait (common.cuh, rule 2).  The consumers wait here, in front of their first write: the flags they set are
-  // zeroed by that kernel, and the bit planes may still be read by the previous run's last kernel.
-  ctr_pdl_enter();
-  for (size_t c = blockIdx.x; c < nchunks; c += gridDim.x, ++it) {
-    const int s = it % TMA_STAGES;
-    const unsigned ph = (it / TMA_STAGES) & 1u;
-    const size_t off = c * (size_t)TMA_CHUNK;
-    const unsigned bytes = (unsigned)((nbytes - off) < (size_t)TMA_CHUNK ? (nbytes - off) : (size_t)TMA_CHUNK);
-    const unsigned words_here = bytes / (32u * (unsigned)sizeof(T));
-    const T* sv = reinterpret_cast<const T*>(smem + (size_t)s * TMA_CHUNK) + (size_t)warp * WPW * 32;
-    mbar_wait(&full[s], ph);
-    T val[WPW];
+  T val[WPW];
+
+  __device__ __forceinline__ TmaConsumer(const Thr& th, uint32_t* scratch) : swords(scratch) {
+    // conservative centre / radius form of the hull test: |x - vc| <= vr  (superset of [nlo, nhi])
+    vc = (T)0.5 * th.nlo + (T)0.5 * th.nhi;
+    vr = (th.nhi - th.nlo) * (T)0.55 + fabs(vc) * (T)1e-6 + (T)1e-30;
+  }
+  __device__ __forceinline__ void load(const unsigned char* slice) {
+    const T* sv = reinterpret_cast<const T*>(slice);
 #pragma unroll
-    for (int q = 0; q < WPW; ++q) val[q] = sv[q * 32 + lane];    // conflict-free: lane <-> bank
-    __syncwarp();
-    if (lane == 0) mbar_arrive(&empty[s]);                       // stage is in registers: release it early
-    const unsigned wbase = warp * WPW;
-    const size_t word0 = off / (32 * sizeof(T)) + wbase;
+    for (int q = 0; q < WPW; ++q) val[q] = sv[q * 32 + lane_id()];   // conflict-free: lane <-> bank
+  }
+  __device__ __forceinline__ void step(const Thr& th, size_t word0, unsigned wbase, unsigned words_here, uint32_t* bits,
+                                       uint32_t* nbits, const RowGeom& rg) {
+    const unsigned lane = lane_id();
     if (words_here < (unsigned)NW) {
-      // partial last chunk: samples past the end are stale shared memory; neutralise them
+      // partial last chunk: samples past the end are stale shared memory.  NaN is neither low nor near, fmin / fmax
+      // ignore it, and the words past the end are not stored.
 #pragma unroll
       for (int q = 0; q < WPW; ++q)
-        if (wbase + q >= words_here) val[q] = INFINITY;
+        if (wbase + q >= words_here) val[q] = NAN;
     }
     T dist = INFINITY;
 #pragma unroll
     for (int q = 0; q < WPW; ++q) {
-      const unsigned wl = __ballot_sync(0xffffffffu, val[q] < thr);
+      const unsigned wl = __ballot_sync(0xffffffffu, val[q] < th.thr);
       if (lane == 0) swords[q] = wl;
       dist = fmin(dist, fabs(val[q] - vc));                     // NaN never wins: not near
       if (MINMAX) {
@@ -364,7 +281,7 @@ __global__ void __launch_bounds__((TMA_CONSUMER_WARPS + 1) * 32) k_bitplane_tma(
     if (__any_sync(0xffffffffu, dist <= vr)) {                   // rare: materialise the near words of this warp
 #pragma unroll
       for (int q = 0; q < WPW; ++q) {
-        const unsigned wn = __ballot_sync(0xffffffffu, (val[q] >= near_lo) && (val[q] <= near_hi));
+        const unsigned wn = __ballot_sync(0xffffffffu, (val[q] >= th.nlo) && (val[q] <= th.nhi));
         if ((int)lane == q) {
           mine_n = wn;
           if (wn) flag_rows(rg, (unsigned)(word0 + q));
@@ -378,75 +295,8 @@ __global__ void __launch_bounds__((TMA_CONSUMER_WARPS + 1) * 32) k_bitplane_tma(
     }
     __syncwarp();
   }
-  minmax_commit(mn, mx, anynear, ctr);
-}
-
-// ---- integer samples (uint8 / int16 / uint16) ----------------------------------------------------
-// An integer sample f meets the fp64 predicates on its widened value exactly when it meets integer ones (IntThr, from
-// thresholds_int on the host):   f < v  <=>  f < thr;   v - r <= f <= v + r  <=>  nlo <= f <= nhi.
-struct IntThr {
-  int thr;            // ceil(v) clamped to [min(T), max(T) + 1]
-  int nlo, nhi;       // near samples, clipped to T's range; nlo > nhi: none
+  __device__ __forceinline__ void commit(MinMaxKeys* ctr) { minmax_commit(mn, mx, ctr); }
 };
-
-__device__ __forceinline__ void minmax_commit_int(int mn, int mx, MinMaxKeys* ctr) {
-  mn = __reduce_min_sync(0xffffffffu, mn);
-  mx = __reduce_max_sync(0xffffffffu, mx);
-  if (lane_id() == 0 && mn <= mx) {
-    atomicMin(&ctr->min_key, order_key((double)mn));
-    atomicMax(&ctr->max_key, order_key((double)mx));
-  }
-}
-
-// any shape: one warp converts 32 samples per step (the integer twin of k_bitplane_generic, also used for
-// CTR_BITPLANE=vec)
-template <typename T, int UNROLL, bool MINMAX>
-__global__ void __launch_bounds__(256) k_bitplane_generic_int(const T* __restrict__ f, unsigned nrows, int n2, int W,
-                                                              IntThr th, uint32_t* __restrict__ bits,
-                                                              uint32_t* __restrict__ nbits, RowGeom rg, MinMaxKeys* ctr) {
-  ctr_pdl_enter();
-  const unsigned lane = lane_id();
-  const unsigned nwords = nrows * (unsigned)W;
-  const unsigned warps = gridDim.x * (blockDim.x >> 5);
-  unsigned g = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  int mn = INT_MAX, mx = INT_MIN;
-  for (; g < nwords; g += warps * UNROLL) {
-    int val[UNROLL];
-    bool ok[UNROLL];
-#pragma unroll
-    for (int u = 0; u < UNROLL; ++u) {
-      unsigned gu = g + (unsigned)u * warps;
-      ok[u] = false;
-      val[u] = 0;
-      if (gu < nwords) {
-        unsigned row = gu / (unsigned)W;
-        int k = (int)(gu - row * (unsigned)W) * 32 + (int)lane;
-        if (k < n2) {
-          ok[u] = true;
-          val[u] = (int)__ldg(f + (size_t)row * n2 + k);
-        }
-      }
-    }
-#pragma unroll
-    for (int u = 0; u < UNROLL; ++u) {
-      unsigned gu = g + (unsigned)u * warps;
-      if (gu < nwords) {                       // warp-uniform
-        unsigned wl = __ballot_sync(0xffffffffu, ok[u] && (val[u] < th.thr));
-        unsigned wn = __ballot_sync(0xffffffffu, ok[u] && (val[u] >= th.nlo) && (val[u] <= th.nhi));
-        if (lane == 0) {
-          bits[gu] = wl;
-          nbits[gu] = wn;
-          if (wn) flag_rows(rg, gu);
-        }
-        if (MINMAX && ok[u]) {
-          mn = min(mn, val[u]);
-          mx = max(mx, val[u]);
-        }
-      }
-    }
-  }
-  minmax_commit_int(mn, mx, ctr);
-}
 
 // SIMD view of one 32-bit register holding N = 4 (uint8) or 2 (int16 / uint16) samples.  Compares give 0 / all-ones
 // per sample; pack() turns that into N bits, sample q at bit q; zeros() is non-zero iff some sample of t is 0 (the
@@ -502,73 +352,34 @@ struct IntThrRep {
   int nnear;          // 0, 1 or 2
 };
 
-// The same ring, producer and PDL placement as k_bitplane_tma; the consumers read 16 bytes (16 / 8 samples) per lane and
-// load, compare 4 / 2 samples per instruction sequence (Simd<T>) and assemble each 32-bit word from the bit groups of
-// 2 / 4 neighbouring lanes.  A warp's 2 KiB of a stage is 4 passes of 512 bytes: pass q, lane l has the samples of word
-// q * WPP + l / GROUP, bits (l % GROUP) * S ...
+// uint8 / int16 / uint16: the consumers read 16 bytes (16 / 8 samples) per lane and load, compare 4 / 2 samples per
+// instruction sequence (Simd<T>) and assemble each 32-bit word from the bit groups of 2 / 4 neighbouring lanes.  A
+// warp's 2 KiB of a stage is 4 passes of 512 bytes: pass q, lane l has the samples of word q * WPP + l / GROUP, bits
+// (l % GROUP) * S ...
 template <typename T, bool MINMAX>
-__global__ void __launch_bounds__((TMA_CONSUMER_WARPS + 1) * 32) k_bitplane_tma_int(const T* __restrict__ f, size_t nbytes,
-                                                                                      IntThrRep th, uint32_t* __restrict__ bits,
-                                                                                      uint32_t* __restrict__ nbits, RowGeom rg,
-                                                                                      MinMaxKeys* ctr, int TMA_STAGES, int l2_hint) {
+struct TmaConsumer<T, MINMAX, false> {
+  typedef IntThrRep Thr;
   typedef Simd<T> V;
-  constexpr int S = 16 / (int)sizeof(T);                        // samples per lane and pass
-  constexpr int GROUP = 32 / S;                                 // lanes per bit word
-  constexpr int WPP = 32 / GROUP;                               // words per warp and pass
-  constexpr int WARP_BYTES = TMA_CHUNK / TMA_CONSUMER_WARPS;
-  constexpr int PASSES = WARP_BYTES / 512;
-  constexpr int WPW = PASSES * WPP;                             // words per warp per stage
-  static_assert(PASSES * 512 == WARP_BYTES && WPW * 32 * (int)sizeof(T) == WARP_BYTES, "stage geometry");
-  extern __shared__ __align__(128) unsigned char smem[];
-  uint64_t* full = reinterpret_cast<uint64_t*>(smem + (size_t)TMA_STAGES * TMA_CHUNK);
-  uint64_t* empty = full + TMA_STAGES;
-  const unsigned warp = threadIdx.x >> 5, lane = lane_id();
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < TMA_STAGES; ++s) {
-      mbar_init(&full[s], 1);
-      mbar_init(&empty[s], TMA_CONSUMER_WARPS);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncthreads();
-  const size_t nchunks = (nbytes + TMA_CHUNK - 1) / TMA_CHUNK;
-  const unsigned char* src = reinterpret_cast<const unsigned char*>(f);
-  if (warp == TMA_CONSUMER_WARPS) {
-    if (lane == 0) {
-      unsigned it = 0;
-      const uint64_t pol = l2_evict_first_policy();
-      for (size_t c = blockIdx.x; c < nchunks; c += gridDim.x, ++it) {
-        const int s = it % TMA_STAGES;
-        const unsigned ph = (it / TMA_STAGES) & 1u;
-        mbar_wait(&empty[s], ph ^ 1u);
-        size_t off = c * (size_t)TMA_CHUNK;
-        unsigned bytes = (unsigned)((nbytes - off) < (size_t)TMA_CHUNK ? (nbytes - off) : (size_t)TMA_CHUNK);
-        mbar_expect_tx(&full[s], bytes);
-        if (l2_hint) tma_bulk_g2s_hint(smem + (size_t)s * TMA_CHUNK, src + off, bytes, &full[s], pol);
-        else tma_bulk_g2s(smem + (size_t)s * TMA_CHUNK, src + off, bytes, &full[s]);
-      }
-    }
-    return;
-  }
-  const unsigned sub = lane % GROUP;
+  static constexpr int S = 16 / (int)sizeof(T);                 // samples per lane and pass
+  static constexpr int GROUP = 32 / S;                          // lanes per bit word
+  static constexpr int WPP = 32 / GROUP;                        // words per warp and pass
+  static constexpr int PASSES = TMA_WARP_BYTES / 512;
+  static constexpr int WPW = PASSES * WPP;                      // words per warp per stage
+  static_assert(PASSES * 512 == TMA_WARP_BYTES && WPW * 32 * (int)sizeof(T) == TMA_WARP_BYTES, "stage geometry");
+  static constexpr int SCRATCH = 0;
+  static constexpr int MIN_CTAS = 0;                             // no bound: ptxas picks the register count
   unsigned vmn = V::rep(V::MAX), vmx = V::rep(V::MIN);        // identities of V::mn / V::mx
-  unsigned it = 0;
-  ctr_pdl_enter();                                              // see k_bitplane_tma
-  for (size_t c = blockIdx.x; c < nchunks; c += gridDim.x, ++it) {
-    const int s = it % TMA_STAGES;
-    const unsigned ph = (it / TMA_STAGES) & 1u;
-    const size_t off = c * (size_t)TMA_CHUNK;
-    const unsigned bytes = (unsigned)((nbytes - off) < (size_t)TMA_CHUNK ? (nbytes - off) : (size_t)TMA_CHUNK);
-    const unsigned words_here = bytes / (32u * (unsigned)sizeof(T));
-    const uint4* sv = reinterpret_cast<const uint4*>(smem + (size_t)s * TMA_CHUNK + (size_t)warp * WARP_BYTES);
-    mbar_wait(&full[s], ph);
-    uint4 v[PASSES];
+  uint4 v[PASSES];
+
+  __device__ __forceinline__ TmaConsumer(const Thr&, uint32_t*) {}
+  __device__ __forceinline__ void load(const unsigned char* slice) {
+    const uint4* sv = reinterpret_cast<const uint4*>(slice);
 #pragma unroll
-    for (int q = 0; q < PASSES; ++q) v[q] = sv[q * 32 + lane];   // 16 bytes per lane: conflict-free
-    __syncwarp();
-    if (lane == 0) mbar_arrive(&empty[s]);
-    const unsigned wbase = warp * WPW;
-    const size_t word0 = off / (32 * sizeof(T)) + wbase;
+    for (int q = 0; q < PASSES; ++q) v[q] = sv[q * 32 + lane_id()];   // 16 bytes per lane: conflict-free
+  }
+  __device__ __forceinline__ void step(const Thr& th, size_t word0, unsigned wbase, unsigned words_here, uint32_t* bits,
+                                       uint32_t* nbits, const RowGeom& rg) {
+    const unsigned lane = lane_id(), sub = lane % GROUP;
     unsigned lo[PASSES], zacc = 0;
     bool ok[PASSES];
 #pragma unroll
@@ -622,12 +433,74 @@ __global__ void __launch_bounds__((TMA_CONSUMER_WARPS + 1) * 32) k_bitplane_tma_
     for (int q = 0; q < PASSES; ++q)
       if (sub == 0 && ok[q]) nbits[word0 + q * WPP + lane / GROUP] = nr[q];
   }
-  int mn = INT_MAX, mx = INT_MIN;
-  if (MINMAX) {
-    mn = V::hmin(vmn);
-    mx = V::hmax(vmx);
+  __device__ __forceinline__ void commit(MinMaxKeys* ctr) {
+    int mn = INT_MAX, mx = INT_MIN;
+    if (MINMAX) {
+      mn = V::hmin(vmn);
+      mx = V::hmax(vmx);
+    }
+    minmax_commit(mn, mx, ctr);
   }
-  minmax_commit_int(mn, mx, ctr);
+};
+
+// dynamic shared memory of k_bitplane_tma<T>: the ring, its full / empty barriers, the consumers' scratch
+template <typename T>
+constexpr int tma_smem_bytes() {
+  return TMA_STAGES * TMA_CHUNK + 2 * TMA_STAGES * 8 + TmaConsumer<T, false>::SCRATCH;
+}
+
+template <typename T, bool MINMAX>
+__global__ void __launch_bounds__((TMA_CONSUMER_WARPS + 1) * 32, TmaConsumer<T, MINMAX>::MIN_CTAS)
+    k_bitplane_tma(const T* __restrict__ f, size_t nbytes, typename TmaConsumer<T, MINMAX>::Thr th, uint32_t* __restrict__ bits,
+                   uint32_t* __restrict__ nbits, RowGeom rg, MinMaxKeys* ctr) {
+  extern __shared__ __align__(128) unsigned char smem[];
+  uint64_t* full = reinterpret_cast<uint64_t*>(smem + TMA_STAGES * TMA_CHUNK);
+  uint64_t* empty = full + TMA_STAGES;
+  const unsigned warp = threadIdx.x >> 5, lane = lane_id();
+  if (threadIdx.x == 0) {
+    for (int s = 0; s < TMA_STAGES; ++s) {
+      mbar_init(&full[s], 1);
+      mbar_init(&empty[s], TMA_CONSUMER_WARPS);
+    }
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  __syncthreads();
+  const unsigned nchunks = (unsigned)((nbytes + TMA_CHUNK - 1) / TMA_CHUNK);   // fewer than the (32-bit) word indices
+  if (warp == TMA_CONSUMER_WARPS) {
+    if (lane == 0) {
+      unsigned it = 0;
+      const uint64_t pol = l2_evict_first_policy();
+      for (unsigned c = blockIdx.x; c < nchunks; c += gridDim.x, ++it) {
+        const int s = it % TMA_STAGES;
+        const unsigned ph = (it / TMA_STAGES) & 1u;
+        mbar_wait(&empty[s], ph ^ 1u);                           // first round passes immediately
+        const size_t off = c * (size_t)TMA_CHUNK;
+        const unsigned bytes = (unsigned)((nbytes - off) < (size_t)TMA_CHUNK ? (nbytes - off) : (size_t)TMA_CHUNK);
+        mbar_expect_tx(&full[s], bytes);
+        tma_bulk_g2s(smem + s * TMA_CHUNK, reinterpret_cast<const unsigned char*>(f) + off, bytes, &full[s], pol);
+      }
+    }
+    return;
+  }
+  TmaConsumer<T, MINMAX> cons(th, reinterpret_cast<uint32_t*>(empty + TMA_STAGES) + warp * 32);
+  const unsigned wbase = warp * cons.WPW;
+  unsigned it = 0;
+  // The producer above starts fetching at once: the field is complete before the kernel in front of this one passed its
+  // own wait (common.cuh, rule 2).  The consumers wait here, in front of their first write: the flags they set are
+  // zeroed by that kernel, and the bit planes may still be read by the previous run's last kernel.
+  ctr_pdl_enter();
+  for (unsigned c = blockIdx.x; c < nchunks; c += gridDim.x, ++it) {
+    const int s = it % TMA_STAGES;
+    const unsigned ph = (it / TMA_STAGES) & 1u;
+    const size_t off = c * (size_t)TMA_CHUNK;
+    const unsigned bytes = (unsigned)((nbytes - off) < (size_t)TMA_CHUNK ? (nbytes - off) : (size_t)TMA_CHUNK);
+    mbar_wait(&full[s], ph);
+    cons.load(smem + s * TMA_CHUNK + warp * TMA_WARP_BYTES);
+    __syncwarp();
+    if (lane == 0) mbar_arrive(&empty[s]);                       // stage is in registers: release it early
+    cons.step(th, off / (32 * sizeof(T)) + wbase, wbase, bytes / (32u * (unsigned)sizeof(T)), bits, nbits, rg);
+  }
+  cons.commit(ctr);
 }
 
 
@@ -679,18 +552,6 @@ IntThr thresholds_int(double v) {
   return t;
 }
 
-enum BitplaneKind { BP_AUTO = 0, BP_GENERIC = 1, BP_VEC = 2, BP_TMA = 3 };
-
-BitplaneKind bitplane_choice() {
-  const char* e = getenv("CTR_BITPLANE");
-  if (!e) return BP_AUTO;
-  if (!strcmp(e, "generic")) return BP_GENERIC;
-  if (!strcmp(e, "vec")) return BP_VEC;
-  if (!strcmp(e, "tma")) return BP_TMA;
-  return BP_AUTO;
-}
-
-// host-side pieces shared by the float and the integer launchers
 RowGeom row_geom(uint8_t* rowflag, uint32_t* wordflag, int W, int rb, int rc) {
   RowGeom rg;
   rg.rowflag = rowflag;
@@ -706,117 +567,55 @@ RowGeom row_geom(uint8_t* rowflag, uint32_t* wordflag, int W, int rb, int rc) {
   return rg;
 }
 
-struct TmaKnobs {
-  int stages, ctas_per_sm, l2_hint;
-};
-const TmaKnobs& tma_knobs() {
-  static const TmaKnobs k = {getenv("CTR_BP_STAGES") ? atoi(getenv("CTR_BP_STAGES")) : TMA_STAGES_DEFAULT,
-                             getenv("CTR_BP_CTAS") ? atoi(getenv("CTR_BP_CTAS")) : 3,
-                             getenv("CTR_BP_L2HINT") ? atoi(getenv("CTR_BP_L2HINT")) : 1};   // L2 hint: 0.428 -> 0.418 ms per 512^3 step
-  return k;
-}
-
-// grid of the generic kernels: 256 threads, 4 words per warp and round, at most 8 blocks per SM
-int generic_blocks(const ctr_ctx* ctx, size_t nwords) {
-  const size_t need = (nwords + 8 * 4 - 1) / (8 * 4);
-  return (int)std::min<size_t>(std::max<size_t>(need, 1), (size_t)ctx->sm_count * 8);
-}
-
-template <typename T, bool MINMAX>
-std::enable_if_t<std::is_floating_point<T>::value, int> launch_bitplane(ctr_ctx* ctx, const T* dfield, unsigned nrows, int n2, int W, int rb, int rc, double iso,
-                    uint32_t* bits, uint32_t* nbits, uint8_t* rowflag, MinMaxKeys* dctr, bool clear_rowflag = true,
-                    uint32_t* wordflag = nullptr) {
+// Stage 1 over float, double, uint8, int16 or uint16 samples.  The TMA kernel takes the field when it is one linear
+// stream of whole words (rows a multiple of 32 samples, 16-byte aligned) and, for integer samples, at most two sample
+// values are near; the generic kernel takes any other field.
+template <typename T>
+int launch_bitplane(ctr_ctx* ctx, const T* dfield, unsigned nrows, int n2, int W, int rb, int rc, double iso,
+                    uint32_t* bits, uint32_t* nbits, uint8_t* rowflag, MinMaxKeys* dctr, bool minmax,
+                    bool clear_rowflag = true, uint32_t* wordflag = nullptr) {
+  static_assert(std::is_floating_point<T>::value || std::is_same<T, uint8_t>::value || std::is_same<T, int16_t>::value ||
+                    std::is_same<T, uint16_t>::value,
+                "samples: float, double, uint8, int16, uint16");
   cudaStream_t st = ctx->stream;
-  T thr, nlo, nhi;
-  thresholds<T>(iso, thr, nlo, nhi);
-  const size_t nsamp = (size_t)nrows * n2;
-  const size_t nwords = (size_t)nrows * W;
-  const bool linear_ok = (n2 % 32 == 0) && (((uintptr_t)dfield) % 16 == 0);
-  BitplaneKind kind = bitplane_choice();
-  if (kind == BP_AUTO) kind = linear_ok ? BP_TMA : BP_GENERIC;
-  if (!linear_ok) kind = BP_GENERIC;
-  const RowGeom rg = row_geom(rowflag, wordflag, W, rb, rc);
-  if (clear_rowflag) CTR_CUDA(ctx, cudaMemsetAsync(rg.rowflag, 0, (size_t)nrows, st));
-  if (kind == BP_TMA) {
-    const TmaKnobs& kn = tma_knobs();
-    const int TMA_STAGES = kn.stages, ctas_per_sm = kn.ctas_per_sm, l2_hint = kn.l2_hint;
-    const int smem = TMA_STAGES * TMA_CHUNK + 2 * TMA_STAGES * 8 + TMA_CONSUMER_WARPS * 32 * 4 + 64;
-    // this header is compiled into two translation units (anonymous namespaces): each has its own kernel instances
-    const int ti = CTR_BP_ATTR_BASE + (sizeof(T) == 4 ? 0 : 1) + (MINMAX ? 2 : 0);
-    if (!(ctx->attr_mask & (1u << ti))) {
-      CTR_CUDA(ctx, cudaFuncSetAttribute(k_bitplane_tma<T, MINMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, 8 * TMA_CHUNK + 1024));
-      ctx->attr_mask |= 1u << ti;
-    }
-    const size_t nbytes = nsamp * sizeof(T);
-    const size_t nchunks = (nbytes + TMA_CHUNK - 1) / TMA_CHUNK;
-    int blocks = (int)std::min<size_t>(nchunks, (size_t)ctx->sm_count * ctas_per_sm);
-    ctr_launch_dep(k_bitplane_tma<T, MINMAX>, blocks, (TMA_CONSUMER_WARPS + 1) * 32, smem, st, dfield, nbytes, thr, nlo, nhi, bits, nbits, rg,
-                   dctr, (int)TMA_STAGES, (int)l2_hint);
-  } else if (kind == BP_VEC) {
-    const size_t nchunks = (nsamp + 32 * Vec16<T>::VEC - 1) / (32 * Vec16<T>::VEC);
-    size_t need = (nchunks + 8 * 4 - 1) / (8 * 4);
-    int blocks = (int)std::min<size_t>(std::max<size_t>(need, 1), (size_t)ctx->sm_count * 8);
-    k_bitplane_vec<T, 4, MINMAX><<<blocks, 256, 0, st>>>(dfield, nsamp, thr, nlo, nhi, bits, nbits, rg, dctr);
+  bool tma = (n2 % 32 == 0) && (((uintptr_t)dfield) % 16 == 0);
+  typename Stage1<T>::Thr th;
+  typename TmaConsumer<T, false>::Thr tth;
+  if constexpr (std::is_floating_point<T>::value) {
+    thresholds<T>(iso, th.thr, th.nlo, th.nhi);
+    tth = th;
   } else {
-    const int blocks = generic_blocks(ctx, nwords);
-    k_bitplane_generic<T, 4, MINMAX><<<blocks, 256, 0, st>>>(dfield, nrows, n2, W, thr, nlo, nhi, bits, nbits, rg, dctr);
-  }
-  ctx->launches++;
-  CTR_CUDA(ctx, cudaGetLastError());
-  return 0;
-}
-
-#ifdef CTR_BP_ATTR_INT_BASE
-// uint8 / int16 / uint16 samples, for translation units that define the attribute bits of these instances:
-// CTR_BP_ATTR_INT_BASE + 2 * (0 uint8, 1 int16, 2 uint16) + MINMAX.
-template <typename T, bool MINMAX>
-std::enable_if_t<std::is_integral<T>::value, int> launch_bitplane(ctr_ctx* ctx, const T* dfield, unsigned nrows, int n2, int W,
-                                                                   int rb, int rc, double iso, uint32_t* bits, uint32_t* nbits,
-                                                                   uint8_t* rowflag, MinMaxKeys* dctr, bool clear_rowflag = true,
-                                                                   uint32_t* wordflag = nullptr) {
-  static_assert(std::is_same<T, uint8_t>::value || std::is_same<T, int16_t>::value || std::is_same<T, uint16_t>::value,
-                "integer samples: uint8, int16, uint16");
-  cudaStream_t st = ctx->stream;
-  const IntThr th = thresholds_int<T>(iso);
-  const size_t nsamp = (size_t)nrows * n2;
-  const size_t nwords = (size_t)nrows * W;
-  // the TMA consumers compare against at most two near values: always so for these types (r < 0.66 inside their range)
-  const bool linear_ok = (n2 % 32 == 0) && (((uintptr_t)dfield) % 16 == 0) && (th.nlo > th.nhi || th.nhi - th.nlo <= 1);
-  BitplaneKind kind = bitplane_choice();
-  if (kind == BP_AUTO) kind = linear_ok ? BP_TMA : BP_GENERIC;
-  if (!linear_ok || kind == BP_VEC) kind = BP_GENERIC;
-  const RowGeom rg = row_geom(rowflag, wordflag, W, rb, rc);
-  if (clear_rowflag) CTR_CUDA(ctx, cudaMemsetAsync(rg.rowflag, 0, (size_t)nrows, st));
-  if (kind == BP_TMA) {
-    const TmaKnobs& kn = tma_knobs();
-    const int TMA_STAGES = kn.stages, ctas_per_sm = kn.ctas_per_sm, l2_hint = kn.l2_hint;
-    const int smem = TMA_STAGES * TMA_CHUNK + 2 * TMA_STAGES * 8 + 64;
-    const int ti = CTR_BP_ATTR_INT_BASE + 2 * (sizeof(T) == 1 ? 0 : std::is_signed<T>::value ? 1 : 2) + (MINMAX ? 1 : 0);
-    if (!(ctx->attr_mask & (1u << ti))) {
-      CTR_CUDA(ctx, cudaFuncSetAttribute(k_bitplane_tma_int<T, MINMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, 8 * TMA_CHUNK + 1024));
-      ctx->attr_mask |= 1u << ti;
-    }
+    th = thresholds_int<T>(iso);
+    // the TMA consumers compare against at most two near values: always so for these types (r < 0.66 inside their range)
+    tma = tma && (th.nlo > th.nhi || th.nhi - th.nlo <= 1);
     typedef Simd<T> V;
     const int tmax = (int)std::numeric_limits<T>::max();
-    IntThrRep tr;
-    tr.thr = V::rep(std::min(th.thr, tmax));
-    tr.lowall = th.thr > tmax ? 0xffffffffu : 0u;
-    tr.nnear = th.nlo > th.nhi ? 0 : th.nhi - th.nlo + 1;
-    tr.near0 = V::rep(th.nlo);
-    tr.near1 = V::rep(th.nhi);
-    const size_t nbytes = nsamp * sizeof(T);
+    tth.thr = V::rep(std::min(th.thr, tmax));
+    tth.lowall = th.thr > tmax ? 0xffffffffu : 0u;
+    tth.nnear = th.nlo > th.nhi ? 0 : th.nhi - th.nlo + 1;
+    tth.near0 = V::rep(th.nlo);
+    tth.near1 = V::rep(th.nhi);
+  }
+  const RowGeom rg = row_geom(rowflag, wordflag, W, rb, rc);
+  if (clear_rowflag) CTR_CUDA(ctx, cudaMemsetAsync(rg.rowflag, 0, (size_t)nrows, st));
+  if (tma) {
+    const auto kern = minmax ? k_bitplane_tma<T, true> : k_bitplane_tma<T, false>;
+    constexpr int smem = tma_smem_bytes<T>();
+    CTR_CUDA(ctx, ctr_smem_optin(ctx, kern, smem));
+    const size_t nbytes = (size_t)nrows * n2 * sizeof(T);
     const size_t nchunks = (nbytes + TMA_CHUNK - 1) / TMA_CHUNK;
-    int blocks = (int)std::min<size_t>(nchunks, (size_t)ctx->sm_count * ctas_per_sm);
-    ctr_launch_dep(k_bitplane_tma_int<T, MINMAX>, blocks, (TMA_CONSUMER_WARPS + 1) * 32, smem, st, dfield, nbytes, tr, bits, nbits,
-                   rg, dctr, (int)TMA_STAGES, (int)l2_hint);
+    const int blocks = (int)std::min<size_t>(nchunks, (size_t)ctx->sm_count * TMA_CTAS_PER_SM);
+    ctr_launch_dep(kern, blocks, (TMA_CONSUMER_WARPS + 1) * 32, smem, st, dfield, nbytes, tth, bits, nbits, rg, dctr);
   } else {
-    const int blocks = generic_blocks(ctx, nwords);
-    k_bitplane_generic_int<T, 4, MINMAX><<<blocks, 256, 0, st>>>(dfield, nrows, n2, W, th, bits, nbits, rg, dctr);
+    // 256 threads, 4 words per warp and round, at most 8 blocks per SM
+    const size_t need = ((size_t)nrows * W + 8 * 4 - 1) / (8 * 4);
+    const int blocks = (int)std::min<size_t>(std::max<size_t>(need, 1), (size_t)ctx->sm_count * 8);
+    const auto kern = minmax ? k_bitplane_generic<T, true> : k_bitplane_generic<T, false>;
+    ctr_launch_dep(kern, blocks, 256, 0, st, dfield, nrows, n2, W, th, bits, nbits, rg, dctr);
   }
   ctx->launches++;
   CTR_CUDA(ctx, cudaGetLastError());
   return 0;
 }
-#endif
 
 }  // namespace

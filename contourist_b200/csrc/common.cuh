@@ -6,6 +6,7 @@
 #include <stdio.h>
 #include <string>
 #include <utility>
+#include <vector>
 
 #include "../../include/contourist_b200.h"
 
@@ -33,7 +34,7 @@ struct ctr_ctx {
   bool ev_set[CTR_NSTAGE + 1] = {};
   float stage_ms[CTR_NSTAGE] = {};
   int sm_count = 148;
-  unsigned attr_mask = 0;    // cudaFuncSetAttribute calls already made on this context's device (the attribute is per device)
+  std::vector<const void*> smem_optin;   // kernels ctr_smem_optin has set up on this context's device
 
   // staging + shared scratch
   DevBuf field;              // device copy of a host field
@@ -163,6 +164,19 @@ static inline cudaError_t ctr_launch_dep(void (*kern)(KArgs...), dim3 grid, dim3
   cfg.attrs = at;
   cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
+}
+
+// Lets `kernel` take `bytes` of dynamic shared memory (above the default 48 KiB), the first time this context launches
+// it.  The attribute belongs to the device and to the kernel instance (a header's kernels are instantiated in every
+// translation unit that includes it), so each context keeps its own list of the kernels it has set.
+template <typename... KArgs>
+static inline cudaError_t ctr_smem_optin(ctr_ctx* ctx, void (*kernel)(KArgs...), int bytes) {
+  const void* k = reinterpret_cast<const void*>(kernel);
+  for (const void* done : ctx->smem_optin)
+    if (done == k) return cudaSuccess;
+  const cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+  if (e == cudaSuccess) ctx->smem_optin.push_back(k);
+  return e;
 }
 
 __device__ __forceinline__ unsigned long long warp_incl_scan_u64(unsigned long long v) {

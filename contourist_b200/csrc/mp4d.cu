@@ -11,7 +11,8 @@
 //   k4_slice               : morph_geometry.py:145-237 slicing, single pass (look-back scan, smem-staged output), with
 //                            the instant / tiny filter (pentatopes.py:171-189, tetrahedral.py:353-375) folded in when
 //                            the integer time bins decide it; k4_tet_filter is the general (fp64) form of that filter.
-#define CTR_BP_ATTR_BASE 4   // bits of ctr_ctx::attr_mask used by this file's bitplane kernels
+#include <stdlib.h>
+
 #include "bitplane.cuh"
 #include "tables.h"
 
@@ -1150,12 +1151,8 @@ int run4d(ctr_ctx* ctx, const ctr_mp4d_params* p, ctr_mp4d_counts* out) {
   memcpy(ctx->counters_host, &init, sizeof init);
   CTR_CUDA(ctx, cudaMemcpyAsync(ctx->counters.p, ctx->counters_host, sizeof init, cudaMemcpyHostToDevice, st));
   Counters4* dctr = (Counters4*)ctx->counters.p;
-  if (p->flags & CTR_WANT_MINMAX)
-    rc = launch_bitplane<T, true>(ctx, df, (unsigned)nrows, n3, W, n1, n2, p->isovalue, (uint32_t*)ctx->bits.p,
-                                  (uint32_t*)ctx->nbits.p, (uint8_t*)B.rowflag.p, (MinMaxKeys*)dctr);
-  else
-    rc = launch_bitplane<T, false>(ctx, df, (unsigned)nrows, n3, W, n1, n2, p->isovalue, (uint32_t*)ctx->bits.p,
-                                   (uint32_t*)ctx->nbits.p, (uint8_t*)B.rowflag.p, (MinMaxKeys*)dctr);
+  rc = launch_bitplane<T>(ctx, df, (unsigned)nrows, n3, W, n1, n2, p->isovalue, (uint32_t*)ctx->bits.p, (uint32_t*)ctx->nbits.p,
+                          (uint8_t*)B.rowflag.p, (MinMaxKeys*)dctr, (p->flags & CTR_WANT_MINMAX) != 0);
   if (rc) return rc;
   ctr_stage_mark(ctx, 2);
   Grid4<T> g;
@@ -1306,11 +1303,8 @@ int run4d(ctr_ctx* ctx, const ctr_mp4d_params* p, ctr_mp4d_counts* out) {
       for (int attempt = 0; attempt < 3; ++attempt) {
         if ((rc = ctr_ensure(ctx, B.mtris, want * 24))) return rc;
         const unsigned cap = (unsigned)std::min<size_t>(B.mtris.cap / 24, 0x7fffffffu);
-        if (!(ctx->attr_mask & (1u << 8))) {
-          CTR_CUDA(ctx, cudaFuncSetAttribute(k4_slice<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, SL_SMEM));
-          CTR_CUDA(ctx, cudaFuncSetAttribute(k4_slice<int>, cudaFuncAttributeMaxDynamicSharedMemorySize, SL_SMEM));
-          ctx->attr_mask |= 1u << 8;
-        }
+        CTR_CUDA(ctx, ctr_smem_optin(ctx, k4_slice<double>, SL_SMEM));
+        CTR_CUDA(ctx, ctr_smem_optin(ctx, k4_slice<int>, SL_SMEM));
         SlCounters* slc = (SlCounters*)((char*)B.slstate.p + (size_t)sl_tiles * 8);
         unsigned long long* ptab = (unsigned long long*)((char*)B.slstate.p + (((size_t)sl_tiles * 8 + 64 + 255) & ~(size_t)255));
         CTR_CUDA(ctx, cudaMemsetAsync(B.slstate.p, 0, (size_t)sl_tiles * 8 + 32, st));

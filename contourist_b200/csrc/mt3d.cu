@@ -28,8 +28,6 @@
 #include <algorithm>
 #include <vector>
 
-#define CTR_BP_ATTR_BASE 0   // bits of ctr_ctx::attr_mask used by this file's bitplane kernels
-#define CTR_BP_ATTR_INT_BASE 9   // bits 9-14: its integer-sample bitplane kernels
 #include "bitplane.cuh"
 #include "tables.h"
 #include "uf_hash.cuh"
@@ -1526,12 +1524,8 @@ int run_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts* out, int 
                    (uint4*)ctx->aux[35].p, (size_t)(nrows + 3) / 4, st_vt, (size_t)ntiles);
     ctx->launches++;
     CTR_DBG(ctx, "k_reset3");
-    if (p->flags & CTR_WANT_MINMAX)
-      rc = launch_bitplane<T, true>(ctx, dfield, (unsigned)nrows, n2, W, n0, n1, p->isovalue, (uint32_t*)ctx->bits.p,
-                                    (uint32_t*)ctx->nbits.p, (uint8_t*)ctx->aux[4].p, (MinMaxKeys*)dctr, false, (uint32_t*)ctx->aux[32].p);
-    else
-      rc = launch_bitplane<T, false>(ctx, dfield, (unsigned)nrows, n2, W, n0, n1, p->isovalue, (uint32_t*)ctx->bits.p,
-                                     (uint32_t*)ctx->nbits.p, (uint8_t*)ctx->aux[4].p, (MinMaxKeys*)dctr, false, (uint32_t*)ctx->aux[32].p);
+    rc = launch_bitplane<T>(ctx, dfield, (unsigned)nrows, n2, W, n0, n1, p->isovalue, (uint32_t*)ctx->bits.p, (uint32_t*)ctx->nbits.p,
+                            (uint8_t*)ctx->aux[4].p, (MinMaxKeys*)dctr, (p->flags & CTR_WANT_MINMAX) != 0, false, (uint32_t*)ctx->aux[32].p);
     if (rc) return rc;
     CTR_DBG(ctx, "k_bitplane");
     ctr_stage_mark(ctx, 2);

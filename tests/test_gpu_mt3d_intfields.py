@@ -27,12 +27,12 @@ def _run(engine, field, value, flags, **kw):
 
 
 def _assert_same(a, b):
-    # fmin / fmax are checked against numpy in check_int_field, not against the float runs: the float stage-1 kernel
-    # reports fmax = +inf when the field's size is not a multiple of its 16 KiB chunk (the neutralised samples of the
-    # partial last chunk take part in the max)
     (ca, oa), (cb, ob) = a, b
     for name in ("n_verts", "n_tris", "n_active_cells", "n_crossings", "n_codes"):
         assert getattr(ca, name) == getattr(cb, name), name
+    for name in ("fmin", "fmax"):                             # NaN both: the run did not ask for them
+        x, y = getattr(ca, name), getattr(cb, name)
+        assert x == y or (np.isnan(x) and np.isnan(y)), (name, x, y)
     for name in ("verts", "normals", "tris", "keys", "lowmin"):
         if oa[name] is not None or ob[name] is not None:
             assert oa[name].dtype == ob[name].dtype and np.array_equal(oa[name], ob[name]), name
@@ -133,43 +133,103 @@ def test_misaligned_device_pointer(engine):
     _assert_same((c, engine.mt3d_fetch()), want)
 
 
-@pytest.mark.parametrize("kind", ["tma", "generic", "vec"])
+def _off_alignment(field):
+    """A device copy of `field` one sample past a 16-byte boundary: (buffer to keep alive, pointer)."""
+    import torch
+    tdt = {np.uint8: torch.uint8, np.int16: torch.int16, np.uint16: torch.uint16, np.float32: torch.float32,
+           np.float64: torch.float64}[field.dtype.type]
+    buf = torch.zeros(field.size + 16, dtype=tdt, device="cuda")
+    flat = field.reshape(-1)
+    src = torch.from_numpy(flat.astype(np.int32) if flat.dtype.kind in "iu" else flat)
+    buf[1:1 + field.size] = src.to("cuda").to(tdt)
+    torch.cuda.synchronize()
+    return buf, buf.data_ptr() + field.itemsize
+
+
+@pytest.mark.parametrize("layout", ["aligned", "off_alignment", "rows129"])
 @pytest.mark.parametrize("dt", INTS, ids=[np.dtype(d).name for d in INTS])
-def test_stage1_choice(engine, monkeypatch, kind, dt):
-    """Every CTR_BITPLANE choice gives the float64 result (integer fields have no vec kernel: it falls back to generic)."""
+def test_stage1_choice(engine, layout, dt):
+    """Both stage-1 kernels give the float64 result: rows a multiple of 32 samples from an aligned buffer (TMA), the same
+    field from a device pointer one sample off alignment and rows of 129 samples (generic)."""
+    from contourist_b200 import engine as E
     rng = np.random.default_rng(7)
-    f, mid = _random_field(rng, (12, 10, 64), dt)
-    monkeypatch.setenv("CTR_BITPLANE", kind)
+    f, mid = _random_field(rng, (12, 10, 129 if layout == "rows129" else 64), dt)
     for v in (mid, mid + 0.5, mid - 2.0):
         for geom64 in (True, False):
-            check_int_field(engine, f, float(v), geom64)
+            if layout != "off_alignment":
+                check_int_field(engine, f, float(v), geom64)
+                continue
+            flags = _flags(geom64)
+            buf, ptr = _off_alignment(f)
+            c = engine.mt3d_run(ptr, float(v), flags=flags | E.FIELD_ON_DEVICE, shape=f.shape, dtype=dt)
+            ri = (c, engine.mt3d_fetch())
+            del buf
+            assert c.fmin == f.min() and c.fmax == f.max()
+            _assert_same(ri, _run(engine, f.astype(np.float64), float(v), flags))
+            if not geom64:
+                _assert_same(ri, _run(engine, f.astype(np.float32), float(v), flags))
 
 
-def _stage1_kernels(engine, field, value):
+def _stage1_kernels(engine, field, value, off_alignment=False):
+    """The stage-1 kernel instances of one run, as `k_bitplane_<path><first template argument`."""
+    import re
     import torch
     from torch.profiler import ProfilerActivity, profile
+    from contourist_b200 import engine as E
+    flags = _flags(False, codes=False, minmax=False)
+    arg, kw = field, {}
+    if off_alignment:
+        buf, arg = _off_alignment(field)
+        flags |= E.FIELD_ON_DEVICE
+        kw = dict(shape=field.shape, dtype=field.dtype.type)
     torch.cuda.synchronize()
     with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        engine.mt3d_run(field, value, flags=_flags(False, codes=False, minmax=False))
+        engine.mt3d_run(arg, value, flags=flags, **kw)
         torch.cuda.synchronize()
     names = [e.name for e in prof.events()]
     assert any("k_emit_verts" in n for n in names), "the profiler did not see the extraction's kernels"
-    return sorted({n.split("<")[0].split("::")[-1] for n in names if "k_bitplane" in n})
+    return sorted({m.group(1) for n in names for m in [re.search(r"(k_bitplane_\w+<[^,>]+)", n)] if m})
 
 
-@pytest.mark.parametrize("dt", INTS, ids=[np.dtype(d).name for d in INTS])
-def test_stage1_kernel_that_runs(engine, monkeypatch, dt):
-    """Rows of 32k samples from an aligned buffer take the integer TMA kernel; other rows, and CTR_BITPLANE=vec, the
-    integer generic kernel.  The float32 copy still takes the float TMA kernel."""
-    monkeypatch.delenv("CTR_BITPLANE", raising=False)
+FLOATS = [np.float32, np.float64]
+CTYPE = {np.uint8: "unsigned char", np.int16: "short", np.uint16: "unsigned short", np.float32: "float",
+         np.float64: "double"}
+
+
+def _field(rng, shape, dt):
+    if dt in FLOATS:
+        return rng.standard_normal(shape).astype(dt), 0.0
+    return _random_field(rng, shape, dt)
+
+
+@pytest.mark.parametrize("layout", ["aligned", "off_alignment", "rows129"])
+@pytest.mark.parametrize("dt", INTS + FLOATS, ids=[np.dtype(d).name for d in INTS + FLOATS])
+def test_stage1_kernel_that_runs(engine, dt, layout):
+    """Rows of 32k samples from an aligned buffer take the TMA kernel of the field's sample type; the same rows from a
+    device pointer one sample off alignment, and rows of 129 samples, its generic kernel."""
     rng = np.random.default_rng(9)
-    f, mid = _random_field(rng, (16, 12, 64), dt)
-    assert _stage1_kernels(engine, f, mid + 0.5) == ["k_bitplane_tma_int"]
-    assert _stage1_kernels(engine, f.astype(np.float32), mid + 0.5) == ["k_bitplane_tma"]
-    g, _ = _random_field(rng, (9, 9, 129), dt)
-    assert _stage1_kernels(engine, g, mid + 0.5) == ["k_bitplane_generic_int"]
-    monkeypatch.setenv("CTR_BITPLANE", "vec")
-    assert _stage1_kernels(engine, f, mid + 0.5) == ["k_bitplane_generic_int"]
+    f, mid = _field(rng, (9, 9, 129) if layout == "rows129" else (16, 12, 64), dt)
+    kind = "tma" if layout == "aligned" else "generic"
+    got = _stage1_kernels(engine, f, mid + 0.5, off_alignment=layout == "off_alignment")
+    assert got == ["k_bitplane_%s<%s" % (kind, CTYPE[dt])]
+
+
+@pytest.mark.parametrize("dt", FLOATS, ids=[np.dtype(d).name for d in FLOATS])
+def test_minmax_partial_last_chunk(engine, dt):
+    """fmin / fmax of float fields on the TMA path whose size in bytes is not a multiple of the kernel's 16 KiB chunk:
+    the stale tail of the last chunk takes no part, in 3D and in 4D."""
+    from contourist_b200 import engine as E
+    rng = np.random.default_rng(13)
+    for shape in ((5, 7, 64), (9, 33, 96)):
+        f = (rng.standard_normal(shape) + 1.0).astype(dt)
+        assert f.nbytes % 16384 != 0
+        c = engine.mt3d_run(f, 1.0, flags=E.WANT_MINMAX)
+        assert (c.fmin, c.fmax) == (f.min(), f.max()), shape
+    for shape in ((4, 5, 6, 64), (3, 4, 5, 96)):
+        f = (rng.standard_normal(shape) + 1.0).astype(dt)
+        assert f.nbytes % 16384 != 0
+        c = engine.mp4d_run(f, 1.0, flags=E.WANT_MINMAX)
+        assert (c.fmin, c.fmax) == (f.min(), f.max()), shape
 
 
 # ---------------------------------------------------------------------------------------------- 3. near hull
