@@ -146,6 +146,7 @@ int interp_typed(ctr_ctx* ctx, const ctr_attr_params* ap, int64_t* n_verts) {
   CTR_CUDA(ctx, cudaStreamSynchronize(st));
   ctx->attr_rows = nV;
   ctx->attr_ncomp = ap->ncomp;
+  ctx->attr_gen = ctx->mesh_gen;
   if (n_verts) *n_verts = (int64_t)nV;
   return 0;
 }

@@ -57,7 +57,11 @@ struct ctr_ctx {
   int64_t poly_counts[2] = {};            // 2D: polylines / points of the last ctr_mt2d_polylines
   unsigned char last3_params[160] = {};   // parameters of the last completed ctr_mt3d_run
   long long* publish3 = nullptr;          // ctr_mt3d_publish_counts: device {n_verts, n_tris} behind every 3D run
-  unsigned last3_edited = 0;              // passes that have rewritten the device mesh of that run: 1 seeded selection, 2 clean-up
+  unsigned last3_edited = 0;              // passes that have rewritten the device mesh of that run: 1 seeded selection, 2 clean-up,
+                                          // 4 component filter
+  // bumped by every 3D run and every pass that removes or renumbers mesh rows (selection, clean-up, offset_ids,
+  // component filter); the vertex values and the components below record the generation they were computed on
+  uint64_t mesh_gen = 0;
   // 3D: an extraction enqueued by ctr_mt3d_enqueue and not yet finished
   bool pending3 = false;
   alignas(8) unsigned char pending3_params[160] = {};
@@ -68,9 +72,11 @@ struct ctr_ctx {
   // 3D vertex values (ctr_mt3d_interpolate): rows and components of aux[43]; 0 = none since the last 3D run
   size_t attr_rows = 0;
   int attr_ncomp = 0;
+  uint64_t attr_gen = 0;
   // 3D connected components (ctr_mt3d_components): triangles and components of aux[44] / aux[45]; -1 = none since the
   // last 3D run
   int64_t comp_tris = 0, comp_count = -1;
+  uint64_t comp_gen = 0;
 
   // 2D / 4D extra outputs are declared in their own translation units via these generic slots
   DevBuf aux[48];            // 0-4, 32-35, 41: 3D; 5-10: 2D; 12-26: 4D; 27-31: mesh passes; 36-40: 2D polylines;

@@ -247,6 +247,7 @@ int components_typed(ctr_ctx* ctx, int64_t* n_components) {
   if (nt == 0) {
     ctx->comp_tris = 0;
     ctx->comp_count = 0;
+    ctx->comp_gen = ctx->mesh_gen;
     return 0;
   }
   size_t nslots = 1;
@@ -302,6 +303,7 @@ int components_typed(ctr_ctx* ctx, int64_t* n_components) {
   CTR_CUDA(ctx, cudaStreamSynchronize(st));
   ctx->comp_tris = nt;
   ctx->comp_count = nc;
+  ctx->comp_gen = ctx->mesh_gen;
   if (n_components) *n_components = nc;
   return 0;
 }

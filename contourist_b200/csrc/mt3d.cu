@@ -1666,6 +1666,7 @@ int run_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts* out, int 
 }
 
 #include "mt3d_select.cuh"
+#include "mt3d_keep.cuh"
 #include "mt3d_clean.cuh"
 #include "attr3d.cuh"
 
@@ -1691,6 +1692,7 @@ static int mt3d_dispatch(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
   if (out) memset(out, 0, sizeof *out);
   ctx->last_kind = 0;
+  ctx->mesh_gen++;
   ctx->attr_ncomp = 0;                                 // vertex values of the previous run are gone
   ctx->comp_count = -1;                                // ... and so are its components
   switch (p->dtype) {
@@ -1738,6 +1740,7 @@ extern "C" int ctr_mt3d_offset_ids(ctr_ctx* ctx, int64_t base) {
   if (base < 0 || base > 0x7fffffffll) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "id base out of range");
   const size_t n = (size_t)ctx->last_counts[1] * 3;
   if (!n || !base) return 0;
+  ctx->mesh_gen++;
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
   k_offset_ids<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>((int*)ctx->tris.p, n, (int)base);
   ctx->launches++;
@@ -1809,7 +1812,8 @@ extern "C" int ctr_mt3d_select_seeded(ctr_ctx* ctx, const int32_t* seed_voxels, 
   // the selection compacts the run's mesh in place while the voxel work list keeps its per-voxel triangle offsets: it
   // can be applied once per run
   if (ctx->last3_edited)
-    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has already been selected from or cleaned; run ctr_mt3d_run again");
+    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has already been selected from, cleaned or filtered; run ctr_mt3d_run again");
+  ctx->mesh_gen++;
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
   switch (p->dtype) {
     case CTR_F32: return select_typed<float>(ctx, p, seed_voxels, n_seeds, n_verts, n_tris, n_voxels);
@@ -1819,6 +1823,19 @@ extern "C" int ctr_mt3d_select_seeded(ctr_ctx* ctx, const int32_t* seed_voxels, 
     case CTR_U16: return select_typed<uint16_t>(ctx, p, seed_voxels, n_seeds, n_verts, n_tris, n_voxels);
   }
   return ctr_fail(ctx, CTR_ERR_BAD_ARG, "unknown dtype");
+}
+
+extern "C" int ctr_mt3d_keep_components(ctr_ctx* ctx, const uint8_t* keep, int64_t n_keep, int64_t* n_verts, int64_t* n_tris) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (ctx->last_kind != 3 || ctx->comp_count < 0)
+    return ctr_fail(ctx, CTR_ERR_STATE, "no ctr_mt3d_components since the last 3D run");
+  if (ctx->comp_gen != ctx->mesh_gen)
+    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh was edited after ctr_mt3d_components (selection, clean-up or offset_ids): "
+                                        "call ctr_mt3d_components again");
+  if (n_keep != ctx->comp_count || (!keep && n_keep > 0))
+    return ctr_fail(ctx, CTR_ERR_BAD_ARG, "keep must hold one byte per component of the last ctr_mt3d_components call");
+  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
+  return keep_components_run(ctx, keep, n_verts, n_tris);
 }
 
 extern "C" int ctr_mt3d_clean(ctr_ctx* ctx, const ctr_clean_params* cp, ctr_clean_counts* out) {
@@ -1839,6 +1856,7 @@ extern "C" int ctr_mt3d_clean(ctr_ctx* ctx, const ctr_clean_params* cp, ctr_clea
   }
   if (cp->divisions < 1 || cp->divisions >= (1 << 21)) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "divisions must be in [1, 2^21)");
   if (!(cp->epsilon == cp->epsilon)) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "epsilon is NaN");
+  ctx->mesh_gen++;
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
   if (ctx->last_flags & CTR_GEOM_F64) return clean_typed<double>(ctx, cp, out);
   return clean_typed<float>(ctx, cp, out);

@@ -148,6 +148,8 @@ def load_library():
     lib.ctr_mt3d_components.restype = i32
     lib.ctr_mt3d_components_fetch.argtypes = [vp, vp, vp]
     lib.ctr_mt3d_components_fetch.restype = i32
+    lib.ctr_mt3d_keep_components.argtypes = [vp, vp, i64, ctypes.POINTER(i64), ctypes.POINTER(i64)]
+    lib.ctr_mt3d_keep_components.restype = i32
     lib.ctr_mt3d_interpolate.argtypes = [vp, ctypes.POINTER(AttrParams), ctypes.POINTER(i64)]
     lib.ctr_mt3d_interpolate.restype = i32
     lib.ctr_mt3d_interpolate_fetch.argtypes = [vp, vp]
@@ -436,15 +438,55 @@ class Engine(object):
         COMPONENT_DTYPE), numbered by smallest triangle index (ctr_mt3d_components).  Per component: triangle, vertex
         and edge counts (n_verts - n_edges + n_tris is the Euler characteristic), boundary and non-manifold edges, fp64
         area, signed enclosed volume (> 0 around a region below the isovalue on the raw mesh, >= 0 for closed
-        components after orientation) and the box lo / hi.  Not updated by a later selection or clean-up."""
+        components after orientation) and the box lo / hi.  Not updated by a later selection or clean-up
+        (mt3d_keep_components updates them)."""
         n = ctypes.c_int64()
+        self._comp_shape = None
         self._check(self.lib.ctr_mt3d_components(self.h, ctypes.byref(n)), "ctr_mt3d_components")
-        _, c = self._last3
-        labels = np.empty(int(c.n_tris), np.int32)
-        table = np.empty(int(n.value), COMPONENT_DTYPE)
-        self._check(self.lib.ctr_mt3d_components_fetch(self.h, _ptr(labels) if len(labels) else None,
-                                                       _ptr(table) if len(table) else None), "ctr_mt3d_components_fetch")
+        self._comp_shape = (int(self._last3[1].n_tris), int(n.value))
+        return self.mt3d_components_fetch()
+
+    def mt3d_components_fetch(self):
+        """The current (tri_component, table) of the last mt3d_components(), as a later mt3d_keep_components() left
+        them, without measuring again (ctr_mt3d_components_fetch)."""
+        T, C = getattr(self, "_comp_shape", None) or (0, 0)   # (no results: the library refuses the fetch)
+        labels = np.empty(T, np.int32)
+        table = np.empty(C, COMPONENT_DTYPE)
+        self._check(self.lib.ctr_mt3d_components_fetch(self.h, _ptr(labels) if T else None, _ptr(table) if C else None),
+                    "ctr_mt3d_components_fetch")
         return labels, table
+
+    def mt3d_keep_components(self, keep):
+        """Keep the components named by `keep` on the device mesh and drop the others (ctr_mt3d_keep_components):
+        `keep` is a boolean mask with one entry per component of the last mt3d_components(), or an array of component
+        indices.  Kept triangles and vertices stay in order, ids renumbered; normals, keys and the values of an
+        mt3d_interpolate() made on this mesh are compacted with them, and the component results are renumbered
+        0..K-1 (mt3d_components_fetch()).  Returns (n_verts, n_tris); fetch afterwards."""
+        C = (getattr(self, "_comp_shape", None) or (0, -1))[1]
+        k = np.asarray(keep)
+        if k.dtype == np.bool_:
+            if C >= 0 and k.shape != (C,):
+                raise ValueError("keep mask of shape %r: the last mt3d_components() found %d components" % (k.shape, C))
+            mask = k.astype(np.uint8)
+        elif k.size == 0 or np.issubdtype(k.dtype, np.integer):
+            idx = k.astype(np.int64).reshape(-1)
+            if len(idx) and (idx.min() < 0 or idx.max() >= max(C, 0)):
+                raise ValueError("component index outside [0, %d)" % max(C, 0))
+            mask = np.zeros(max(C, 0), np.uint8)
+            mask[idx] = 1
+        else:
+            raise TypeError("keep: a boolean mask or integer component indices, not %s" % k.dtype)
+        mask = np.ascontiguousarray(mask)
+        nv, nt = ctypes.c_int64(), ctypes.c_int64()
+        self.run_serial += 1
+        self._check(self.lib.ctr_mt3d_keep_components(self.h, _ptr(mask) if len(mask) else None, len(mask), ctypes.byref(nv),
+                                                      ctypes.byref(nt)), "ctr_mt3d_keep_components")
+        flags, c = self._last3
+        c = type(c).from_buffer_copy(c)                                # the caller keeps the full scan's counts
+        c.n_verts, c.n_tris = int(nv.value), int(nt.value)             # what mt3d_fetch sizes its arrays from
+        self._last3 = (flags, c)
+        self._comp_shape = (int(nt.value), int(mask.astype(bool).sum()))
+        return int(nv.value), int(nt.value)
 
     def mt3d_interpolate(self, field, shape=None, dtype=None):
         """Values of another field at the vertices of the last 3D run's mesh as it stands now (after a selection or
@@ -453,7 +495,7 @@ class Engine(object):
         the run's array shape [n0, n1, n2] or [n0, n1, n2, c] (c = 1..4), or an integer device pointer with shape and
         dtype.  Host arrays of float32 / float64 / uint8 / int16 / uint16 are read as they are, other types are widened
         to float64.  Returns [V] (or [V, c]) in the run's geometry type.  Values are not compacted by a later selection
-        or clean-up: interpolate after the last one."""
+        or clean-up: interpolate after the last one (mt3d_keep_components does compact them)."""
         p = AttrParams()
         codes = tuple(DTYPE_CODES.values())
         if isinstance(field, np.ndarray):

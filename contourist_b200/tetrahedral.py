@@ -22,6 +22,8 @@ extract_surface_geometry().  Differences, all documented in DESIGN.md section 2:
   * search_for_endpoints() already runs the extraction (the crossing scan is its first two stages);
     get_points_and_triangles() then only post-processes and fetches that run.
 """
+import numbers
+
 import numpy as np
 
 from . import engine as E
@@ -96,6 +98,19 @@ def initial_voxels(samples, value, end_points):
     return np.array(sorted(set(found)), dtype=np.int32).reshape(-1, 3)
 
 
+def components_to_keep(table, rule):
+    """What GridContour3d.keep_components asks for, on a component table (engine.COMPONENT_DTYPE): an int k names the k
+    components with the most triangles (ties: the smaller component number; triangle counts are exact, so the choice
+    is deterministic), a callable is called with the table and returns a boolean mask or component indices."""
+    if isinstance(rule, numbers.Integral) and not isinstance(rule, bool):
+        if rule < 0:
+            raise ValueError("keep_components = %d: a number of components >= 0" % rule)
+        return np.argsort(-table["n_tris"], kind="stable")[:int(rule)]
+    if callable(rule):
+        return rule(table)
+    raise TypeError("keep_components: None, an int or a callable, not %r" % (rule,))
+
+
 class GridContour3d(object):
     """Grid-coordinate engine front end (reference: GridContour + GridContour3d, tetrahedral.py:109-621).
 
@@ -126,6 +141,10 @@ class GridContour3d(object):
     measure_components = False
     triangle_components = None
     component_table = None
+    # keep_components: None (everything), an int k (the k components with the most triangles) or a callable
+    # table -> boolean mask or component indices; get_points_and_triangles() then returns only those components
+    # (ctr_mt3d_keep_components), and vertex_values / triangle_components / component_table describe that mesh
+    keep_components = None
 
     def __init__(self, corner, function, value, segment_endpoints, linear_interpolate=True, callback=None,
                  origin=(0.0, 0.0, 0.0), delta=(1.0, 1.0, 1.0)):
@@ -198,6 +217,10 @@ class GridContour3d(object):
         elif self.reference_orientation:
             # surface_geometry.py:52-140 on the device mesh: one keep / reverse decision per edge-connected component
             self.components, self.flipped = eng.mt3d_orient_reference()
+        if self.keep_components is not None:
+            # after every pass that edits the mesh, before the values and the measurement below
+            _, table = eng.mt3d_components()
+            eng.mt3d_keep_components(components_to_keep(table, self.keep_components))
         if self.vertex_fields is not None:
             # after every pass that edits the mesh: the values line up with the points fetched below
             many = isinstance(self.vertex_fields, (list, tuple))
@@ -205,8 +228,9 @@ class GridContour3d(object):
                     for f in (self.vertex_fields if many else [self.vertex_fields])]
             self.vertex_values = vals if many else vals[0]
         if self.measure_components:
-            # after every pass that edits the mesh, like the values above
-            self.triangle_components, self.component_table = eng.mt3d_components()
+            # after every pass that edits the mesh, like the values above; the filter has already measured this mesh
+            self.triangle_components, self.component_table = \
+                eng.mt3d_components_fetch() if self.keep_components is not None else eng.mt3d_components()
         out = eng.mt3d_fetch()
         self.normals = out["normals"]
         points, triangles = out["verts"], out["tris"]
@@ -261,7 +285,7 @@ class Delta3DContour(object):
     def _configure(self, maker):
         "options set on this driver (before or after the maker was built) reach the maker"
         for name in ("post_process", "geometry_dtype", "want_normals", "reference_orientation", "quantize_divisions",
-                     "tiny_epsilon", "vertex_fields", "measure_components"):
+                     "tiny_epsilon", "vertex_fields", "measure_components", "keep_components"):
             if hasattr(self, name):
                 setattr(maker, name, getattr(self, name))
         maker.field_grid = self.grid

@@ -193,7 +193,7 @@ CTR_API int ctr_mt3d_orient_reference(ctr_ctx* ctx, int64_t* n_components, int64
  *   _components      : *n_components (may be NULL) receives C
  *   _components_fetch: tri_component [n_tris] (the component of every triangle, row for row with ctr_mt3d_fetch's
  *                      triangles) and components [C]; either may be NULL.  These are the results of the last call: a
- *                      later selection or clean-up does not update them.                                             */
+ *                      later selection or clean-up does not update them (ctr_mt3d_keep_components does).             */
 typedef struct {
   int64_t n_tris, n_verts, n_edges;          /* faces, distinct vertices, distinct undirected edges of the component  */
   int64_t n_boundary_edges;                  /* edges used by exactly one triangle                                     */
@@ -205,6 +205,31 @@ typedef struct {
 } ctr_mt3d_component;                        /* 112 bytes */
 CTR_API int ctr_mt3d_components(ctr_ctx* ctx, int64_t* n_components);
 CTR_API int ctr_mt3d_components_fetch(ctr_ctx* ctx, int32_t* tri_component, ctr_mt3d_component* components);
+
+/* Keeps the components whose keep[c] is non-zero and drops the others, on the LAST 3D run's device mesh as the last
+ * ctr_mt3d_components call measured it (engine extension, like VTK's vtkPolyDataConnectivityFilter with specified
+ * regions; oracle/mt3d_filter.py:keep_components is the definition).  Synchronous on return.
+ *   - keep: host array of n_keep == C bytes, indexed by the component numbers of the last ctr_mt3d_components call.
+ *     *n_verts and *n_tris (either may be NULL) receive the new counts; fetch afterwards.
+ *   - A triangle stays when its component is kept; kept triangles stay in their order.  A vertex stays when a kept
+ *     triangle uses it (also one that a kept and a dropped component share); kept vertices stay in their order and the
+ *     ids in the triangles are rewritten.  Positions, normals (CTR_WANT_NORMALS), keys / lowmin (CTR_WANT_KEYS) and the
+ *     values of a ctr_mt3d_interpolate made on the current mesh are compacted in place, so _interpolate_fetch stays
+ *     row for row with ctr_mt3d_fetch.  Cells and codes stay those of the full scan, as after a selection.
+ *   - The component results are updated, not dropped: the kept components are renumbered 0..K-1 in their old order,
+ *     tri_component is compacted and relabelled, the table rows are compacted with first_tri the compacted index (still
+ *     the component's smallest triangle).  Every other field is carried over: a component is kept whole, so they stay
+ *     true.  ctr_mt3d_components_fetch returns the filtered results; calling this again filters further.
+ *   - The device buffers are rewritten in place: pointers from ctr_mt3d_device_ptrs and
+ *     ctr_mt3d_interpolate_device_ptr stay valid.  The counts published by ctr_mt3d_publish_counts stay those of the
+ *     run.
+ *   - A seeded selection after this call returns CTR_ERR_STATE; ctr_mt3d_clean, ctr_mt3d_orient_reference,
+ *     ctr_mt3d_components and ctr_mt3d_interpolate are accepted.
+ *   - CTR_ERR_BAD_ARG: n_keep != C, or keep == NULL with C > 0.  CTR_ERR_STATE: no 3D run, a CTR_NO_GEOMETRY run or no
+ *     ctr_mt3d_components since the last run; or the mesh was edited after that call by ctr_mt3d_select_seeded,
+ *     ctr_mt3d_clean or ctr_mt3d_offset_ids (ctr_mt3d_orient_reference only swaps corners inside triangles: the labels
+ *     stay valid).  An empty mesh (C = 0) is a valid no-op; keeping nothing leaves an empty mesh.                      */
+CTR_API int ctr_mt3d_keep_components(ctr_ctx* ctx, const uint8_t* keep, int64_t n_keep, int64_t* n_verts, int64_t* n_tris);
 
 /* Seeded extraction (SURVEY.md 8(f3)): restricts the LAST full-volume run's mesh to what the reference's tracker
  *   tetrahedral.py:443-469  expand_voxels / in_range  (flood fill over the 26-neighbourhood of border voxels)
