@@ -58,9 +58,10 @@ struct ctr_ctx {
   unsigned char last3_params[160] = {};   // parameters of the last completed ctr_mt3d_run
   long long* publish3 = nullptr;          // ctr_mt3d_publish_counts: device {n_verts, n_tris} behind every 3D run
   unsigned last3_edited = 0;              // passes that have rewritten the device mesh of that run: 1 seeded selection, 2 clean-up,
-                                          // 4 component filter
+                                          // 4 component filter, 8 smoothing
   // bumped by every 3D run and every pass that removes or renumbers mesh rows (selection, clean-up, offset_ids,
-  // component filter); the vertex values and the components below record the generation they were computed on
+  // component filter) or moves vertices (smoothing); the vertex values and the components below record the generation
+  // they were computed on
   uint64_t mesh_gen = 0;
   // 3D: an extraction enqueued by ctr_mt3d_enqueue and not yet finished
   bool pending3 = false;
@@ -81,7 +82,8 @@ struct ctr_ctx {
   // 2D / 4D extra outputs are declared in their own translation units via these generic slots
   DevBuf aux[48];            // 0-4, 32-35, 41: 3D; 5-10: 2D; 12-26: 4D; 27-31: mesh passes; 36-40: 2D polylines;
                              // 42-43: 3D vertex values (staged attribute field, values);
-                             // 44-45: 3D connected components (triangle labels, component table)
+                             // 44-45: 3D connected components (triangle labels, component table);
+                             // 46-47: smoothing's fp64 working copies
 };
 
 static inline int ctr_fail(ctr_ctx* ctx, int code, const char* what, const char* detail = "") {

@@ -12,6 +12,7 @@
 //   k_o_decide / k_o_flip : reverse the triangles of components whose seed has cross.x < 0.
 // Components are joined through shared EDGES, as in the reference (two sheets touching in one vertex stay apart).
 // components3d.cuh (ctr_mt3d_components) reuses the edge table and k_o_union to number and measure the components.
+// smooth3d.cuh (ctr_mt3d_smooth) builds the same edge table with its use counts for the fixed vertices and neighbour lists.
 #include <math.h>
 #include <string.h>
 
@@ -220,6 +221,7 @@ int orient_typed(ctr_ctx* ctx, int64_t* n_components, int64_t* n_flipped) {
 }
 
 #include "components3d.cuh"
+#include "smooth3d.cuh"
 
 }  // namespace
 
@@ -244,6 +246,24 @@ extern "C" int ctr_mt3d_components(ctr_ctx* ctx, int64_t* n_components) {
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
   if (ctx->last_flags & CTR_GEOM_F64) return components_typed<double>(ctx, n_components);
   return components_typed<float>(ctx, n_components);
+}
+
+extern "C" int ctr_mt3d_smooth(ctr_ctx* ctx, const ctr_smooth_params* sp, ctr_smooth_counts* out) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (!sp || !out) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  memset(out, 0, sizeof *out);
+  if (sp->iterations < 0 || sp->iterations > 1000) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "iterations must be in [0, 1000]");
+  if (sp->reserved != 0) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "reserved must be 0");
+  if (!(sp->lambda > 0.0 && sp->lambda <= 1.0)) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "lambda must be in (0, 1]");
+  if (!(sp->mu >= -1.0 && sp->mu <= 0.0)) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "mu must be in [-1, 0]");
+  if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
+    return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to smooth");
+  const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
+  if (p->i_lo != 0 || p->i_hi != p->n0 || p->vert_id_base != 0)
+    return ctr_fail(ctx, CTR_ERR_STATE, "smoothing needs a full-volume run with vert_id_base 0 (a slab's halo ids belong to another shard)");
+  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
+  if (ctx->last_flags & CTR_GEOM_F64) return smooth_typed<double>(ctx, sp, out);
+  return smooth_typed<float>(ctx, sp, out);
 }
 
 extern "C" int ctr_mt3d_components_fetch(ctr_ctx* ctx, int32_t* tri_component, ctr_mt3d_component* components) {

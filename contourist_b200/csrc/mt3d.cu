@@ -1812,7 +1812,7 @@ extern "C" int ctr_mt3d_select_seeded(ctr_ctx* ctx, const int32_t* seed_voxels, 
   // the selection compacts the run's mesh in place while the voxel work list keeps its per-voxel triangle offsets: it
   // can be applied once per run
   if (ctx->last3_edited)
-    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has already been selected from, cleaned or filtered; run ctr_mt3d_run again");
+    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has already been selected from, cleaned, filtered or smoothed; run ctr_mt3d_run again");
   ctx->mesh_gen++;
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
   switch (p->dtype) {
@@ -1830,7 +1830,7 @@ extern "C" int ctr_mt3d_keep_components(ctr_ctx* ctx, const uint8_t* keep, int64
   if (ctx->last_kind != 3 || ctx->comp_count < 0)
     return ctr_fail(ctx, CTR_ERR_STATE, "no ctr_mt3d_components since the last 3D run");
   if (ctx->comp_gen != ctx->mesh_gen)
-    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh was edited after ctr_mt3d_components (selection, clean-up or offset_ids): "
+    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh was edited after ctr_mt3d_components (selection, clean-up, smoothing or offset_ids): "
                                         "call ctr_mt3d_components again");
   if (n_keep != ctx->comp_count || (!keep && n_keep > 0))
     return ctr_fail(ctx, CTR_ERR_BAD_ARG, "keep must hold one byte per component of the last ctr_mt3d_components call");
@@ -1845,6 +1845,8 @@ extern "C" int ctr_mt3d_clean(ctr_ctx* ctx, const ctr_clean_params* cp, ctr_clea
   if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
     return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to clean");
   if (ctx->last3_edited & 2u) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has already been cleaned");
+  // the reference's clean-up (quantize, tiny simplices) is defined on the interpolated positions
+  if (ctx->last3_edited & 8u) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has been smoothed: clean it up before smoothing");
   const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
   if (p->i_lo != 0 || p->i_hi != p->n0 || p->vert_id_base != 0)
     return ctr_fail(ctx, CTR_ERR_UNSUPPORTED, "mesh clean-up needs a full-volume run (merges cross slab faces)");

@@ -86,6 +86,15 @@ class CleanCounts(ctypes.Structure):
                 ("n_flipped", ctypes.c_int64)]
 
 
+class SmoothParams(ctypes.Structure):
+    _fields_ = [("iterations", ctypes.c_int32), ("reserved", ctypes.c_uint32), ("lam", ctypes.c_double),
+                ("mu", ctypes.c_double)]
+
+
+class SmoothCounts(ctypes.Structure):
+    _fields_ = [("n_edges", ctypes.c_int64), ("n_fixed_verts", ctypes.c_int64)]
+
+
 class PolyCounts(ctypes.Structure):
     _fields_ = [("n_polylines", ctypes.c_int64), ("n_points", ctypes.c_int64), ("junction_levels", ctypes.c_uint64)]
 
@@ -150,6 +159,8 @@ def load_library():
     lib.ctr_mt3d_components_fetch.restype = i32
     lib.ctr_mt3d_keep_components.argtypes = [vp, vp, i64, ctypes.POINTER(i64), ctypes.POINTER(i64)]
     lib.ctr_mt3d_keep_components.restype = i32
+    lib.ctr_mt3d_smooth.argtypes = [vp, ctypes.POINTER(SmoothParams), ctypes.POINTER(SmoothCounts)]
+    lib.ctr_mt3d_smooth.restype = i32
     lib.ctr_mt3d_interpolate.argtypes = [vp, ctypes.POINTER(AttrParams), ctypes.POINTER(i64)]
     lib.ctr_mt3d_interpolate.restype = i32
     lib.ctr_mt3d_interpolate_fetch.argtypes = [vp, vp]
@@ -487,6 +498,22 @@ class Engine(object):
         self._last3 = (flags, c)
         self._comp_shape = (int(nt.value), int(mask.astype(bool).sum()))
         return int(nv.value), int(nt.value)
+
+    def mt3d_smooth(self, iterations=10, lam=0.5, mu=-0.53):
+        """Taubin lambda|mu smoothing of the last 3D run's device mesh as it stands now, in place (ctr_mt3d_smooth;
+        oracle/mt3d_smooth.py is the definition): each iteration moves every free vertex by lam, then by mu, towards
+        the average of its edge neighbours (mu=0: plain Laplacian smoothing, which shrinks).  Vertices on boundary or
+        non-manifold edges stay bit for bit; normals (WANT_NORMALS) are recomputed; triangles and keys do not change.
+        Afterwards mt3d_components() must measure again before mt3d_keep_components(), and mt3d_select_seeded() /
+        mt3d_clean() are refused.  Returns SmoothCounts (n_edges, n_fixed_verts); fetch afterwards."""
+        p = SmoothParams()
+        p.iterations = int(iterations)
+        p.lam = float(lam)
+        p.mu = float(mu)
+        c = SmoothCounts()
+        self.run_serial += 1
+        self._check(self.lib.ctr_mt3d_smooth(self.h, ctypes.byref(p), ctypes.byref(c)), "ctr_mt3d_smooth")
+        return c
 
     def mt3d_interpolate(self, field, shape=None, dtype=None):
         """Values of another field at the vertices of the last 3D run's mesh as it stands now (after a selection or

@@ -145,6 +145,13 @@ class GridContour3d(object):
     # table -> boolean mask or component indices; get_points_and_triangles() then returns only those components
     # (ctr_mt3d_keep_components), and vertex_values / triangle_components / component_table describe that mesh
     keep_components = None
+    # smooth_iterations > 0: get_points_and_triangles() smooths the mesh on the device (Taubin lambda|mu,
+    # ctr_mt3d_smooth) after the component filter and before vertex_fields / measure_components, which then describe
+    # the smoothed mesh; vertices on boundary or non-manifold edges stay put.  `smooth` (the reference's
+    # smooth_interpolations) is a different algorithm and still raises.
+    smooth_iterations = 0
+    smooth_lambda = 0.5
+    smooth_mu = -0.53
 
     def __init__(self, corner, function, value, segment_endpoints, linear_interpolate=True, callback=None,
                  origin=(0.0, 0.0, 0.0), delta=(1.0, 1.0, 1.0)):
@@ -221,6 +228,11 @@ class GridContour3d(object):
             # after every pass that edits the mesh, before the values and the measurement below
             _, table = eng.mt3d_components()
             eng.mt3d_keep_components(components_to_keep(table, self.keep_components))
+        smoothed = self.smooth_iterations > 0
+        if smoothed:
+            # after the filter (its components are measured on the unsmoothed mesh), before the values and the
+            # measurement below
+            eng.mt3d_smooth(self.smooth_iterations, self.smooth_lambda, self.smooth_mu)
         if self.vertex_fields is not None:
             # after every pass that edits the mesh: the values line up with the points fetched below
             many = isinstance(self.vertex_fields, (list, tuple))
@@ -228,9 +240,10 @@ class GridContour3d(object):
                     for f in (self.vertex_fields if many else [self.vertex_fields])]
             self.vertex_values = vals if many else vals[0]
         if self.measure_components:
-            # after every pass that edits the mesh, like the values above; the filter has already measured this mesh
+            # after every pass that edits the mesh, like the values above; the filter has already measured this mesh,
+            # unless smoothing has moved it since
             self.triangle_components, self.component_table = \
-                eng.mt3d_components_fetch() if self.keep_components is not None else eng.mt3d_components()
+                eng.mt3d_components_fetch() if self.keep_components is not None and not smoothed else eng.mt3d_components()
         out = eng.mt3d_fetch()
         self.normals = out["normals"]
         points, triangles = out["verts"], out["tris"]
@@ -285,7 +298,8 @@ class Delta3DContour(object):
     def _configure(self, maker):
         "options set on this driver (before or after the maker was built) reach the maker"
         for name in ("post_process", "geometry_dtype", "want_normals", "reference_orientation", "quantize_divisions",
-                     "tiny_epsilon", "vertex_fields", "measure_components", "keep_components"):
+                     "tiny_epsilon", "vertex_fields", "measure_components", "keep_components", "smooth_iterations",
+                     "smooth_lambda", "smooth_mu"):
             if hasattr(self, name):
                 setattr(maker, name, getattr(self, name))
         maker.field_grid = self.grid

@@ -227,9 +227,48 @@ CTR_API int ctr_mt3d_components_fetch(ctr_ctx* ctx, int32_t* tri_component, ctr_
  *     ctr_mt3d_components and ctr_mt3d_interpolate are accepted.
  *   - CTR_ERR_BAD_ARG: n_keep != C, or keep == NULL with C > 0.  CTR_ERR_STATE: no 3D run, a CTR_NO_GEOMETRY run or no
  *     ctr_mt3d_components since the last run; or the mesh was edited after that call by ctr_mt3d_select_seeded,
- *     ctr_mt3d_clean or ctr_mt3d_offset_ids (ctr_mt3d_orient_reference only swaps corners inside triangles: the labels
- *     stay valid).  An empty mesh (C = 0) is a valid no-op; keeping nothing leaves an empty mesh.                      */
+ *     ctr_mt3d_clean, ctr_mt3d_smooth or ctr_mt3d_offset_ids (ctr_mt3d_orient_reference only swaps corners inside
+ *     triangles: the labels stay valid; after smoothing the areas and volumes are stale, so measure again).  An empty
+ *     mesh (C = 0) is a valid no-op; keeping nothing leaves an empty mesh.                                             */
 CTR_API int ctr_mt3d_keep_components(ctr_ctx* ctx, const uint8_t* keep, int64_t n_keep, int64_t* n_verts, int64_t* n_tris);
+
+/* Taubin lambda|mu smoothing of the LAST 3D run's device mesh as it stands now (after a selection, clean-up, orientation
+ * or component filter too), in place (engine extension, the smoothing step of VTK-style pipelines; the reference's
+ * smooth_interpolations is not reproduced -- oracle/mt3d_smooth.py:smooth is the definition).  Synchronous on return.
+ *   - An edge is {a, b}, a != b, of some triangle; its uses are the triangle edge slots on it.  A vertex on an edge used
+ *     once (boundary) or three or more times (non-manifold), or on no edge, is FIXED: it never moves and keeps its
+ *     position bit for bit -- a surface cut by the volume's box stays exactly on the box faces.
+ *   - Every free vertex moves towards the average of its distinct edge neighbours (fixed ones included), summed in
+ *     ascending id order: x' = x + w * (avg - x), multiply and add rounded apart.  A step is a Jacobi step (all vertices
+ *     read the positions from before the step); one iteration is a step with w = lambda, then one with w = mu (skipped
+ *     when mu == 0: plain Laplacian smoothing, which shrinks the surface; lambda 0.5 / mu -0.53 does not).  All in fp64
+ *     on a copy widened from the geometry type, rounded back once at the end: the positions equal the definition bit for
+ *     bit, and with CTR_GEOM_F64 n iterations followed by m equal n + m.
+ *   - Normals (CTR_WANT_NORMALS) are recomputed: per vertex the sum of cross(b - a, c - a) over its triangles (fp64, in
+ *     an unspecified order: equal to the definition within rounding), normalised, its sign chosen so that it does not
+ *     point against the old gradient normal (up the field, whatever the winding); a zero sum keeps the old normal.
+ *   - Nothing else changes: triangles, keys / lowmin, cells / codes, the counts, the counts published by
+ *     ctr_mt3d_publish_counts and every device pointer handed out before.
+ *   - After a call with iterations > 0 on a non-empty mesh: component results of an earlier ctr_mt3d_components are
+ *     stale (ctr_mt3d_keep_components returns CTR_ERR_STATE until ctr_mt3d_components measures again); vertex values of
+ *     an earlier ctr_mt3d_interpolate are not compacted by a later filter; ctr_mt3d_select_seeded and ctr_mt3d_clean
+ *     return CTR_ERR_STATE (the clean-up is defined on the interpolated positions: clean up first).
+ *     ctr_mt3d_orient_reference, ctr_mt3d_components, ctr_mt3d_interpolate and further smoothing are accepted; values
+ *     interpolated afterwards are still those at each vertex's edge crossing (the keys did not move).
+ *   - *out receives n_edges (distinct undirected edges, self-edges of degenerate triangles excluded) and n_fixed_verts,
+ *     also for iterations == 0, which writes nothing.
+ *   - CTR_ERR_BAD_ARG: a NULL argument, iterations outside [0, 1000], lambda outside (0, 1], mu outside [-1, 0], a NaN
+ *     parameter, reserved != 0.  CTR_ERR_STATE: no 3D run or a CTR_NO_GEOMETRY run; a slab run (i_lo != 0 or i_hi != n0)
+ *     or vert_id_base != 0; a triangle id outside [0, n_verts) (e.g. after ctr_mt3d_offset_ids), detected before
+ *     anything is written.  An empty mesh is a valid no-op.                                                            */
+typedef struct {
+  int32_t iterations;   /* lambda|mu pairs, 0..1000 (0: nothing is written, the counts are reported) */
+  uint32_t reserved;    /* 0 */
+  double lambda;        /* (0, 1], e.g. 0.5   */
+  double mu;            /* [-1, 0], e.g. -0.53; 0 = Laplacian (mu step skipped) */
+} ctr_smooth_params;
+typedef struct { int64_t n_edges, n_fixed_verts; } ctr_smooth_counts;
+CTR_API int ctr_mt3d_smooth(ctr_ctx* ctx, const ctr_smooth_params* p, ctr_smooth_counts* out);
 
 /* Seeded extraction (SURVEY.md 8(f3)): restricts the LAST full-volume run's mesh to what the reference's tracker
  *   tetrahedral.py:443-469  expand_voxels / in_range  (flood fill over the 26-neighbourhood of border voxels)
@@ -239,7 +278,7 @@ CTR_API int ctr_mt3d_keep_components(ctr_ctx* ctx, const uint8_t* keep, int64_t 
  * are compacted in place (order kept, ids renumbered); case codes / cells stay those of the full scan.  Returns the
  * new counts and the number of emitting voxels selected; fetch afterwards.  With CTR_FIELD_ON_DEVICE the field must
  * still be resident.  ONE-SHOT: the run's mesh is rewritten, so a second call on the same run (or a call after
- * ctr_mt3d_clean) returns CTR_ERR_STATE until the next ctr_mt3d_run.                                              */
+ * ctr_mt3d_clean, ctr_mt3d_keep_components or ctr_mt3d_smooth) returns CTR_ERR_STATE until the next ctr_mt3d_run.  */
 CTR_API int ctr_mt3d_select_seeded(ctr_ctx* ctx, const int32_t* seed_voxels, int64_t n_seeds, int64_t* n_verts,
                                    int64_t* n_tris, int64_t* n_voxels);
 
@@ -301,7 +340,9 @@ CTR_API int ctr_gathered_fetch(ctr_ctx* ctx, void* verts, void* normals, int32_t
  * which is what GridContour3d.get_points_and_triangles(clean=True) returns (tetrahedral.py:541-552).  The run must have
  * been made in GRID coordinates (origin 0, delta 1), over the full volume, with vert_id_base 0.  Where the reference's
  * result depends on CPython dict / set order the vertex of smallest id survives (oracle/post3d.py states the rules).
- * Vertices, normals, keys and triangles are compacted in place (order kept); fetch afterwards.  One-shot per run.  */
+ * Vertices, normals, keys and triangles are compacted in place (order kept); fetch afterwards.  One-shot per run, and
+ * not after ctr_mt3d_smooth (CTR_ERR_STATE: quantizing and the tiny-simplex test are defined on interpolated
+ * positions; clean up first, then smooth).                                                                           */
 #define CTR_CLEAN_ORIENT 1u        /* run the orientation pass before the transform                         */
 #define CTR_CLEAN_NO_TRIANGLES 2u  /* skip clean_triangles (get_points_and_triangles(clean=False))          */
 typedef struct {
