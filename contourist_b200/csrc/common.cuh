@@ -58,10 +58,10 @@ struct ctr_ctx {
   unsigned char last3_params[160] = {};   // parameters of the last completed ctr_mt3d_run
   long long* publish3 = nullptr;          // ctr_mt3d_publish_counts: device {n_verts, n_tris} behind every 3D run
   unsigned last3_edited = 0;              // passes that have rewritten the device mesh of that run: 1 seeded selection, 2 clean-up,
-                                          // 4 component filter, 8 smoothing
+                                          // 4 component filter, 8 smoothing, 16 decimation
   // bumped by every 3D run and every pass that removes or renumbers mesh rows (selection, clean-up, offset_ids,
-  // component filter) or moves vertices (smoothing); the vertex values and the components below record the generation
-  // they were computed on
+  // component filter, decimation) or moves vertices (smoothing); the vertex values and the components below record the
+  // generation they were computed on
   uint64_t mesh_gen = 0;
   // 3D: an extraction enqueued by ctr_mt3d_enqueue and not yet finished
   bool pending3 = false;

@@ -140,14 +140,6 @@ __global__ void k_m_table_init(ctr_mt3d_component* comp, unsigned nc) {
 }
 
 template <typename G>
-__device__ __forceinline__ void tri_corners(const G* __restrict__ verts, const int v[3], double p[3][3]) {
-#pragma unroll
-  for (int q = 0; q < 3; ++q)
-#pragma unroll
-    for (int a = 0; a < 3; ++a) p[q][a] = (double)verts[(size_t)v[q] * 3 + a];
-}
-
-template <typename G>
 __global__ void __launch_bounds__(M_THREADS) k_m_tris(const G* __restrict__ verts, const int* __restrict__ tris, unsigned nt,
                                                       const int* __restrict__ parent, const int* __restrict__ rank, EdgeSlot* etab,
                                                       EdgeSlot* vtab, size_t mask, int* __restrict__ label, ctr_mt3d_component* comp) {

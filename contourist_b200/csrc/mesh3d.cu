@@ -220,6 +220,7 @@ int orient_typed(ctr_ctx* ctx, int64_t* n_components, int64_t* n_flipped) {
   return 0;
 }
 
+#include "normals3d.cuh"
 #include "components3d.cuh"
 #include "smooth3d.cuh"
 

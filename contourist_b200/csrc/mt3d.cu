@@ -1668,6 +1668,8 @@ int run_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts* out, int 
 #include "mt3d_select.cuh"
 #include "mt3d_keep.cuh"
 #include "mt3d_clean.cuh"
+#include "normals3d.cuh"
+#include "decimate3d.cuh"
 #include "attr3d.cuh"
 
 }  // namespace
@@ -1812,7 +1814,8 @@ extern "C" int ctr_mt3d_select_seeded(ctr_ctx* ctx, const int32_t* seed_voxels, 
   // the selection compacts the run's mesh in place while the voxel work list keeps its per-voxel triangle offsets: it
   // can be applied once per run
   if (ctx->last3_edited)
-    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has already been selected from, cleaned, filtered or smoothed; run ctr_mt3d_run again");
+    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has already been selected from, cleaned, filtered, smoothed or decimated; "
+                                        "run ctr_mt3d_run again");
   ctx->mesh_gen++;
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
   switch (p->dtype) {
@@ -1830,8 +1833,8 @@ extern "C" int ctr_mt3d_keep_components(ctr_ctx* ctx, const uint8_t* keep, int64
   if (ctx->last_kind != 3 || ctx->comp_count < 0)
     return ctr_fail(ctx, CTR_ERR_STATE, "no ctr_mt3d_components since the last 3D run");
   if (ctx->comp_gen != ctx->mesh_gen)
-    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh was edited after ctr_mt3d_components (selection, clean-up, smoothing or offset_ids): "
-                                        "call ctr_mt3d_components again");
+    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh was edited after ctr_mt3d_components (selection, clean-up, smoothing, decimation "
+                                        "or offset_ids): call ctr_mt3d_components again");
   if (n_keep != ctx->comp_count || (!keep && n_keep > 0))
     return ctr_fail(ctx, CTR_ERR_BAD_ARG, "keep must hold one byte per component of the last ctr_mt3d_components call");
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
@@ -1847,6 +1850,7 @@ extern "C" int ctr_mt3d_clean(ctr_ctx* ctx, const ctr_clean_params* cp, ctr_clea
   if (ctx->last3_edited & 2u) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has already been cleaned");
   // the reference's clean-up (quantize, tiny simplices) is defined on the interpolated positions
   if (ctx->last3_edited & 8u) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has been smoothed: clean it up before smoothing");
+  if (ctx->last3_edited & 16u) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has been decimated: clean it up before decimating");
   const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
   if (p->i_lo != 0 || p->i_hi != p->n0 || p->vert_id_base != 0)
     return ctr_fail(ctx, CTR_ERR_UNSUPPORTED, "mesh clean-up needs a full-volume run (merges cross slab faces)");
@@ -1862,6 +1866,24 @@ extern "C" int ctr_mt3d_clean(ctr_ctx* ctx, const ctr_clean_params* cp, ctr_clea
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
   if (ctx->last_flags & CTR_GEOM_F64) return clean_typed<double>(ctx, cp, out);
   return clean_typed<float>(ctx, cp, out);
+}
+
+extern "C" int ctr_mt3d_decimate(ctr_ctx* ctx, const ctr_decimate_params* dp, ctr_decimate_counts* out) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (!dp || !out) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  memset(out, 0, sizeof *out);
+  for (int a = 0; a < 3; ++a) {
+    if (!(dp->cell[a] > 0.0 && isfinite(dp->cell[a]))) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "cell must be > 0 and finite on every axis");
+    if (!isfinite(dp->origin[a])) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "origin must be finite");
+  }
+  if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
+    return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to decimate");
+  const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
+  if (p->i_lo != 0 || p->i_hi != p->n0 || p->vert_id_base != 0)
+    return ctr_fail(ctx, CTR_ERR_STATE, "decimation needs a full-volume run with vert_id_base 0 (clusters cross slab faces)");
+  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
+  if (ctx->last_flags & CTR_GEOM_F64) return decimate_typed<double>(ctx, dp, out);
+  return decimate_typed<float>(ctx, dp, out);
 }
 
 extern "C" int ctr_mt3d_interpolate(ctr_ctx* ctx, const ctr_attr_params* a, int64_t* n_verts) {

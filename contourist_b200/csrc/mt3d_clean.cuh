@@ -43,9 +43,13 @@ __device__ __forceinline__ unsigned long long quantum_key(const G* __restrict__ 
   return key;
 }
 
-struct Expander {
+struct Expander {                                     // quantize's cell key (also the scale of the tiny-simplex test)
   double ex[3];
   double inv[3];
+  template <typename G>
+  __device__ __forceinline__ unsigned long long operator()(const G* __restrict__ verts, unsigned v) const {
+    return quantum_key(verts, v, ex);
+  }
 };
 
 __global__ void k_c_init(ufh::Slot* tab_v, size_t nslots_v, ufh::Slot* tab_t, size_t nslots_t, int* parent_a, int* parent_b,
@@ -60,18 +64,19 @@ __global__ void k_c_init(ufh::Slot* tab_v, size_t nslots_v, ufh::Slot* tab_t, si
   }
 }
 
-template <typename G>
-__global__ void k_c_qinsert(const G* __restrict__ verts, unsigned nv, Expander e, ufh::Slot* tab, size_t mask) {
+// Key: a functor (verts, v) -> 63-bit cell key of vertex v (Expander here, CellKey in decimate3d.cuh)
+template <typename G, typename Key>
+__global__ void k_c_qinsert(const G* __restrict__ verts, unsigned nv, Key key, ufh::Slot* tab, size_t mask) {
   const unsigned v = blockIdx.x * blockDim.x + threadIdx.x;
   if (v >= nv) return;
-  atomicMin(&ufh::hash_slot(tab, mask, quantum_key(verts, v, e.ex), true)->tri, (int)v);
+  atomicMin(&ufh::hash_slot(tab, mask, key(verts, v), true)->tri, (int)v);
 }
 
-template <typename G>
-__global__ void k_c_qmap(const G* __restrict__ verts, unsigned nv, Expander e, ufh::Slot* tab, size_t mask, int* __restrict__ rep) {
+template <typename G, typename Key>
+__global__ void k_c_qmap(const G* __restrict__ verts, unsigned nv, Key key, ufh::Slot* tab, size_t mask, int* __restrict__ rep) {
   const unsigned v = blockIdx.x * blockDim.x + threadIdx.x;
   if (v >= nv) return;
-  rep[v] = ufh::hash_slot(tab, mask, quantum_key(verts, v, e.ex), false)->tri;
+  rep[v] = ufh::hash_slot(tab, mask, key(verts, v), false)->tri;
 }
 
 __device__ __forceinline__ void sort3(int& a, int& b, int& c) {
@@ -247,13 +252,137 @@ __global__ void k_c_transform(G* __restrict__ verts, G* __restrict__ normals, un
   }
 }
 
+// Scratch of the passes that cluster vertices by cell (clean-up, decimation), carved from aux[28]: the cell and triangle
+// tables, the representative map, union-find parents, flags, mapped triangles, compaction indices and scan words, the
+// selection's counters, a `head` block for the pass's own counters, an `extra` block, and the staging rows of the
+// compaction.
+struct ClusterBufs {
+  ufh::Slot *tab_v, *tab_t;
+  size_t nslots_v, nslots_t;
+  int *rep, *parent_a, *parent_b, *tris2;
+  uint8_t *used_v, *keep_t;
+  uint32_t *idx_t, *idx_v;
+  unsigned long long *st_t, *st_v;
+  int tiles_t, tiles_v;
+  SelCounters* dsel;
+  void *head, *extra, *tmp;
+};
+
+static int cluster_bufs(ctr_ctx* ctx, unsigned nV, unsigned nT, size_t gsz, size_t head_bytes, size_t extra_bytes, ClusterBufs& b) {
+  b.nslots_v = 1024;
+  b.nslots_t = 1024;
+  while (b.nslots_v < (size_t)nV * 2) b.nslots_v <<= 1;
+  while (b.nslots_t < (size_t)nT * 2) b.nslots_t <<= 1;
+  b.tiles_t = (int)(((size_t)nT + SC_TILE - 1) / SC_TILE);
+  b.tiles_v = (int)(((size_t)nV + SC_TILE - 1) / SC_TILE);
+  size_t off = 0;
+  auto carve = [&](size_t bytes) {
+    const size_t o = off;
+    off += (bytes + 255) & ~(size_t)255;
+    return o;
+  };
+  const size_t o_tv = carve(b.nslots_v * sizeof(ufh::Slot)), o_tt = carve(b.nslots_t * sizeof(ufh::Slot)),
+               o_rep = carve((size_t)nV * 4 + 4), o_pa = carve((size_t)nV * 4 + 4), o_pb = carve((size_t)nV * 4 + 4),
+               o_used = carve((size_t)nV + 8), o_keep = carve((size_t)nT + 8), o_t2 = carve((size_t)nT * 12 + 16),
+               o_it = carve((size_t)nT * 4 + 4), o_iv = carve((size_t)nV * 4 + 4), o_st = carve((size_t)b.tiles_t * 8 + 8),
+               o_sv = carve((size_t)b.tiles_v * 8 + 8), o_sel = carve(sizeof(SelCounters) + 64), o_head = carve(head_bytes + 64),
+               o_extra = carve(extra_bytes), o_out = carve(std::max<size_t>((size_t)nV * 3 * gsz, (size_t)nT * 12) + 16);
+  DevBuf& b_s = ctx->aux[28];
+  int rc;
+  if ((rc = ctr_ensure(ctx, b_s, off))) return rc;
+  char* base = (char*)b_s.p;
+  b.tab_v = (ufh::Slot*)(base + o_tv);
+  b.tab_t = (ufh::Slot*)(base + o_tt);
+  b.rep = (int*)(base + o_rep);
+  b.parent_a = (int*)(base + o_pa);
+  b.parent_b = (int*)(base + o_pb);
+  b.used_v = (uint8_t*)(base + o_used);
+  b.keep_t = (uint8_t*)(base + o_keep);
+  b.tris2 = (int*)(base + o_t2);
+  b.idx_t = (uint32_t*)(base + o_it);
+  b.idx_v = (uint32_t*)(base + o_iv);
+  b.st_t = (unsigned long long*)(base + o_st);
+  b.st_v = (unsigned long long*)(base + o_sv);
+  b.dsel = (SelCounters*)(base + o_sel);
+  b.head = base + o_head;
+  b.extra = base + o_extra;
+  b.tmp = base + o_out;
+  return 0;
+}
+
+// k_c_init, every vertex's representative (the smallest vertex id in its cell of `key`), the triangles through that map
+// and their de-duplication; retried with another seed while the triangle table reports a hash collision.  `head` (hbytes)
+// starts with the CleanCounters that k_c_qdedupe counts into: it is zeroed before each attempt and copied to `h` at
+// the sync that checks for collisions.
+template <typename G, typename Key>
+int cluster_tris(ctr_ctx* ctx, const G* verts, unsigned nV, const int* tris, unsigned nT, const Key& key, const ClusterBufs& b,
+                 void* h, size_t hbytes) {
+  cudaStream_t st = ctx->stream;
+  const unsigned vb = (nV + 255) / 256, tb = (nT + 255) / 256;
+  CleanCounters* dcc = (CleanCounters*)b.head;
+  for (int attempt = 0;; ++attempt) {
+    const unsigned long long seed = 0x51ed270b1a2c3d4full * (unsigned long long)(attempt + 1);
+    CTR_CUDA(ctx, cudaMemsetAsync(b.head, 0, hbytes, st));
+    k_c_init<<<ctx->sm_count * 8, 256, 0, st>>>(b.tab_v, b.nslots_v, b.tab_t, b.nslots_t, b.parent_a, b.parent_b, b.used_v, nV);
+    k_c_qinsert<G><<<vb, 256, 0, st>>>(verts, nV, key, b.tab_v, b.nslots_v - 1);
+    k_c_qmap<G><<<vb, 256, 0, st>>>(verts, nV, key, b.tab_v, b.nslots_v - 1, b.rep);
+    ctx->launches += 3;
+    if (nT) {
+      k_c_qtris<<<tb, 256, 0, st>>>(tris, nT, b.rep, b.tris2, b.keep_t, b.tab_t, b.nslots_t - 1, seed);
+      k_c_qdedupe<<<tb, 256, 0, st>>>(b.tris2, nT, b.keep_t, b.tab_t, b.nslots_t - 1, seed, dcc);
+      ctx->launches += 2;
+    }
+    CTR_CUDA(ctx, cudaMemcpyAsync(h, b.head, hbytes, cudaMemcpyDeviceToHost, st));
+    CTR_CUDA(ctx, cudaStreamSynchronize(st));
+    if (!((const CleanCounters*)h)->collision) return 0;
+    if (attempt == 3) return ctr_fail(ctx, CTR_ERR_STATE, "triangle de-duplication: hash collisions under four seeds");
+  }
+}
+
+// Order-preserving compaction in place: the triangles with keep_t (their ids, representatives in tris2, renumbered
+// through idx_v) and the vertices with used_v (positions, normals, keys / lowmin as the run has them).  Synchronous;
+// newV / newT receive the new counts.
+static int compact_mesh(ctr_ctx* ctx, const ClusterBufs& b, unsigned nV, unsigned nT, size_t gsz, size_t& newV, size_t& newT) {
+  cudaStream_t st = ctx->stream;
+  const uint32_t fl = ctx->last_flags;
+  const unsigned vb = (nV + 255) / 256, tb = (nT + 255) / 256;
+  SelCounters hs;
+  CTR_CUDA(ctx, cudaMemsetAsync(b.dsel, 0, sizeof(SelCounters), st));
+  CTR_CUDA(ctx, cudaMemsetAsync(b.st_t, 0, (size_t)b.tiles_t * 8 + 8, st));
+  CTR_CUDA(ctx, cudaMemsetAsync(b.st_v, 0, (size_t)b.tiles_v * 8 + 8, st));
+  k_flag_scan<<<b.tiles_t, SC_THREADS, 0, st>>>(b.keep_t, nT, b.idx_t, b.st_t, &b.dsel->ticket[0], &b.dsel->total[0], b.tiles_t);
+  k_flag_scan<<<b.tiles_v, SC_THREADS, 0, st>>>(b.used_v, nV, b.idx_v, b.st_v, &b.dsel->ticket[1], &b.dsel->total[1], b.tiles_v);
+  ctx->launches += 2;
+  CTR_CUDA(ctx, cudaGetLastError());
+  CTR_CUDA(ctx, cudaMemcpyAsync(&hs, b.dsel, sizeof hs, cudaMemcpyDeviceToHost, st));
+  CTR_CUDA(ctx, cudaStreamSynchronize(st));
+  newT = (size_t)hs.total[0];
+  newV = (size_t)hs.total[1];
+  auto rows = [&](DevBuf& d, int wpr, size_t row_bytes) -> int {
+    if (!d.p) return 0;
+    k_sel_rows<<<vb, 256, 0, st>>>((const uint32_t*)d.p, (uint32_t*)b.tmp, b.used_v, b.idx_v, nV, wpr);
+    ctx->launches++;
+    if (newV) CTR_CUDA(ctx, cudaMemcpyAsync(d.p, b.tmp, newV * row_bytes, cudaMemcpyDeviceToDevice, st));
+    return 0;
+  };
+  int rc;
+  if ((rc = rows(ctx->verts, (int)(3 * gsz / 4), 3 * gsz))) return rc;
+  if ((fl & CTR_WANT_NORMALS) && (rc = rows(ctx->normals, (int)(3 * gsz / 4), 3 * gsz))) return rc;
+  if ((fl & CTR_WANT_KEYS) && (rc = rows(ctx->keys, 2, 8))) return rc;
+  if ((fl & CTR_WANT_KEYS) && (rc = rows(ctx->lowmin, 0, 1))) return rc;
+  k_c_tris_out<<<tb, 256, 0, st>>>(b.tris2, (int*)b.tmp, b.keep_t, b.idx_t, b.idx_v, nT);
+  ctx->launches++;
+  if (newT) CTR_CUDA(ctx, cudaMemcpyAsync(ctx->tris.p, b.tmp, newT * 12, cudaMemcpyDeviceToDevice, st));
+  CTR_CUDA(ctx, cudaGetLastError());
+  CTR_CUDA(ctx, cudaStreamSynchronize(st));
+  return 0;
+}
+
 template <typename G>
 int clean_typed(ctr_ctx* ctx, const ctr_clean_params* cp, ctr_clean_counts* out) {
   cudaStream_t st = ctx->stream;
   const unsigned nV = (unsigned)ctx->last_counts[0], nT = (unsigned)ctx->last_counts[1];
-  const uint32_t fl = ctx->last_flags;
-  const size_t gsz = sizeof(G);
-  const bool want_n = (fl & CTR_WANT_NORMALS) != 0, want_k = (fl & CTR_WANT_KEYS) != 0;
+  const bool want_n = (ctx->last_flags & CTR_WANT_NORMALS) != 0;
   Expander e;
   for (int a = 0; a < 3; ++a) {
     e.ex[a] = (double)(long long)(((double)cp->divisions * 1.0) / (double)cp->corner[a]);   // tetrahedral.py:192
@@ -268,95 +397,24 @@ int clean_typed(ctr_ctx* ctx, const ctr_clean_params* cp, ctr_clean_counts* out)
     identity = identity && cp->origin[a] == 0.0 && cp->delta[a] == 1.0;
   }
   int rc;
-  size_t nslots_v = 1024, nslots_t = 1024;
-  while (nslots_v < (size_t)nV * 2) nslots_v <<= 1;
-  while (nslots_t < (size_t)nT * 2) nslots_t <<= 1;
-  const int tiles_t = (int)(((size_t)nT + SC_TILE - 1) / SC_TILE), tiles_v = (int)(((size_t)nV + SC_TILE - 1) / SC_TILE);
-  size_t off = 0;
-  auto carve = [&](size_t bytes) {
-    const size_t o = off;
-    off += (bytes + 255) & ~(size_t)255;
-    return o;
-  };
-  const size_t o_tv = carve(nslots_v * sizeof(ufh::Slot)), o_tt = carve(nslots_t * sizeof(ufh::Slot)),
-               o_rep = carve((size_t)nV * 4 + 4), o_pa = carve((size_t)nV * 4 + 4), o_pb = carve((size_t)nV * 4 + 4),
-               o_used = carve((size_t)nV + 8), o_keep = carve((size_t)nT + 8), o_t2 = carve((size_t)nT * 12 + 16),
-               o_it = carve((size_t)nT * 4 + 4), o_iv = carve((size_t)nV * 4 + 4), o_st = carve((size_t)tiles_t * 8 + 8),
-               o_sv = carve((size_t)tiles_v * 8 + 8), o_sel = carve(sizeof(SelCounters) + 64), o_cc = carve(sizeof(CleanCounters) + 64),
-               o_out = carve(std::max<size_t>((size_t)nV * 3 * gsz, (size_t)nT * 12) + 16);
-  DevBuf& b_s = ctx->aux[28];
-  if ((rc = ctr_ensure(ctx, b_s, off))) return rc;
-  char* base = (char*)b_s.p;
-  ufh::Slot* tab_v = (ufh::Slot*)(base + o_tv);
-  ufh::Slot* tab_t = (ufh::Slot*)(base + o_tt);
-  int* rep = (int*)(base + o_rep);
-  int* parent_a = (int*)(base + o_pa);
-  int* parent_b = (int*)(base + o_pb);
-  uint8_t* used_v = (uint8_t*)(base + o_used);
-  uint8_t* keep_t = (uint8_t*)(base + o_keep);
-  int* tris2 = (int*)(base + o_t2);
-  uint32_t* idx_t = (uint32_t*)(base + o_it);
-  uint32_t* idx_v = (uint32_t*)(base + o_iv);
-  unsigned long long* st_t = (unsigned long long*)(base + o_st);
-  unsigned long long* st_v = (unsigned long long*)(base + o_sv);
-  SelCounters* dsel = (SelCounters*)(base + o_sel);
-  CleanCounters* dcc = (CleanCounters*)(base + o_cc);
-  void* tmp = base + o_out;
+  ClusterBufs b;
+  if ((rc = cluster_bufs(ctx, nV, nT, sizeof(G), sizeof(CleanCounters), 0, b))) return rc;
+  CleanCounters* dcc = (CleanCounters*)b.head;
   G* verts = (G*)ctx->verts.p;
   const int* tris = (const int*)ctx->tris.p;
   const unsigned vb = (nV + 255) / 256, tb = (nT + 255) / 256;
   CleanCounters hc;
   memset(&hc, 0, sizeof hc);
-  SelCounters hs;
-  memset(&hs, 0, sizeof hs);
+  size_t newV = 0, newT = 0;
   if (nV && nT) {
-    for (int attempt = 0;; ++attempt) {
-      const unsigned long long seed = 0x51ed270b1a2c3d4full * (unsigned long long)(attempt + 1);
-      CTR_CUDA(ctx, cudaMemsetAsync(dcc, 0, sizeof(CleanCounters), st));
-      k_c_init<<<ctx->sm_count * 8, 256, 0, st>>>(tab_v, nslots_v, tab_t, nslots_t, parent_a, parent_b, used_v, nV);
-      k_c_qinsert<G><<<vb, 256, 0, st>>>(verts, nV, e, tab_v, nslots_v - 1);
-      k_c_qmap<G><<<vb, 256, 0, st>>>(verts, nV, e, tab_v, nslots_v - 1, rep);
-      k_c_qtris<<<tb, 256, 0, st>>>(tris, nT, rep, tris2, keep_t, tab_t, nslots_t - 1, seed);
-      k_c_qdedupe<<<tb, 256, 0, st>>>(tris2, nT, keep_t, tab_t, nslots_t - 1, seed, dcc);
-      ctx->launches += 5;
-      CTR_CUDA(ctx, cudaMemcpyAsync(&hc, dcc, sizeof hc, cudaMemcpyDeviceToHost, st));
-      CTR_CUDA(ctx, cudaStreamSynchronize(st));
-      if (!hc.collision) break;
-      if (attempt == 3) return ctr_fail(ctx, CTR_ERR_STATE, "triangle de-duplication: hash collisions under four seeds");
-    }
-    k_c_tiny<G><<<tb, 256, 0, st>>>(verts, tris2, nT, keep_t, e, cp->epsilon, parent_a, dcc);
-    k_c_tinypos<G><<<vb, 256, 0, st>>>(verts, nV, parent_a);
-    if (!(cp->flags & CTR_CLEAN_NO_TRIANGLES)) k_c_flat<G><<<tb, 256, 0, st>>>(verts, tris2, nT, keep_t, parent_b, dcc);
-    k_c_final<<<tb, 256, 0, st>>>(tris2, nT, keep_t, parent_b, used_v, dcc);
-    CTR_CUDA(ctx, cudaMemsetAsync(dsel, 0, sizeof(SelCounters), st));
-    CTR_CUDA(ctx, cudaMemsetAsync(st_t, 0, (size_t)tiles_t * 8 + 8, st));
-    CTR_CUDA(ctx, cudaMemsetAsync(st_v, 0, (size_t)tiles_v * 8 + 8, st));
-    k_flag_scan<<<tiles_t, SC_THREADS, 0, st>>>(keep_t, nT, idx_t, st_t, &dsel->ticket[0], &dsel->total[0], tiles_t);
-    k_flag_scan<<<tiles_v, SC_THREADS, 0, st>>>(used_v, nV, idx_v, st_v, &dsel->ticket[1], &dsel->total[1], tiles_v);
-    ctx->launches += 6;
-    CTR_CUDA(ctx, cudaGetLastError());
-    CTR_CUDA(ctx, cudaMemcpyAsync(&hc, dcc, sizeof hc, cudaMemcpyDeviceToHost, st));
-    CTR_CUDA(ctx, cudaMemcpyAsync(&hs, dsel, sizeof hs, cudaMemcpyDeviceToHost, st));
-    CTR_CUDA(ctx, cudaStreamSynchronize(st));
-  }
-  const size_t newT = (size_t)hs.total[0], newV = (size_t)hs.total[1];
-  auto rows = [&](DevBuf& b, int wpr, size_t row_bytes) -> int {
-    if (!nV || !b.p) return 0;
-    k_sel_rows<<<vb, 256, 0, st>>>((const uint32_t*)b.p, (uint32_t*)tmp, used_v, idx_v, nV, wpr);
-    ctx->launches++;
-    if (newV) CTR_CUDA(ctx, cudaMemcpyAsync(b.p, tmp, newV * row_bytes, cudaMemcpyDeviceToDevice, st));
-    return 0;
-  };
-  if (nV && nT) {
-    if ((rc = rows(ctx->verts, (int)(3 * gsz / 4), 3 * gsz))) return rc;
-    if (want_n && (rc = rows(ctx->normals, (int)(3 * gsz / 4), 3 * gsz))) return rc;
-    if (want_k && (rc = rows(ctx->keys, 2, 8))) return rc;
-    if (want_k && (rc = rows(ctx->lowmin, 0, 1))) return rc;
-    k_c_tris_out<<<tb, 256, 0, st>>>(tris2, (int*)tmp, keep_t, idx_t, idx_v, nT);
-    ctx->launches++;
-    if (newT) CTR_CUDA(ctx, cudaMemcpyAsync(ctx->tris.p, tmp, newT * 12, cudaMemcpyDeviceToDevice, st));
-    CTR_CUDA(ctx, cudaGetLastError());
-    CTR_CUDA(ctx, cudaStreamSynchronize(st));
+    if ((rc = cluster_tris<G>(ctx, verts, nV, tris, nT, e, b, &hc, sizeof hc))) return rc;
+    k_c_tiny<G><<<tb, 256, 0, st>>>(verts, b.tris2, nT, b.keep_t, e, cp->epsilon, b.parent_a, dcc);
+    k_c_tinypos<G><<<vb, 256, 0, st>>>(verts, nV, b.parent_a);
+    if (!(cp->flags & CTR_CLEAN_NO_TRIANGLES)) k_c_flat<G><<<tb, 256, 0, st>>>(verts, b.tris2, nT, b.keep_t, b.parent_b, dcc);
+    k_c_final<<<tb, 256, 0, st>>>(b.tris2, nT, b.keep_t, b.parent_b, b.used_v, dcc);
+    ctx->launches += 4;
+    CTR_CUDA(ctx, cudaMemcpyAsync(&hc, dcc, sizeof hc, cudaMemcpyDeviceToHost, st));   // (synchronised by compact_mesh)
+    if ((rc = compact_mesh(ctx, b, nV, nT, sizeof(G), newV, newT))) return rc;
   }
   ctx->last_counts[0] = (int64_t)newV;
   ctx->last_counts[1] = (int64_t)newT;

@@ -13,8 +13,8 @@
 //   k_s_widen  : geometry type -> both fp64 working copies (fixed vertices are never written again);
 //   k_s_step   : one Jacobi step, one thread per free vertex, reading one copy and writing the other;
 //   k_s_store  : the result rounded into ctx->verts in place;
-//   k_s_nsum / k_s_nfin : (CTR_WANT_NORMALS) per-triangle cross products summed into the corners (fp64 atomicAdd), then
-//                normalised with the sign of the old gradient normal.
+//   k_s_nsum / k_s_nfin (normals3d.cuh): (CTR_WANT_NORMALS) per-triangle cross products summed into the corners (fp64
+//                atomicAdd), then normalised with the sign of the old gradient normal.
 // Scratch: aux[27] edge table, aux[28] per-vertex offsets / cursors / fixed flags, aux[29] neighbour lists, aux[30]
 // counters and look-back words, aux[46] / aux[47] the two fp64 copies.  aux[42..45] (vertex values, component labels
 // and table) are not touched.
@@ -166,48 +166,6 @@ __global__ void k_s_store(const double* __restrict__ x, size_t n, G* __restrict_
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   verts[i] = (G)x[i];
-}
-
-template <typename G>
-__global__ void __launch_bounds__(S_THREADS) k_s_nsum(const G* __restrict__ verts, const int* __restrict__ tris, unsigned nt,
-                                                      double* __restrict__ sum) {
-  const unsigned t = blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= nt) return;
-  const int v[3] = {tris[(size_t)t * 3], tris[(size_t)t * 3 + 1], tris[(size_t)t * 3 + 2]};
-  double p[3][3];
-  tri_corners(verts, v, p);
-  const double ux = __dsub_rn(p[1][0], p[0][0]), uy = __dsub_rn(p[1][1], p[0][1]), uz = __dsub_rn(p[1][2], p[0][2]);
-  const double wx = __dsub_rn(p[2][0], p[0][0]), wy = __dsub_rn(p[2][1], p[0][1]), wz = __dsub_rn(p[2][2], p[0][2]);
-  const double cx = __dsub_rn(__dmul_rn(uy, wz), __dmul_rn(uz, wy));
-  const double cy = __dsub_rn(__dmul_rn(uz, wx), __dmul_rn(ux, wz));
-  const double cz = __dsub_rn(__dmul_rn(ux, wy), __dmul_rn(uy, wx));
-#pragma unroll
-  for (int q = 0; q < 3; ++q) {
-    double* s = sum + (size_t)v[q] * 3;
-    atomicAdd(s, cx);
-    atomicAdd(s + 1, cy);
-    atomicAdd(s + 2, cz);
-  }
-}
-
-template <typename G>
-__global__ void k_s_nfin(const double* __restrict__ sum, unsigned nv, G* __restrict__ normals) {
-  const unsigned v = blockIdx.x * blockDim.x + threadIdx.x;
-  if (v >= nv) return;
-  const double sx = sum[(size_t)v * 3], sy = sum[(size_t)v * 3 + 1], sz = sum[(size_t)v * 3 + 2];
-  if (sx == 0.0 && sy == 0.0 && sz == 0.0) return;    // no face normal here: the old normal stays
-  const double len = sqrt(__dadd_rn(__dadd_rn(__dmul_rn(sx, sx), __dmul_rn(sy, sy)), __dmul_rn(sz, sz)));
-  double nx = __ddiv_rn(sx, len), ny = __ddiv_rn(sy, len), nz = __ddiv_rn(sz, len);
-  G* o = normals + (size_t)v * 3;
-  const double dot = __dadd_rn(__dadd_rn(__dmul_rn(nx, (double)o[0]), __dmul_rn(ny, (double)o[1])), __dmul_rn(nz, (double)o[2]));
-  if (dot < 0.0) {                                    // keep pointing up the field, whatever the winding
-    nx = -nx;
-    ny = -ny;
-    nz = -nz;
-  }
-  o[0] = (G)nx;
-  o[1] = (G)ny;
-  o[2] = (G)nz;
 }
 
 template <typename G>

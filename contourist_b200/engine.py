@@ -95,6 +95,15 @@ class SmoothCounts(ctypes.Structure):
     _fields_ = [("n_edges", ctypes.c_int64), ("n_fixed_verts", ctypes.c_int64)]
 
 
+class DecimateParams(ctypes.Structure):
+    _fields_ = [("cell", ctypes.c_double * 3), ("origin", ctypes.c_double * 3)]
+
+
+class DecimateCounts(ctypes.Structure):
+    _fields_ = [("n_verts", ctypes.c_int64), ("n_tris", ctypes.c_int64), ("n_clusters", ctypes.c_int64),
+                ("n_collapsed", ctypes.c_int64), ("n_duplicate", ctypes.c_int64)]
+
+
 class PolyCounts(ctypes.Structure):
     _fields_ = [("n_polylines", ctypes.c_int64), ("n_points", ctypes.c_int64), ("junction_levels", ctypes.c_uint64)]
 
@@ -161,6 +170,8 @@ def load_library():
     lib.ctr_mt3d_keep_components.restype = i32
     lib.ctr_mt3d_smooth.argtypes = [vp, ctypes.POINTER(SmoothParams), ctypes.POINTER(SmoothCounts)]
     lib.ctr_mt3d_smooth.restype = i32
+    lib.ctr_mt3d_decimate.argtypes = [vp, ctypes.POINTER(DecimateParams), ctypes.POINTER(DecimateCounts)]
+    lib.ctr_mt3d_decimate.restype = i32
     lib.ctr_mt3d_interpolate.argtypes = [vp, ctypes.POINTER(AttrParams), ctypes.POINTER(i64)]
     lib.ctr_mt3d_interpolate.restype = i32
     lib.ctr_mt3d_interpolate_fetch.argtypes = [vp, vp]
@@ -513,6 +524,32 @@ class Engine(object):
         c = SmoothCounts()
         self.run_serial += 1
         self._check(self.lib.ctr_mt3d_smooth(self.h, ctypes.byref(p), ctypes.byref(c)), "ctr_mt3d_smooth")
+        return c
+
+    def mt3d_decimate(self, cell, origin=(0.0, 0.0, 0.0)):
+        """Quadric vertex-clustering decimation of the last 3D run's device mesh as it stands now, in place
+        (ctr_mt3d_decimate; oracle/mt3d_decimate.py is the definition): the vertices in one cell of the grid of edge
+        lengths `cell` (a number or 3 numbers, in the units of the current positions) with its corner at `origin`
+        become one vertex, placed where the planes of the triangles around it meet best (a corner or ridge inside a
+        cell survives) and clamped to the cell.  Triangles left with fewer than three cells, and repeats of an earlier
+        triangle's three cells, are dropped; the rest keep their order.  Each output vertex carries the keys of its
+        cell's smallest vertex id (mt3d_interpolate() then samples the field there); normals (WANT_NORMALS) are
+        recomputed.  Afterwards mt3d_components() must measure again before mt3d_keep_components(), and
+        mt3d_select_seeded() / mt3d_clean() are refused.  Returns DecimateCounts (n_verts, n_tris, n_clusters,
+        n_collapsed, n_duplicate); fetch afterwards."""
+        p = DecimateParams()
+        cell = np.broadcast_to(np.asarray(cell, np.float64), (3,))
+        origin = np.broadcast_to(np.asarray(origin, np.float64), (3,))
+        for a in range(3):
+            p.cell[a] = float(cell[a])
+            p.origin[a] = float(origin[a])
+        c = DecimateCounts()
+        self.run_serial += 1
+        self._check(self.lib.ctr_mt3d_decimate(self.h, ctypes.byref(p), ctypes.byref(c)), "ctr_mt3d_decimate")
+        flags, c3 = self._last3
+        c3 = type(c3).from_buffer_copy(c3)                             # the caller keeps the full scan's counts
+        c3.n_verts, c3.n_tris = int(c.n_verts), int(c.n_tris)          # what mt3d_fetch sizes its arrays from
+        self._last3 = (flags, c3)
         return c
 
     def mt3d_interpolate(self, field, shape=None, dtype=None):

@@ -152,6 +152,12 @@ class GridContour3d(object):
     smooth_iterations = 0
     smooth_lambda = 0.5
     smooth_mu = -0.53
+    # decimate_cell (a number or 3 numbers, in voxels): get_points_and_triangles() reduces the mesh on the device by
+    # quadric vertex clustering (ctr_mt3d_decimate) on cells of decimate_cell * |delta| aligned with the voxel grid,
+    # after the component filter and smoothing and before vertex_fields / measure_components, which then describe the
+    # decimated mesh.  `flatten` (the reference's LP-based collapse_flat_segments) is a different algorithm and still
+    # raises.
+    decimate_cell = None
 
     def __init__(self, corner, function, value, segment_endpoints, linear_interpolate=True, callback=None,
                  origin=(0.0, 0.0, 0.0), delta=(1.0, 1.0, 1.0)):
@@ -194,6 +200,9 @@ class GridContour3d(object):
 
     def get_points_and_triangles(self, clean=True):
         if self.flatten or self.smooth:
+            # the reference's flatten solves an LP per edge, serially, and smooth is its own smoothing: the engine's
+            # smoothing and decimation are other algorithms behind their own options (smooth_iterations,
+            # decimate_cell), so these keep raising rather than silently giving a different mesh
             raise NotImplementedError("flatten / smooth (LP-based decimation, tetrahedral.py:217-351) are out of scope")
         eng = E.default_engine()
         flags = (E.GEOM_F64 if np.dtype(self.geometry_dtype) == np.float64 else 0) | (E.WANT_NORMALS if self.want_normals else 0)
@@ -233,6 +242,12 @@ class GridContour3d(object):
             # after the filter (its components are measured on the unsmoothed mesh), before the values and the
             # measurement below
             eng.mt3d_smooth(self.smooth_iterations, self.smooth_lambda, self.smooth_mu)
+        decimated = self.decimate_cell is not None
+        if decimated:
+            # after the filter and smoothing, before the values and the measurement below; cells of decimate_cell
+            # voxels in the world coordinates the mesh has by now, aligned with the voxel grid
+            cell = np.asarray(self.decimate_cell, np.float64) * np.abs(np.asarray(self.delta, np.float64))
+            eng.mt3d_decimate(cell, origin=tuple(float(x) for x in self.origin))
         if self.vertex_fields is not None:
             # after every pass that edits the mesh: the values line up with the points fetched below
             many = isinstance(self.vertex_fields, (list, tuple))
@@ -241,9 +256,10 @@ class GridContour3d(object):
             self.vertex_values = vals if many else vals[0]
         if self.measure_components:
             # after every pass that edits the mesh, like the values above; the filter has already measured this mesh,
-            # unless smoothing has moved it since
+            # unless smoothing or decimation has changed it since
             self.triangle_components, self.component_table = \
-                eng.mt3d_components_fetch() if self.keep_components is not None and not smoothed else eng.mt3d_components()
+                eng.mt3d_components_fetch() if self.keep_components is not None and not (smoothed or decimated) \
+                else eng.mt3d_components()
         out = eng.mt3d_fetch()
         self.normals = out["normals"]
         points, triangles = out["verts"], out["tris"]
@@ -299,7 +315,7 @@ class Delta3DContour(object):
         "options set on this driver (before or after the maker was built) reach the maker"
         for name in ("post_process", "geometry_dtype", "want_normals", "reference_orientation", "quantize_divisions",
                      "tiny_epsilon", "vertex_fields", "measure_components", "keep_components", "smooth_iterations",
-                     "smooth_lambda", "smooth_mu"):
+                     "smooth_lambda", "smooth_mu", "decimate_cell"):
             if hasattr(self, name):
                 setattr(maker, name, getattr(self, name))
         maker.field_grid = self.grid

@@ -270,6 +270,54 @@ typedef struct {
 typedef struct { int64_t n_edges, n_fixed_verts; } ctr_smooth_counts;
 CTR_API int ctr_mt3d_smooth(ctr_ctx* ctx, const ctr_smooth_params* p, ctr_smooth_counts* out);
 
+/* Quadric vertex-clustering decimation of the LAST 3D run's device mesh as it stands now (after a selection, clean-up,
+ * orientation, component filter or smoothing too), in place (engine extension: Lindstrom's quadric clustering, as in
+ * VTK's vtkQuadricClustering; the reference's flatten is not reproduced -- oracle/mt3d_decimate.py:decimate is the
+ * definition).  Synchronous on return.  All arithmetic is fp64 on positions widened from the geometry type, each
+ * operation rounded on its own (no fused multiply-add).
+ *   - Cluster of a vertex: q[a] = floor((p[a] - origin[a]) / cell[a]) (subtract, then divide), which must lie in
+ *     [-2^20, 2^20) on every axis; the cell corner is lo[a] = origin[a] + q[a] * cell[a] (multiply, then add).
+ *   - Quadrics: every triangle (a, b, c) of the input, also one that collapses below, has n = cross(P_b - P_a, P_c - P_a)
+ *     (unnormalised: the quadric is weighted by area squared).  For each corner, with k its cluster and
+ *     d = -(n . (P_a - lo_k)), cluster k gets A_k += n n^T and g_k += d n (a triangle with two corners in k adds twice).
+ *   - Position: m_k = mean of (P - lo_k) over the cluster's vertices, lambda_k = 1e-3 * trace(A_k); x = m_k when
+ *     lambda_k == 0, else the solution of (A_k + lambda_k I) x = lambda_k m_k - g_k (the minimiser of
+ *     sum (n . x + d)^2 + lambda |x - m|^2: exact on flat clusters, keeps a corner or ridge inside a cell, and pulled to
+ *     the mean only along directions no plane constrains).  Each axis of x is clamped to [0, cell[a]]; the position is
+ *     lo_k + x, rounded to the geometry type once.
+ *   - Triangles map to the clusters of their corners.  One with fewer than three distinct clusters is dropped
+ *     (n_collapsed); of triangles with the same set of three clusters (either winding) the first in triangle order stays
+ *     (n_duplicate: the rules of the clean-up's quantize step).  Kept triangles keep their order and corner order.
+ *   - Each cluster a kept triangle uses becomes one vertex.  Clusters are ordered by their smallest member vertex id,
+ *     and that member is the cluster's representative: keys / lowmin (CTR_WANT_KEYS) are its rows, so a later
+ *     ctr_mt3d_interpolate gives the value at the representative's edge crossing -- a sample of the cluster, not its
+ *     average.  Normals (CTR_WANT_NORMALS) are recomputed as ctr_mt3d_smooth does, signed by the representative's old
+ *     normal.
+ *   - Counts, triangles, vertex order, keys and lowmin are exact; positions and normals equal the definition within
+ *     rounding (the sums run in an unspecified order).  Cells and codes stay those of the full scan.
+ *   - The device buffers are compacted in place: pointers from ctr_mt3d_device_ptrs stay valid.  The counts published
+ *     by ctr_mt3d_publish_counts stay those of the run.
+ *   - After a call on a non-empty mesh: component results of an earlier ctr_mt3d_components are stale
+ *     (ctr_mt3d_keep_components returns CTR_ERR_STATE until ctr_mt3d_components measures again) and so are vertex values
+ *     of an earlier ctr_mt3d_interpolate; ctr_mt3d_select_seeded and ctr_mt3d_clean return CTR_ERR_STATE (the clean-up
+ *     is defined on the interpolated positions: clean up first).  ctr_mt3d_orient_reference, ctr_mt3d_components,
+ *     ctr_mt3d_interpolate, ctr_mt3d_smooth and further decimation are accepted.
+ *   - CTR_ERR_BAD_ARG: a NULL argument; a cell <= 0, NaN or infinite; an origin that is not finite; a cell index out of
+ *     range.  CTR_ERR_STATE: no 3D run or a CTR_NO_GEOMETRY run; a slab run (i_lo != 0 or i_hi != n0) or
+ *     vert_id_base != 0; a triangle id outside [0, n_verts) (e.g. after ctr_mt3d_offset_ids).  All are detected before
+ *     anything is written.  An empty mesh is a valid no-op.                                                             */
+typedef struct {
+  double cell[3];     /* > 0 and finite: edge lengths of the clustering cells, in the units of the current positions */
+  double origin[3];   /* finite: the corner of cell (0, 0, 0)                                                         */
+} ctr_decimate_params;                       /* 48 bytes */
+typedef struct {
+  int64_t n_verts, n_tris;                   /* the decimated mesh                                                    */
+  int64_t n_clusters;                        /* occupied cells: cells holding at least one vertex of the input        */
+  int64_t n_collapsed;                       /* triangles dropped because two or three corners share a cluster        */
+  int64_t n_duplicate;                       /* triangles dropped because an earlier kept triangle has the same three clusters */
+} ctr_decimate_counts;                       /* 40 bytes */
+CTR_API int ctr_mt3d_decimate(ctr_ctx* ctx, const ctr_decimate_params* p, ctr_decimate_counts* out);
+
 /* Seeded extraction (SURVEY.md 8(f3)): restricts the LAST full-volume run's mesh to what the reference's tracker
  *   tetrahedral.py:443-469  expand_voxels / in_range  (flood fill over the 26-neighbourhood of border voxels)
  * reaches from the given start voxels (the output of find_initial_voxels, tetrahedral.py:396-441, which the binding
