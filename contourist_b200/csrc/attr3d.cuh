@@ -116,11 +116,11 @@ int interp_typed(ctr_ctx* ctx, const ctr_attr_params* ap, int64_t* n_verts) {
     src = (const char*)ap->field;
   } else {
     // a buffer of its own: ctx->field still holds the run's staged samples, which the ratio needs
-    if ((rc = ctr_ensure(ctx, ctx->aux[42], npts * rb))) return rc;
-    CTR_CUDA(ctx, cudaMemcpyAsync(ctx->aux[42].p, ap->field, npts * rb, cudaMemcpyHostToDevice, st));
-    src = (const char*)ctx->aux[42].p;
+    if ((rc = ctr_ensure(ctx, ctx->aux[AUX_ATTR_FIELD], npts * rb))) return rc;
+    CTR_CUDA(ctx, cudaMemcpyAsync(ctx->aux[AUX_ATTR_FIELD].p, ap->field, npts * rb, cudaMemcpyHostToDevice, st));
+    src = (const char*)ctx->aux[AUX_ATTR_FIELD].p;
   }
-  if ((rc = ctr_ensure(ctx, ctx->aux[43], nV * (size_t)ap->ncomp * gsz))) return rc;
+  if ((rc = ctr_ensure(ctx, ctx->aux[AUX_VALUES], nV * (size_t)ap->ncomp * gsz))) return rc;
   AttrSrc a;
   a.p = src;
   a.dtype = ap->dtype;
@@ -135,11 +135,11 @@ int interp_typed(ctr_ctx* ctx, const ctr_attr_params* ap, int64_t* n_verts) {
     if (f64)
       k_interp_attr<T, double><<<nb, 256, 0, st>>>(f, (int)p->n1, (int)p->n2, off, p->isovalue,
                                                     (const unsigned long long*)ctx->keys.p, (const uint8_t*)ctx->lowmin.p,
-                                                    (unsigned)nV, a, (double*)ctx->aux[43].p);
+                                                    (unsigned)nV, a, (double*)ctx->aux[AUX_VALUES].p);
     else
       k_interp_attr<T, float><<<nb, 256, 0, st>>>(f, (int)p->n1, (int)p->n2, off, p->isovalue,
                                                    (const unsigned long long*)ctx->keys.p, (const uint8_t*)ctx->lowmin.p,
-                                                   (unsigned)nV, a, (float*)ctx->aux[43].p);
+                                                   (unsigned)nV, a, (float*)ctx->aux[AUX_VALUES].p);
     ctx->launches++;
   }
   CTR_CUDA(ctx, cudaGetLastError());

@@ -19,6 +19,41 @@ struct DevBuf {
 
 struct ctr_comm_state;                    // comm.cu: NCCL communicator + gathered mesh of a context
 
+// The 3D slots of ctr_ctx::aux (the 2D and 4D paths number theirs in their own translation units).
+enum Aux3 : int {
+  // the extraction's work lists and flags, rewritten by every ctr_mt3d_run; the seeded selection reads them
+  AUX_OWN_LIST = 0,          // (owner id, vertex offset) per active owner
+  AUX_CELL_LIST = 2,         // id of every emitting voxel
+  AUX_ROW_FLAGS = 4,         // per voxel row: some sample near the isovalue
+  AUX_WORD_FLAGS = 32,       // per word: near flags
+  AUX_WORD_RECS = 33,        // records of the listed interesting words
+  AUX_TILE_WORDS = 34,       // (first entry, entries) of the word list per tile
+  AUX_EXACT_FLAGS = 35,      // per word: "exact test differs" flags
+  AUX_WORD_SLOTS = 41,       // first work-list slots of the listed words
+  // scratch of the mesh passes: any pass may overwrite them
+  AUX_SCRATCH0 = 27,
+  AUX_SCRATCH1 = 28,
+  AUX_SCRATCH2 = 29,
+  AUX_SCRATCH3 = 30,
+  AUX_SCRATCH4 = 31,
+  AUX_ATTR_FIELD = 42,       // ctr_mt3d_interpolate's staged host field
+  AUX_SMOOTH_X0 = 46,        // smoothing's two fp64 working copies
+  AUX_SMOOTH_X1 = 47,
+  // results that outlive the pass that made them: no pass uses them as scratch
+  AUX_VALUES = 43,           // vertex values (ctr_mt3d_interpolate)
+  AUX_LABELS = 44,           // component of every triangle (ctr_mt3d_components)
+  AUX_COMPONENTS = 45,       // component table
+};
+
+// ctr_ctx::last3_edited: the passes that have rewritten the device mesh of the last 3D run
+enum Edit3 : unsigned {
+  EDIT_SELECT = 1u,          // seeded selection
+  EDIT_CLEAN = 2u,           // clean-up
+  EDIT_KEEP = 4u,            // component filter
+  EDIT_SMOOTH = 8u,          // smoothing
+  EDIT_DECIMATE = 16u,       // decimation
+};
+
 struct ctr_ctx {
   int device = 0;
   ctr_comm_state* comm = nullptr;
@@ -57,8 +92,7 @@ struct ctr_ctx {
   int64_t poly_counts[2] = {};            // 2D: polylines / points of the last ctr_mt2d_polylines
   unsigned char last3_params[160] = {};   // parameters of the last completed ctr_mt3d_run
   long long* publish3 = nullptr;          // ctr_mt3d_publish_counts: device {n_verts, n_tris} behind every 3D run
-  unsigned last3_edited = 0;              // passes that have rewritten the device mesh of that run: 1 seeded selection, 2 clean-up,
-                                          // 4 component filter, 8 smoothing, 16 decimation
+  unsigned last3_edited = 0;              // Edit3 bits of the passes that have rewritten the device mesh of that run
   // bumped by every 3D run and every pass that removes or renumbers mesh rows (selection, clean-up, offset_ids,
   // component filter, decimation) or moves vertices (smoothing); the vertex values and the components below record the
   // generation they were computed on
@@ -70,20 +104,17 @@ struct ctr_ctx {
   size_t spec_v = 0, spec_t = 0, spec_own = 0, spec_cell = 0, last_own = 0, last_cell = 0, cover_own = 0, cover_cell = 0;
   size_t spec_w = 0, last_w = 0, cover_w = 0;   // interesting-word list of the split stage 2
   DevBuf wlist;
-  // 3D vertex values (ctr_mt3d_interpolate): rows and components of aux[43]; 0 = none since the last 3D run
+  // 3D vertex values (ctr_mt3d_interpolate): rows and components of AUX_VALUES; 0 = none since the last 3D run
   size_t attr_rows = 0;
   int attr_ncomp = 0;
   uint64_t attr_gen = 0;
-  // 3D connected components (ctr_mt3d_components): triangles and components of aux[44] / aux[45]; -1 = none since the
-  // last 3D run
+  // 3D connected components (ctr_mt3d_components): triangles and components of AUX_LABELS / AUX_COMPONENTS; -1 = none
+  // since the last 3D run
   int64_t comp_tris = 0, comp_count = -1;
   uint64_t comp_gen = 0;
 
-  // 2D / 4D extra outputs are declared in their own translation units via these generic slots
-  DevBuf aux[48];            // 0-4, 32-35, 41: 3D; 5-10: 2D; 12-26: 4D; 27-31: mesh passes; 36-40: 2D polylines;
-                             // 42-43: 3D vertex values (staged attribute field, values);
-                             // 44-45: 3D connected components (triangle labels, component table);
-                             // 46-47: smoothing's fp64 working copies
+  // extra outputs and scratch in generic slots: 3D (Aux3 above, 1 and 3 unused); 5-10: 2D; 12-26: 4D; 36-40: 2D polylines
+  DevBuf aux[48];
 };
 
 static inline int ctr_fail(ctr_ctx* ctx, int code, const char* what, const char* detail = "") {
@@ -128,6 +159,28 @@ static inline int ctr_ensure(ctr_ctx* ctx, DevBuf& b, size_t bytes, bool exact =
     return ctr_fail(ctx, CTR_ERR_OOM, m);
   }
   b.cap = want;
+  return 0;
+}
+
+// 256-byte-aligned pieces of one DevBuf.  `pieces` names each piece once, as carve(pointer, bytes); ctr_carve_buf calls
+// it twice: to add up the size (the pointers stay null), then, after ctr_ensure, to point every piece into the buffer.
+struct ctr_carve {
+  char* base = nullptr;
+  size_t off = 0;
+  template <typename P>
+  void operator()(P*& p, size_t bytes) {
+    p = base ? reinterpret_cast<P*>(base + off) : nullptr;
+    off += (bytes + 255) & ~(size_t)255;
+  }
+};
+
+template <typename F>
+static inline int ctr_carve_buf(ctr_ctx* ctx, DevBuf& b, F&& pieces) {
+  ctr_carve c;
+  pieces(c);
+  if (int rc = ctr_ensure(ctx, b, c.off)) return rc;
+  c = ctr_carve{(char*)b.p, 0};
+  pieces(c);
   return 0;
 }
 

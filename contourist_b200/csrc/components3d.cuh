@@ -247,12 +247,12 @@ int components_typed(ctr_ctx* ctx, int64_t* n_components) {
                                                       // vertex) pairs: about nt / 2 (3 nt at worst): load <= 3/4
   const unsigned blocks = (nt + M_THREADS - 1) / M_THREADS;   // also the look-back tiles of k_m_roots
   int rc;
-  DevBuf& b_etab = ctx->aux[27];
-  DevBuf& b_vtab = ctx->aux[28];
-  DevBuf& b_par = ctx->aux[29];
-  DevBuf& b_scan = ctx->aux[30];
-  DevBuf& b_label = ctx->aux[44];
-  DevBuf& b_comp = ctx->aux[45];
+  DevBuf& b_etab = ctx->aux[AUX_SCRATCH0];
+  DevBuf& b_vtab = ctx->aux[AUX_SCRATCH1];
+  DevBuf& b_par = ctx->aux[AUX_SCRATCH2];
+  DevBuf& b_scan = ctx->aux[AUX_SCRATCH3];
+  DevBuf& b_label = ctx->aux[AUX_LABELS];
+  DevBuf& b_comp = ctx->aux[AUX_COMPONENTS];
   if ((rc = ctr_ensure(ctx, b_etab, nslots * sizeof(EdgeSlot)))) return rc;
   if ((rc = ctr_ensure(ctx, b_vtab, nslots * sizeof(EdgeSlot)))) return rc;
   if ((rc = ctr_ensure(ctx, b_par, (size_t)nt * 8))) return rc;

@@ -2,9 +2,10 @@
 // DeCoro & Tatarchuk 2007, VTK's vtkQuadricClustering).
 //
 // Included into mt3d.cu after mt3d_clean.cuh, inside its anonymous namespace: clustering is the clean-up's quantize
-// step with another cell key, so the pass runs that step's kernels through its helpers (cluster_bufs, cluster_tris,
-// compact_mesh) and the normals of normals3d.cuh.  The definition is oracle/mt3d_decimate.py:decimate (positions within
-// rounding: the sums below are fp64 atomics in an unspecified order; everything else exactly).
+// step with another cell key, so the pass runs that step's kernels through its helpers (cluster_bufs, cluster_tris),
+// compacts with compact_mesh (compact3d.cuh) and takes the normals of normals3d.cuh.  The definition is
+// oracle/mt3d_decimate.py:decimate (positions within rounding: the sums below are fp64 atomics in an unspecified order;
+// everything else exactly).
 //   k_d_ids               : every triangle id in [0, n_verts), checked (and synchronised) before anything else runs;
 //   k_c_qinsert / k_c_qmap: with CellKey, every vertex's cluster = the smallest vertex id in its cell (out-of-range cell
 //                           indices flagged there); k_c_qtris / k_c_qdedupe: triangles through that map, those with
@@ -15,11 +16,11 @@
 //   k_c_final             : (identity parents) flags the clusters the kept triangles use;
 //   k_d_place             : per used cluster, the regularised 3 x 3 solve by the adjugate and the clamp to the cell,
 //                           written into the representative's row of ctx->verts (every read of old positions is done);
-//   compact_mesh          : k_flag_scan x 2, k_sel_rows, k_c_tris_out: vertices in the order of their representative;
+//   compact_mesh          : vertices in the order of their representative, triangles through the cluster map;
 //   k_s_nsum / k_s_nfin   : (CTR_WANT_NORMALS) normals of the decimated mesh, signed by the representative's old normal.
 // The warp's lanes combine the rows they add to one cluster before the fp64 atomics (warp_add_row): triangles come out of
 // the engine by owner word, so the lanes of a warp mostly hit the same few clusters.
-// Scratch: aux[28] only (cluster_bufs; its extra block holds the 13 fp64 sums per vertex row, reused for the normal
+// Scratch: AUX_SCRATCH1 only (cluster_bufs; its extra block holds the 13 fp64 sums per vertex row, reused for the normal
 // sums after compaction).  No other aux slot is touched: vertex values and component results stay (stale).
 
 constexpr int D_ROW = 13;                              // A: xx xy xz yy yz zz, g: x y z, position sums: x y z, count
@@ -219,31 +220,27 @@ int decimate_typed(ctr_ctx* ctx, const ctr_decimate_params* dp, ctr_decimate_cou
   if ((rc = cluster_tris<G>(ctx, verts, nV, tris, nT, key, b, &h, sizeof h))) return rc;
   if (h.out_of_range) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "a cell index (p - origin) / cell lies outside [-2^20, 2^20)");
   ctx->mesh_gen++;                                    // from here on the mesh is edited
-  ctx->last3_edited |= 16u;
+  ctx->last3_edited |= EDIT_DECIMATE;
   CTR_CUDA(ctx, cudaMemsetAsync(acc, 0, (size_t)nV * D_ROW * 8, st));
   k_d_vsum<G><<<vb, 256, 0, st>>>(verts, nV, b.rep, d, acc, dc);
   ctx->launches++;
   if (nT) {
     k_d_quadric<G><<<tb, 256, 0, st>>>(verts, tris, nT, b.rep, d, acc, dc);
-    k_c_final<<<tb, 256, 0, st>>>(b.tris2, nT, b.keep_t, b.parent_b, b.used_v, &dc->c);   // parent_b: identity (k_c_init)
-    k_d_place<G><<<vb, 256, 0, st>>>(verts, nV, b.used_v, d, acc);
+    k_c_final<<<tb, 256, 0, st>>>(b.tris2, nT, b.cb.keep_t, b.parent_b, b.cb.used_v, &dc->c);   // parent_b: identity (k_c_init)
+    k_d_place<G><<<vb, 256, 0, st>>>(verts, nV, b.cb.used_v, d, acc);
     ctx->launches += 3;
   }
   CTR_CUDA(ctx, cudaMemcpyAsync(&h, dc, sizeof h, cudaMemcpyDeviceToHost, st));   // (synchronised by compact_mesh)
   size_t newV = 0, newT = 0;
-  if (nT) {
-    if ((rc = compact_mesh(ctx, b, nV, nT, sizeof(G), newV, newT))) return rc;
-  } else {
-    CTR_CUDA(ctx, cudaStreamSynchronize(st));
-  }
+  if (nT && (rc = compact_mesh(ctx, b.cb, nV, nT, b.tris2, 0u, false, nullptr, newV, newT))) return rc;
   if ((ctx->last_flags & CTR_WANT_NORMALS) && newT) {
     CTR_CUDA(ctx, cudaMemsetAsync(acc, 0, newV * 3 * 8, st));
     k_s_nsum<G><<<(unsigned)((newT + N_THREADS - 1) / N_THREADS), N_THREADS, 0, st>>>(verts, tris, (unsigned)newT, acc);
     k_s_nfin<G><<<(unsigned)((newV + N_THREADS - 1) / N_THREADS), N_THREADS, 0, st>>>(acc, (unsigned)newV, (G*)ctx->normals.p);
     ctx->launches += 2;
-    CTR_CUDA(ctx, cudaGetLastError());
-    CTR_CUDA(ctx, cudaStreamSynchronize(st));
   }
+  CTR_CUDA(ctx, cudaGetLastError());
+  CTR_CUDA(ctx, cudaStreamSynchronize(st));
   ctx->last_counts[0] = (int64_t)newV;
   ctx->last_counts[1] = (int64_t)newT;
   out->n_verts = (int64_t)newV;

@@ -184,9 +184,9 @@ int orient_typed(ctr_ctx* ctx, int64_t* n_components, int64_t* n_flipped) {
   size_t nslots = 1;
   while (nslots < (size_t)nt * 4) nslots <<= 1;       // 1.5 nt distinct edges on closed sheets (3 nt at worst): load <= 3/8 (3/4)
   int rc;
-  DevBuf& b_tab = ctx->aux[27];
-  DevBuf& b_par = ctx->aux[29];
-  DevBuf& b_comp = ctx->aux[30];
+  DevBuf& b_tab = ctx->aux[AUX_SCRATCH0];
+  DevBuf& b_par = ctx->aux[AUX_SCRATCH2];
+  DevBuf& b_comp = ctx->aux[AUX_SCRATCH3];
   if ((rc = ctr_ensure(ctx, b_tab, nslots * sizeof(EdgeSlot)))) return rc;
   if ((rc = ctr_ensure(ctx, b_par, (size_t)nt * 8))) return rc;
   if ((rc = ctr_ensure(ctx, b_comp, (size_t)nt * (8 + 8 + 4) + 64))) return rc;
@@ -273,9 +273,9 @@ extern "C" int ctr_mt3d_components_fetch(ctr_ctx* ctx, int32_t* tri_component, c
     return ctr_fail(ctx, CTR_ERR_STATE, "no ctr_mt3d_components since the last 3D run");
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
   if (tri_component && ctx->comp_tris)
-    CTR_CUDA(ctx, cudaMemcpyAsync(tri_component, ctx->aux[44].p, (size_t)ctx->comp_tris * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CTR_CUDA(ctx, cudaMemcpyAsync(tri_component, ctx->aux[AUX_LABELS].p, (size_t)ctx->comp_tris * 4, cudaMemcpyDeviceToHost, ctx->stream));
   if (components && ctx->comp_count)
-    CTR_CUDA(ctx, cudaMemcpyAsync(components, ctx->aux[45].p, (size_t)ctx->comp_count * sizeof(ctr_mt3d_component),
+    CTR_CUDA(ctx, cudaMemcpyAsync(components, ctx->aux[AUX_COMPONENTS].p, (size_t)ctx->comp_count * sizeof(ctr_mt3d_component),
                                   cudaMemcpyDeviceToHost, ctx->stream));
   CTR_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return 0;

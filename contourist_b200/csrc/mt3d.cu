@@ -1461,16 +1461,16 @@ int run_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts* out, int 
     CTR_CUDA(ctx, cudaStreamSynchronize(st));
   }
   if ((rc = ctr_ensure(ctx, ctx->counters, sizeof(Counters)))) return rc;
-  if ((rc = ctr_ensure(ctx, ctx->aux[4], (size_t)nrows + 32))) return rc;
-  if ((rc = ctr_ensure(ctx, ctx->aux[32], (size_t)nrows * 4 + 64))) return rc;      // word-level near flags
-  if ((rc = ctr_ensure(ctx, ctx->aux[35], (size_t)nrows * 4 + 64))) return rc;      // word-level "exact differs" flags
+  if ((rc = ctr_ensure(ctx, ctx->aux[AUX_ROW_FLAGS], (size_t)nrows + 32))) return rc;
+  if ((rc = ctr_ensure(ctx, ctx->aux[AUX_WORD_FLAGS], (size_t)nrows * 4 + 64))) return rc;
+  if ((rc = ctr_ensure(ctx, ctx->aux[AUX_EXACT_FLAGS], (size_t)nrows * 4 + 64))) return rc;
   if ((rc = ctr_ensure(ctx, ctx->tile_state, (size_t)ntiles * 16 + 16))) return rc;
   if (!ctx->counters_host) CTR_CUDA(ctx, cudaMallocHost(&ctx->counters_host, 1024));
   g.bits = (const uint32_t*)ctx->bits.p;
   g.nbits = (const uint32_t*)ctx->nbits.p;
-  g.rowflag = (const uint8_t*)ctx->aux[4].p;
-  g.wordflag = (const uint32_t*)ctx->aux[32].p;
-  g.exactflag = (uint32_t*)ctx->aux[35].p;
+  g.rowflag = (const uint8_t*)ctx->aux[AUX_ROW_FLAGS].p;
+  g.wordflag = (const uint32_t*)ctx->aux[AUX_WORD_FLAGS].p;
+  g.exactflag = (uint32_t*)ctx->aux[AUX_EXACT_FLAGS].p;
   g.wshift = 0;
   while ((W >> g.wshift) > 32) ++g.wshift;
   Counters* dctr = (Counters*)ctx->counters.p;
@@ -1490,8 +1490,8 @@ int run_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts* out, int 
   // every stage is enqueued against them without waiting for the counts -- kernels read the list lengths from the
   // device counters and never write past a capacity -- and the counts are checked after the single synchronisation
   // at the end.  Only when a capacity turns out too small are the buffers grown and the affected stages redone.
-  DevBuf& b_own = ctx->aux[0];
-  DevBuf& b_cell_id = ctx->aux[2];
+  DevBuf& b_own = ctx->aux[AUX_OWN_LIST];
+  DevBuf& b_cell_id = ctx->aux[AUX_CELL_LIST];
   if (!ctx->spec_w) ctx->spec_w = std::max<size_t>((size_t)nwords / 4, 1 << 14);
   if (!ctx->spec_own) ctx->spec_own = std::max<size_t>((size_t)nwords / 2, 1 << 14);
   if (!ctx->spec_cell) ctx->spec_cell = ctx->spec_own;
@@ -1503,9 +1503,9 @@ int run_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts* out, int 
     if ((rc = ctr_ensure(ctx, b_own, ctx->spec_own * 16, true))) return rc;
     if ((rc = ctr_ensure(ctx, b_cell_id, ctx->spec_cell * 8, true))) return rc;
     if ((rc = ctr_ensure(ctx, ctx->wlist, ctx->spec_w * 4, true))) return rc;
-    if ((rc = ctr_ensure(ctx, ctx->aux[33], ctx->spec_w * 4, true))) return rc;                 // records of the listed words
-    if ((rc = ctr_ensure(ctx, ctx->aux[41], ctx->spec_w * 8, true))) return rc;                 // their first slots in the work lists
-    if ((rc = ctr_ensure(ctx, ctx->aux[34], (size_t)ntiles * 8 + 16))) return rc;               // (first entry, entries) per tile
+    if ((rc = ctr_ensure(ctx, ctx->aux[AUX_WORD_RECS], ctx->spec_w * 4, true))) return rc;
+    if ((rc = ctr_ensure(ctx, ctx->aux[AUX_WORD_SLOTS], ctx->spec_w * 8, true))) return rc;
+    if ((rc = ctr_ensure(ctx, ctx->aux[AUX_TILE_WORDS], (size_t)ntiles * 8 + 16))) return rc;
     if (geom) {
       if ((rc = ctr_ensure(ctx, ctx->verts, ctx->spec_v * 3 * gsz, true))) return rc;
       if (want_n && (rc = ctr_ensure(ctx, ctx->normals, ctx->spec_v * 3 * gsz, true))) return rc;
@@ -1520,23 +1520,25 @@ int run_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts* out, int 
     const unsigned cap_w = (unsigned)std::min<size_t>(ctx->spec_w, 0x7fffffffu);
 
     if (!(phase == 2 && attempt == 0)) {                 // phase 2: attempt 0 was enqueued by phase 1
-    ctr_launch_dep(k_reset3, 64, 256, 0, st, dctr, (uint4*)ctx->aux[4].p, (size_t)(nrows + 15) / 16, (uint4*)ctx->aux[32].p,
-                   (uint4*)ctx->aux[35].p, (size_t)(nrows + 3) / 4, st_vt, (size_t)ntiles);
+    ctr_launch_dep(k_reset3, 64, 256, 0, st, dctr, (uint4*)ctx->aux[AUX_ROW_FLAGS].p, (size_t)(nrows + 15) / 16,
+                   (uint4*)ctx->aux[AUX_WORD_FLAGS].p, (uint4*)ctx->aux[AUX_EXACT_FLAGS].p, (size_t)(nrows + 3) / 4, st_vt,
+                   (size_t)ntiles);
     ctx->launches++;
     CTR_DBG(ctx, "k_reset3");
     rc = launch_bitplane<T>(ctx, dfield, (unsigned)nrows, n2, W, n0, n1, p->isovalue, (uint32_t*)ctx->bits.p, (uint32_t*)ctx->nbits.p,
-                            (uint8_t*)ctx->aux[4].p, (MinMaxKeys*)dctr, (p->flags & CTR_WANT_MINMAX) != 0, false, (uint32_t*)ctx->aux[32].p);
+                            (uint8_t*)ctx->aux[AUX_ROW_FLAGS].p, (MinMaxKeys*)dctr, (p->flags & CTR_WANT_MINMAX) != 0, false,
+                            (uint32_t*)ctx->aux[AUX_WORD_FLAGS].p);
     if (rc) return rc;
     CTR_DBG(ctx, "k_bitplane");
     ctr_stage_mark(ctx, 2);
     if (ntiles > 0) {
-      ctr_launch_dep(k_count_a<T>, ntiles, CS_THREADS, 0, st, g, word0, nscan, (uint32_t*)ctx->wlist.p, (uint2*)ctx->aux[41].p,
-                     (uint2*)ctx->aux[34].p, cap_w, dctr);
+      ctr_launch_dep(k_count_a<T>, ntiles, CS_THREADS, 0, st, g, word0, nscan, (uint32_t*)ctx->wlist.p,
+                     (uint2*)ctx->aux[AUX_WORD_SLOTS].p, (uint2*)ctx->aux[AUX_TILE_WORDS].p, cap_w, dctr);
       CTR_DBG(ctx, "k_count_a");
       // the grid covers the expected list length (last run's, with head-room); blocks past the real length only take a ticket
       const unsigned wb = (unsigned)((std::min<size_t>(cap_w, ctx->last_w + ctx->last_w / 8 + 4096) + CB_THREADS - 1) / CB_THREADS);
-      ctr_launch_dep(k_count_b<T>, wb, CB_THREADS, 0, st, g, word0, (const uint32_t*)ctx->wlist.p, (const uint2*)ctx->aux[41].p, cap_w,
-                     (uint32_t*)ctx->aux[33].p,
+      ctr_launch_dep(k_count_b<T>, wb, CB_THREADS, 0, st, g, word0, (const uint32_t*)ctx->wlist.p,
+                     (const uint2*)ctx->aux[AUX_WORD_SLOTS].p, cap_w, (uint32_t*)ctx->aux[AUX_WORD_RECS].p,
                      (uint4*)ctx->wdir.p, (ulonglong2*)b_own.p, (unsigned long long*)b_cell_id.p, cap_own, cap_cell, st_vt, dctr, ntiles);
       const int fused = ntiles <= SCAN_FUSE_TILES ? 1 : 0;
       if (!fused) ctr_launch_dep(k_tile_scan3, 1, 1024, 0, st, st_vt, ntiles, dctr);
@@ -1544,7 +1546,8 @@ int run_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts* out, int 
       ctx->cover_w = (size_t)wb * CB_THREADS;
       CTR_DBG(ctx, "k_count_b");
       ctr_launch_dep(k_scan<T>, (ntiles + SCAN_WARPS - 1) / SCAN_WARPS, SCAN_WARPS * 32, 0, st,
-                     g, word0, ntiles, (const uint32_t*)ctx->wlist.p, (const uint32_t*)ctx->aux[33].p, (const uint2*)ctx->aux[34].p, cap_w,
+                     g, word0, ntiles, (const uint32_t*)ctx->wlist.p, (const uint32_t*)ctx->aux[AUX_WORD_RECS].p,
+                     (const uint2*)ctx->aux[AUX_TILE_WORDS].p, cap_w,
                      (const unsigned long long*)st_vt, (uint4*)ctx->wdir.p, dctr, fused);
       ctx->launches++;
       CTR_DBG(ctx, "k_scan");
@@ -1665,6 +1668,7 @@ int run_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts* out, int 
   return 0;
 }
 
+#include "compact3d.cuh"
 #include "mt3d_select.cuh"
 #include "mt3d_keep.cuh"
 #include "mt3d_clean.cuh"
@@ -1847,10 +1851,10 @@ extern "C" int ctr_mt3d_clean(ctr_ctx* ctx, const ctr_clean_params* cp, ctr_clea
   memset(out, 0, sizeof *out);
   if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
     return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to clean");
-  if (ctx->last3_edited & 2u) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has already been cleaned");
+  if (ctx->last3_edited & EDIT_CLEAN) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has already been cleaned");
   // the reference's clean-up (quantize, tiny simplices) is defined on the interpolated positions
-  if (ctx->last3_edited & 8u) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has been smoothed: clean it up before smoothing");
-  if (ctx->last3_edited & 16u) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has been decimated: clean it up before decimating");
+  if (ctx->last3_edited & EDIT_SMOOTH) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has been smoothed: clean it up before smoothing");
+  if (ctx->last3_edited & EDIT_DECIMATE) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has been decimated: clean it up before decimating");
   const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
   if (p->i_lo != 0 || p->i_hi != p->n0 || p->vert_id_base != 0)
     return ctr_fail(ctx, CTR_ERR_UNSUPPORTED, "mesh clean-up needs a full-volume run (merges cross slab faces)");
@@ -1920,7 +1924,7 @@ extern "C" int ctr_mt3d_interpolate_fetch(ctr_ctx* ctx, void* values) {
   if (rc) return rc;
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
   const size_t bytes = ctx->attr_rows * (size_t)ctx->attr_ncomp * ((ctx->last_flags & CTR_GEOM_F64) ? 8 : 4);
-  if (bytes) CTR_CUDA(ctx, cudaMemcpyAsync(values, ctx->aux[43].p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  if (bytes) CTR_CUDA(ctx, cudaMemcpyAsync(values, ctx->aux[AUX_VALUES].p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
   CTR_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return 0;
 }
@@ -1930,6 +1934,6 @@ extern "C" int ctr_mt3d_interpolate_device_ptr(ctr_ctx* ctx, void** values) {
   if (!values) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
   int rc = interp_check(ctx);
   if (rc) return rc;
-  *values = ctx->aux[43].p;
+  *values = ctx->aux[AUX_VALUES].p;
   return 0;
 }

@@ -1,5 +1,5 @@
 // The reference's mesh post-processing on the device mesh of the last ctr_mt3d_run (SURVEY.md 8 a10, a11, a13, f1) --
-// included by mt3d.cu inside its anonymous namespace, after mt3d_select.cuh (whose scan / compaction kernels it uses).
+// included by mt3d.cu inside its anonymous namespace, after compact3d.cuh.
 //
 //   tetrahedral.py:190-215    quantize_interpolations : interpolations that truncate to the same cell of the
 //                             `divisions` grid become one vertex; simplices that lose a vertex, or equal another, go;
@@ -21,7 +21,7 @@
 //   k_c_tiny / k_c_tinypos : extent test, union of the three vertices, positions of non-roots overwritten by their root's;
 //   k_c_flat / k_c_final   : cross-product test, union of np.allclose vertex pairs of flat triangles, kept triangles
 //                            mapped through the merge and checked for lost vertices; used-vertex flags;
-//   k_flag_scan x 2, k_sel_rows, k_c_tris_out : order-preserving compaction of vertices, normals, keys and triangles;
+//   compact_mesh           : order-preserving compaction of vertices, normals, keys and the mapped triangles;
 //   k_c_transform          : grid -> world (grid_field.py:89-93) at the very end, after the optional orientation pass,
 //                            which the reference also runs in grid coordinates (tetrahedral.py:611-617).
 
@@ -223,15 +223,6 @@ __global__ void k_c_final(int* __restrict__ tris2, unsigned nt, uint8_t* __restr
   }
 }
 
-__global__ void k_c_tris_out(const int* __restrict__ tris2, int* __restrict__ dst, const uint8_t* __restrict__ keep,
-                             const uint32_t* __restrict__ idx_t, const uint32_t* __restrict__ idx_v, unsigned nt) {
-  const unsigned t = blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= nt || !keep[t]) return;
-  const size_t d = idx_t[t];
-#pragma unroll
-  for (int q = 0; q < 3; ++q) dst[d * 3 + q] = (int)idx_v[tris2[(size_t)t * 3 + q]];
-}
-
 template <typename G>
 __global__ void k_c_transform(G* __restrict__ verts, G* __restrict__ normals, unsigned nv, Xform xf) {
   const unsigned v = blockIdx.x * blockDim.x + threadIdx.x;
@@ -252,20 +243,15 @@ __global__ void k_c_transform(G* __restrict__ verts, G* __restrict__ normals, un
   }
 }
 
-// Scratch of the passes that cluster vertices by cell (clean-up, decimation), carved from aux[28]: the cell and triangle
-// tables, the representative map, union-find parents, flags, mapped triangles, compaction indices and scan words, the
-// selection's counters, a `head` block for the pass's own counters, an `extra` block, and the staging rows of the
-// compaction.
+// Scratch of the passes that cluster vertices by cell (clean-up, decimation), carved from AUX_SCRATCH1: the cell and
+// triangle tables, the representative map, union-find parents, the compaction's pieces, mapped triangles, a `head`
+// block for the pass's own counters, an `extra` block, and the staging rows.
 struct ClusterBufs {
   ufh::Slot *tab_v, *tab_t;
   size_t nslots_v, nslots_t;
   int *rep, *parent_a, *parent_b, *tris2;
-  uint8_t *used_v, *keep_t;
-  uint32_t *idx_t, *idx_v;
-  unsigned long long *st_t, *st_v;
-  int tiles_t, tiles_v;
-  SelCounters* dsel;
-  void *head, *extra, *tmp;
+  void *head, *extra;
+  CompactBufs cb;
 };
 
 static int cluster_bufs(ctr_ctx* ctx, unsigned nV, unsigned nT, size_t gsz, size_t head_bytes, size_t extra_bytes, ClusterBufs& b) {
@@ -273,41 +259,18 @@ static int cluster_bufs(ctr_ctx* ctx, unsigned nV, unsigned nT, size_t gsz, size
   b.nslots_t = 1024;
   while (b.nslots_v < (size_t)nV * 2) b.nslots_v <<= 1;
   while (b.nslots_t < (size_t)nT * 2) b.nslots_t <<= 1;
-  b.tiles_t = (int)(((size_t)nT + SC_TILE - 1) / SC_TILE);
-  b.tiles_v = (int)(((size_t)nV + SC_TILE - 1) / SC_TILE);
-  size_t off = 0;
-  auto carve = [&](size_t bytes) {
-    const size_t o = off;
-    off += (bytes + 255) & ~(size_t)255;
-    return o;
-  };
-  const size_t o_tv = carve(b.nslots_v * sizeof(ufh::Slot)), o_tt = carve(b.nslots_t * sizeof(ufh::Slot)),
-               o_rep = carve((size_t)nV * 4 + 4), o_pa = carve((size_t)nV * 4 + 4), o_pb = carve((size_t)nV * 4 + 4),
-               o_used = carve((size_t)nV + 8), o_keep = carve((size_t)nT + 8), o_t2 = carve((size_t)nT * 12 + 16),
-               o_it = carve((size_t)nT * 4 + 4), o_iv = carve((size_t)nV * 4 + 4), o_st = carve((size_t)b.tiles_t * 8 + 8),
-               o_sv = carve((size_t)b.tiles_v * 8 + 8), o_sel = carve(sizeof(SelCounters) + 64), o_head = carve(head_bytes + 64),
-               o_extra = carve(extra_bytes), o_out = carve(std::max<size_t>((size_t)nV * 3 * gsz, (size_t)nT * 12) + 16);
-  DevBuf& b_s = ctx->aux[28];
-  int rc;
-  if ((rc = ctr_ensure(ctx, b_s, off))) return rc;
-  char* base = (char*)b_s.p;
-  b.tab_v = (ufh::Slot*)(base + o_tv);
-  b.tab_t = (ufh::Slot*)(base + o_tt);
-  b.rep = (int*)(base + o_rep);
-  b.parent_a = (int*)(base + o_pa);
-  b.parent_b = (int*)(base + o_pb);
-  b.used_v = (uint8_t*)(base + o_used);
-  b.keep_t = (uint8_t*)(base + o_keep);
-  b.tris2 = (int*)(base + o_t2);
-  b.idx_t = (uint32_t*)(base + o_it);
-  b.idx_v = (uint32_t*)(base + o_iv);
-  b.st_t = (unsigned long long*)(base + o_st);
-  b.st_v = (unsigned long long*)(base + o_sv);
-  b.dsel = (SelCounters*)(base + o_sel);
-  b.head = base + o_head;
-  b.extra = base + o_extra;
-  b.tmp = base + o_out;
-  return 0;
+  return ctr_carve_buf(ctx, ctx->aux[AUX_SCRATCH1], [&](ctr_carve& c) {
+    c(b.tab_v, b.nslots_v * sizeof(ufh::Slot));
+    c(b.tab_t, b.nslots_t * sizeof(ufh::Slot));
+    c(b.rep, (size_t)nV * 4 + 4);
+    c(b.parent_a, (size_t)nV * 4 + 4);
+    c(b.parent_b, (size_t)nV * 4 + 4);
+    compact_carve(c, nV, nT, 0, b.cb);
+    c(b.tris2, (size_t)nT * 12 + 16);
+    c(b.head, head_bytes + 64);
+    c(b.extra, extra_bytes);
+    c(b.cb.stage, std::max<size_t>((size_t)nV * 3 * gsz, (size_t)nT * 12) + 16);
+  });
 }
 
 // k_c_init, every vertex's representative (the smallest vertex id in its cell of `key`), the triangles through that map
@@ -323,13 +286,13 @@ int cluster_tris(ctr_ctx* ctx, const G* verts, unsigned nV, const int* tris, uns
   for (int attempt = 0;; ++attempt) {
     const unsigned long long seed = 0x51ed270b1a2c3d4full * (unsigned long long)(attempt + 1);
     CTR_CUDA(ctx, cudaMemsetAsync(b.head, 0, hbytes, st));
-    k_c_init<<<ctx->sm_count * 8, 256, 0, st>>>(b.tab_v, b.nslots_v, b.tab_t, b.nslots_t, b.parent_a, b.parent_b, b.used_v, nV);
+    k_c_init<<<ctx->sm_count * 8, 256, 0, st>>>(b.tab_v, b.nslots_v, b.tab_t, b.nslots_t, b.parent_a, b.parent_b, b.cb.used_v, nV);
     k_c_qinsert<G><<<vb, 256, 0, st>>>(verts, nV, key, b.tab_v, b.nslots_v - 1);
     k_c_qmap<G><<<vb, 256, 0, st>>>(verts, nV, key, b.tab_v, b.nslots_v - 1, b.rep);
     ctx->launches += 3;
     if (nT) {
-      k_c_qtris<<<tb, 256, 0, st>>>(tris, nT, b.rep, b.tris2, b.keep_t, b.tab_t, b.nslots_t - 1, seed);
-      k_c_qdedupe<<<tb, 256, 0, st>>>(b.tris2, nT, b.keep_t, b.tab_t, b.nslots_t - 1, seed, dcc);
+      k_c_qtris<<<tb, 256, 0, st>>>(tris, nT, b.rep, b.tris2, b.cb.keep_t, b.tab_t, b.nslots_t - 1, seed);
+      k_c_qdedupe<<<tb, 256, 0, st>>>(b.tris2, nT, b.cb.keep_t, b.tab_t, b.nslots_t - 1, seed, dcc);
       ctx->launches += 2;
     }
     CTR_CUDA(ctx, cudaMemcpyAsync(h, b.head, hbytes, cudaMemcpyDeviceToHost, st));
@@ -337,45 +300,6 @@ int cluster_tris(ctr_ctx* ctx, const G* verts, unsigned nV, const int* tris, uns
     if (!((const CleanCounters*)h)->collision) return 0;
     if (attempt == 3) return ctr_fail(ctx, CTR_ERR_STATE, "triangle de-duplication: hash collisions under four seeds");
   }
-}
-
-// Order-preserving compaction in place: the triangles with keep_t (their ids, representatives in tris2, renumbered
-// through idx_v) and the vertices with used_v (positions, normals, keys / lowmin as the run has them).  Synchronous;
-// newV / newT receive the new counts.
-static int compact_mesh(ctr_ctx* ctx, const ClusterBufs& b, unsigned nV, unsigned nT, size_t gsz, size_t& newV, size_t& newT) {
-  cudaStream_t st = ctx->stream;
-  const uint32_t fl = ctx->last_flags;
-  const unsigned vb = (nV + 255) / 256, tb = (nT + 255) / 256;
-  SelCounters hs;
-  CTR_CUDA(ctx, cudaMemsetAsync(b.dsel, 0, sizeof(SelCounters), st));
-  CTR_CUDA(ctx, cudaMemsetAsync(b.st_t, 0, (size_t)b.tiles_t * 8 + 8, st));
-  CTR_CUDA(ctx, cudaMemsetAsync(b.st_v, 0, (size_t)b.tiles_v * 8 + 8, st));
-  k_flag_scan<<<b.tiles_t, SC_THREADS, 0, st>>>(b.keep_t, nT, b.idx_t, b.st_t, &b.dsel->ticket[0], &b.dsel->total[0], b.tiles_t);
-  k_flag_scan<<<b.tiles_v, SC_THREADS, 0, st>>>(b.used_v, nV, b.idx_v, b.st_v, &b.dsel->ticket[1], &b.dsel->total[1], b.tiles_v);
-  ctx->launches += 2;
-  CTR_CUDA(ctx, cudaGetLastError());
-  CTR_CUDA(ctx, cudaMemcpyAsync(&hs, b.dsel, sizeof hs, cudaMemcpyDeviceToHost, st));
-  CTR_CUDA(ctx, cudaStreamSynchronize(st));
-  newT = (size_t)hs.total[0];
-  newV = (size_t)hs.total[1];
-  auto rows = [&](DevBuf& d, int wpr, size_t row_bytes) -> int {
-    if (!d.p) return 0;
-    k_sel_rows<<<vb, 256, 0, st>>>((const uint32_t*)d.p, (uint32_t*)b.tmp, b.used_v, b.idx_v, nV, wpr);
-    ctx->launches++;
-    if (newV) CTR_CUDA(ctx, cudaMemcpyAsync(d.p, b.tmp, newV * row_bytes, cudaMemcpyDeviceToDevice, st));
-    return 0;
-  };
-  int rc;
-  if ((rc = rows(ctx->verts, (int)(3 * gsz / 4), 3 * gsz))) return rc;
-  if ((fl & CTR_WANT_NORMALS) && (rc = rows(ctx->normals, (int)(3 * gsz / 4), 3 * gsz))) return rc;
-  if ((fl & CTR_WANT_KEYS) && (rc = rows(ctx->keys, 2, 8))) return rc;
-  if ((fl & CTR_WANT_KEYS) && (rc = rows(ctx->lowmin, 0, 1))) return rc;
-  k_c_tris_out<<<tb, 256, 0, st>>>(b.tris2, (int*)b.tmp, b.keep_t, b.idx_t, b.idx_v, nT);
-  ctx->launches++;
-  if (newT) CTR_CUDA(ctx, cudaMemcpyAsync(ctx->tris.p, b.tmp, newT * 12, cudaMemcpyDeviceToDevice, st));
-  CTR_CUDA(ctx, cudaGetLastError());
-  CTR_CUDA(ctx, cudaStreamSynchronize(st));
-  return 0;
 }
 
 template <typename G>
@@ -408,17 +332,18 @@ int clean_typed(ctr_ctx* ctx, const ctr_clean_params* cp, ctr_clean_counts* out)
   size_t newV = 0, newT = 0;
   if (nV && nT) {
     if ((rc = cluster_tris<G>(ctx, verts, nV, tris, nT, e, b, &hc, sizeof hc))) return rc;
-    k_c_tiny<G><<<tb, 256, 0, st>>>(verts, b.tris2, nT, b.keep_t, e, cp->epsilon, b.parent_a, dcc);
+    k_c_tiny<G><<<tb, 256, 0, st>>>(verts, b.tris2, nT, b.cb.keep_t, e, cp->epsilon, b.parent_a, dcc);
     k_c_tinypos<G><<<vb, 256, 0, st>>>(verts, nV, b.parent_a);
-    if (!(cp->flags & CTR_CLEAN_NO_TRIANGLES)) k_c_flat<G><<<tb, 256, 0, st>>>(verts, b.tris2, nT, b.keep_t, b.parent_b, dcc);
-    k_c_final<<<tb, 256, 0, st>>>(b.tris2, nT, b.keep_t, b.parent_b, b.used_v, dcc);
+    if (!(cp->flags & CTR_CLEAN_NO_TRIANGLES)) k_c_flat<G><<<tb, 256, 0, st>>>(verts, b.tris2, nT, b.cb.keep_t, b.parent_b, dcc);
+    k_c_final<<<tb, 256, 0, st>>>(b.tris2, nT, b.cb.keep_t, b.parent_b, b.cb.used_v, dcc);
     ctx->launches += 4;
     CTR_CUDA(ctx, cudaMemcpyAsync(&hc, dcc, sizeof hc, cudaMemcpyDeviceToHost, st));   // (synchronised by compact_mesh)
-    if ((rc = compact_mesh(ctx, b, nV, nT, sizeof(G), newV, newT))) return rc;
+    if ((rc = compact_mesh(ctx, b.cb, nV, nT, b.tris2, 0u, false, nullptr, newV, newT))) return rc;
+    CTR_CUDA(ctx, cudaStreamSynchronize(st));
   }
   ctx->last_counts[0] = (int64_t)newV;
   ctx->last_counts[1] = (int64_t)newT;
-  ctx->last3_edited |= 2u;
+  ctx->last3_edited |= EDIT_CLEAN;
   out->n_verts = (int64_t)newV;
   out->n_tris = (int64_t)newT;
   out->n_quantized = hc.n_quant;

@@ -12,17 +12,10 @@
 //                neighbours and unites with the ones that exist (lock-free union-find, uf_hash.cuh);
 //   k_sel_seeds : the components of the seed voxels get flagged;
 //   k_sel_mark  : every emitting voxel copies its component's flag to its triangles (contiguous in the output);
-//   k_sel_used, k_flag_scan x 2, k_sel_rows / k_sel_tris : the kept triangles and the vertices they use are compacted
-//                in place order (single-pass look-back scans), ids rewritten.
-constexpr int SC_THREADS = 256;
-constexpr int SC_PER = 8;
-constexpr int SC_TILE = SC_THREADS * SC_PER;
+//   k_sel_used  : the vertices of the kept triangles; then compact_mesh (compact3d.cuh) compacts both in place, in order.
 
 struct SelCounters {
   unsigned n_extra;                  // connector voxels found
-  unsigned ticket[2];                // tile tickets of the two scans
-  unsigned pad;
-  unsigned long long total[2];       // kept triangles, used vertices
 };
 
 template <typename T>
@@ -136,81 +129,6 @@ __global__ void k_sel_mark(const unsigned long long* __restrict__ cell_id, unsig
     if (t0 + q < n_tris) keep_t[t0 + q] = 1;
 }
 
-__global__ void k_sel_used(const int* __restrict__ tris, unsigned n_tris, const uint8_t* __restrict__ keep_t, unsigned id_base,
-                           uint8_t* __restrict__ used_v, unsigned n_verts) {
-  const unsigned t = blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= n_tris || !keep_t[t]) return;
-#pragma unroll
-  for (int q = 0; q < 3; ++q) {
-    const unsigned v = (unsigned)tris[(size_t)t * 3 + q] - id_base;
-    if (v < n_verts) used_v[v] = 1;
-  }
-}
-
-// idx[q] = number of set flags before q; *total = number of set flags.  Tiles take tickets, prefixes by look-back.
-__global__ void __launch_bounds__(SC_THREADS) k_flag_scan(const uint8_t* __restrict__ flags, unsigned n, uint32_t* __restrict__ idx,
-                                                          unsigned long long* status, unsigned* ticket,
-                                                          unsigned long long* total, int ntiles) {
-  __shared__ unsigned s_tile;
-  __shared__ unsigned s_warp[SC_THREADS / 32];
-  __shared__ unsigned long long s_excl;
-  if (threadIdx.x == 0) s_tile = atomicAdd(ticket, 1u);
-  __syncthreads();
-  const int tile = (int)s_tile;
-  const unsigned lane = lane_id(), warp = threadIdx.x >> 5;
-  const unsigned q0 = (unsigned)tile * SC_TILE + threadIdx.x * SC_PER;
-  unsigned f[SC_PER], cnt = 0;
-#pragma unroll
-  for (int u = 0; u < SC_PER; ++u) {
-    f[u] = (q0 + u < n && flags[q0 + u]) ? 1u : 0u;
-    cnt += f[u];
-  }
-  const unsigned inc = warp_incl_scan_u32(cnt);
-  if (lane == 31) s_warp[warp] = inc;
-  __syncthreads();
-  unsigned woff = 0, blk = 0;
-#pragma unroll
-  for (int w = 0; w < SC_THREADS / 32; ++w) {
-    if (w < (int)warp) woff += s_warp[w];
-    blk += s_warp[w];
-  }
-  if (warp == 0) {
-    const unsigned long long e = lb_lookback(status, tile, (unsigned long long)blk);
-    if (lane == 0) s_excl = e;
-  }
-  __syncthreads();
-  unsigned run = (unsigned)s_excl + woff + inc - cnt;
-#pragma unroll
-  for (int u = 0; u < SC_PER; ++u) {
-    if (q0 + u < n) idx[q0 + u] = run;
-    run += f[u];
-  }
-  if (tile == ntiles - 1 && threadIdx.x == 0) *total = s_excl + blk;
-}
-
-// rows of `wpr` 32-bit words (or single bytes when wpr == 0): dst[idx[r]] = src[r] for flagged rows
-__global__ void k_sel_rows(const uint32_t* __restrict__ src, uint32_t* __restrict__ dst, const uint8_t* __restrict__ flags,
-                           const uint32_t* __restrict__ idx, unsigned n, int wpr) {
-  const unsigned r = blockIdx.x * blockDim.x + threadIdx.x;
-  if (r >= n || !flags[r]) return;
-  const size_t d = idx[r];
-  if (wpr == 0) {
-    reinterpret_cast<uint8_t*>(dst)[d] = reinterpret_cast<const uint8_t*>(src)[r];
-    return;
-  }
-  for (int q = 0; q < wpr; ++q) dst[d * wpr + q] = src[(size_t)r * wpr + q];
-}
-
-__global__ void k_sel_tris(const int* __restrict__ src, int* __restrict__ dst, const uint8_t* __restrict__ keep_t,
-                           const uint32_t* __restrict__ idx_t, const uint32_t* __restrict__ idx_v, unsigned n_tris,
-                           unsigned id_base) {
-  const unsigned t = blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= n_tris || !keep_t[t]) return;
-  const size_t d = idx_t[t];
-#pragma unroll
-  for (int q = 0; q < 3; ++q) dst[d * 3 + q] = (int)(idx_v[(unsigned)src[(size_t)t * 3 + q] - id_base] + id_base);
-}
-
 template <typename T>
 int select_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, const int32_t* seeds, int64_t n_seeds, int64_t* out_verts,
                  int64_t* out_tris, int64_t* out_voxels) {
@@ -231,18 +149,17 @@ int select_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, const int32_t* seeds, i
   g.divN1.init((unsigned)n1);
   g.bits = (const uint32_t*)ctx->bits.p;
   g.nbits = (const uint32_t*)ctx->nbits.p;
-  g.rowflag = (const uint8_t*)ctx->aux[4].p;
-  g.wordflag = (const uint32_t*)ctx->aux[32].p;
-  g.exactflag = (uint32_t*)ctx->aux[35].p;
+  g.rowflag = (const uint8_t*)ctx->aux[AUX_ROW_FLAGS].p;
+  g.wordflag = (const uint32_t*)ctx->aux[AUX_WORD_FLAGS].p;
+  g.exactflag = (uint32_t*)ctx->aux[AUX_EXACT_FLAGS].p;
   g.wshift = 0;
   while ((W >> g.wshift) > 32) ++g.wshift;
   const unsigned nV = (unsigned)ctx->last_counts[0], nT = (unsigned)ctx->last_counts[1];
   const unsigned n_cell = (unsigned)ctx->last_cell;
-  const uint32_t fl = p->flags;
-  const size_t gsz = (fl & CTR_GEOM_F64) ? 8 : 4;
-  const bool want_n = (fl & CTR_WANT_NORMALS) != 0, want_k = (fl & CTR_WANT_KEYS) != 0;
+  const size_t gsz = (p->flags & CTR_GEOM_F64) ? 8 : 4;
+  const unsigned long long* cell_id = (const unsigned long long*)ctx->aux[AUX_CELL_LIST].p;
   int rc;
-  DevBuf& b_ctr = ctx->aux[31];
+  DevBuf& b_ctr = ctx->aux[AUX_SCRATCH4];
   if ((rc = ctr_ensure(ctx, b_ctr, sizeof(SelCounters) + 64))) return rc;
   SelCounters* dctr = (SelCounters*)b_ctr.p;
   SelCounters h;
@@ -258,42 +175,30 @@ int select_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, const int32_t* seeds, i
   if (n_nodes >= 0x7fffffffull) return ctr_fail(ctx, CTR_ERR_OVERFLOW, "too many border voxels for one selection");
   size_t nslots = 1024;
   while (nslots < n_nodes * 2) nslots <<= 1;
-  const int tiles_t = (int)(((size_t)nT + SC_TILE - 1) / SC_TILE), tiles_v = (int)(((size_t)nV + SC_TILE - 1) / SC_TILE);
-  // one scratch allocation, carved (256-byte aligned pieces)
-  size_t off = 0;
-  auto carve = [&](size_t bytes) {
-    const size_t o = off;
-    off += (bytes + 255) & ~(size_t)255;
-    return o;
-  };
-  const size_t o_vox = carve(n_nodes * 8 + 8), o_tab = carve(nslots * sizeof(ufh::Slot)), o_par = carve(n_nodes * 4 + 4),
-               o_flag = carve(n_nodes + 1), o_keep = carve((size_t)nT + 8), o_used = carve((size_t)nV + 8),
-               o_it = carve((size_t)nT * 4 + 4), o_iv = carve((size_t)nV * 4 + 4), o_st = carve((size_t)tiles_t * 8 + 8),
-               o_sv = carve((size_t)tiles_v * 8 + 8), o_out = carve(std::max<size_t>((size_t)nV * 3 * gsz, (size_t)nT * 12) + 16);
-  DevBuf& b_s = ctx->aux[30];
-  if ((rc = ctr_ensure(ctx, b_s, off))) return rc;
-  char* base = (char*)b_s.p;
-  unsigned long long* node_vox = (unsigned long long*)(base + o_vox);
-  ufh::Slot* tab = (ufh::Slot*)(base + o_tab);
-  int* parent = (int*)(base + o_par);
-  uint8_t* flag = (uint8_t*)(base + o_flag);
-  uint8_t* keep_t = (uint8_t*)(base + o_keep);
-  uint8_t* used_v = (uint8_t*)(base + o_used);
-  uint32_t* idx_t = (uint32_t*)(base + o_it);
-  uint32_t* idx_v = (uint32_t*)(base + o_iv);
-  unsigned long long* st_t = (unsigned long long*)(base + o_st);
-  unsigned long long* st_v = (unsigned long long*)(base + o_sv);
-  void* tmp = base + o_out;
-  DevBuf& b_seeds = ctx->aux[29];
+  unsigned long long* node_vox;
+  ufh::Slot* tab;
+  int* parent;
+  uint8_t* flag;
+  CompactBufs cb;
+  if ((rc = ctr_carve_buf(ctx, ctx->aux[AUX_SCRATCH3], [&](ctr_carve& c) {
+         c(node_vox, n_nodes * 8 + 8);
+         c(tab, nslots * sizeof(ufh::Slot));
+         c(parent, n_nodes * 4 + 4);
+         c(flag, n_nodes + 1);
+         compact_carve(c, nV, nT, sizeof(unsigned), cb);
+         c(cb.stage, std::max<size_t>((size_t)nV * 3 * gsz, (size_t)nT * 12) + 16);
+       })))
+    return rc;
+  DevBuf& b_seeds = ctx->aux[AUX_SCRATCH2];
   if ((rc = ctr_ensure(ctx, b_seeds, (size_t)std::max<int64_t>(n_seeds, 1) * 12))) return rc;
   if (n_seeds) CTR_CUDA(ctx, cudaMemcpyAsync(b_seeds.p, seeds, (size_t)n_seeds * 12, cudaMemcpyHostToDevice, st));
+  unsigned* n_voxels = (unsigned*)cb.scan;           // emitting voxels selected: the pass's counter of the scan piece
   CTR_CUDA(ctx, cudaMemsetAsync(dctr, 0, sizeof(SelCounters), st));
-  CTR_CUDA(ctx, cudaMemsetAsync(keep_t, 0, (size_t)nT + 8, st));
-  CTR_CUDA(ctx, cudaMemsetAsync(used_v, 0, (size_t)nV + 8, st));
-  CTR_CUDA(ctx, cudaMemsetAsync(st_t, 0, (size_t)tiles_t * 8 + 8, st));
-  CTR_CUDA(ctx, cudaMemsetAsync(st_v, 0, (size_t)tiles_v * 8 + 8, st));
-  const unsigned nb = (unsigned)((n_nodes + 255) / 256), cb = (n_cell + 255) / 256, tb = (nT + 255) / 256, vb = (nV + 255) / 256;
-  if (n_cell) k_sel_cells<T><<<cb, 256, 0, st>>>(g, (const unsigned long long*)ctx->aux[2].p, n_cell, node_vox);
+  CTR_CUDA(ctx, cudaMemsetAsync(n_voxels, 0, sizeof(unsigned), st));
+  CTR_CUDA(ctx, cudaMemsetAsync(cb.keep_t, 0, (size_t)nT + 8, st));
+  CTR_CUDA(ctx, cudaMemsetAsync(cb.used_v, 0, (size_t)nV + 8, st));
+  const unsigned nb = (unsigned)((n_nodes + 255) / 256), cblk = (n_cell + 255) / 256;
+  if (n_cell) k_sel_cells<T><<<cblk, 256, 0, st>>>(g, cell_id, n_cell, node_vox);
   if (n_extra) k_sel_connectors<T><<<wb, 256, 0, st>>>(g, (unsigned)nwords, node_vox, n_cell, (unsigned)n_nodes, &dctr->n_extra);
   k_sel_init<<<ctx->sm_count * 8, 256, 0, st>>>(tab, nslots, parent, flag, (unsigned)n_nodes);
   if (n_nodes) {
@@ -304,42 +209,19 @@ int select_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, const int32_t* seeds, i
     k_sel_seeds<<<(unsigned)((n_seeds + 255) / 256), 256, 0, st>>>((const int*)b_seeds.p, (unsigned)n_seeds, n0, n1, n2, tab,
                                                                     nslots - 1, parent, flag);
   if (n_cell)
-    k_sel_mark<<<cb, 256, 0, st>>>((const unsigned long long*)ctx->aux[2].p, n_cell,
-                                   (const uint4*)ctx->wdir.p, parent, flag, keep_t, nT, &dctr->pad);
-  if (nT) {
-    k_sel_used<<<tb, 256, 0, st>>>((const int*)ctx->tris.p, nT, keep_t, g.id_base, used_v, nV);
-    k_flag_scan<<<tiles_t, SC_THREADS, 0, st>>>(keep_t, nT, idx_t, st_t, &dctr->ticket[0], &dctr->total[0], tiles_t);
-  }
-  if (nV) k_flag_scan<<<tiles_v, SC_THREADS, 0, st>>>(used_v, nV, idx_v, st_v, &dctr->ticket[1], &dctr->total[1], tiles_v);
-  ctx->launches += 9;
+    k_sel_mark<<<cblk, 256, 0, st>>>(cell_id, n_cell, (const uint4*)ctx->wdir.p, parent, flag, cb.keep_t, nT, n_voxels);
+  if (nT) k_sel_used<<<(nT + 255) / 256, 256, 0, st>>>((const int*)ctx->tris.p, nT, cb.keep_t, g.id_base, cb.used_v, nV);
+  ctx->launches += 1 + (n_cell ? 2 : 0) + (n_extra ? 1 : 0) + (n_nodes ? 2 : 0) + (n_seeds ? 1 : 0) + (nT ? 1 : 0);
   CTR_CUDA(ctx, cudaGetLastError());
-  CTR_CUDA(ctx, cudaMemcpyAsync(&h, dctr, sizeof h, cudaMemcpyDeviceToHost, st));
-  CTR_CUDA(ctx, cudaStreamSynchronize(st));
-  const size_t newT = (size_t)h.total[0], newV = (size_t)h.total[1];
-  // compaction through the scratch piece, array by array
-  auto rows = [&](DevBuf& b, int wpr, size_t row_bytes) -> int {
-    if (!nV || !b.p) return 0;
-    k_sel_rows<<<vb, 256, 0, st>>>((const uint32_t*)b.p, (uint32_t*)tmp, used_v, idx_v, nV, wpr);
-    ctx->launches++;
-    if (newV) CTR_CUDA(ctx, cudaMemcpyAsync(b.p, tmp, newV * row_bytes, cudaMemcpyDeviceToDevice, st));
-    return 0;
-  };
-  if ((rc = rows(ctx->verts, (int)(3 * gsz / 4), 3 * gsz))) return rc;
-  if (want_n && (rc = rows(ctx->normals, (int)(3 * gsz / 4), 3 * gsz))) return rc;
-  if (want_k && (rc = rows(ctx->keys, 2, 8))) return rc;
-  if (want_k && (rc = rows(ctx->lowmin, 0, 1))) return rc;
-  if (nT) {
-    k_sel_tris<<<tb, 256, 0, st>>>((const int*)ctx->tris.p, (int*)tmp, keep_t, idx_t, idx_v, nT, g.id_base);
-    ctx->launches++;
-    if (newT) CTR_CUDA(ctx, cudaMemcpyAsync(ctx->tris.p, tmp, newT * 12, cudaMemcpyDeviceToDevice, st));
-  }
-  CTR_CUDA(ctx, cudaGetLastError());
+  unsigned h_voxels = 0;
+  size_t newV, newT;
+  if ((rc = compact_mesh(ctx, cb, nV, nT, (const int*)ctx->tris.p, g.id_base, false, &h_voxels, newV, newT))) return rc;
   CTR_CUDA(ctx, cudaStreamSynchronize(st));
   ctx->last_counts[0] = (int64_t)newV;
   ctx->last_counts[1] = (int64_t)newT;
-  ctx->last3_edited |= 1u;
+  ctx->last3_edited |= EDIT_SELECT;
   if (out_verts) *out_verts = (int64_t)newV;
   if (out_tris) *out_tris = (int64_t)newT;
-  if (out_voxels) *out_voxels = (int64_t)h.pad;
+  if (out_voxels) *out_voxels = (int64_t)h_voxels;
   return 0;
 }

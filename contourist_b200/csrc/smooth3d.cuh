@@ -15,13 +15,12 @@
 //   k_s_store  : the result rounded into ctx->verts in place;
 //   k_s_nsum / k_s_nfin (normals3d.cuh): (CTR_WANT_NORMALS) per-triangle cross products summed into the corners (fp64
 //                atomicAdd), then normalised with the sign of the old gradient normal.
-// Scratch: aux[27] edge table, aux[28] per-vertex offsets / cursors / fixed flags, aux[29] neighbour lists, aux[30]
-// counters and look-back words, aux[46] / aux[47] the two fp64 copies.  aux[42..45] (vertex values, component labels
-// and table) are not touched.
+// Scratch: AUX_SCRATCH0 edge table, AUX_SCRATCH1 per-vertex offsets / cursors / fixed flags, AUX_SCRATCH2 neighbour
+// lists, AUX_SCRATCH3 counters and look-back words, AUX_SMOOTH_X0 / AUX_SMOOTH_X1 the two fp64 copies.
 
 constexpr int S_THREADS = 256;
 
-struct SCounters {                                    // head of aux[30], then one look-back word per vertex tile
+struct SCounters {                                    // head of AUX_SCRATCH3, then one look-back word per vertex tile
   MCounters m;                                        // k_m_edges' bad-id flag; the scan's ticket and total degree
   unsigned long long n_edges, n_fixed;
 };
@@ -181,12 +180,12 @@ int smooth_typed(ctr_ctx* ctx, const ctr_smooth_params* sp, ctr_smooth_counts* o
   const unsigned blocks_t = (nt + S_THREADS - 1) / S_THREADS, tiles_v = (nv + S_THREADS - 1) / S_THREADS;
   const unsigned slot_blocks = (unsigned)ctx->sm_count * 8;
   int rc;
-  DevBuf& b_etab = ctx->aux[27];
-  DevBuf& b_vert = ctx->aux[28];
-  DevBuf& b_nbr = ctx->aux[29];
-  DevBuf& b_scan = ctx->aux[30];
-  DevBuf& b_x0 = ctx->aux[46];
-  DevBuf& b_x1 = ctx->aux[47];
+  DevBuf& b_etab = ctx->aux[AUX_SCRATCH0];
+  DevBuf& b_vert = ctx->aux[AUX_SCRATCH1];
+  DevBuf& b_nbr = ctx->aux[AUX_SCRATCH2];
+  DevBuf& b_scan = ctx->aux[AUX_SCRATCH3];
+  DevBuf& b_x0 = ctx->aux[AUX_SMOOTH_X0];
+  DevBuf& b_x1 = ctx->aux[AUX_SMOOTH_X1];
   const size_t vbytes = (size_t)(nv + 1) * 4 + (size_t)nv * 4 + nv;   // off, cur, fixed
   if ((rc = ctr_ensure(ctx, b_etab, nslots * sizeof(EdgeSlot)))) return rc;
   if ((rc = ctr_ensure(ctx, b_vert, vbytes))) return rc;
@@ -224,7 +223,7 @@ int smooth_typed(ctr_ctx* ctx, const ctr_smooth_params* sp, ctr_smooth_counts* o
   if ((rc = ctr_ensure(ctx, b_x0, n3 * 8))) return rc;
   if ((rc = ctr_ensure(ctx, b_x1, n3 * 8))) return rc;
   ctx->mesh_gen++;                                    // from here on the mesh is edited
-  ctx->last3_edited |= 8u;
+  ctx->last3_edited |= EDIT_SMOOTH;
   int* nbr = (int*)b_nbr.p;
   double* x = (double*)b_x0.p;
   double* y = (double*)b_x1.p;

@@ -416,6 +416,13 @@ class Engine(object):
         self._check(self.lib.ctr_mt3d_orient_reference(self.h, ctypes.byref(nc), ctypes.byref(nf)), "ctr_mt3d_orient_reference")
         return int(nc.value), int(nf.value)
 
+    def _mesh_edited(self, n_verts, n_tris):
+        "a pass has dropped rows of the device mesh: the new counts, which mt3d_fetch sizes its arrays from"
+        flags, c = self._last3
+        c = type(c).from_buffer_copy(c)                                # the caller keeps the full scan's counts
+        c.n_verts, c.n_tris = int(n_verts), int(n_tris)
+        self._last3 = (flags, c)
+
     def mt3d_select_seeded(self, start_voxels):
         """Keep only what the reference's flood fill reaches from these voxel origins ([n, 3] ints, the output of
         find_initial_voxels): tetrahedral.py:443-469 on the device mesh of the last full-volume run.
@@ -425,10 +432,7 @@ class Engine(object):
         self.run_serial += 1
         self._check(self.lib.ctr_mt3d_select_seeded(self.h, _ptr(sv) if len(sv) else None, len(sv), ctypes.byref(nv),
                                                     ctypes.byref(nt), ctypes.byref(nc)), "ctr_mt3d_select_seeded")
-        flags, c = self._last3
-        c = type(c).from_buffer_copy(c)                                # the caller keeps the full scan's counts
-        c.n_verts, c.n_tris = int(nv.value), int(nt.value)             # what mt3d_fetch sizes its arrays from
-        self._last3 = (flags, c)
+        self._mesh_edited(nv.value, nt.value)
         return int(nv.value), int(nt.value), int(nc.value)
 
     def mt3d_clean(self, corner, origin=(0.0, 0.0, 0.0), delta=(1.0, 1.0, 1.0), divisions=10000, epsilon=1e-4, orient=False,
@@ -448,10 +452,7 @@ class Engine(object):
         c = CleanCounts()
         self.run_serial += 1
         self._check(self.lib.ctr_mt3d_clean(self.h, ctypes.byref(p), ctypes.byref(c)), "ctr_mt3d_clean")
-        flags, c3 = self._last3
-        c3 = type(c3).from_buffer_copy(c3)
-        c3.n_verts, c3.n_tris = int(c.n_verts), int(c.n_tris)
-        self._last3 = (flags, c3)
+        self._mesh_edited(c.n_verts, c.n_tris)
         return c
 
     def mt3d_components(self):
@@ -503,10 +504,7 @@ class Engine(object):
         self.run_serial += 1
         self._check(self.lib.ctr_mt3d_keep_components(self.h, _ptr(mask) if len(mask) else None, len(mask), ctypes.byref(nv),
                                                       ctypes.byref(nt)), "ctr_mt3d_keep_components")
-        flags, c = self._last3
-        c = type(c).from_buffer_copy(c)                                # the caller keeps the full scan's counts
-        c.n_verts, c.n_tris = int(nv.value), int(nt.value)             # what mt3d_fetch sizes its arrays from
-        self._last3 = (flags, c)
+        self._mesh_edited(nv.value, nt.value)
         self._comp_shape = (int(nt.value), int(mask.astype(bool).sum()))
         return int(nv.value), int(nt.value)
 
@@ -546,10 +544,7 @@ class Engine(object):
         c = DecimateCounts()
         self.run_serial += 1
         self._check(self.lib.ctr_mt3d_decimate(self.h, ctypes.byref(p), ctypes.byref(c)), "ctr_mt3d_decimate")
-        flags, c3 = self._last3
-        c3 = type(c3).from_buffer_copy(c3)                             # the caller keeps the full scan's counts
-        c3.n_verts, c3.n_tris = int(c.n_verts), int(c.n_tris)          # what mt3d_fetch sizes its arrays from
-        self._last3 = (flags, c3)
+        self._mesh_edited(c.n_verts, c.n_tris)
         return c
 
     def mt3d_interpolate(self, field, shape=None, dtype=None):

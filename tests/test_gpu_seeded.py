@@ -112,6 +112,30 @@ def test_many_seeds_and_no_seeds(engine):
     assert n_sel == n_full
 
 
+def test_select_keeps_the_vertex_id_base(engine):
+    """A run with vert_id_base B numbers its vertices from B: the selection compacts in that range, so it gives the
+    base-0 selection's mesh with every triangle id shifted by B."""
+    from contourist_b200 import engine as E
+    from contourist_b200 import tetrahedral
+    n, B = 30, 1000
+    x, y, z = np.meshgrid(*(np.arange(n, dtype=np.float64),) * 3, indexing="ij")
+    f = np.exp(-((x - 8) ** 2 + (y - 9) ** 2 + (z - 10) ** 2) / 12.0) + \
+        np.exp(-((x - 21) ** 2 + (y - 20) ** 2 + (z - 19) ** 2) / 10.0)
+    start = tetrahedral.initial_voxels(f, 0.5, [[(8, 9, 10), (8, 9, 0)]])
+    flags = E.WANT_KEYS | E.WANT_NORMALS | E.GEOM_F64
+    out = []
+    for base in (0, B):
+        full = engine.mt3d_run(f, 0.5, flags=flags, vert_id_base=base)
+        nv, nt, _ = engine.mt3d_select_seeded(start)
+        assert 0 < nt < int(full.n_tris)                        # the second blob is dropped
+        out.append(engine.mt3d_fetch())
+    a, b = out
+    for k in ("verts", "normals", "keys", "lowmin"):
+        assert np.array_equal(a[k], b[k])
+    assert b["tris"].min() >= B
+    assert np.array_equal(b["tris"], a["tris"] + B)
+
+
 def test_facade_two_dots_seeded_is_the_reference_known_answer(engine):
     """test_tetrahedral.py:13-37 at the grid level: only the seeded dot comes back (minus the two leak triangles)."""
     from contourist_b200 import tetrahedral
