@@ -52,6 +52,7 @@ enum Edit3 : unsigned {
   EDIT_KEEP = 4u,            // component filter
   EDIT_SMOOTH = 8u,          // smoothing
   EDIT_DECIMATE = 16u,       // decimation
+  EDIT_CAP = 32u,            // caps at the box faces
 };
 
 struct ctr_ctx {
@@ -93,6 +94,9 @@ struct ctr_ctx {
   unsigned char last3_params[160] = {};   // parameters of the last completed ctr_mt3d_run
   long long* publish3 = nullptr;          // ctr_mt3d_publish_counts: device {n_verts, n_tris} behind every 3D run
   unsigned last3_edited = 0;              // Edit3 bits of the passes that have rewritten the device mesh of that run
+  // ctr_mt3d_orient_reference has rewound that mesh: kept apart from last3_edited, which the seeded selection refuses
+  // (it accepts an oriented run); ctr_mt3d_cap refuses it (the rim no longer faces the high side)
+  bool last3_oriented = false;
   // bumped by every 3D run and every pass that removes or renumbers mesh rows (selection, clean-up, offset_ids,
   // component filter, decimation) or moves vertices (smoothing); the vertex values and the components below record the
   // generation they were computed on
@@ -159,6 +163,23 @@ static inline int ctr_ensure(ctr_ctx* ctx, DevBuf& b, size_t bytes, bool exact =
     return ctr_fail(ctx, CTR_ERR_OOM, m);
   }
   b.cap = want;
+  return 0;
+}
+
+// ctr_ensure for a buffer whose first `keep` bytes must survive: a larger buffer is allocated, the content copied over
+// on the device and the old buffer freed.  The buffer's address changes when it grows.
+static inline int ctr_grow_keep(ctr_ctx* ctx, DevBuf& b, size_t bytes, size_t keep) {
+  if (bytes <= b.cap && b.p) return 0;
+  DevBuf n;
+  if (int rc = ctr_ensure(ctx, n, bytes)) return rc;
+  cudaError_t e = keep ? cudaMemcpyAsync(n.p, b.p, keep, cudaMemcpyDeviceToDevice, ctx->stream) : cudaSuccess;
+  if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+  if (e != cudaSuccess) {
+    cudaFree(n.p);
+    CTR_CUDA(ctx, e);
+  }
+  cudaFree(b.p);
+  b = n;
   return 0;
 }
 

@@ -230,6 +230,7 @@ extern "C" int ctr_mt3d_orient_reference(ctr_ctx* ctx, int64_t* n_components, in
   if (!ctx) return CTR_ERR_BAD_ARG;
   if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
     return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to orient");
+  ctx->last3_oriented = true;                         // (also when the call fails below: it may have rewound a part)
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
   if (ctx->last_flags & CTR_GEOM_F64) return orient_typed<double>(ctx, n_components, n_flipped);
   return orient_typed<float>(ctx, n_components, n_flipped);

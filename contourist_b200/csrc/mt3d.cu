@@ -1660,6 +1660,7 @@ int run_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts* out, int 
   }
   ctx->last_kind = 3;
   ctx->last3_edited = 0;
+  ctx->last3_oriented = false;
   ctx->last_flags = p->flags;
   ctx->last_counts[0] = (int64_t)nV;
   ctx->last_counts[1] = (int64_t)totT;
@@ -1675,6 +1676,7 @@ int run_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts* out, int 
 #include "normals3d.cuh"
 #include "decimate3d.cuh"
 #include "attr3d.cuh"
+#include "cap3d.cuh"
 
 }  // namespace
 
@@ -1818,7 +1820,7 @@ extern "C" int ctr_mt3d_select_seeded(ctr_ctx* ctx, const int32_t* seed_voxels, 
   // the selection compacts the run's mesh in place while the voxel work list keeps its per-voxel triangle offsets: it
   // can be applied once per run
   if (ctx->last3_edited)
-    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has already been selected from, cleaned, filtered, smoothed or decimated; "
+    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has already been selected from, cleaned, filtered, smoothed, decimated or capped; "
                                         "run ctr_mt3d_run again");
   ctx->mesh_gen++;
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
@@ -1855,6 +1857,7 @@ extern "C" int ctr_mt3d_clean(ctr_ctx* ctx, const ctr_clean_params* cp, ctr_clea
   // the reference's clean-up (quantize, tiny simplices) is defined on the interpolated positions
   if (ctx->last3_edited & EDIT_SMOOTH) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has been smoothed: clean it up before smoothing");
   if (ctx->last3_edited & EDIT_DECIMATE) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has been decimated: clean it up before decimating");
+  if (ctx->last3_edited & EDIT_CAP) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has been capped: clean it up before capping");
   const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
   if (p->i_lo != 0 || p->i_hi != p->n0 || p->vert_id_base != 0)
     return ctr_fail(ctx, CTR_ERR_UNSUPPORTED, "mesh clean-up needs a full-volume run (merges cross slab faces)");
@@ -1888,6 +1891,39 @@ extern "C" int ctr_mt3d_decimate(ctr_ctx* ctx, const ctr_decimate_params* dp, ct
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
   if (ctx->last_flags & CTR_GEOM_F64) return decimate_typed<double>(ctx, dp, out);
   return decimate_typed<float>(ctx, dp, out);
+}
+
+template <typename T>
+static int cap_dispatch(ctr_ctx* ctx, const ctr_cap_params* cp, ctr_cap_counts* out) {
+  if (ctx->last_flags & CTR_GEOM_F64) return cap_typed<T, double>(ctx, cp, out);
+  return cap_typed<T, float>(ctx, cp, out);
+}
+
+extern "C" int ctr_mt3d_cap(ctr_ctx* ctx, const ctr_cap_params* cp, ctr_cap_counts* out) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (!cp || !out) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  memset(out, 0, sizeof *out);
+  if (cp->side != CTR_CAP_HIGH && cp->side != CTR_CAP_LOW) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "side must be CTR_CAP_HIGH or CTR_CAP_LOW");
+  if (cp->reserved != 0) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "reserved must be 0");
+  if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
+    return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to cap");
+  if (!(ctx->last_flags & CTR_WANT_KEYS)) return ctr_fail(ctx, CTR_ERR_STATE, "the run did not keep its keys: run with CTR_WANT_KEYS");
+  const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
+  if (p->i_lo != 0 || p->i_hi != p->n0 || p->plane_offset != 0 || p->vert_id_base != 0)
+    return ctr_fail(ctx, CTR_ERR_STATE, "caps need a full-volume run with plane_offset 0 and vert_id_base 0 (the box of a slab is not the volume's)");
+  // after these passes the field no longer tells where the mesh's rim is or which way it faces: cap first
+  if ((ctx->last3_edited & ~(unsigned)EDIT_SMOOTH) || ctx->last3_oriented)
+    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has been selected from, cleaned, filtered, decimated, oriented or capped: "
+                                        "cap it before those passes");
+  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
+  switch (p->dtype) {
+    case CTR_F32: return cap_dispatch<float>(ctx, cp, out);
+    case CTR_F64: return cap_dispatch<double>(ctx, cp, out);
+    case CTR_U8: return cap_dispatch<uint8_t>(ctx, cp, out);
+    case CTR_I16: return cap_dispatch<int16_t>(ctx, cp, out);
+    case CTR_U16: return cap_dispatch<uint16_t>(ctx, cp, out);
+  }
+  return ctr_fail(ctx, CTR_ERR_BAD_ARG, "unknown dtype");
 }
 
 extern "C" int ctr_mt3d_interpolate(ctr_ctx* ctx, const ctr_attr_params* a, int64_t* n_verts) {

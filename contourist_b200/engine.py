@@ -104,6 +104,18 @@ class DecimateCounts(ctypes.Structure):
                 ("n_collapsed", ctypes.c_int64), ("n_duplicate", ctypes.c_int64)]
 
 
+class CapParams(ctypes.Structure):
+    _fields_ = [("side", ctypes.c_int32), ("reserved", ctypes.c_uint32)]
+
+
+class CapCounts(ctypes.Structure):
+    _fields_ = [("n_verts", ctypes.c_int64), ("n_tris", ctypes.c_int64), ("n_cap_verts", ctypes.c_int64),
+                ("n_cap_tris", ctypes.c_int64), ("n_missing", ctypes.c_int64)]
+
+
+CAP_SIDES = {"high": 0, "low": 1}
+
+
 class PolyCounts(ctypes.Structure):
     _fields_ = [("n_polylines", ctypes.c_int64), ("n_points", ctypes.c_int64), ("junction_levels", ctypes.c_uint64)]
 
@@ -172,6 +184,8 @@ def load_library():
     lib.ctr_mt3d_smooth.restype = i32
     lib.ctr_mt3d_decimate.argtypes = [vp, ctypes.POINTER(DecimateParams), ctypes.POINTER(DecimateCounts)]
     lib.ctr_mt3d_decimate.restype = i32
+    lib.ctr_mt3d_cap.argtypes = [vp, ctypes.POINTER(CapParams), ctypes.POINTER(CapCounts)]
+    lib.ctr_mt3d_cap.restype = i32
     lib.ctr_mt3d_interpolate.argtypes = [vp, ctypes.POINTER(AttrParams), ctypes.POINTER(i64)]
     lib.ctr_mt3d_interpolate.restype = i32
     lib.ctr_mt3d_interpolate_fetch.argtypes = [vp, vp]
@@ -544,6 +558,25 @@ class Engine(object):
         c = DecimateCounts()
         self.run_serial += 1
         self._check(self.lib.ctr_mt3d_decimate(self.h, ctypes.byref(p), ctypes.byref(c)), "ctr_mt3d_decimate")
+        self._mesh_edited(c.n_verts, c.n_tris)
+        return c
+
+    def mt3d_cap(self, side):
+        """Close the last 3D run's device mesh at the faces of the volume's box (ctr_mt3d_cap; oracle/mt3d_cap.py is the
+        definition): side "high" closes the region f >= value, "low" the region f < value.  On every box face the part
+        of each face triangle of the tetrahedral grid on that side is appended; its rim vertices are the surface's own,
+        and the box-surface grid points it uses become new vertices (key lin * 8 + 0), so the region's boundary is
+        closed.  The run needs WANT_KEYS; accepted on the mesh as extracted or smoothed (smooth first for flat caps),
+        refused after a selection, clean-up, component filter, decimation, orientation or an earlier cap.  Device
+        pointers must be taken again afterwards.  Returns CapCounts (n_verts, n_tris, n_cap_verts, n_cap_tris,
+        n_missing); fetch afterwards."""
+        if side not in CAP_SIDES:
+            raise ValueError("side must be 'high' or 'low', not %r" % (side,))
+        p = CapParams()
+        p.side = CAP_SIDES[side]
+        c = CapCounts()
+        self.run_serial += 1
+        self._check(self.lib.ctr_mt3d_cap(self.h, ctypes.byref(p), ctypes.byref(c)), "ctr_mt3d_cap")
         self._mesh_edited(c.n_verts, c.n_tris)
         return c
 

@@ -158,6 +158,13 @@ class GridContour3d(object):
     # decimated mesh.  `flatten` (the reference's LP-based collapse_flat_segments) is a different algorithm and still
     # raises.
     decimate_cell = None
+    # cap = "high" / "low" (with post_process = False, on a full scan): get_points_and_triangles() closes the surface at
+    # the faces of the volume's box on the device (ctr_mt3d_cap), right after the run and before the reference
+    # orientation, the component filter, smoothing, decimation, vertex_fields and measure_components: the region
+    # f >= value ("high") or f < value ("low") then has a closed boundary, and its components are enclosed volumes.
+    # Smoothing after the cap rounds the box edges (the cap's rim vertices are no longer fixed); Engine users who want
+    # flat caps smooth first, then cap.
+    cap = None
 
     def __init__(self, corner, function, value, segment_endpoints, linear_interpolate=True, callback=None,
                  origin=(0.0, 0.0, 0.0), delta=(1.0, 1.0, 1.0)):
@@ -206,8 +213,18 @@ class GridContour3d(object):
             raise NotImplementedError("flatten / smooth (LP-based decimation, tetrahedral.py:217-351) are out of scope")
         eng = E.default_engine()
         flags = (E.GEOM_F64 if np.dtype(self.geometry_dtype) == np.float64 else 0) | (E.WANT_NORMALS if self.want_normals else 0)
-        if self.vertex_fields is not None:
-            flags |= E.WANT_KEYS                          # the values are interpolated along the vertices' keys
+        if self.vertex_fields is not None or self.cap is not None:
+            flags |= E.WANT_KEYS                          # the values are interpolated, the rim found, along the keys
+        seeded = not self.full_scan and self.end_points is not None
+        if self.cap is not None:
+            if self.cap not in E.CAP_SIDES:
+                raise ValueError("cap must be None, 'high' or 'low', not %r" % (self.cap,))
+            if self.post_process:
+                raise ValueError("cap needs post_process = False: the reference's post-processing would merge and rewind "
+                                 "the capped mesh")
+            if seeded:
+                raise ValueError("cap needs a full scan: a seeded selection keeps part of the surface, whose rim the caps "
+                                 "would not meet")
         field = self._field()
         identity = tuple(float(x) for x in self.origin) == (0.0, 0.0, 0.0) and tuple(float(x) for x in self.delta) == (1.0, 1.0, 1.0)
         # with post-processing the run is made in grid coordinates and ctr_mt3d_clean applies the transform last, like
@@ -220,11 +237,14 @@ class GridContour3d(object):
             self.counts = pre[3]                          # search_for_endpoints() made this very run: nothing to redo
         else:
             self.counts = eng.mt3d_run(field, self.value, origin=run_origin, delta=run_delta, flags=flags)
-        if not self.full_scan and self.end_points is not None:
+        if seeded:
             # seeded tracking: only what the flood fill reaches from the seeds' start voxels (no seeds: nothing)
             self.start_voxels = initial_voxels(field, self.value, self.end_points) if len(self.end_points) else \
                 np.zeros((0, 3), np.int32)
             self.selected = eng.mt3d_select_seeded(self.start_voxels)
+        if self.cap is not None:
+            # on the mesh as extracted: the field still tells where its rim is and which way it faces
+            self.capped = eng.mt3d_cap(self.cap)
         if self.post_process:
             # tetrahedral.py:541-552 on the device mesh: quantize, tiny, clean (if asked), orient, grid -> world
             self.cleaned = eng.mt3d_clean(self.corner, origin=self.origin, delta=self.delta, divisions=self.quantize_divisions,
@@ -315,7 +335,7 @@ class Delta3DContour(object):
         "options set on this driver (before or after the maker was built) reach the maker"
         for name in ("post_process", "geometry_dtype", "want_normals", "reference_orientation", "quantize_divisions",
                      "tiny_epsilon", "vertex_fields", "measure_components", "keep_components", "smooth_iterations",
-                     "smooth_lambda", "smooth_mu", "decimate_cell"):
+                     "smooth_lambda", "smooth_mu", "decimate_cell", "cap"):
             if hasattr(self, name):
                 setattr(maker, name, getattr(self, name))
         maker.field_grid = self.grid

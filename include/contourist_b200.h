@@ -184,7 +184,8 @@ CTR_API int ctr_mt3d_orient_reference(ctr_ctx* ctx, int64_t* n_components, int64
  *     closed component has volume > 0 when the region it encloses is below the isovalue and < 0 when it is above (a
  *     blob brighter than its surroundings: negative).  After ctr_mt3d_orient_reference, or ctr_mt3d_clean with
  *     CTR_CLEAN_ORIENT, every closed component faces outward and its volume is >= 0.  For an open component the value
- *     is reported but is not an enclosed volume.
+ *     is reported but is not an enclosed volume.  After ctr_mt3d_cap the components that the box cut are closed by
+ *     their caps, so their volumes are enclosed volumes too.
  *   - The integer fields, first_tri and the box are exact.  area and volume are sums whose order may change between
  *     calls: their last bits may differ.
  *   - CTR_ERR_STATE: no 3D run or a CTR_NO_GEOMETRY run; a slab run (i_lo != 0 or i_hi != n0) or vert_id_base != 0; a
@@ -317,6 +318,57 @@ typedef struct {
   int64_t n_duplicate;                       /* triangles dropped because an earlier kept triangle has the same three clusters */
 } ctr_decimate_counts;                       /* 40 bytes */
 CTR_API int ctr_mt3d_decimate(ctr_ctx* ctx, const ctr_decimate_params* p, ctr_decimate_counts* out);
+
+/* Caps that close the LAST 3D run's device mesh at the faces of the volume's box (engine extension: a surface cut by the
+ * box otherwise ends there in a rim of boundary edges; oracle/mt3d_cap.py:cap is the definition).  The mesh is
+ * extended in place; synchronous on return.
+ *   - side CTR_CAP_HIGH closes the region f >= isovalue (the side the triangles and normals face), CTR_CAP_LOW the
+ *     region f < isovalue ("low" is the extraction's strict f < isovalue).
+ *   - With the Kuhn decomposition each box face square with minimum corner m and in-face axes a < b is cut along its
+ *     min -> max diagonal into the face triangles (m, m + e_a, m + e_a + e_b) and (m, m + e_b, m + e_a + e_b).  The cap
+ *     is the part of every face triangle on the chosen side: the whole triangle, a corner and its two crossings, or a
+ *     quad split by the fan from its first vertex (corners and crossings listed in the face triangle's corner order).
+ *     Its rim vertices are the surface's own crossing vertices, found by edge key: the rim is shared exactly.
+ *   - Cap triangles face into the box for CTR_CAP_HIGH and out of it for CTR_CAP_LOW (in grid coordinates), so every rim
+ *     edge is crossed in opposite directions by its surface and cap triangles.
+ *   - New vertices: one per box-surface grid point that some cap triangle uses (the faces share those on box edges and
+ *     corners), appended after the existing vertices in ascending key order.  Key lin*8 + 0: d = 0 names the grid
+ *     point itself, and ctr_mt3d_interpolate gives exactly the attribute's sample there.  lowmin 1 when the point is
+ *     low.  Position grid*delta + origin, rounded per operation in the geometry type as the extraction's.  Normal
+ *     (CTR_WANT_NORMALS) the normalised sum of the unit world normals of the cap triangles of the box faces the point
+ *     lies on.  Existing vertices keep their rows.
+ *   - New triangles are appended after the existing ones, by face (axis 0 lo, axis 0 hi, axis 1 lo, ..., axis 2 hi),
+ *     then face square (row-major over (a, b)), then face triangle, then piece.
+ *   - A face triangle whose crossing vertex is not in the mesh adds nothing and counts in n_missing: the surface has a
+ *     gap there (a tetrahedron skipped by allclose).  Not watertight either: a face sample exactly equal to the
+ *     isovalue gives a crossing vertex at ratio 1 that is not merged with the cap's grid vertex at the same position.
+ *     Otherwise every edge of the capped mesh is used by exactly two triangles.
+ *   - Accepted on the mesh as extracted and after ctr_mt3d_smooth, which keeps the triangles, the keys and the rim's
+ *     positions bit for bit: smooth, then cap, gives flat caps.  Also after ctr_mt3d_interpolate and
+ *     ctr_mt3d_components, whose results then become stale.
+ *   - Afterwards: the published counts, cells and codes stay those of the run; the output buffers may have been
+ *     reallocated, so take device pointers (ctr_mt3d_device_ptrs) again.  Component results and vertex values are
+ *     stale.  ctr_mt3d_select_seeded and ctr_mt3d_clean return CTR_ERR_STATE; ctr_mt3d_components,
+ *     ctr_mt3d_keep_components (after measuring again), ctr_mt3d_smooth (which then rounds the box edges),
+ *     ctr_mt3d_decimate, ctr_mt3d_interpolate and ctr_mt3d_orient_reference are accepted.
+ *   - CTR_ERR_BAD_ARG: a NULL argument, side not CTR_CAP_HIGH / CTR_CAP_LOW, reserved != 0.  CTR_ERR_STATE: no 3D run or
+ *     a CTR_NO_GEOMETRY run; a run without CTR_WANT_KEYS; a slab run (i_lo != 0, i_hi != n0 or plane_offset != 0) or
+ *     vert_id_base != 0; a triangle id outside [0, n_verts) (e.g. after ctr_mt3d_offset_ids); a mesh already selected
+ *     from, cleaned, filtered, decimated, oriented or capped (the field no longer tells where its rim is or which way it
+ *     faces: cap first).  CTR_ERR_OVERFLOW: 2^31 or more vertices or triangles after capping.  All are detected before
+ *     anything is written.                                                                                              */
+#define CTR_CAP_HIGH 0
+#define CTR_CAP_LOW 1
+typedef struct {
+  int32_t side;       /* CTR_CAP_HIGH or CTR_CAP_LOW */
+  uint32_t reserved;  /* 0 */
+} ctr_cap_params;                            /* 8 bytes */
+typedef struct {
+  int64_t n_verts, n_tris;                   /* the capped mesh                                                       */
+  int64_t n_cap_verts, n_cap_tris;           /* added by the caps                                                     */
+  int64_t n_missing;                         /* face triangles left open because a crossing vertex is not in the mesh */
+} ctr_cap_counts;                            /* 40 bytes */
+CTR_API int ctr_mt3d_cap(ctr_ctx* ctx, const ctr_cap_params* p, ctr_cap_counts* out);
 
 /* Seeded extraction (SURVEY.md 8(f3)): restricts the LAST full-volume run's mesh to what the reference's tracker
  *   tetrahedral.py:443-469  expand_voxels / in_range  (flood fill over the 26-neighbourhood of border voxels)
