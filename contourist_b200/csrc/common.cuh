@@ -43,6 +43,8 @@ enum Aux3 : int {
   AUX_VALUES = 43,           // vertex values (ctr_mt3d_interpolate)
   AUX_LABELS = 44,           // component of every triangle (ctr_mt3d_components)
   AUX_COMPONENTS = 45,       // component table
+  AUX_SECTION_SEGS = 1,      // plane sections (ctr_mt3d_section): segments and junction planes
+  AUX_SECTION_POLYS = 3,     // ... polylines, their points and measures
 };
 
 // ctr_ctx::last3_edited: the passes that have rewritten the device mesh of the last 3D run
@@ -116,8 +118,12 @@ struct ctr_ctx {
   // since the last 3D run
   int64_t comp_tris = 0, comp_count = -1;
   uint64_t comp_gen = 0;
+  // 3D plane sections (ctr_mt3d_section) in AUX_SECTION_SEGS / AUX_SECTION_POLYS: segments (-1 = none since the last 3D
+  // run), polylines, points, junction planes; and the number of planes
+  int64_t sect_count[4] = {-1, 0, 0, 0};
+  int32_t sect_nplanes = 0;
 
-  // extra outputs and scratch in generic slots: 3D (Aux3 above, 1 and 3 unused); 5-10: 2D; 12-26: 4D; 36-40: 2D polylines
+  // extra outputs and scratch in generic slots: 3D (Aux3 above); 5-10: 2D; 12-26: 4D; 36-40: 2D polylines
   DevBuf aux[48];
 };
 

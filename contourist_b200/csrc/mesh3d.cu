@@ -13,6 +13,7 @@
 // Components are joined through shared EDGES, as in the reference (two sheets touching in one vertex stay apart).
 // components3d.cuh (ctr_mt3d_components) reuses the edge table and k_o_union to number and measure the components.
 // smooth3d.cuh (ctr_mt3d_smooth) builds the same edge table with its use counts for the fixed vertices and neighbour lists.
+// section3d.cuh (ctr_mt3d_section) names the crossing vertices of its plane sections by their slots in that table.
 #include <math.h>
 #include <string.h>
 
@@ -223,6 +224,7 @@ int orient_typed(ctr_ctx* ctx, int64_t* n_components, int64_t* n_flipped) {
 #include "normals3d.cuh"
 #include "components3d.cuh"
 #include "smooth3d.cuh"
+#include "section3d.cuh"
 
 }  // namespace
 
@@ -279,5 +281,77 @@ extern "C" int ctr_mt3d_components_fetch(ctr_ctx* ctx, int32_t* tri_component, c
     CTR_CUDA(ctx, cudaMemcpyAsync(components, ctx->aux[AUX_COMPONENTS].p, (size_t)ctx->comp_count * sizeof(ctr_mt3d_component),
                                   cudaMemcpyDeviceToHost, ctx->stream));
   CTR_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return 0;
+}
+
+extern "C" int ctr_mt3d_section(ctr_ctx* ctx, const ctr_section_params* sp, ctr_section_counts* out) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (!sp || !out || !sp->offsets) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  memset(out, 0, sizeof *out);
+  const double* n = sp->normal;
+  if (!(isfinite(n[0]) && isfinite(n[1]) && isfinite(n[2])) || (n[0] == 0.0 && n[1] == 0.0 && n[2] == 0.0))
+    return ctr_fail(ctx, CTR_ERR_BAD_ARG, "normal must be finite and not zero");
+  if (sp->nplanes < 1 || sp->nplanes > 65536) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "nplanes must be in [1, 65536]");
+  if (sp->reserved != 0) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "reserved must be 0");
+  for (int32_t l = 0; l < sp->nplanes; ++l)
+    if (!isfinite(sp->offsets[l]) || (l > 0 && !(sp->offsets[l] > sp->offsets[l - 1])))
+      return ctr_fail(ctx, CTR_ERR_BAD_ARG, "offsets must be finite and strictly increasing");
+  ctx->sect_count[0] = -1;                            // the buffers are rewritten: earlier results are gone
+  if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
+    return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to cut");
+  const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
+  if (p->i_lo != 0 || p->i_hi != p->n0 || p->vert_id_base != 0)
+    return ctr_fail(ctx, CTR_ERR_STATE, "sections need a full-volume run with vert_id_base 0 (a slab's halo ids belong to another shard)");
+  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
+  if (ctx->last_flags & CTR_GEOM_F64) return section_typed<double>(ctx, sp, out);
+  return section_typed<float>(ctx, sp, out);
+}
+
+extern "C" int ctr_mt3d_section_segments_fetch(ctr_ctx* ctx, int32_t* plane, int32_t* edges, void* points) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (ctx->last_kind != 3 || ctx->sect_count[0] < 0) return ctr_fail(ctx, CTR_ERR_STATE, "no ctr_mt3d_section since the last 3D run");
+  const size_t S = (size_t)ctx->sect_count[0], gsz = (ctx->last_flags & CTR_GEOM_F64) ? 8 : 4;
+  if (!S) return 0;
+  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  SecSegs sg;
+  ctr_carve c{(char*)ctx->aux[AUX_SECTION_SEGS].p, 0};
+  sg.carve(c, S, gsz, (size_t)ctx->sect_nplanes);
+  if (plane) CTR_CUDA(ctx, cudaMemcpyAsync(plane, sg.plane, S * 4, cudaMemcpyDeviceToHost, st));
+  if (edges) CTR_CUDA(ctx, cudaMemcpyAsync(edges, sg.edges, S * 16, cudaMemcpyDeviceToHost, st));
+  if (points) CTR_CUDA(ctx, cudaMemcpyAsync(points, sg.pts, S * 6 * gsz, cudaMemcpyDeviceToHost, st));
+  CTR_CUDA(ctx, cudaStreamSynchronize(st));
+  return 0;
+}
+
+extern "C" int ctr_mt3d_section_polylines_fetch(ctr_ctx* ctx, int32_t* plane, uint8_t* flags, uint64_t* start_key, uint32_t* offset,
+                                                uint32_t* length, double* measures, void* points, uint8_t* junction) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (ctx->last_kind != 3 || ctx->sect_count[0] < 0) return ctr_fail(ctx, CTR_ERR_STATE, "no ctr_mt3d_section since the last 3D run");
+  const size_t S = (size_t)ctx->sect_count[0], P = (size_t)ctx->sect_count[1], N = (size_t)ctx->sect_count[2];
+  const size_t np = (size_t)ctx->sect_nplanes, gsz = (ctx->last_flags & CTR_GEOM_F64) ? 8 : 4;
+  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  std::vector<uint32_t> jp(junction ? np : 0);
+  if (junction) {
+    SecSegs sg;
+    ctr_carve c{(char*)ctx->aux[AUX_SECTION_SEGS].p, 0};
+    sg.carve(c, S, gsz, np);
+    CTR_CUDA(ctx, cudaMemcpyAsync(jp.data(), sg.jplane, np * 4, cudaMemcpyDeviceToHost, st));
+  }
+  if (P) {
+    SecPolys pg;
+    ctr_carve c{(char*)ctx->aux[AUX_SECTION_POLYS].p, 0};
+    pg.carve(c, P, N, gsz);
+    if (plane) CTR_CUDA(ctx, cudaMemcpyAsync(plane, pg.plane, P * 4, cudaMemcpyDeviceToHost, st));
+    if (flags) CTR_CUDA(ctx, cudaMemcpyAsync(flags, pg.flags, P, cudaMemcpyDeviceToHost, st));
+    if (start_key) CTR_CUDA(ctx, cudaMemcpyAsync(start_key, pg.key, P * 8, cudaMemcpyDeviceToHost, st));
+    if (offset) CTR_CUDA(ctx, cudaMemcpyAsync(offset, pg.off, P * 4, cudaMemcpyDeviceToHost, st));
+    if (length) CTR_CUDA(ctx, cudaMemcpyAsync(length, pg.len, P * 4, cudaMemcpyDeviceToHost, st));
+    if (measures) CTR_CUDA(ctx, cudaMemcpyAsync(measures, pg.meas, P * 16, cudaMemcpyDeviceToHost, st));
+    if (points && N) CTR_CUDA(ctx, cudaMemcpyAsync(points, pg.pts, N * 3 * gsz, cudaMemcpyDeviceToHost, st));
+  }
+  CTR_CUDA(ctx, cudaStreamSynchronize(st));
+  for (size_t l = 0; l < jp.size(); ++l) junction[l] = jp[l] ? 1 : 0;
   return 0;
 }

@@ -1703,6 +1703,7 @@ static int mt3d_dispatch(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts
   ctx->mesh_gen++;
   ctx->attr_ncomp = 0;                                 // vertex values of the previous run are gone
   ctx->comp_count = -1;                                // ... and so are its components
+  ctx->sect_count[0] = -1;                             // ... and its plane sections
   switch (p->dtype) {
     case CTR_F32: return run_typed<float>(ctx, p, out, phase);
     case CTR_F64: return run_typed<double>(ctx, p, out, phase);

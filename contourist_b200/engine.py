@@ -116,6 +116,16 @@ class CapCounts(ctypes.Structure):
 CAP_SIDES = {"high": 0, "low": 1}
 
 
+class SectionParams(ctypes.Structure):
+    _fields_ = [("normal", ctypes.c_double * 3), ("offsets", ctypes.c_void_p), ("nplanes", ctypes.c_int32),
+                ("reserved", ctypes.c_uint32)]
+
+
+class SectionCounts(ctypes.Structure):
+    _fields_ = [("n_segments", ctypes.c_int64), ("n_polylines", ctypes.c_int64), ("n_points", ctypes.c_int64),
+                ("n_junction_planes", ctypes.c_int64)]
+
+
 class PolyCounts(ctypes.Structure):
     _fields_ = [("n_polylines", ctypes.c_int64), ("n_points", ctypes.c_int64), ("junction_levels", ctypes.c_uint64)]
 
@@ -186,6 +196,12 @@ def load_library():
     lib.ctr_mt3d_decimate.restype = i32
     lib.ctr_mt3d_cap.argtypes = [vp, ctypes.POINTER(CapParams), ctypes.POINTER(CapCounts)]
     lib.ctr_mt3d_cap.restype = i32
+    lib.ctr_mt3d_section.argtypes = [vp, ctypes.POINTER(SectionParams), ctypes.POINTER(SectionCounts)]
+    lib.ctr_mt3d_section.restype = i32
+    lib.ctr_mt3d_section_segments_fetch.argtypes = [vp] * 4
+    lib.ctr_mt3d_section_segments_fetch.restype = i32
+    lib.ctr_mt3d_section_polylines_fetch.argtypes = [vp] * 9
+    lib.ctr_mt3d_section_polylines_fetch.restype = i32
     lib.ctr_mt3d_interpolate.argtypes = [vp, ctypes.POINTER(AttrParams), ctypes.POINTER(i64)]
     lib.ctr_mt3d_interpolate.restype = i32
     lib.ctr_mt3d_interpolate_fetch.argtypes = [vp, vp]
@@ -579,6 +595,43 @@ class Engine(object):
         self._check(self.lib.ctr_mt3d_cap(self.h, ctypes.byref(p), ctypes.byref(c)), "ctr_mt3d_cap")
         self._mesh_edited(c.n_verts, c.n_tris)
         return c
+
+    def mt3d_section(self, normal, offsets):
+        """Sections of the last 3D run's device mesh as it stands now with the planes {x : normal . x == offsets[l]}
+        (ctr_mt3d_section; oracle/mt3d_section.py is the definition), `offsets` strictly increasing, in the units of
+        the current positions.  The mesh is not edited.  Returns (segments, polylines):
+          segments  = dict(plane [S] int32, edges [S, 2, 2] int32 (vertex-id pairs (min, max), start edge first),
+                      points [S, 2, 3] in the geometry type), by triangle, then plane;
+          polylines = one list per plane of (closed, consistent, points [k, 3], length, area), open ones first, then by
+                      start key, or None for a junction plane (one that crosses a non-manifold edge: its segments are
+                      not chained).  An outward-oriented closed surface gives counter-clockwise sections seen from
+                      +normal, with area > 0 (the raw mesh is wound towards the high side)."""
+        n = np.asarray(normal, np.float64).reshape(3)
+        off = np.ascontiguousarray(np.asarray(offsets, np.float64).reshape(-1))
+        p = SectionParams()
+        for a in range(3):
+            p.normal[a] = float(n[a])
+        p.offsets = off.ctypes.data if len(off) else None
+        p.nplanes = len(off)
+        c = SectionCounts()
+        self._check(self.lib.ctr_mt3d_section(self.h, ctypes.byref(p), ctypes.byref(c)), "ctr_mt3d_section")
+        flags, _ = self._last3
+        gd = np.float64 if flags & GEOM_F64 else np.float32
+        S, P, N = int(c.n_segments), int(c.n_polylines), int(c.n_points)
+        seg = dict(plane=np.empty(S, np.int32), edges=np.empty((S, 2, 2), np.int32), points=np.empty((S, 2, 3), gd))
+        self._check(self.lib.ctr_mt3d_section_segments_fetch(self.h, _ptr(seg["plane"]), _ptr(seg["edges"]),
+                                                             _ptr(seg["points"])), "ctr_mt3d_section_segments_fetch")
+        plane, fl, key = np.empty(P, np.int32), np.empty(P, np.uint8), np.empty(P, np.uint64)
+        o, ln, meas = np.empty(P, np.uint32), np.empty(P, np.uint32), np.empty((P, 2), np.float64)
+        pts, junction = np.empty((N, 3), gd), np.empty(len(off), np.uint8)
+        self._check(self.lib.ctr_mt3d_section_polylines_fetch(self.h, _ptr(plane), _ptr(fl), _ptr(key), _ptr(o), _ptr(ln),
+                                                              _ptr(meas), _ptr(pts), _ptr(junction)),
+                    "ctr_mt3d_section_polylines_fetch")
+        out = [None if junction[l] else [] for l in range(len(off))]
+        for q in np.lexsort((key, fl & 1, plane)):
+            out[int(plane[q])].append((bool(fl[q] & 1), bool(fl[q] & 2), pts[int(o[q]):int(o[q]) + int(ln[q])],
+                                       float(meas[q, 0]), float(meas[q, 1])))
+        return seg, out
 
     def mt3d_interpolate(self, field, shape=None, dtype=None):
         """Values of another field at the vertices of the last 3D run's mesh as it stands now (after a selection or

@@ -165,6 +165,12 @@ class GridContour3d(object):
     # Smoothing after the cap rounds the box edges (the cap's rim vertices are no longer fixed); Engine users who want
     # flat caps smooth first, then cap.
     cap = None
+    # sections = (normal, offsets) in world units: get_points_and_triangles() then cuts the returned mesh with the planes
+    # {x : normal . x == offsets[l]} on the device (ctr_mt3d_section), after every other pass, and leaves in
+    # section_polylines one list per plane of (closed, consistent, points, length, area), or None for a plane through a
+    # non-manifold edge
+    sections = None
+    section_polylines = None
 
     def __init__(self, corner, function, value, segment_endpoints, linear_interpolate=True, callback=None,
                  origin=(0.0, 0.0, 0.0), delta=(1.0, 1.0, 1.0)):
@@ -280,6 +286,9 @@ class GridContour3d(object):
             self.triangle_components, self.component_table = \
                 eng.mt3d_components_fetch() if self.keep_components is not None and not (smoothed or decimated) \
                 else eng.mt3d_components()
+        if self.sections is not None:
+            normal, offsets = self.sections
+            self.section_polylines = eng.mt3d_section(normal, offsets)[1]
         out = eng.mt3d_fetch()
         self.normals = out["normals"]
         points, triangles = out["verts"], out["tris"]
@@ -335,7 +344,7 @@ class Delta3DContour(object):
         "options set on this driver (before or after the maker was built) reach the maker"
         for name in ("post_process", "geometry_dtype", "want_normals", "reference_orientation", "quantize_divisions",
                      "tiny_epsilon", "vertex_fields", "measure_components", "keep_components", "smooth_iterations",
-                     "smooth_lambda", "smooth_mu", "decimate_cell", "cap"):
+                     "smooth_lambda", "smooth_mu", "decimate_cell", "cap", "sections"):
             if hasattr(self, name):
                 setattr(maker, name, getattr(self, name))
         maker.field_grid = self.grid
@@ -353,6 +362,7 @@ class Delta3DContour(object):
         self.vertex_values = maker.vertex_values       # values of vertex_fields (when set) at the returned points
         self.triangle_components = maker.triangle_components   # with measure_components: aligned with the triangles
         self.component_table = maker.component_table
+        self.section_polylines = maker.section_polylines
         return result
 
 

@@ -370,6 +370,57 @@ typedef struct {
 } ctr_cap_counts;                            /* 40 bytes */
 CTR_API int ctr_mt3d_cap(ctr_ctx* ctx, const ctr_cap_params* p, ctr_cap_counts* out);
 
+/* Sections of the LAST 3D run's device mesh as it stands now (after a selection, clean-up, orientation, component filter,
+ * smoothing, decimation or cap too) with a stack of parallel planes (engine extension, like VTK's vtkCutter on polydata;
+ * oracle/mt3d_section.py:section is the definition).  Reads the mesh only; synchronous on return.
+ *   - Plane l is {x : n . x == offsets[l]}, n as given.  A vertex is high for plane l when s = (n0 x + n1 y) + n2 z >=
+ *     offsets[l] and low otherwise (fp64 on positions widened from the geometry type, each operation rounded on its own):
+ *     the extraction's strict rule, so no vertex is ever on a plane.
+ *   - A triangle whose corners are not all on one side of plane l gives one segment.  Its two crossing edges are
+ *     {a, b} with a the low end: t = (d - s_a) / (s_b - s_a), p = p_a + t * (p_b - p_a) per axis, fp64, rounded once to
+ *     the geometry type, so both triangles on an edge give the same point.  The segment runs from the crossing on the
+ *     edge the corner walk takes from high to low to the one on the edge it takes from low to high: along n x (triangle
+ *     normal).  Seen from +n an outward-oriented closed surface gives counter-clockwise sections; the raw engine mesh
+ *     (wound towards the high side) runs clockwise around a region above the isovalue.
+ *   - Segments come by triangle, then plane; each has its plane, its two crossing edges as vertex-id pairs (min, max),
+ *     start edge first, and its two points.
+ *   - Polylines: the vertices are the pairs (plane, undirected edge); segments are chained by the rules of
+ *     ctr_mt2d_polylines without its allclose dedupe.  An open chain starts at its smaller end key, a closed one at its
+ *     smallest key towards the smaller neighbour (edge key a << 32 | b; a closed chain of two segments between the same
+ *     two vertices runs along its first segment).  When the first segment then runs from its point 1 to its point 0 the
+ *     polyline is reversed: an open one starts at its other end, a closed one keeps its first point and lists the rest
+ *     in reverse.  Flags: bit 0 closed, bit 1 consistent (every segment runs from point i to point i + 1, the closing one
+ *     included; a consistently wound manifold mesh gives consistent polylines).  start_key: the edge key of point 0.
+ *     Measures in fp64 from the output points: length (the closing segment included), and area
+ *     1/2 sum ((p_i - p_0) x (p_{i+1} - p_0)) . n / |n| (reported for open polylines too, where it encloses nothing;
+ *     both are sums in an unspecified order, equal to the definition within rounding).  Polylines come in no particular
+ *     order; their points are contiguous from offset.
+ *   - Junction planes: a plane that crosses an edge used by three or more triangles (a crossing vertex on three or more
+ *     segments) has junction[l] = 1 and none of its segments is chained; the segments are still returned.  A segment
+ *     whose two crossing edges are one edge (a triangle with a repeated vertex) is returned and not chained.
+ *   - The call edits nothing: the mesh, its generation, component results, vertex values and device pointers are
+ *     untouched, and every other pass accepts the mesh as before.  The results are those of this call until the next
+ *     call or 3D run.
+ *   - CTR_ERR_BAD_ARG: a NULL argument, a zero or non-finite normal, nplanes outside [1, 65536], offsets not finite or
+ *     not strictly increasing, reserved != 0.  CTR_ERR_STATE: no 3D run or a CTR_NO_GEOMETRY run; a slab run (i_lo != 0
+ *     or i_hi != n0) or vert_id_base != 0; a triangle id outside [0, n_verts) (e.g. after ctr_mt3d_offset_ids); a _fetch
+ *     with no ctr_mt3d_section since the last run.  CTR_ERR_OVERFLOW: 2^31 or more segments or points.  All are detected
+ *     before anything is written.  An empty mesh gives zero counts.
+ *   _section_segments_fetch : plane [S], edges [S][2][2], points [S][2][3] in the geometry type;
+ *   _section_polylines_fetch: plane, flags, start_key, offset, length, measures [P][2] (length, area) per polyline,
+ *                             points [N][3] in the geometry type, junction [nplanes].  Any pointer may be NULL.       */
+typedef struct {
+  double normal[3];          /* finite, not zero                                                                       */
+  const double* offsets;     /* host, nplanes values, strictly increasing, in the units of the current positions       */
+  int32_t nplanes;           /* 1..65536                                                                               */
+  uint32_t reserved;         /* 0                                                                                      */
+} ctr_section_params;                        /* 40 bytes */
+typedef struct { int64_t n_segments, n_polylines, n_points, n_junction_planes; } ctr_section_counts;   /* 32 bytes */
+CTR_API int ctr_mt3d_section(ctr_ctx* ctx, const ctr_section_params* p, ctr_section_counts* out);
+CTR_API int ctr_mt3d_section_segments_fetch(ctr_ctx* ctx, int32_t* plane, int32_t* edges, void* points);
+CTR_API int ctr_mt3d_section_polylines_fetch(ctr_ctx* ctx, int32_t* plane, uint8_t* flags, uint64_t* start_key, uint32_t* offset,
+                                             uint32_t* length, double* measures, void* points, uint8_t* junction);
+
 /* Seeded extraction (SURVEY.md 8(f3)): restricts the LAST full-volume run's mesh to what the reference's tracker
  *   tetrahedral.py:443-469  expand_voxels / in_range  (flood fill over the 26-neighbourhood of border voxels)
  * reaches from the given start voxels (the output of find_initial_voxels, tetrahedral.py:396-441, which the binding
