@@ -1,4 +1,4 @@
-// Per-vertex values of another field on the 3D mesh (ctr_mt3d_interpolate; included by mt3d.cu inside its namespace).
+// Per-vertex values of another field on the 3D mesh (ctr_mt3d_interpolate; included by mesh3d.cu inside its namespace).
 //
 //   k_interp_attr : thread per vertex of the last run's mesh (device keys, in vertex order = owner-word order, so
 //                   neighbouring lanes gather from neighbouring rows): the edge's two run samples give the ratio exactly
@@ -101,12 +101,11 @@ __global__ void __launch_bounds__(256) k_interp_attr(const T* __restrict__ f, in
   }
 }
 
-template <typename T>
+template <typename T, typename G>
 int interp_typed(ctr_ctx* ctx, const ctr_attr_params* ap, int64_t* n_verts) {
   const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
   const size_t nV = (size_t)ctx->last_counts[0];
-  const bool f64 = (ctx->last_flags & CTR_GEOM_F64) != 0;
-  const size_t gsz = f64 ? 8 : 4;
+  const size_t gsz = sizeof(G);
   const size_t rb = attr_sample_bytes(ap->dtype) * (size_t)ap->ncomp;
   const size_t npts = (size_t)p->n0 * (size_t)p->n1 * (size_t)p->n2;
   cudaStream_t st = ctx->stream;
@@ -132,14 +131,8 @@ int interp_typed(ctr_ctx* ctx, const ctr_attr_params* ap, int64_t* n_verts) {
   const long long off = p->plane_offset * p->n1 * p->n2;
   if (nV) {
     const unsigned nb = (unsigned)((nV + 255) / 256);
-    if (f64)
-      k_interp_attr<T, double><<<nb, 256, 0, st>>>(f, (int)p->n1, (int)p->n2, off, p->isovalue,
-                                                    (const unsigned long long*)ctx->keys.p, (const uint8_t*)ctx->lowmin.p,
-                                                    (unsigned)nV, a, (double*)ctx->aux[AUX_VALUES].p);
-    else
-      k_interp_attr<T, float><<<nb, 256, 0, st>>>(f, (int)p->n1, (int)p->n2, off, p->isovalue,
-                                                   (const unsigned long long*)ctx->keys.p, (const uint8_t*)ctx->lowmin.p,
-                                                   (unsigned)nV, a, (float*)ctx->aux[AUX_VALUES].p);
+    k_interp_attr<T, G><<<nb, 256, 0, st>>>(f, (int)p->n1, (int)p->n2, off, p->isovalue, (const unsigned long long*)ctx->keys.p,
+                                            (const uint8_t*)ctx->lowmin.p, (unsigned)nV, a, (G*)ctx->aux[AUX_VALUES].p);
     ctx->launches++;
   }
   CTR_CUDA(ctx, cudaGetLastError());

@@ -1,4 +1,4 @@
-// Caps that close the 3D device mesh at the faces of the volume (ctr_mt3d_cap; included by mt3d.cu inside its anonymous
+// Caps that close the 3D device mesh at the faces of the volume (ctr_mt3d_cap; included by mesh3d.cu inside its anonymous
 // namespace, after decimate3d.cuh, whose k_d_ids it runs).  The definition is oracle/mt3d_cap.py:cap (exact; new
 // normals within rounding of the normalisation).
 //
@@ -331,14 +331,12 @@ int cap_typed(ctr_ctx* ctx, const ctr_cap_params* cp, ctr_cap_counts* out) {
   CapCounters h;
   CTR_CUDA(ctx, cudaMemcpyAsync(&h, ctr, sizeof h, cudaMemcpyDeviceToHost, st));
   CTR_CUDA(ctx, cudaStreamSynchronize(st));
-  if (h.ids.bad_ids) return ctr_fail(ctx, CTR_ERR_STATE, "triangle ids outside [0, n_verts): the ids were shifted (ctr_mt3d_offset_ids)");
+  if (h.ids.bad_ids) return fail_shifted_ids(ctx);
   const size_t capT = (size_t)h.total[0], capV = (size_t)h.total[1];
   const size_t newV = nV + capV, newT = nT + capT;
   if (newV > 0x7fffffffull || newT > 0x7fffffffull)
     return ctr_fail(ctx, CTR_ERR_OVERFLOW, "the capped mesh would have 2^31 or more vertices or triangles");
-  // from here on the mesh is edited
-  ctx->mesh_gen++;
-  ctx->last3_edited |= EDIT_CAP;
+  mesh_edited(ctx, EDIT_CAP);
   const size_t gsz = sizeof(G);
   if ((rc = ctr_grow_keep(ctx, ctx->verts, newV * 3 * gsz, nV * 3 * gsz))) return rc;
   if ((ctx->last_flags & CTR_WANT_NORMALS) && (rc = ctr_grow_keep(ctx, ctx->normals, newV * 3 * gsz, nV * 3 * gsz))) return rc;

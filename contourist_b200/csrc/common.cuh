@@ -55,7 +55,51 @@ enum Edit3 : unsigned {
   EDIT_SMOOTH = 8u,          // smoothing
   EDIT_DECIMATE = 16u,       // decimation
   EDIT_CAP = 32u,            // caps at the box faces
+  EDIT_ORIENT = 64u,         // reference orientation (rewinds triangles only: the mesh generation stays)
 };
+
+// What a pass on the device mesh of the last 3D run needs of that run, and which earlier passes refuse it: one row per
+// pass, checked by check_pass.  Every pass needs a completed run with geometry (CTR_ERR_STATE).
+// Slab conditions, each including the one before: i_lo == 0 and i_hi == n0; vert_id_base == 0; plane_offset == 0.
+enum Slab3 : int { ANY_RUN, FULL, FULL_ID0, FULL_ID0_PLANE0 };
+
+struct PassRule {
+  const char* verb;          // ends "no completed ctr_mt3d_run with geometry<verb>"
+  bool keys;                 // needs the run's CTR_WANT_KEYS outputs
+  Slab3 slab;
+  int slab_code;             // the error of a run that misses the slab condition
+  const char* slab_msg;
+  unsigned refused_after;    // Edit3 bits of the passes that must not have run before this one
+  const char* order_msg;     // what to do instead, after the list of those passes
+};
+
+constexpr PassRule PASS_ORIENT = {" to orient", false, ANY_RUN, 0, nullptr, 0u, nullptr};
+constexpr PassRule PASS_COMPONENTS = {" to measure", false, FULL_ID0, CTR_ERR_STATE,
+                                      "components need a full-volume run with vert_id_base 0 (components cross slab faces)", 0u, nullptr};
+constexpr PassRule PASS_SMOOTH = {" to smooth", false, FULL_ID0, CTR_ERR_STATE,
+                                  "smoothing needs a full-volume run with vert_id_base 0 (a slab's halo ids belong to another shard)", 0u, nullptr};
+constexpr PassRule PASS_SECTION = {" to cut", false, FULL_ID0, CTR_ERR_STATE,
+                                   "sections need a full-volume run with vert_id_base 0 (a slab's halo ids belong to another shard)", 0u, nullptr};
+constexpr PassRule PASS_DECIMATE = {" to decimate", false, FULL_ID0, CTR_ERR_STATE,
+                                    "decimation needs a full-volume run with vert_id_base 0 (clusters cross slab faces)", 0u, nullptr};
+// the selection compacts the run's mesh in place while the voxel work list keeps its per-voxel triangle offsets: it can
+// be applied once per run, and before any other edit (an oriented mesh has the same rows)
+constexpr PassRule PASS_SELECT = {" to select from", false, FULL, CTR_ERR_UNSUPPORTED,
+                                  "seeded selection needs a full-volume run (components cross slab faces)",
+                                  EDIT_SELECT | EDIT_CLEAN | EDIT_KEEP | EDIT_SMOOTH | EDIT_DECIMATE | EDIT_CAP,
+                                  "run ctr_mt3d_run again"};
+// the reference's clean-up (quantize, tiny simplices) is defined on the interpolated positions
+constexpr PassRule PASS_CLEAN = {" to clean", false, FULL_ID0, CTR_ERR_UNSUPPORTED,
+                                 "mesh clean-up needs a full-volume run (merges cross slab faces)",
+                                 EDIT_CLEAN | EDIT_SMOOTH | EDIT_DECIMATE | EDIT_CAP,
+                                 "clean it up once, before smoothing, decimating or capping"};
+// after these passes the field no longer tells where the mesh's rim is or which way it faces
+constexpr PassRule PASS_CAP = {" to cap", true, FULL_ID0_PLANE0, CTR_ERR_STATE,
+                               "caps need a full-volume run with plane_offset 0 and vert_id_base 0 (the box of a slab is not the volume's)",
+                               EDIT_SELECT | EDIT_CLEAN | EDIT_KEEP | EDIT_DECIMATE | EDIT_CAP | EDIT_ORIENT,
+                               "cap it before those passes"};
+constexpr PassRule PASS_INTERPOLATE = {" to interpolate on", true, ANY_RUN, 0, nullptr, 0u, nullptr};
+constexpr PassRule PASS_OFFSET_IDS = {"", false, ANY_RUN, 0, nullptr, 0u, nullptr};
 
 struct ctr_ctx {
   int device = 0;
@@ -96,12 +140,8 @@ struct ctr_ctx {
   unsigned char last3_params[160] = {};   // parameters of the last completed ctr_mt3d_run
   long long* publish3 = nullptr;          // ctr_mt3d_publish_counts: device {n_verts, n_tris} behind every 3D run
   unsigned last3_edited = 0;              // Edit3 bits of the passes that have rewritten the device mesh of that run
-  // ctr_mt3d_orient_reference has rewound that mesh: kept apart from last3_edited, which the seeded selection refuses
-  // (it accepts an oriented run); ctr_mt3d_cap refuses it (the rim no longer faces the high side)
-  bool last3_oriented = false;
-  // bumped by every 3D run and every pass that removes or renumbers mesh rows (selection, clean-up, offset_ids,
-  // component filter, decimation) or moves vertices (smoothing); the vertex values and the components below record the
-  // generation they were computed on
+  // bumped by every 3D run and by mesh_edited (every pass that writes the mesh, orientation aside); the vertex values
+  // and the components below record the generation they were computed on
   uint64_t mesh_gen = 0;
   // 3D: an extraction enqueued by ctr_mt3d_enqueue and not yet finished
   bool pending3 = false;
@@ -211,6 +251,56 @@ static inline int ctr_carve_buf(ctr_ctx* ctx, DevBuf& b, F&& pieces) {
   return 0;
 }
 
+// 0 when the last 3D run and the passes since allow the pass of row `r`, and the context's device is then current; else
+// the error, with the message set
+static inline int check_pass(ctr_ctx* ctx, const PassRule& r) {
+  if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
+    return ctr_fail(ctx, CTR_ERR_STATE, (std::string("no completed ctr_mt3d_run with geometry") + r.verb).c_str());
+  if (r.keys && !(ctx->last_flags & CTR_WANT_KEYS))
+    return ctr_fail(ctx, CTR_ERR_STATE, "the run did not keep its keys: run with CTR_WANT_KEYS");
+  const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
+  if ((r.slab >= FULL && (p->i_lo != 0 || p->i_hi != p->n0)) || (r.slab >= FULL_ID0 && p->vert_id_base != 0) ||
+      (r.slab >= FULL_ID0_PLANE0 && p->plane_offset != 0))
+    return ctr_fail(ctx, r.slab_code, r.slab_msg);
+  if (const unsigned done = ctx->last3_edited & r.refused_after) {
+    static const char* const names[] = {"selected from", "cleaned", "filtered", "smoothed", "decimated", "capped", "oriented"};
+    std::string list;
+    for (int b = 0; b < 7; ++b)
+      if (done & (1u << b)) list += std::string(list.empty() ? "" : ", ") + names[b];
+    return ctr_fail(ctx, CTR_ERR_STATE, ("the mesh of this run has been " + list).c_str(), r.order_msg);
+  }
+  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
+  return 0;
+}
+
+// A pass is about to write the device mesh of the last 3D run (a mesh buffer or its counts): results recorded against
+// the mesh generation (components, vertex values) no longer describe it, and check_pass refuses the passes that must
+// come before `edit` (0: a change no pass refuses, such as ctr_mt3d_offset_ids).
+static inline void mesh_edited(ctr_ctx* ctx, unsigned edit) {
+  ctx->mesh_gen++;
+  ctx->last3_edited |= edit;
+}
+
+// f(T{}) for the sample type T of `dtype`
+template <typename F>
+static inline int with_sample_type(ctr_ctx* ctx, int dtype, F&& f) {
+  switch (dtype) {
+    case CTR_F32: return f(float{});
+    case CTR_F64: return f(double{});
+    case CTR_U8: return f(uint8_t{});
+    case CTR_I16: return f(int16_t{});
+    case CTR_U16: return f(uint16_t{});
+  }
+  return ctr_fail(ctx, CTR_ERR_BAD_ARG, "unknown dtype");
+}
+
+// f(G{}) for the geometry type G of the last run (double with CTR_GEOM_F64, else float)
+template <typename F>
+static inline int with_geom_type(ctr_ctx* ctx, F&& f) {
+  if (ctx->last_flags & CTR_GEOM_F64) return f(double{});
+  return f(float{});
+}
+
 static inline void ctr_stage_mark(ctr_ctx* ctx, int idx) {
   if (!ctx->timing) return;
   if (!ctx->ev[idx]) cudaEventCreate(&ctx->ev[idx]);
@@ -222,6 +312,21 @@ static inline void ctr_stage_mark(ctr_ctx* ctx, int idx) {
 #ifdef __CUDACC__
 
 __device__ __forceinline__ unsigned lane_id() { return threadIdx.x & 31u; }
+
+__device__ __forceinline__ double mul_rn(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ float mul_rn(float a, float b) { return __fmul_rn(a, b); }
+__device__ __forceinline__ double add_rn(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ float add_rn(float a, float b) { return __fadd_rn(a, b); }
+
+struct Xform {
+  double origin[3], delta[3], inv_delta[3];
+};
+
+// geometry-mode arithmetic: IEEE in fp64 mode (positions bit-exact vs the oracle); fast approximations in fp32 mode (1e-4 rel)
+__device__ __forceinline__ double quot(double a, double b) { return a / b; }
+__device__ __forceinline__ float quot(float a, float b) { return __fdividef(a, b); }
+__device__ __forceinline__ double inv_sqrt(double a) { return 1.0 / sqrt(a); }
+__device__ __forceinline__ float inv_sqrt(float a) { return rsqrtf(a); }
 
 // Programmatic dependent launch.  The kernels of one extraction run back to back on one stream, several of them for a
 // few microseconds only; launched with ctr_launch_dep a kernel's blocks may become resident (and run their prologue:

@@ -1,6 +1,6 @@
-// Order-preserving compaction of the 3D device mesh in place -- included by mt3d.cu inside its anonymous namespace,
-// before the passes that drop triangles and the vertices no kept triangle uses: the seeded selection, the component
-// filter, the clean-up and the decimation.  A pass carves the pieces below out of its scratch (compact_carve), flags the
+// Order-preserving compaction of the 3D device mesh in place, for the passes that drop triangles and the vertices no kept
+// triangle uses -- included inside the anonymous namespace of mt3d.cu (the seeded selection) and of mesh3d.cu (the
+// component filter, the clean-up and the decimation).  A pass carves the pieces below out of its scratch (compact_carve), flags the
 // triangles it keeps (keep_t) and the vertices they use (used_v: k_sel_used, or the pass's own kernel), then calls
 // compact_mesh:
 //   k_flag_scan x 2 : new triangle and vertex indices, single-pass look-back scans;

@@ -242,9 +242,7 @@ int components_typed(ctr_ctx* ctx, int64_t* n_components) {
     ctx->comp_gen = ctx->mesh_gen;
     return 0;
   }
-  size_t nslots = 1;
-  while (nslots < (size_t)nt * 4) nslots <<= 1;       // edges: 1.5 nt on closed sheets (3 nt at worst); (component,
-                                                      // vertex) pairs: about nt / 2 (3 nt at worst): load <= 3/4
+  const size_t nslots = edge_slots(nt);               // also the (component, vertex) table: about nt / 2 pairs (3 nt at worst)
   const unsigned blocks = (nt + M_THREADS - 1) / M_THREADS;   // also the look-back tiles of k_m_roots
   int rc;
   DevBuf& b_etab = ctx->aux[AUX_SCRATCH0];
@@ -275,7 +273,7 @@ int components_typed(ctr_ctx* ctx, int64_t* n_components) {
   MCounters h;
   CTR_CUDA(ctx, cudaMemcpyAsync(&h, ctr, sizeof h, cudaMemcpyDeviceToHost, st));
   CTR_CUDA(ctx, cudaStreamSynchronize(st));
-  if (h.bad) return ctr_fail(ctx, CTR_ERR_STATE, "triangle ids outside [0, n_verts): the ids were shifted (ctr_mt3d_offset_ids)");
+  if (h.bad) return fail_shifted_ids(ctx);
   k_o_union<<<blocks, M_THREADS, 0, st>>>(tris, nt, etab, nslots - 1, parent);
   k_m_roots<<<blocks, M_THREADS, 0, st>>>(parent, nt, rank, status, ctr, (int)blocks);
   ctx->launches += 2;

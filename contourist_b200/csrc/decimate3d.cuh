@@ -1,7 +1,7 @@
 // Quadric vertex-clustering decimation of the 3D device mesh (ctr_mt3d_decimate; Lindstrom 2000, the GPU form of
 // DeCoro & Tatarchuk 2007, VTK's vtkQuadricClustering).
 //
-// Included into mt3d.cu after mt3d_clean.cuh, inside its anonymous namespace: clustering is the clean-up's quantize
+// Included into mesh3d.cu after mt3d_clean.cuh, inside its anonymous namespace: clustering is the clean-up's quantize
 // step with another cell key, so the pass runs that step's kernels through its helpers (cluster_bufs, cluster_tris),
 // compacts with compact_mesh (compact3d.cuh) and takes the normals of normals3d.cuh.  The definition is
 // oracle/mt3d_decimate.py:decimate (positions within rounding: the sums below are fp64 atomics in an unspecified order;
@@ -215,12 +215,11 @@ int decimate_typed(ctr_ctx* ctx, const ctr_decimate_params* dp, ctr_decimate_cou
     ctx->launches++;
     CTR_CUDA(ctx, cudaMemcpyAsync(&h, dc, sizeof h, cudaMemcpyDeviceToHost, st));
     CTR_CUDA(ctx, cudaStreamSynchronize(st));
-    if (h.bad_ids) return ctr_fail(ctx, CTR_ERR_STATE, "triangle ids outside [0, n_verts): the ids were shifted (ctr_mt3d_offset_ids)");
+    if (h.bad_ids) return fail_shifted_ids(ctx);
   }
   if ((rc = cluster_tris<G>(ctx, verts, nV, tris, nT, key, b, &h, sizeof h))) return rc;
   if (h.out_of_range) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "a cell index (p - origin) / cell lies outside [-2^20, 2^20)");
-  ctx->mesh_gen++;                                    // from here on the mesh is edited
-  ctx->last3_edited |= EDIT_DECIMATE;
+  mesh_edited(ctx, EDIT_DECIMATE);
   CTR_CUDA(ctx, cudaMemsetAsync(acc, 0, (size_t)nV * D_ROW * 8, st));
   k_d_vsum<G><<<vb, 256, 0, st>>>(verts, nV, b.rep, d, acc, dc);
   ctx->launches++;

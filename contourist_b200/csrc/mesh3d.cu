@@ -17,6 +17,8 @@
 #include <math.h>
 #include <string.h>
 
+#include <algorithm>
+
 #include "common.cuh"
 #include "uf_hash.cuh"
 
@@ -34,6 +36,18 @@ __device__ __forceinline__ unsigned long long edge_key(int a, int b) {
 
 __device__ __forceinline__ EdgeSlot* edge_slot(EdgeSlot* tab, size_t mask, unsigned long long key, bool insert) {
   return ufh::hash_slot(tab, mask, key, insert);
+}
+
+// slots of the edge table of nt triangles: 1.5 nt distinct edges on closed sheets (3 nt at worst): load <= 3/8 (3/4)
+static inline size_t edge_slots(unsigned nt) {
+  size_t n = 1;
+  while (n < (size_t)nt * 4) n <<= 1;
+  return n;
+}
+
+// a pass found triangle ids outside [0, n_verts)
+static inline int fail_shifted_ids(ctr_ctx* ctx) {
+  return ctr_fail(ctx, CTR_ERR_STATE, "triangle ids outside [0, n_verts): the ids were shifted (ctr_mt3d_offset_ids)");
 }
 
 __global__ void k_o_init(EdgeSlot* tab, size_t nslots, int* parent, unsigned nt, unsigned long long* comp_key,
@@ -182,8 +196,7 @@ int orient_typed(ctr_ctx* ctx, int64_t* n_components, int64_t* n_flipped) {
   if (n_components) *n_components = 0;
   if (n_flipped) *n_flipped = 0;
   if (nt == 0) return 0;
-  size_t nslots = 1;
-  while (nslots < (size_t)nt * 4) nslots <<= 1;       // 1.5 nt distinct edges on closed sheets (3 nt at worst): load <= 3/8 (3/4)
+  const size_t nslots = edge_slots(nt);
   int rc;
   DevBuf& b_tab = ctx->aux[AUX_SCRATCH0];
   DevBuf& b_par = ctx->aux[AUX_SCRATCH2];
@@ -225,31 +238,28 @@ int orient_typed(ctr_ctx* ctx, int64_t* n_components, int64_t* n_flipped) {
 #include "components3d.cuh"
 #include "smooth3d.cuh"
 #include "section3d.cuh"
+#include "compact3d.cuh"
+#include "mt3d_keep.cuh"
+#include "mt3d_clean.cuh"
+#include "decimate3d.cuh"
+#include "attr3d.cuh"
+#include "cap3d.cuh"
 
 }  // namespace
 
 extern "C" int ctr_mt3d_orient_reference(ctr_ctx* ctx, int64_t* n_components, int64_t* n_flipped) {
   if (!ctx) return CTR_ERR_BAD_ARG;
-  if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
-    return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to orient");
-  ctx->last3_oriented = true;                         // (also when the call fails below: it may have rewound a part)
-  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
-  if (ctx->last_flags & CTR_GEOM_F64) return orient_typed<double>(ctx, n_components, n_flipped);
-  return orient_typed<float>(ctx, n_components, n_flipped);
+  if (int rc = check_pass(ctx, PASS_ORIENT)) return rc;
+  ctx->last3_edited |= EDIT_ORIENT;                   // (also when the call fails below: it may have rewound a part)
+  return with_geom_type(ctx, [&](auto g) { return orient_typed<decltype(g)>(ctx, n_components, n_flipped); });
 }
 
 extern "C" int ctr_mt3d_components(ctr_ctx* ctx, int64_t* n_components) {
   if (!ctx) return CTR_ERR_BAD_ARG;
   if (n_components) *n_components = 0;
   ctx->comp_count = -1;                               // the buffers are rewritten: earlier results are gone
-  if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
-    return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to measure");
-  const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
-  if (p->i_lo != 0 || p->i_hi != p->n0 || p->vert_id_base != 0)
-    return ctr_fail(ctx, CTR_ERR_STATE, "components need a full-volume run with vert_id_base 0 (components cross slab faces)");
-  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
-  if (ctx->last_flags & CTR_GEOM_F64) return components_typed<double>(ctx, n_components);
-  return components_typed<float>(ctx, n_components);
+  if (int rc = check_pass(ctx, PASS_COMPONENTS)) return rc;
+  return with_geom_type(ctx, [&](auto g) { return components_typed<decltype(g)>(ctx, n_components); });
 }
 
 extern "C" int ctr_mt3d_smooth(ctr_ctx* ctx, const ctr_smooth_params* sp, ctr_smooth_counts* out) {
@@ -260,14 +270,8 @@ extern "C" int ctr_mt3d_smooth(ctr_ctx* ctx, const ctr_smooth_params* sp, ctr_sm
   if (sp->reserved != 0) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "reserved must be 0");
   if (!(sp->lambda > 0.0 && sp->lambda <= 1.0)) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "lambda must be in (0, 1]");
   if (!(sp->mu >= -1.0 && sp->mu <= 0.0)) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "mu must be in [-1, 0]");
-  if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
-    return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to smooth");
-  const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
-  if (p->i_lo != 0 || p->i_hi != p->n0 || p->vert_id_base != 0)
-    return ctr_fail(ctx, CTR_ERR_STATE, "smoothing needs a full-volume run with vert_id_base 0 (a slab's halo ids belong to another shard)");
-  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
-  if (ctx->last_flags & CTR_GEOM_F64) return smooth_typed<double>(ctx, sp, out);
-  return smooth_typed<float>(ctx, sp, out);
+  if (int rc = check_pass(ctx, PASS_SMOOTH)) return rc;
+  return with_geom_type(ctx, [&](auto g) { return smooth_typed<decltype(g)>(ctx, sp, out); });
 }
 
 extern "C" int ctr_mt3d_components_fetch(ctr_ctx* ctx, int32_t* tri_component, ctr_mt3d_component* components) {
@@ -297,14 +301,8 @@ extern "C" int ctr_mt3d_section(ctr_ctx* ctx, const ctr_section_params* sp, ctr_
     if (!isfinite(sp->offsets[l]) || (l > 0 && !(sp->offsets[l] > sp->offsets[l - 1])))
       return ctr_fail(ctx, CTR_ERR_BAD_ARG, "offsets must be finite and strictly increasing");
   ctx->sect_count[0] = -1;                            // the buffers are rewritten: earlier results are gone
-  if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
-    return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to cut");
-  const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
-  if (p->i_lo != 0 || p->i_hi != p->n0 || p->vert_id_base != 0)
-    return ctr_fail(ctx, CTR_ERR_STATE, "sections need a full-volume run with vert_id_base 0 (a slab's halo ids belong to another shard)");
-  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
-  if (ctx->last_flags & CTR_GEOM_F64) return section_typed<double>(ctx, sp, out);
-  return section_typed<float>(ctx, sp, out);
+  if (int rc = check_pass(ctx, PASS_SECTION)) return rc;
+  return with_geom_type(ctx, [&](auto g) { return section_typed<decltype(g)>(ctx, sp, out); });
 }
 
 extern "C" int ctr_mt3d_section_segments_fetch(ctr_ctx* ctx, int32_t* plane, int32_t* edges, void* points) {
@@ -353,5 +351,98 @@ extern "C" int ctr_mt3d_section_polylines_fetch(ctr_ctx* ctx, int32_t* plane, ui
   }
   CTR_CUDA(ctx, cudaStreamSynchronize(st));
   for (size_t l = 0; l < jp.size(); ++l) junction[l] = jp[l] ? 1 : 0;
+  return 0;
+}
+
+extern "C" int ctr_mt3d_keep_components(ctr_ctx* ctx, const uint8_t* keep, int64_t n_keep, int64_t* n_verts, int64_t* n_tris) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (ctx->last_kind != 3 || ctx->comp_count < 0)
+    return ctr_fail(ctx, CTR_ERR_STATE, "no ctr_mt3d_components since the last 3D run");
+  if (ctx->comp_gen != ctx->mesh_gen)
+    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh was edited after ctr_mt3d_components (selection, clean-up, smoothing, decimation "
+                                        "or offset_ids): call ctr_mt3d_components again");
+  if (n_keep != ctx->comp_count || (!keep && n_keep > 0))
+    return ctr_fail(ctx, CTR_ERR_BAD_ARG, "keep must hold one byte per component of the last ctr_mt3d_components call");
+  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
+  return keep_components_run(ctx, keep, n_verts, n_tris);
+}
+
+extern "C" int ctr_mt3d_clean(ctr_ctx* ctx, const ctr_clean_params* cp, ctr_clean_counts* out) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (!cp || !out) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  memset(out, 0, sizeof *out);
+  if (int rc = check_pass(ctx, PASS_CLEAN)) return rc;
+  const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
+  for (int a = 0; a < 3; ++a) {
+    if (p->origin[a] != 0.0 || p->delta[a] != 1.0)
+      return ctr_fail(ctx, CTR_ERR_STATE, "mesh clean-up works in grid coordinates: run with origin 0, delta 1 and pass the transform here");
+    if (cp->corner[a] < 1) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "corner must be >= 1 on every axis");
+    if (cp->delta[a] == 0.0) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "delta must be non-zero");
+  }
+  if (cp->divisions < 1 || cp->divisions >= (1 << 21)) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "divisions must be in [1, 2^21)");
+  if (!(cp->epsilon == cp->epsilon)) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "epsilon is NaN");
+  return with_geom_type(ctx, [&](auto g) { return clean_typed<decltype(g)>(ctx, cp, out); });
+}
+
+extern "C" int ctr_mt3d_decimate(ctr_ctx* ctx, const ctr_decimate_params* dp, ctr_decimate_counts* out) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (!dp || !out) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  memset(out, 0, sizeof *out);
+  for (int a = 0; a < 3; ++a) {
+    if (!(dp->cell[a] > 0.0 && isfinite(dp->cell[a]))) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "cell must be > 0 and finite on every axis");
+    if (!isfinite(dp->origin[a])) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "origin must be finite");
+  }
+  if (int rc = check_pass(ctx, PASS_DECIMATE)) return rc;
+  return with_geom_type(ctx, [&](auto g) { return decimate_typed<decltype(g)>(ctx, dp, out); });
+}
+
+extern "C" int ctr_mt3d_cap(ctr_ctx* ctx, const ctr_cap_params* cp, ctr_cap_counts* out) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (!cp || !out) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  memset(out, 0, sizeof *out);
+  if (cp->side != CTR_CAP_HIGH && cp->side != CTR_CAP_LOW) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "side must be CTR_CAP_HIGH or CTR_CAP_LOW");
+  if (cp->reserved != 0) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "reserved must be 0");
+  if (int rc = check_pass(ctx, PASS_CAP)) return rc;
+  return with_sample_type(ctx, ((const ctr_mt3d_params*)ctx->last3_params)->dtype, [&](auto t) {
+    return with_geom_type(ctx, [&](auto g) { return cap_typed<decltype(t), decltype(g)>(ctx, cp, out); });
+  });
+}
+
+extern "C" int ctr_mt3d_interpolate(ctr_ctx* ctx, const ctr_attr_params* a, int64_t* n_verts) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (!a || !a->field) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  if (a->ncomp < 1 || a->ncomp > 4) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "ncomp must be 1..4");
+  if (a->dtype != CTR_F32 && a->dtype != CTR_F64 && a->dtype != CTR_U8 && a->dtype != CTR_I16 && a->dtype != CTR_U16)
+    return ctr_fail(ctx, CTR_ERR_BAD_ARG, "dtype must be CTR_F32, CTR_F64, CTR_U8, CTR_I16 or CTR_U16");
+  if (int rc = check_pass(ctx, PASS_INTERPOLATE)) return rc;
+  ctx->attr_ncomp = 0;                                 // the buffer is rewritten: earlier values are gone
+  return with_sample_type(ctx, ((const ctr_mt3d_params*)ctx->last3_params)->dtype, [&](auto t) {
+    return with_geom_type(ctx, [&](auto g) { return interp_typed<decltype(t), decltype(g)>(ctx, a, n_verts); });
+  });
+}
+
+static int interp_check(ctr_ctx* ctx) {
+  if (ctx->last_kind != 3 || !ctx->attr_ncomp) return ctr_fail(ctx, CTR_ERR_STATE, "no ctr_mt3d_interpolate since the last 3D run");
+  return 0;
+}
+
+extern "C" int ctr_mt3d_interpolate_fetch(ctr_ctx* ctx, void* values) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (!values) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  int rc = interp_check(ctx);
+  if (rc) return rc;
+  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
+  const size_t bytes = ctx->attr_rows * (size_t)ctx->attr_ncomp * ((ctx->last_flags & CTR_GEOM_F64) ? 8 : 4);
+  if (bytes) CTR_CUDA(ctx, cudaMemcpyAsync(values, ctx->aux[AUX_VALUES].p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  CTR_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return 0;
+}
+
+extern "C" int ctr_mt3d_interpolate_device_ptr(ctr_ctx* ctx, void** values) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (!values) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  int rc = interp_check(ctx);
+  if (rc) return rc;
+  *values = ctx->aux[AUX_VALUES].p;
   return 0;
 }

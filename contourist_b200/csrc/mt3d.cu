@@ -961,22 +961,9 @@ __device__ __forceinline__ void grad_at(const Grid<T>& g, int i, int j, int k, G
   }
 }
 
-__device__ __forceinline__ double mul_rn(double a, double b) { return __dmul_rn(a, b); }
-__device__ __forceinline__ float mul_rn(float a, float b) { return __fmul_rn(a, b); }
-__device__ __forceinline__ double add_rn(double a, double b) { return __dadd_rn(a, b); }
-__device__ __forceinline__ float add_rn(float a, float b) { return __fadd_rn(a, b); }
 __device__ __forceinline__ double shfl_g(double v, int src) { return __shfl_sync(0xffffffffu, v, src); }
 __device__ __forceinline__ float shfl_g(float v, int src) { return __shfl_sync(0xffffffffu, v, src); }
 
-struct Xform {
-  double origin[3], delta[3], inv_delta[3];
-};
-
-// geometry-mode arithmetic: IEEE in fp64 mode (positions bit-exact vs the oracle); fast approximations in fp32 mode (1e-4 rel)
-__device__ __forceinline__ double quot(double a, double b) { return a / b; }
-__device__ __forceinline__ float quot(float a, float b) { return __fdividef(a, b); }
-__device__ __forceinline__ double inv_sqrt(double a) { return 1.0 / sqrt(a); }
-__device__ __forceinline__ float inv_sqrt(float a) { return rsqrtf(a); }
 // n-th (0-based) set bit of a 7-bit mask (__fns costs ~50 instructions)
 __device__ __forceinline__ int nth_set_bit7(unsigned m, unsigned n) {
   int b = 0;
@@ -1660,7 +1647,6 @@ int run_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts* out, int 
   }
   ctx->last_kind = 3;
   ctx->last3_edited = 0;
-  ctx->last3_oriented = false;
   ctx->last_flags = p->flags;
   ctx->last_counts[0] = (int64_t)nV;
   ctx->last_counts[1] = (int64_t)totT;
@@ -1671,12 +1657,6 @@ int run_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts* out, int 
 
 #include "compact3d.cuh"
 #include "mt3d_select.cuh"
-#include "mt3d_keep.cuh"
-#include "mt3d_clean.cuh"
-#include "normals3d.cuh"
-#include "decimate3d.cuh"
-#include "attr3d.cuh"
-#include "cap3d.cuh"
 
 }  // namespace
 
@@ -1704,14 +1684,7 @@ static int mt3d_dispatch(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts
   ctx->attr_ncomp = 0;                                 // vertex values of the previous run are gone
   ctx->comp_count = -1;                                // ... and so are its components
   ctx->sect_count[0] = -1;                             // ... and its plane sections
-  switch (p->dtype) {
-    case CTR_F32: return run_typed<float>(ctx, p, out, phase);
-    case CTR_F64: return run_typed<double>(ctx, p, out, phase);
-    case CTR_U8: return run_typed<uint8_t>(ctx, p, out, phase);
-    case CTR_I16: return run_typed<int16_t>(ctx, p, out, phase);
-    case CTR_U16: return run_typed<uint16_t>(ctx, p, out, phase);
-  }
-  return ctr_fail(ctx, CTR_ERR_BAD_ARG, "unknown dtype");
+  return with_sample_type(ctx, p->dtype, [&](auto t) { return run_typed<decltype(t)>(ctx, p, out, phase); });
 }
 
 extern "C" int ctr_mt3d_run(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts* out) {
@@ -1745,12 +1718,11 @@ extern "C" int ctr_mt3d_finish(ctr_ctx* ctx, ctr_mt3d_counts* out) {
 
 extern "C" int ctr_mt3d_offset_ids(ctr_ctx* ctx, int64_t base) {
   if (!ctx) return CTR_ERR_BAD_ARG;
-  if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY)) return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry");
+  if (int rc = check_pass(ctx, PASS_OFFSET_IDS)) return rc;
   if (base < 0 || base > 0x7fffffffll) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "id base out of range");
   const size_t n = (size_t)ctx->last_counts[1] * 3;
   if (!n || !base) return 0;
-  ctx->mesh_gen++;
-  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
+  mesh_edited(ctx, 0u);
   k_offset_ids<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>((int*)ctx->tris.p, n, (int)base);
   ctx->launches++;
   CTR_CUDA(ctx, cudaGetLastError());
@@ -1813,164 +1785,9 @@ extern "C" int ctr_mt3d_select_seeded(ctr_ctx* ctx, const int32_t* seed_voxels, 
                                       int64_t* n_tris, int64_t* n_voxels) {
   if (!ctx) return CTR_ERR_BAD_ARG;
   if (n_seeds < 0 || (n_seeds > 0 && !seed_voxels)) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "bad seed list");
-  if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
-    return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to select from");
+  if (int rc = check_pass(ctx, PASS_SELECT)) return rc;
   const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
-  if (p->i_lo != 0 || p->i_hi != p->n0)
-    return ctr_fail(ctx, CTR_ERR_UNSUPPORTED, "seeded selection needs a full-volume run (components cross slab faces)");
-  // the selection compacts the run's mesh in place while the voxel work list keeps its per-voxel triangle offsets: it
-  // can be applied once per run
-  if (ctx->last3_edited)
-    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has already been selected from, cleaned, filtered, smoothed, decimated or capped; "
-                                        "run ctr_mt3d_run again");
-  ctx->mesh_gen++;
-  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
-  switch (p->dtype) {
-    case CTR_F32: return select_typed<float>(ctx, p, seed_voxels, n_seeds, n_verts, n_tris, n_voxels);
-    case CTR_F64: return select_typed<double>(ctx, p, seed_voxels, n_seeds, n_verts, n_tris, n_voxels);
-    case CTR_U8: return select_typed<uint8_t>(ctx, p, seed_voxels, n_seeds, n_verts, n_tris, n_voxels);
-    case CTR_I16: return select_typed<int16_t>(ctx, p, seed_voxels, n_seeds, n_verts, n_tris, n_voxels);
-    case CTR_U16: return select_typed<uint16_t>(ctx, p, seed_voxels, n_seeds, n_verts, n_tris, n_voxels);
-  }
-  return ctr_fail(ctx, CTR_ERR_BAD_ARG, "unknown dtype");
-}
-
-extern "C" int ctr_mt3d_keep_components(ctr_ctx* ctx, const uint8_t* keep, int64_t n_keep, int64_t* n_verts, int64_t* n_tris) {
-  if (!ctx) return CTR_ERR_BAD_ARG;
-  if (ctx->last_kind != 3 || ctx->comp_count < 0)
-    return ctr_fail(ctx, CTR_ERR_STATE, "no ctr_mt3d_components since the last 3D run");
-  if (ctx->comp_gen != ctx->mesh_gen)
-    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh was edited after ctr_mt3d_components (selection, clean-up, smoothing, decimation "
-                                        "or offset_ids): call ctr_mt3d_components again");
-  if (n_keep != ctx->comp_count || (!keep && n_keep > 0))
-    return ctr_fail(ctx, CTR_ERR_BAD_ARG, "keep must hold one byte per component of the last ctr_mt3d_components call");
-  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
-  return keep_components_run(ctx, keep, n_verts, n_tris);
-}
-
-extern "C" int ctr_mt3d_clean(ctr_ctx* ctx, const ctr_clean_params* cp, ctr_clean_counts* out) {
-  if (!ctx) return CTR_ERR_BAD_ARG;
-  if (!cp || !out) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
-  memset(out, 0, sizeof *out);
-  if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
-    return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to clean");
-  if (ctx->last3_edited & EDIT_CLEAN) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has already been cleaned");
-  // the reference's clean-up (quantize, tiny simplices) is defined on the interpolated positions
-  if (ctx->last3_edited & EDIT_SMOOTH) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has been smoothed: clean it up before smoothing");
-  if (ctx->last3_edited & EDIT_DECIMATE) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has been decimated: clean it up before decimating");
-  if (ctx->last3_edited & EDIT_CAP) return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has been capped: clean it up before capping");
-  const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
-  if (p->i_lo != 0 || p->i_hi != p->n0 || p->vert_id_base != 0)
-    return ctr_fail(ctx, CTR_ERR_UNSUPPORTED, "mesh clean-up needs a full-volume run (merges cross slab faces)");
-  for (int a = 0; a < 3; ++a) {
-    if (p->origin[a] != 0.0 || p->delta[a] != 1.0)
-      return ctr_fail(ctx, CTR_ERR_STATE, "mesh clean-up works in grid coordinates: run with origin 0, delta 1 and pass the transform here");
-    if (cp->corner[a] < 1) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "corner must be >= 1 on every axis");
-    if (cp->delta[a] == 0.0) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "delta must be non-zero");
-  }
-  if (cp->divisions < 1 || cp->divisions >= (1 << 21)) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "divisions must be in [1, 2^21)");
-  if (!(cp->epsilon == cp->epsilon)) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "epsilon is NaN");
-  ctx->mesh_gen++;
-  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
-  if (ctx->last_flags & CTR_GEOM_F64) return clean_typed<double>(ctx, cp, out);
-  return clean_typed<float>(ctx, cp, out);
-}
-
-extern "C" int ctr_mt3d_decimate(ctr_ctx* ctx, const ctr_decimate_params* dp, ctr_decimate_counts* out) {
-  if (!ctx) return CTR_ERR_BAD_ARG;
-  if (!dp || !out) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
-  memset(out, 0, sizeof *out);
-  for (int a = 0; a < 3; ++a) {
-    if (!(dp->cell[a] > 0.0 && isfinite(dp->cell[a]))) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "cell must be > 0 and finite on every axis");
-    if (!isfinite(dp->origin[a])) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "origin must be finite");
-  }
-  if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
-    return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to decimate");
-  const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
-  if (p->i_lo != 0 || p->i_hi != p->n0 || p->vert_id_base != 0)
-    return ctr_fail(ctx, CTR_ERR_STATE, "decimation needs a full-volume run with vert_id_base 0 (clusters cross slab faces)");
-  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
-  if (ctx->last_flags & CTR_GEOM_F64) return decimate_typed<double>(ctx, dp, out);
-  return decimate_typed<float>(ctx, dp, out);
-}
-
-template <typename T>
-static int cap_dispatch(ctr_ctx* ctx, const ctr_cap_params* cp, ctr_cap_counts* out) {
-  if (ctx->last_flags & CTR_GEOM_F64) return cap_typed<T, double>(ctx, cp, out);
-  return cap_typed<T, float>(ctx, cp, out);
-}
-
-extern "C" int ctr_mt3d_cap(ctr_ctx* ctx, const ctr_cap_params* cp, ctr_cap_counts* out) {
-  if (!ctx) return CTR_ERR_BAD_ARG;
-  if (!cp || !out) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
-  memset(out, 0, sizeof *out);
-  if (cp->side != CTR_CAP_HIGH && cp->side != CTR_CAP_LOW) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "side must be CTR_CAP_HIGH or CTR_CAP_LOW");
-  if (cp->reserved != 0) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "reserved must be 0");
-  if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
-    return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to cap");
-  if (!(ctx->last_flags & CTR_WANT_KEYS)) return ctr_fail(ctx, CTR_ERR_STATE, "the run did not keep its keys: run with CTR_WANT_KEYS");
-  const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
-  if (p->i_lo != 0 || p->i_hi != p->n0 || p->plane_offset != 0 || p->vert_id_base != 0)
-    return ctr_fail(ctx, CTR_ERR_STATE, "caps need a full-volume run with plane_offset 0 and vert_id_base 0 (the box of a slab is not the volume's)");
-  // after these passes the field no longer tells where the mesh's rim is or which way it faces: cap first
-  if ((ctx->last3_edited & ~(unsigned)EDIT_SMOOTH) || ctx->last3_oriented)
-    return ctr_fail(ctx, CTR_ERR_STATE, "the mesh of this run has been selected from, cleaned, filtered, decimated, oriented or capped: "
-                                        "cap it before those passes");
-  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
-  switch (p->dtype) {
-    case CTR_F32: return cap_dispatch<float>(ctx, cp, out);
-    case CTR_F64: return cap_dispatch<double>(ctx, cp, out);
-    case CTR_U8: return cap_dispatch<uint8_t>(ctx, cp, out);
-    case CTR_I16: return cap_dispatch<int16_t>(ctx, cp, out);
-    case CTR_U16: return cap_dispatch<uint16_t>(ctx, cp, out);
-  }
-  return ctr_fail(ctx, CTR_ERR_BAD_ARG, "unknown dtype");
-}
-
-extern "C" int ctr_mt3d_interpolate(ctr_ctx* ctx, const ctr_attr_params* a, int64_t* n_verts) {
-  if (!ctx) return CTR_ERR_BAD_ARG;
-  if (!a || !a->field) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
-  if (a->ncomp < 1 || a->ncomp > 4) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "ncomp must be 1..4");
-  if (a->dtype != CTR_F32 && a->dtype != CTR_F64 && a->dtype != CTR_U8 && a->dtype != CTR_I16 && a->dtype != CTR_U16)
-    return ctr_fail(ctx, CTR_ERR_BAD_ARG, "dtype must be CTR_F32, CTR_F64, CTR_U8, CTR_I16 or CTR_U16");
-  if (ctx->last_kind != 3 || (ctx->last_flags & CTR_NO_GEOMETRY))
-    return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt3d_run with geometry to interpolate on");
-  if (!(ctx->last_flags & CTR_WANT_KEYS)) return ctr_fail(ctx, CTR_ERR_STATE, "the run did not keep its keys: run with CTR_WANT_KEYS");
-  ctx->attr_ncomp = 0;                                 // the buffer is rewritten: earlier values are gone
-  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
-  const ctr_mt3d_params* p = (const ctr_mt3d_params*)ctx->last3_params;
-  switch (p->dtype) {
-    case CTR_F32: return interp_typed<float>(ctx, a, n_verts);
-    case CTR_F64: return interp_typed<double>(ctx, a, n_verts);
-    case CTR_U8: return interp_typed<uint8_t>(ctx, a, n_verts);
-    case CTR_I16: return interp_typed<int16_t>(ctx, a, n_verts);
-    case CTR_U16: return interp_typed<uint16_t>(ctx, a, n_verts);
-  }
-  return ctr_fail(ctx, CTR_ERR_BAD_ARG, "unknown dtype");
-}
-
-static int interp_check(ctr_ctx* ctx) {
-  if (ctx->last_kind != 3 || !ctx->attr_ncomp) return ctr_fail(ctx, CTR_ERR_STATE, "no ctr_mt3d_interpolate since the last 3D run");
-  return 0;
-}
-
-extern "C" int ctr_mt3d_interpolate_fetch(ctr_ctx* ctx, void* values) {
-  if (!ctx) return CTR_ERR_BAD_ARG;
-  if (!values) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
-  int rc = interp_check(ctx);
-  if (rc) return rc;
-  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
-  const size_t bytes = ctx->attr_rows * (size_t)ctx->attr_ncomp * ((ctx->last_flags & CTR_GEOM_F64) ? 8 : 4);
-  if (bytes) CTR_CUDA(ctx, cudaMemcpyAsync(values, ctx->aux[AUX_VALUES].p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-  CTR_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  return 0;
-}
-
-extern "C" int ctr_mt3d_interpolate_device_ptr(ctr_ctx* ctx, void** values) {
-  if (!ctx) return CTR_ERR_BAD_ARG;
-  if (!values) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
-  int rc = interp_check(ctx);
-  if (rc) return rc;
-  *values = ctx->aux[AUX_VALUES].p;
-  return 0;
+  return with_sample_type(ctx, p->dtype, [&](auto t) {
+    return select_typed<decltype(t)>(ctx, p, seed_voxels, n_seeds, n_verts, n_tris, n_voxels);
+  });
 }

@@ -1,5 +1,5 @@
 // The reference's mesh post-processing on the device mesh of the last ctr_mt3d_run (SURVEY.md 8 a10, a11, a13, f1) --
-// included by mt3d.cu inside its anonymous namespace, after compact3d.cuh.
+// included by mesh3d.cu inside its anonymous namespace, after compact3d.cuh.
 //
 //   tetrahedral.py:190-215    quantize_interpolations : interpolations that truncate to the same cell of the
 //                             `divisions` grid become one vertex; simplices that lose a vertex, or equal another, go;
@@ -330,8 +330,9 @@ int clean_typed(ctr_ctx* ctx, const ctr_clean_params* cp, ctr_clean_counts* out)
   CleanCounters hc;
   memset(&hc, 0, sizeof hc);
   size_t newV = 0, newT = 0;
+  if (nV && nT && (rc = cluster_tris<G>(ctx, verts, nV, tris, nT, e, b, &hc, sizeof hc))) return rc;
+  mesh_edited(ctx, EDIT_CLEAN);
   if (nV && nT) {
-    if ((rc = cluster_tris<G>(ctx, verts, nV, tris, nT, e, b, &hc, sizeof hc))) return rc;
     k_c_tiny<G><<<tb, 256, 0, st>>>(verts, b.tris2, nT, b.cb.keep_t, e, cp->epsilon, b.parent_a, dcc);
     k_c_tinypos<G><<<vb, 256, 0, st>>>(verts, nV, b.parent_a);
     if (!(cp->flags & CTR_CLEAN_NO_TRIANGLES)) k_c_flat<G><<<tb, 256, 0, st>>>(verts, b.tris2, nT, b.cb.keep_t, b.parent_b, dcc);
@@ -343,7 +344,6 @@ int clean_typed(ctr_ctx* ctx, const ctr_clean_params* cp, ctr_clean_counts* out)
   }
   ctx->last_counts[0] = (int64_t)newV;
   ctx->last_counts[1] = (int64_t)newT;
-  ctx->last3_edited |= EDIT_CLEAN;
   out->n_verts = (int64_t)newV;
   out->n_tris = (int64_t)newT;
   out->n_quantized = hc.n_quant;

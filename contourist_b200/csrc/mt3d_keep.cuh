@@ -1,4 +1,4 @@
-// Component filter (ctr_mt3d_keep_components) -- included by mt3d.cu after compact3d.cuh, inside its anonymous
+// Component filter (ctr_mt3d_keep_components) -- included by mesh3d.cu after compact3d.cuh, inside its anonymous
 // namespace.
 //
 // The labels (AUX_LABELS) and the table (AUX_COMPONENTS) of the last ctr_mt3d_components call say which component every
@@ -45,7 +45,6 @@ int keep_components_run(ctr_ctx* ctx, const uint8_t* keep, int64_t* out_verts, i
   // values interpolated on this very mesh are compacted with it; older ones are left as they are
   const bool values = ctx->attr_ncomp > 0 && ctx->attr_gen == ctx->mesh_gen;
   const size_t vrow = std::max<size_t>(3 * gsz, values ? (size_t)ctx->attr_ncomp * gsz : 0);   // widest vertex row
-  ctx->mesh_gen++;                                    // from here on the mesh is edited
   cudaStream_t st = ctx->stream;
   int rc;
   const int tiles_c = (int)(((size_t)nC + SC_TILE - 1) / SC_TILE);
@@ -82,6 +81,7 @@ int keep_components_run(ctr_ctx* ctx, const uint8_t* keep, int64_t* out_verts, i
   CTR_CUDA(ctx, cudaGetLastError());
   KeepCounters h;
   size_t newV, newT;
+  mesh_edited(ctx, EDIT_KEEP);
   if ((rc = compact_mesh(ctx, cb, nV, nT, (const int*)ctx->tris.p, 0u, values, &h, newV, newT))) return rc;
   const size_t newC = (size_t)h.total;
   if (nT) {
@@ -98,7 +98,6 @@ int keep_components_run(ctr_ctx* ctx, const uint8_t* keep, int64_t* out_verts, i
   CTR_CUDA(ctx, cudaStreamSynchronize(st));
   ctx->last_counts[0] = (int64_t)newV;
   ctx->last_counts[1] = (int64_t)newT;
-  ctx->last3_edited |= EDIT_KEEP;
   ctx->comp_tris = (int64_t)newT;
   ctx->comp_count = (int64_t)newC;
   ctx->comp_gen = ctx->mesh_gen;

@@ -215,11 +215,11 @@ int select_typed(ctr_ctx* ctx, const ctr_mt3d_params* p, const int32_t* seeds, i
   CTR_CUDA(ctx, cudaGetLastError());
   unsigned h_voxels = 0;
   size_t newV, newT;
+  mesh_edited(ctx, EDIT_SELECT);
   if ((rc = compact_mesh(ctx, cb, nV, nT, (const int*)ctx->tris.p, g.id_base, false, &h_voxels, newV, newT))) return rc;
   CTR_CUDA(ctx, cudaStreamSynchronize(st));
   ctx->last_counts[0] = (int64_t)newV;
   ctx->last_counts[1] = (int64_t)newT;
-  ctx->last3_edited |= EDIT_SELECT;
   if (out_verts) *out_verts = (int64_t)newV;
   if (out_tris) *out_tris = (int64_t)newT;
   if (out_voxels) *out_voxels = (int64_t)h_voxels;

@@ -1,6 +1,5 @@
 // Face-normal sums and per-vertex normals of a 3D device mesh, shared by the passes that move vertices: smoothing
-// (smooth3d.cuh, mesh3d.cu) and decimation (decimate3d.cuh, mt3d.cu).  Included inside each translation unit's
-// anonymous namespace.  The definition is oracle/mt3d_smooth.py:normals (within rounding: the face normals are summed
+// (smooth3d.cuh) and decimation (decimate3d.cuh).  Included by mesh3d.cu inside its anonymous namespace.  The definition is oracle/mt3d_smooth.py:normals (within rounding: the face normals are summed
 // with atomics).
 //   k_s_nsum : per triangle, cross(b - a, c - a) in fp64 added to its three corners (fp64 atomicAdd);
 //   k_s_nfin : per vertex, the sum normalised, its sign chosen so that it does not point against the old normal; a zero

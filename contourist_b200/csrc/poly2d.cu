@@ -259,8 +259,7 @@ extern "C" int ctr_mt2d_polylines(ctr_ctx* ctx, ctr_poly_counts* out) {
   if (ctx->last_kind != 2 || (ctx->last_flags & CTR_NO_GEOMETRY))
     return ctr_fail(ctx, CTR_ERR_STATE, "no completed ctr_mt2d_run with geometry to chain");
   CTR_CUDA(ctx, cudaSetDevice(ctx->device));
-  if (ctx->last_flags & CTR_GEOM_F64) return polylines_typed<double>(ctx, out);
-  return polylines_typed<float>(ctx, out);
+  return with_geom_type(ctx, [&](auto g) { return polylines_typed<decltype(g)>(ctx, out); });
 }
 
 extern "C" int ctr_mt2d_polylines_fetch(ctr_ctx* ctx, int32_t* level, uint8_t* closed, uint64_t* start_key, uint32_t* offset,

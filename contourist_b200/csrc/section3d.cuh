@@ -3,7 +3,7 @@
 // Included into mesh3d.cu after components3d.cuh and smooth3d.cuh, inside its anonymous namespace.  The definition is
 // oracle/mt3d_section.py:section.  Plane l is {x : n . x == offsets[l]}; a vertex is high for it when
 // s = (n0 x + n1 y) + n2 z >= offsets[l] (fp64, every operation rounded on its own).
-//   k_o_init / k_m_edges : the components pass's edge table: every undirected edge once, triangle ids checked;
+//   k_m_init / k_m_edges : the components pass's edge table: every undirected edge once, triangle ids checked;
 //   k_sec_count : per triangle the planes it crosses, [first, first + count), by binary search of its side range over
 //                 the offsets (every 2^shift-th offset staged in shared memory, the last steps in global memory);
 //   k_s_scan    : (smoothing's) counts -> the first segment of every triangle, with the exact 64-bit total;
@@ -295,8 +295,7 @@ int section_typed(ctr_ctx* ctx, const ctr_section_params* sp, ctr_section_counts
     return finish(0, 0, 0, 0);
   }
   // ---- edge table, crossings per triangle, their scan; one host wait for the total
-  size_t nslots = 1;
-  while (nslots < (size_t)nt * 4) nslots <<= 1;       // as in components_typed
+  const size_t nslots = edge_slots(nt);
   const unsigned blocks = (nt + SEC_THREADS - 1) / SEC_THREADS;   // also the look-back tiles of k_s_scan
   DevBuf& b_etab = ctx->aux[AUX_SCRATCH0];
   DevBuf& b_tri = ctx->aux[AUX_SCRATCH1];
@@ -318,7 +317,8 @@ int section_typed(ctr_ctx* ctx, const ctr_section_params* sp, ctr_section_counts
   while (((P.np + (1 << P.shift) - 1) >> P.shift) > SEC_STAGE) ++P.shift;
   const G* verts = (const G*)ctx->verts.p;
   const int* tris = (const int*)ctx->tris.p;
-  k_o_init<<<ctx->sm_count * 8, 256, 0, st>>>(etab, nslots, nullptr, 0u, nullptr, nullptr);
+  // the (component, vertex) table of k_m_init aliases the edge table: this pass does not read slot.tri
+  k_m_init<<<ctx->sm_count * 8, 256, 0, st>>>(etab, etab, nslots, nullptr, 0u);
   k_m_edges<<<blocks, M_THREADS, 0, st>>>(tris, nt, nv, etab, nslots - 1, &ctr->m);
   k_sec_count<G><<<std::min(blocks, (unsigned)ctx->sm_count * 4), SEC_THREADS, 0, st>>>(verts, tris, nt, nv, P, cnt, first);
   k_s_scan<<<blocks, S_THREADS, 0, st>>>(cnt, nt, seg_off, status, ctr, (int)blocks);
@@ -327,7 +327,7 @@ int section_typed(ctr_ctx* ctx, const ctr_section_params* sp, ctr_section_counts
   SCounters h;
   CTR_CUDA(ctx, cudaMemcpyAsync(&h, ctr, sizeof h, cudaMemcpyDeviceToHost, st));
   CTR_CUDA(ctx, cudaStreamSynchronize(st));
-  if (h.m.bad) return ctr_fail(ctx, CTR_ERR_STATE, "triangle ids outside [0, n_verts): the ids were shifted (ctr_mt3d_offset_ids)");
+  if (h.m.bad) return fail_shifted_ids(ctx);
   if (h.m.total >= (1ull << 31)) return ctr_fail(ctx, CTR_ERR_OVERFLOW, "2^31 or more section segments: use fewer planes");
   const size_t S = (size_t)h.m.total, nd = 2 * S;
   if ((rc = ctr_carve_buf(ctx, ctx->aux[AUX_SECTION_SEGS], [&](ctr_carve& c) { sg.carve(c, S, gsz, nplanes); }))) return rc;

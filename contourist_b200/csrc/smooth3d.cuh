@@ -175,8 +175,7 @@ int smooth_typed(ctr_ctx* ctx, const ctr_smooth_params* sp, ctr_smooth_counts* o
     out->n_fixed_verts = nv;
     return 0;
   }
-  size_t nslots = 1;
-  while (nslots < (size_t)nt * 4) nslots <<= 1;       // the components pass's table size: load <= 3/4
+  const size_t nslots = edge_slots(nt);
   const unsigned blocks_t = (nt + S_THREADS - 1) / S_THREADS, tiles_v = (nv + S_THREADS - 1) / S_THREADS;
   const unsigned slot_blocks = (unsigned)ctx->sm_count * 8;
   int rc;
@@ -207,7 +206,7 @@ int smooth_typed(ctr_ctx* ctx, const ctr_smooth_params* sp, ctr_smooth_counts* o
   SCounters h;
   CTR_CUDA(ctx, cudaMemcpyAsync(&h, ctr, sizeof h, cudaMemcpyDeviceToHost, st));
   CTR_CUDA(ctx, cudaStreamSynchronize(st));
-  if (h.m.bad) return ctr_fail(ctx, CTR_ERR_STATE, "triangle ids outside [0, n_verts): the ids were shifted (ctr_mt3d_offset_ids)");
+  if (h.m.bad) return fail_shifted_ids(ctx);
   k_s_fixed<<<slot_blocks, 256, 0, st>>>(etab, nslots, fixed, ctr);
   k_s_degree<<<slot_blocks, 256, 0, st>>>(etab, nslots, fixed, cur);
   k_s_scan<<<tiles_v, S_THREADS, 0, st>>>(cur, nv, off, status, ctr, (int)tiles_v);   // (nv > 0: the ids were checked)
@@ -222,8 +221,7 @@ int smooth_typed(ctr_ctx* ctx, const ctr_smooth_params* sp, ctr_smooth_counts* o
   if ((rc = ctr_ensure(ctx, b_nbr, (size_t)h.m.total * 4))) return rc;
   if ((rc = ctr_ensure(ctx, b_x0, n3 * 8))) return rc;
   if ((rc = ctr_ensure(ctx, b_x1, n3 * 8))) return rc;
-  ctx->mesh_gen++;                                    // from here on the mesh is edited
-  ctx->last3_edited |= EDIT_SMOOTH;
+  mesh_edited(ctx, EDIT_SMOOTH);
   int* nbr = (int*)b_nbr.p;
   double* x = (double*)b_x0.p;
   double* y = (double*)b_x1.p;
