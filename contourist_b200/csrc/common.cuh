@@ -56,6 +56,7 @@ enum Edit3 : unsigned {
   EDIT_DECIMATE = 16u,       // decimation
   EDIT_CAP = 32u,            // caps at the box faces
   EDIT_ORIENT = 64u,         // reference orientation (rewinds triangles only: the mesh generation stays)
+  EDIT_CLIP = 128u,          // clipping by a plane or a vertex value
 };
 
 // What a pass on the device mesh of the last 3D run needs of that run, and which earlier passes refuse it: one row per
@@ -86,18 +87,21 @@ constexpr PassRule PASS_DECIMATE = {" to decimate", false, FULL_ID0, CTR_ERR_STA
 // be applied once per run, and before any other edit (an oriented mesh has the same rows)
 constexpr PassRule PASS_SELECT = {" to select from", false, FULL, CTR_ERR_UNSUPPORTED,
                                   "seeded selection needs a full-volume run (components cross slab faces)",
-                                  EDIT_SELECT | EDIT_CLEAN | EDIT_KEEP | EDIT_SMOOTH | EDIT_DECIMATE | EDIT_CAP,
+                                  EDIT_SELECT | EDIT_CLEAN | EDIT_KEEP | EDIT_SMOOTH | EDIT_DECIMATE | EDIT_CAP | EDIT_CLIP,
                                   "run ctr_mt3d_run again"};
 // the reference's clean-up (quantize, tiny simplices) is defined on the interpolated positions
 constexpr PassRule PASS_CLEAN = {" to clean", false, FULL_ID0, CTR_ERR_UNSUPPORTED,
                                  "mesh clean-up needs a full-volume run (merges cross slab faces)",
-                                 EDIT_CLEAN | EDIT_SMOOTH | EDIT_DECIMATE | EDIT_CAP,
-                                 "clean it up once, before smoothing, decimating or capping"};
+                                 EDIT_CLEAN | EDIT_SMOOTH | EDIT_DECIMATE | EDIT_CAP | EDIT_CLIP,
+                                 "clean it up once, before smoothing, decimating, capping or clipping"};
 // after these passes the field no longer tells where the mesh's rim is or which way it faces
 constexpr PassRule PASS_CAP = {" to cap", true, FULL_ID0_PLANE0, CTR_ERR_STATE,
                                "caps need a full-volume run with plane_offset 0 and vert_id_base 0 (the box of a slab is not the volume's)",
-                               EDIT_SELECT | EDIT_CLEAN | EDIT_KEEP | EDIT_DECIMATE | EDIT_CAP | EDIT_ORIENT,
+                               EDIT_SELECT | EDIT_CLEAN | EDIT_KEEP | EDIT_DECIMATE | EDIT_CAP | EDIT_ORIENT | EDIT_CLIP,
                                "cap it before those passes"};
+// the clip keeps the part of the mesh on one side: any earlier pass, an earlier clip too (six clips make a box)
+constexpr PassRule PASS_CLIP = {" to clip", false, FULL_ID0, CTR_ERR_STATE,
+                                "clipping needs a full-volume run with vert_id_base 0 (a slab's halo ids belong to another shard)", 0u, nullptr};
 constexpr PassRule PASS_INTERPOLATE = {" to interpolate on", true, ANY_RUN, 0, nullptr, 0u, nullptr};
 constexpr PassRule PASS_OFFSET_IDS = {"", false, ANY_RUN, 0, nullptr, 0u, nullptr};
 
@@ -263,9 +267,10 @@ static inline int check_pass(ctr_ctx* ctx, const PassRule& r) {
       (r.slab >= FULL_ID0_PLANE0 && p->plane_offset != 0))
     return ctr_fail(ctx, r.slab_code, r.slab_msg);
   if (const unsigned done = ctx->last3_edited & r.refused_after) {
-    static const char* const names[] = {"selected from", "cleaned", "filtered", "smoothed", "decimated", "capped", "oriented"};
+    static const char* const names[] = {"selected from", "cleaned", "filtered", "smoothed", "decimated", "capped", "oriented",
+                                              "clipped"};
     std::string list;
-    for (int b = 0; b < 7; ++b)
+    for (int b = 0; b < 8; ++b)
       if (done & (1u << b)) list += std::string(list.empty() ? "" : ", ") + names[b];
     return ctr_fail(ctx, CTR_ERR_STATE, ("the mesh of this run has been " + list).c_str(), r.order_msg);
   }

@@ -14,6 +14,8 @@
 // components3d.cuh (ctr_mt3d_components) reuses the edge table and k_o_union to number and measure the components.
 // smooth3d.cuh (ctr_mt3d_smooth) builds the same edge table with its use counts for the fixed vertices and neighbour lists.
 // section3d.cuh (ctr_mt3d_section) names the crossing vertices of its plane sections by their slots in that table.
+// clip3d.cuh (ctr_mt3d_clip) keeps the part of the mesh on one side of a plane or a vertex value, with the section's side
+// test and crossing point, the caps' corner walk and one new vertex per crossed edge, found in the same kind of table.
 #include <math.h>
 #include <string.h>
 
@@ -244,6 +246,7 @@ int orient_typed(ctr_ctx* ctx, int64_t* n_components, int64_t* n_flipped) {
 #include "decimate3d.cuh"
 #include "attr3d.cuh"
 #include "cap3d.cuh"
+#include "clip3d.cuh"
 
 }  // namespace
 
@@ -406,6 +409,28 @@ extern "C" int ctr_mt3d_cap(ctr_ctx* ctx, const ctr_cap_params* cp, ctr_cap_coun
   return with_sample_type(ctx, ((const ctr_mt3d_params*)ctx->last3_params)->dtype, [&](auto t) {
     return with_geom_type(ctx, [&](auto g) { return cap_typed<decltype(t), decltype(g)>(ctx, cp, out); });
   });
+}
+
+extern "C" int ctr_mt3d_clip(ctr_ctx* ctx, const ctr_clip_params* cp, ctr_clip_counts* out) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (!cp || !out) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  memset(out, 0, sizeof *out);
+  if (cp->source != CTR_CLIP_PLANE && cp->source != CTR_CLIP_VALUE)
+    return ctr_fail(ctx, CTR_ERR_BAD_ARG, "source must be CTR_CLIP_PLANE or CTR_CLIP_VALUE");
+  if (cp->side != CTR_CLIP_HIGH && cp->side != CTR_CLIP_LOW) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "side must be CTR_CLIP_HIGH or CTR_CLIP_LOW");
+  const double* n = cp->normal;
+  if (cp->source == CTR_CLIP_PLANE) {
+    if (!(isfinite(n[0]) && isfinite(n[1]) && isfinite(n[2])) || (n[0] == 0.0 && n[1] == 0.0 && n[2] == 0.0))
+      return ctr_fail(ctx, CTR_ERR_BAD_ARG, "normal must be finite and not zero");
+    if (cp->component != 0) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "component must be 0 for a plane clip");
+  } else {
+    if (n[0] != 0.0 || n[1] != 0.0 || n[2] != 0.0) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "normal must be 0 for a value clip");
+    if (cp->component < 0) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "component must be in [0, ncomp) of the last interpolation");
+  }
+  if (!isfinite(cp->offset)) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "offset must be finite");
+  if (cp->reserved != 0) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "reserved must be 0");
+  if (int rc = check_pass(ctx, PASS_CLIP)) return rc;
+  return with_geom_type(ctx, [&](auto g) { return clip_typed<decltype(g)>(ctx, cp, out); });
 }
 
 extern "C" int ctr_mt3d_interpolate(ctr_ctx* ctx, const ctr_attr_params* a, int64_t* n_verts) {

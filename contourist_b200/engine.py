@@ -126,6 +126,20 @@ class SectionCounts(ctypes.Structure):
                 ("n_junction_planes", ctypes.c_int64)]
 
 
+class ClipParams(ctypes.Structure):
+    _fields_ = [("source", ctypes.c_int32), ("side", ctypes.c_int32), ("normal", ctypes.c_double * 3),
+                ("offset", ctypes.c_double), ("component", ctypes.c_int32), ("reserved", ctypes.c_uint32)]
+
+
+class ClipCounts(ctypes.Structure):
+    _fields_ = [("n_verts", ctypes.c_int64), ("n_tris", ctypes.c_int64), ("n_new_verts", ctypes.c_int64),
+                ("n_cut_tris", ctypes.c_int64), ("n_dropped_tris", ctypes.c_int64)]
+
+
+CLIP_PLANE, CLIP_VALUE = 0, 1
+CLIP_SIDES = {"high": 0, "low": 1}
+
+
 class PolyCounts(ctypes.Structure):
     _fields_ = [("n_polylines", ctypes.c_int64), ("n_points", ctypes.c_int64), ("junction_levels", ctypes.c_uint64)]
 
@@ -202,6 +216,8 @@ def load_library():
     lib.ctr_mt3d_section_segments_fetch.restype = i32
     lib.ctr_mt3d_section_polylines_fetch.argtypes = [vp] * 9
     lib.ctr_mt3d_section_polylines_fetch.restype = i32
+    lib.ctr_mt3d_clip.argtypes = [vp, ctypes.POINTER(ClipParams), ctypes.POINTER(ClipCounts)]
+    lib.ctr_mt3d_clip.restype = i32
     lib.ctr_mt3d_interpolate.argtypes = [vp, ctypes.POINTER(AttrParams), ctypes.POINTER(i64)]
     lib.ctr_mt3d_interpolate.restype = i32
     lib.ctr_mt3d_interpolate_fetch.argtypes = [vp, vp]
@@ -632,6 +648,39 @@ class Engine(object):
             out[int(plane[q])].append((bool(fl[q] & 1), bool(fl[q] & 2), pts[int(o[q]):int(o[q]) + int(ln[q])],
                                        float(meas[q, 0]), float(meas[q, 1])))
         return seg, out
+
+    def mt3d_clip(self, normal=None, offset=0.0, keep="high", component=None):
+        """Keep the part of the last 3D run's device mesh as it stands now on one side of a plane or of a vertex value,
+        in place (ctr_mt3d_clip; oracle/mt3d_clip.py is the definition).  Give exactly one of `normal` (a plane:
+        s = (n0 x + n1 y) + n2 z of each vertex, in the units of the current positions) and `component` (s = that
+        component of the values of an mt3d_interpolate() made on the mesh as it stands).  keep="high" keeps
+        s >= offset, "low" keeps s < offset.  Triangles across the cut are split at one new vertex per crossed edge
+        (positions, normals and carried vertex values interpolated along the edge, keys from the kept end) and keep
+        their winding; kept vertices stay in order, new ones follow.  Every vertex kept: nothing changes.  Accepted after
+        every pass (six clips make a box); afterwards mt3d_select_seeded(), mt3d_clean() and mt3d_cap() are refused, and
+        mt3d_components() must measure again before mt3d_keep_components().  Device pointers (mt3d_device_ptrs(),
+        mt3d_interpolate_device_ptr()) must be taken again.  Returns ClipCounts (n_verts, n_tris, n_new_verts,
+        n_cut_tris, n_dropped_tris); fetch afterwards."""
+        if (normal is None) == (component is None):
+            raise ValueError("give exactly one of normal (a plane clip) and component (a value clip)")
+        if keep not in CLIP_SIDES:
+            raise ValueError("keep must be 'high' or 'low', not %r" % (keep,))
+        p = ClipParams()
+        p.side = CLIP_SIDES[keep]
+        p.offset = float(offset)
+        if normal is not None:
+            n = np.asarray(normal, np.float64).reshape(3)
+            p.source = CLIP_PLANE
+            for a in range(3):
+                p.normal[a] = float(n[a])
+        else:
+            p.source = CLIP_VALUE
+            p.component = int(component)
+        c = ClipCounts()
+        self.run_serial += 1
+        self._check(self.lib.ctr_mt3d_clip(self.h, ctypes.byref(p), ctypes.byref(c)), "ctr_mt3d_clip")
+        self._mesh_edited(c.n_verts, c.n_tris)
+        return c
 
     def mt3d_interpolate(self, field, shape=None, dtype=None):
         """Values of another field at the vertices of the last 3D run's mesh as it stands now (after a selection or

@@ -171,6 +171,11 @@ class GridContour3d(object):
     # non-manifold edge
     sections = None
     section_polylines = None
+    # clip_halfspaces = (A, b), A [m, 3] and b [m] in world units: get_points_and_triangles() keeps the part of the mesh
+    # in {x : A x < b} on the device, one plane clip per row in row order (ctr_mt3d_clip, keep "low"; the convention of
+    # the reference's constraints.py), after decimation and before vertex_fields, measure_components and sections,
+    # which then describe the clipped mesh.  Triangles across a plane are split on it; six rows make a box.
+    clip_halfspaces = None
 
     def __init__(self, corner, function, value, segment_endpoints, linear_interpolate=True, callback=None,
                  origin=(0.0, 0.0, 0.0), delta=(1.0, 1.0, 1.0)):
@@ -217,6 +222,7 @@ class GridContour3d(object):
             # smoothing and decimation are other algorithms behind their own options (smooth_iterations,
             # decimate_cell), so these keep raising rather than silently giving a different mesh
             raise NotImplementedError("flatten / smooth (LP-based decimation, tetrahedral.py:217-351) are out of scope")
+        halfspaces = self._halfspaces()
         eng = E.default_engine()
         flags = (E.GEOM_F64 if np.dtype(self.geometry_dtype) == np.float64 else 0) | (E.WANT_NORMALS if self.want_normals else 0)
         if self.vertex_fields is not None or self.cap is not None:
@@ -274,6 +280,11 @@ class GridContour3d(object):
             # voxels in the world coordinates the mesh has by now, aligned with the voxel grid
             cell = np.asarray(self.decimate_cell, np.float64) * np.abs(np.asarray(self.delta, np.float64))
             eng.mt3d_decimate(cell, origin=tuple(float(x) for x in self.origin))
+        clipped = halfspaces is not None
+        if clipped:
+            # after every other edit, before the values and the measurement below: row i keeps A[i] . x < b[i]
+            for a, b in zip(*halfspaces):
+                eng.mt3d_clip(normal=a, offset=b, keep="low")
         if self.vertex_fields is not None:
             # after every pass that edits the mesh: the values line up with the points fetched below
             many = isinstance(self.vertex_fields, (list, tuple))
@@ -284,7 +295,7 @@ class GridContour3d(object):
             # after every pass that edits the mesh, like the values above; the filter has already measured this mesh,
             # unless smoothing or decimation has changed it since
             self.triangle_components, self.component_table = \
-                eng.mt3d_components_fetch() if self.keep_components is not None and not (smoothed or decimated) \
+                eng.mt3d_components_fetch() if self.keep_components is not None and not (smoothed or decimated or clipped) \
                 else eng.mt3d_components()
         if self.sections is not None:
             normal, offsets = self.sections
@@ -295,6 +306,24 @@ class GridContour3d(object):
         if self.callback:
             self.callback(self)
         return (points, triangles)
+
+    def _halfspaces(self):
+        "clip_halfspaces checked: (A [m, 3], b [m]) as finite fp64 arrays with non-zero rows, or None"
+        if self.clip_halfspaces is None:
+            return None
+        try:
+            A, b = self.clip_halfspaces
+        except (TypeError, ValueError):
+            raise ValueError("clip_halfspaces must be a pair (A [m, 3], b [m])")
+        A = np.asarray(A, np.float64)
+        b = np.asarray(b, np.float64)
+        if A.ndim != 2 or A.shape[1] != 3 or b.shape != (A.shape[0],):
+            raise ValueError("clip_halfspaces: A must be [m, 3] and b [m], not %r and %r" % (A.shape, b.shape))
+        if not (np.isfinite(A).all() and np.isfinite(b).all()):
+            raise ValueError("clip_halfspaces: A and b must be finite")
+        if len(A) and not np.any(A != 0.0, axis=1).all():
+            raise ValueError("clip_halfspaces: every row of A must be non-zero")
+        return A, b
 
     def extract_surface_geometry(self, clean=True):
         points, triangles = self.get_points_and_triangles(clean)
@@ -344,7 +373,7 @@ class Delta3DContour(object):
         "options set on this driver (before or after the maker was built) reach the maker"
         for name in ("post_process", "geometry_dtype", "want_normals", "reference_orientation", "quantize_divisions",
                      "tiny_epsilon", "vertex_fields", "measure_components", "keep_components", "smooth_iterations",
-                     "smooth_lambda", "smooth_mu", "decimate_cell", "cap", "sections"):
+                     "smooth_lambda", "smooth_mu", "decimate_cell", "cap", "sections", "clip_halfspaces"):
             if hasattr(self, name):
                 setattr(maker, name, getattr(self, name))
         maker.field_grid = self.grid

@@ -421,6 +421,60 @@ CTR_API int ctr_mt3d_section_segments_fetch(ctr_ctx* ctx, int32_t* plane, int32_
 CTR_API int ctr_mt3d_section_polylines_fetch(ctr_ctx* ctx, int32_t* plane, uint8_t* flags, uint64_t* start_key, uint32_t* offset,
                                              uint32_t* length, double* measures, void* points, uint8_t* junction);
 
+/* Clipping of the LAST 3D run's device mesh as it stands now by a plane or by a vertex value (engine extension, like
+ * VTK's vtkClipPolyData; oracle/mt3d_clip.py:clip is the definition).  The mesh is rewritten in place; synchronous on
+ * return.
+ *   - Side value of a vertex: CTR_CLIP_PLANE s = (n0 x + n1 y) + n2 z in fp64 on the positions widened from the geometry
+ *     type, each operation rounded on its own (the side test of ctr_mt3d_section); CTR_CLIP_VALUE s = component
+ *     `component` of the vertex values of a ctr_mt3d_interpolate made on the mesh as it stands, widened to fp64.  A
+ *     vertex is high when s >= offset and low otherwise, so no vertex is ever on the cut; it is kept when it is on `side`.
+ *   - Vertices: the kept ones in their order (also one no triangle uses), then one new vertex per distinct undirected
+ *     edge {a, b} of some triangle whose ends are on different sides, ordered by first use (the smallest index of a
+ *     triangle on the edge, then the edge's position (v0,v1), (v1,v2), (v2,v0) in it; a non-manifold edge gets one
+ *     vertex too).  With a the low end, t = (offset - s_a) / (s_b - s_a) and the position is p_a + t * (p_b - p_a) per
+ *     axis, fp64, rounded once to the geometry type: in plane mode the point ctr_mt3d_section gives for that edge and
+ *     offset, bit for bit.  Normal (CTR_WANT_NORMALS): m = n_a + t * (n_b - n_a), then m / sqrt((mx*mx + my*my) + mz*mz)
+ *     rounded once (the kept end's normal where that length is 0).  key and lowmin (CTR_WANT_KEYS): the kept end's, so
+ *     a later ctr_mt3d_interpolate gives a rim vertex its kept end's value and keys are no longer distinct.  Vertex
+ *     values made on the mesh as it stands are carried (kept rows compacted, new rows v_a + t * (v_b - v_a), rounded
+ *     once) and stay valid for the clipped mesh: interpolate first, then clip, for interpolated rim values.
+ *   - Triangles: each input triangle (v0, v1, v2) walks i = 0, 1, 2 and emits corner i if it is kept, then the crossing
+ *     of edge (i, i+1 mod 3) if exactly one end of that edge is kept.  3 tokens give one triangle, 4 the fan
+ *     (p0, p1, p2), (p0, p2, p3), 0 drop it.  Output by input triangle, then piece: every piece has the winding of its
+ *     source triangle.  At most 2 n_tris triangles.
+ *   - Every vertex kept: nothing is written and no state changes (n_new_verts = n_cut_tris = n_dropped_tris = 0).  No
+ *     vertex kept: the mesh becomes empty.
+ *   - Afterwards: the published counts, cells and codes stay those of the run; the output buffers and the vertex values
+ *     may have been reallocated, so take device pointers (ctr_mt3d_device_ptrs, ctr_mt3d_interpolate_device_ptr) again.
+ *     Section results stay; component results are stale.  ctr_mt3d_select_seeded, ctr_mt3d_clean and ctr_mt3d_cap
+ *     return CTR_ERR_STATE (their rules are defined on the field's mesh); every other pass, a further clip included, is
+ *     accepted.  ctr_mt3d_smooth keeps boundary vertices fixed, so clip, then smooth, keeps the cut on the plane.
+ *   - CTR_ERR_BAD_ARG: a NULL argument; source or side not one of the values below; a zero or non-finite normal in plane
+ *     mode, a non-zero normal in value mode; a non-finite offset; component not 0 in plane mode or outside [0, ncomp) in
+ *     value mode; reserved != 0; a NaN side value.  CTR_ERR_STATE: no 3D run or a CTR_NO_GEOMETRY run; a slab run
+ *     (i_lo != 0 or i_hi != n0) or vert_id_base != 0; a triangle id outside [0, n_verts) (e.g. after
+ *     ctr_mt3d_offset_ids); value mode with no ctr_mt3d_interpolate on the mesh as it stands.  CTR_ERR_OVERFLOW: 2^31 or
+ *     more vertices or triangles after the clip.  All are detected before anything is written.                         */
+#define CTR_CLIP_PLANE 0   /* s = (n0 x + n1 y) + n2 z of the vertex position                                            */
+#define CTR_CLIP_VALUE 1   /* s = component `component` of the current vertex values                                     */
+#define CTR_CLIP_HIGH 0    /* keep s >= offset                                                                           */
+#define CTR_CLIP_LOW 1     /* keep s <  offset                                                                           */
+typedef struct {
+  int32_t source;          /* CTR_CLIP_PLANE or CTR_CLIP_VALUE                                                           */
+  int32_t side;            /* CTR_CLIP_HIGH or CTR_CLIP_LOW                                                              */
+  double normal[3];        /* PLANE: finite, not zero; VALUE: all 0                                                      */
+  double offset;           /* finite, in the units of the positions (PLANE) or values                                   */
+  int32_t component;       /* VALUE: 0 .. ncomp-1 of the last interpolation; PLANE: 0                                    */
+  uint32_t reserved;       /* 0                                                                                          */
+} ctr_clip_params;                           /* 48 bytes */
+typedef struct {
+  int64_t n_verts, n_tris;                   /* the clipped mesh                                                      */
+  int64_t n_new_verts;                       /* crossing vertices added, one per distinct crossed edge                */
+  int64_t n_cut_tris;                        /* input triangles with corners on both sides                            */
+  int64_t n_dropped_tris;                    /* input triangles with no corner on the kept side                       */
+} ctr_clip_counts;                           /* 40 bytes */
+CTR_API int ctr_mt3d_clip(ctr_ctx* ctx, const ctr_clip_params* p, ctr_clip_counts* out);
+
 /* Seeded extraction (SURVEY.md 8(f3)): restricts the LAST full-volume run's mesh to what the reference's tracker
  *   tetrahedral.py:443-469  expand_voxels / in_range  (flood fill over the 26-neighbourhood of border voxels)
  * reaches from the given start voxels (the output of find_initial_voxels, tetrahedral.py:396-441, which the binding
