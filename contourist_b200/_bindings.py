@@ -1,4 +1,4 @@
-"""ctypes prototypes for the 2D / 4D / post-processing entry points."""
+"""ctypes prototypes for the 2D / 4D / post-processing entry points and the closest-point query."""
 import ctypes
 
 
@@ -28,6 +28,15 @@ class Mp4dCounts(ctypes.Structure):
                 ("fmin", ctypes.c_double), ("fmax", ctypes.c_double), ("t_min", ctypes.c_double), ("t_max", ctypes.c_double)]
 
 
+class ClosestParams(ctypes.Structure):
+    _fields_ = [("points", ctypes.c_void_p), ("dtype", ctypes.c_int32), ("flags", ctypes.c_uint32),
+                ("n_points", ctypes.c_int64), ("max_distance", ctypes.c_double)]
+
+
+class ClosestCounts(ctypes.Structure):
+    _fields_ = [("n_found", ctypes.c_int64), ("height", ctypes.c_int64)]
+
+
 def bind(lib):
     vp, i32 = ctypes.c_void_p, ctypes.c_int
     lib.ctr_mt2d_run.argtypes = [vp, ctypes.POINTER(Mt2dParams), ctypes.POINTER(Mt2dCounts)]
@@ -38,3 +47,7 @@ def bind(lib):
     lib.ctr_mp4d_run.restype = i32
     lib.ctr_mp4d_fetch.argtypes = [vp] + [vp] * 9
     lib.ctr_mp4d_fetch.restype = i32
+    lib.ctr_mt3d_closest.argtypes = [vp, ctypes.POINTER(ClosestParams), ctypes.POINTER(ClosestCounts)]
+    lib.ctr_mt3d_closest.restype = i32
+    lib.ctr_mt3d_closest_fetch.argtypes = [vp] * 4
+    lib.ctr_mt3d_closest_fetch.restype = i32

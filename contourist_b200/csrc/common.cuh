@@ -45,6 +45,9 @@ enum Aux3 : int {
   AUX_COMPONENTS = 45,       // component table
   AUX_SECTION_SEGS = 1,      // plane sections (ctr_mt3d_section): segments and junction planes
   AUX_SECTION_POLYS = 3,     // ... polylines, their points and measures
+  AUX_CLOSEST_RESULT = 48,   // closest points (ctr_mt3d_closest): distance, triangle, point per query point
+  AUX_CLOSEST_TREE = 49,     // ... the tree of the last call (rebuilt by every call)
+  AUX_CLOSEST_POINTS = 50,   // ... its host query points, staged
 };
 
 // ctr_ctx::last3_edited: the passes that have rewritten the device mesh of the last 3D run
@@ -102,6 +105,10 @@ constexpr PassRule PASS_CAP = {" to cap", true, FULL_ID0_PLANE0, CTR_ERR_STATE,
 // the clip keeps the part of the mesh on one side: any earlier pass, an earlier clip too (six clips make a box)
 constexpr PassRule PASS_CLIP = {" to clip", false, FULL_ID0, CTR_ERR_STATE,
                                 "clipping needs a full-volume run with vert_id_base 0 (a slab's halo ids belong to another shard)", 0u, nullptr};
+// the closest-point query reads the mesh as it stands after any pass
+constexpr PassRule PASS_CLOSEST = {" to query", false, FULL_ID0, CTR_ERR_STATE,
+                                   "closest points need a full-volume run with vert_id_base 0 (a slab's halo ids belong to another shard)",
+                                   0u, nullptr};
 constexpr PassRule PASS_INTERPOLATE = {" to interpolate on", true, ANY_RUN, 0, nullptr, 0u, nullptr};
 constexpr PassRule PASS_OFFSET_IDS = {"", false, ANY_RUN, 0, nullptr, 0u, nullptr};
 
@@ -166,9 +173,12 @@ struct ctr_ctx {
   // run), polylines, points, junction planes; and the number of planes
   int64_t sect_count[4] = {-1, 0, 0, 0};
   int32_t sect_nplanes = 0;
+  // 3D closest points (ctr_mt3d_closest) in AUX_CLOSEST_RESULT: query points of the last successful call; -1 = none since
+  // the last 3D run (or the last call failed)
+  int64_t closest_n = -1;
 
   // extra outputs and scratch in generic slots: 3D (Aux3 above); 5-10: 2D; 12-26: 4D; 36-40: 2D polylines
-  DevBuf aux[48];
+  DevBuf aux[51];
 };
 
 static inline int ctr_fail(ctr_ctx* ctx, int code, const char* what, const char* detail = "") {

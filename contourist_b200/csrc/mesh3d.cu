@@ -16,10 +16,13 @@
 // section3d.cuh (ctr_mt3d_section) names the crossing vertices of its plane sections by their slots in that table.
 // clip3d.cuh (ctr_mt3d_clip) keeps the part of the mesh on one side of a plane or a vertex value, with the section's side
 // test and crossing point, the caps' corner walk and one new vertex per crossed edge, found in the same kind of table.
+// closest3d.cuh (ctr_mt3d_closest) finds the closest point of the mesh to query points through a tree it builds per call.
 #include <math.h>
 #include <string.h>
 
 #include <algorithm>
+
+#include <cub/device/device_radix_sort.cuh>             // header-only, with the toolkit: the sort of closest3d.cuh
 
 #include "common.cuh"
 #include "uf_hash.cuh"
@@ -247,6 +250,7 @@ int orient_typed(ctr_ctx* ctx, int64_t* n_components, int64_t* n_flipped) {
 #include "attr3d.cuh"
 #include "cap3d.cuh"
 #include "clip3d.cuh"
+#include "closest3d.cuh"
 
 }  // namespace
 
@@ -431,6 +435,53 @@ extern "C" int ctr_mt3d_clip(ctr_ctx* ctx, const ctr_clip_params* cp, ctr_clip_c
   if (cp->reserved != 0) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "reserved must be 0");
   if (int rc = check_pass(ctx, PASS_CLIP)) return rc;
   return with_geom_type(ctx, [&](auto g) { return clip_typed<decltype(g)>(ctx, cp, out); });
+}
+
+extern "C" int ctr_mt3d_closest(ctr_ctx* ctx, const ctr_closest_params* cp, ctr_closest_counts* out) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  ctx->closest_n = -1;                                 // a failed call leaves no results
+  if (!cp || !out) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  memset(out, 0, sizeof *out);
+  if (cp->dtype != CTR_F32 && cp->dtype != CTR_F64) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "dtype must be CTR_F32 or CTR_F64");
+  if (cp->flags & ~(uint32_t)CTR_FIELD_ON_DEVICE) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "flags must be 0 or CTR_FIELD_ON_DEVICE");
+  if (cp->n_points < 0 || cp->n_points > 0x7fffffffll) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "n_points must be in [0, 2^31-1]");
+  if (cp->n_points > 0 && !cp->points) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  if (!(cp->max_distance >= 0.0)) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "max_distance must be >= 0 (and not NaN)");
+  const size_t nc = (size_t)cp->n_points * 3;
+  if (!(cp->flags & CTR_FIELD_ON_DEVICE))              // device points are checked on the device, at the first host wait
+    for (size_t i = 0; i < nc; ++i)
+      if (!isfinite(cp->dtype == CTR_F64 ? ((const double*)cp->points)[i] : (double)((const float*)cp->points)[i]))
+        return ctr_fail(ctx, CTR_ERR_BAD_ARG, "query points must be finite");
+  if (int rc = check_pass(ctx, PASS_CLOSEST)) return rc;
+  if ((cp->flags & CTR_FIELD_ON_DEVICE) && nc) {
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, cp->points) != cudaSuccess || at.device != ctx->device ||
+        (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged)) {
+      cudaGetLastError();
+      return ctr_fail(ctx, CTR_ERR_BAD_ARG, "device points must be device memory on the context's device");
+    }
+  }
+  return with_geom_type(ctx, [&](auto g) { return closest_typed<decltype(g)>(ctx, cp, out); });
+}
+
+extern "C" int ctr_mt3d_closest_fetch(ctr_ctx* ctx, double* distance, int32_t* triangle, double* point) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (ctx->last_kind != 3 || ctx->closest_n < 0) return ctr_fail(ctx, CTR_ERR_STATE, "no ctr_mt3d_closest since the last 3D run");
+  const size_t n = (size_t)ctx->closest_n;
+  if (!n) return 0;
+  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  double *dist, *pt;
+  int* tri;
+  ctr_carve c{(char*)ctx->aux[AUX_CLOSEST_RESULT].p, 0};
+  c(dist, n * 8);
+  c(tri, n * 4);
+  c(pt, n * 24);
+  if (distance) CTR_CUDA(ctx, cudaMemcpyAsync(distance, dist, n * 8, cudaMemcpyDefault, st));
+  if (triangle) CTR_CUDA(ctx, cudaMemcpyAsync(triangle, tri, n * 4, cudaMemcpyDefault, st));
+  if (point) CTR_CUDA(ctx, cudaMemcpyAsync(point, pt, n * 24, cudaMemcpyDefault, st));
+  CTR_CUDA(ctx, cudaStreamSynchronize(st));
+  return 0;
 }
 
 extern "C" int ctr_mt3d_interpolate(ctr_ctx* ctx, const ctr_attr_params* a, int64_t* n_verts) {

@@ -1684,6 +1684,7 @@ static int mt3d_dispatch(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts
   ctx->attr_ncomp = 0;                                 // vertex values of the previous run are gone
   ctx->comp_count = -1;                                // ... and so are its components
   ctx->sect_count[0] = -1;                             // ... and its plane sections
+  ctx->closest_n = -1;                                 // ... and its closest points
   return with_sample_type(ctx, p->dtype, [&](auto t) { return run_typed<decltype(t)>(ctx, p, out, phase); });
 }
 

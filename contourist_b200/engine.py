@@ -682,6 +682,43 @@ class Engine(object):
         self._mesh_edited(c.n_verts, c.n_tris)
         return c
 
+    def mt3d_closest(self, points, max_distance=np.inf, n=None, dtype=None):
+        """Closest points of the last 3D run's device mesh as it stands now to query points (ctr_mt3d_closest;
+        oracle/mt3d_closest.py is the definition).  points: numpy [P, 3] in the units of the current positions
+        (float32 / float64 read as they are, other types widened to float64), or an integer device pointer with n and
+        dtype (float32 or float64) -- e.g. another engine's vertices from mt3d_device_ptrs().  For each point: the
+        closest point of the closest triangle (the smallest index on a tie), when it lies within max_distance.  The
+        mesh is not edited; a tree over the triangles is built per call, so batch the points.  Returns
+        (dict(distance [P] float64, triangle [P] int32, point [P, 3] float64), ClosestCounts (n_found, height)); a point
+        not found has distance inf, triangle -1 and point NaN."""
+        from ._bindings import ClosestCounts, ClosestParams
+        p = ClosestParams()
+        if isinstance(points, np.ndarray):
+            if points.ndim != 2 or points.shape[1] != 3:
+                raise ValueError("points of shape (P, 3) expected, not %r" % (points.shape,))
+            if points.dtype not in (np.float32, np.float64):
+                points = points.astype(np.float64)
+            points = np.ascontiguousarray(points)
+            p.points = points.ctypes.data if len(points) else None
+            p.dtype = dtype_code(points.dtype)
+            p.flags = 0
+            P = len(points)
+        else:
+            if n is None or dtype is None:
+                raise ValueError("device points need n and dtype")
+            p.points = int(points)
+            p.dtype = _device_code(dtype, FLOAT_CODES)
+            p.flags = FIELD_ON_DEVICE
+            P = int(n)
+        p.n_points = P
+        p.max_distance = float(max_distance)
+        c = ClosestCounts()
+        self._check(self.lib.ctr_mt3d_closest(self.h, ctypes.byref(p), ctypes.byref(c)), "ctr_mt3d_closest")
+        out = dict(distance=np.empty(P, np.float64), triangle=np.empty(P, np.int32), point=np.empty((P, 3), np.float64))
+        self._check(self.lib.ctr_mt3d_closest_fetch(self.h, _ptr(out["distance"]), _ptr(out["triangle"]), _ptr(out["point"])),
+                    "ctr_mt3d_closest_fetch")
+        return out, c
+
     def mt3d_interpolate(self, field, shape=None, dtype=None):
         """Values of another field at the vertices of the last 3D run's mesh as it stands now (after a selection or
         clean-up too), row for row with mt3d_fetch()'s vertices: a_low + ratio * (a_high - a_low) along each vertex's

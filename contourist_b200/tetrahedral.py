@@ -176,6 +176,11 @@ class GridContour3d(object):
     # the reference's constraints.py), after decimation and before vertex_fields, measure_components and sections,
     # which then describe the clipped mesh.  Triangles across a plane are split on it; six rows make a box.
     clip_halfspaces = None
+    # closest_points = Q, [q, 3] in world units: get_points_and_triangles() then finds, on the device, the closest point
+    # of the returned mesh to each row (ctr_mt3d_closest), after every other pass, sections included, and leaves in
+    # closest dict(distance [q], triangle [q] (into the returned triangles), point [q, 3])
+    closest_points = None
+    closest = None
 
     def __init__(self, corner, function, value, segment_endpoints, linear_interpolate=True, callback=None,
                  origin=(0.0, 0.0, 0.0), delta=(1.0, 1.0, 1.0)):
@@ -223,6 +228,7 @@ class GridContour3d(object):
             # decimate_cell), so these keep raising rather than silently giving a different mesh
             raise NotImplementedError("flatten / smooth (LP-based decimation, tetrahedral.py:217-351) are out of scope")
         halfspaces = self._halfspaces()
+        query = self._closest_points()
         eng = E.default_engine()
         flags = (E.GEOM_F64 if np.dtype(self.geometry_dtype) == np.float64 else 0) | (E.WANT_NORMALS if self.want_normals else 0)
         if self.vertex_fields is not None or self.cap is not None:
@@ -300,6 +306,9 @@ class GridContour3d(object):
         if self.sections is not None:
             normal, offsets = self.sections
             self.section_polylines = eng.mt3d_section(normal, offsets)[1]
+        if query is not None:
+            # after every other pass: the distances are to the mesh returned below
+            self.closest = eng.mt3d_closest(query)[0]
         out = eng.mt3d_fetch()
         self.normals = out["normals"]
         points, triangles = out["verts"], out["tris"]
@@ -324,6 +333,17 @@ class GridContour3d(object):
         if len(A) and not np.any(A != 0.0, axis=1).all():
             raise ValueError("clip_halfspaces: every row of A must be non-zero")
         return A, b
+
+    def _closest_points(self):
+        "closest_points checked: a finite [q, 3] fp64 array, or None"
+        if self.closest_points is None:
+            return None
+        Q = np.asarray(self.closest_points, np.float64)
+        if Q.ndim != 2 or Q.shape[1] != 3:
+            raise ValueError("closest_points must be [q, 3], not %r" % (Q.shape,))
+        if not np.isfinite(Q).all():
+            raise ValueError("closest_points must be finite")
+        return np.ascontiguousarray(Q)
 
     def extract_surface_geometry(self, clean=True):
         points, triangles = self.get_points_and_triangles(clean)
@@ -373,7 +393,8 @@ class Delta3DContour(object):
         "options set on this driver (before or after the maker was built) reach the maker"
         for name in ("post_process", "geometry_dtype", "want_normals", "reference_orientation", "quantize_divisions",
                      "tiny_epsilon", "vertex_fields", "measure_components", "keep_components", "smooth_iterations",
-                     "smooth_lambda", "smooth_mu", "decimate_cell", "cap", "sections", "clip_halfspaces"):
+                     "smooth_lambda", "smooth_mu", "decimate_cell", "cap", "sections", "clip_halfspaces",
+                     "closest_points"):
             if hasattr(self, name):
                 setattr(maker, name, getattr(self, name))
         maker.field_grid = self.grid
@@ -392,6 +413,7 @@ class Delta3DContour(object):
         self.triangle_components = maker.triangle_components   # with measure_components: aligned with the triangles
         self.component_table = maker.component_table
         self.section_polylines = maker.section_polylines
+        self.closest = maker.closest
         return result
 
 

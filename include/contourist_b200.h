@@ -475,6 +475,48 @@ typedef struct {
 } ctr_clip_counts;                           /* 40 bytes */
 CTR_API int ctr_mt3d_clip(ctr_ctx* ctx, const ctr_clip_params* p, ctr_clip_counts* out);
 
+/* Closest points of the LAST 3D run's device mesh as it stands now (after any other pass) to query points (engine
+ * extension; oracle/mt3d_closest.py:closest is the definition, and the result equals it bit for bit).  Reads the mesh
+ * only; synchronous on return.
+ *   - Positions and points are widened to fp64 and every operation is rounded on its own; dot(x, y) = (x0*y0 + x1*y1) +
+ *     x2*y2.  The closest point q of triangle (a, b, c), corners in stored order, is Ericson's region walk (Real-Time
+ *     Collision Detection 5.1.5) in the definition's order; a degenerate or nearly degenerate triangle (a zero
+ *     denominator, or barycentric weights outside [0, 1]) takes the closest of its three edges' points, (a,b) first.
+ *     d2 = dot(p-q, p-q), distance = sqrt(d2) correctly rounded.
+ *   - The winner of a point is the smallest d2, the smallest triangle index on a tie.  A point is found when that
+ *     d2 <= max_distance * max_distance (in fp64; +inf finds every point).  A point not found, and every point on a
+ *     mesh without triangles, gets distance +inf, triangle -1 and point NaN.
+ *   - A linear BVH (Karras) over the triangles is built by every call, from the positions and triangles as they are
+ *     then: positions written through ctr_mt3d_device_ptrs are seen by the next call.  Batch the queries in one call.
+ *   - Device points (CTR_FIELD_ON_DEVICE) may be another context's mesh on the same device (ctr_mt3d_device_ptrs):
+ *     surface-to-surface distances with no host round trip.
+ *   - The call edits nothing: the mesh, its generation, component results, vertex values, section results and device
+ *     pointers are untouched, and every other pass accepts the mesh as before (ctr_mt3d_keep_components too, without
+ *     measuring again).
+ *   - CTR_ERR_BAD_ARG: a NULL argument (points may be NULL when n_points is 0), dtype not CTR_F32 / CTR_F64, flags other
+ *     than CTR_FIELD_ON_DEVICE, n_points outside [0, 2^31-1], max_distance NaN or negative, a non-finite query point
+ *     (checked on the device for device points, read at the first host wait), device points not in device memory of
+ *     the context's device.  CTR_ERR_STATE: no 3D run or a CTR_NO_GEOMETRY run; a slab run (i_lo != 0 or i_hi != n0)
+ *     or vert_id_base != 0; a triangle id outside [0, n_verts) (e.g. after ctr_mt3d_offset_ids); a _fetch with no
+ *     successful ctr_mt3d_closest since the last run.  All are detected before any result is written; a failed call
+ *     leaves no results.
+ *   _closest_fetch: distance [n_points] f64, triangle [n_points] i32, point [n_points][3] f64; any pointer may be NULL.
+ *     Copied with cudaMemcpyDefault, so each destination may be host memory or device memory on the context's device.
+ *     Valid until the next ctr_mt3d_closest or 3D run.                                                                 */
+typedef struct {
+  const void* points;      /* [n_points][3], host or device (CTR_FIELD_ON_DEVICE), in the units of the positions       */
+  int32_t dtype;           /* CTR_F32 or CTR_F64                                                                       */
+  uint32_t flags;          /* CTR_FIELD_ON_DEVICE                                                                      */
+  int64_t n_points;        /* 0 .. 2^31-1                                                                              */
+  double max_distance;     /* >= 0, +inf allowed                                                                       */
+} ctr_closest_params;                        /* 32 bytes */
+typedef struct {
+  int64_t n_found;                           /* points with a triangle within max_distance                            */
+  int64_t height;                            /* of the tree built by this call (0 for one triangle or none)           */
+} ctr_closest_counts;                        /* 16 bytes */
+CTR_API int ctr_mt3d_closest(ctr_ctx* ctx, const ctr_closest_params* p, ctr_closest_counts* out);
+CTR_API int ctr_mt3d_closest_fetch(ctr_ctx* ctx, double* distance, int32_t* triangle, double* point);
+
 /* Seeded extraction (SURVEY.md 8(f3)): restricts the LAST full-volume run's mesh to what the reference's tracker
  *   tetrahedral.py:443-469  expand_voxels / in_range  (flood fill over the 26-neighbourhood of border voxels)
  * reaches from the given start voxels (the output of find_initial_voxels, tetrahedral.py:396-441, which the binding
