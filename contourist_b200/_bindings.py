@@ -1,4 +1,4 @@
-"""ctypes prototypes for the 2D / 4D / post-processing entry points and the closest-point query."""
+"""ctypes prototypes for the 2D / 4D / post-processing entry points, the closest-point query and the ray cast."""
 import ctypes
 
 
@@ -37,6 +37,15 @@ class ClosestCounts(ctypes.Structure):
     _fields_ = [("n_found", ctypes.c_int64), ("height", ctypes.c_int64)]
 
 
+class RayParams(ctypes.Structure):
+    _fields_ = [("origins", ctypes.c_void_p), ("directions", ctypes.c_void_p), ("dtype", ctypes.c_int32),
+                ("flags", ctypes.c_uint32), ("n_rays", ctypes.c_int64), ("t_min", ctypes.c_double), ("t_max", ctypes.c_double)]
+
+
+class RayCounts(ctypes.Structure):
+    _fields_ = [("n_hit", ctypes.c_int64), ("height", ctypes.c_int64)]
+
+
 def bind(lib):
     vp, i32 = ctypes.c_void_p, ctypes.c_int
     lib.ctr_mt2d_run.argtypes = [vp, ctypes.POINTER(Mt2dParams), ctypes.POINTER(Mt2dCounts)]
@@ -51,3 +60,7 @@ def bind(lib):
     lib.ctr_mt3d_closest.restype = i32
     lib.ctr_mt3d_closest_fetch.argtypes = [vp] * 4
     lib.ctr_mt3d_closest_fetch.restype = i32
+    lib.ctr_mt3d_raycast.argtypes = [vp, ctypes.POINTER(RayParams), ctypes.POINTER(RayCounts)]
+    lib.ctr_mt3d_raycast.restype = i32
+    lib.ctr_mt3d_raycast_fetch.argtypes = [vp] * 6
+    lib.ctr_mt3d_raycast_fetch.restype = i32

@@ -24,6 +24,7 @@
 // so no leaf is deeper than 94 and the 96-entry stack cannot overflow.
 // Node: one 64-byte line, both children's boxes (fp32) and links (>= 0: node; < 0: ~triangle).
 // Scratch: AUX_SCRATCH0 (counters, leaf boxes, codes, the sort).  AUX_CLOSEST_TREE: nodes, parents, arrival counters.
+// cq_build is the whole build; ctr_mt3d_raycast (raycast3d.cuh) builds the same tree through it.
 // AUX_CLOSEST_RESULT: distance, triangle, point.  AUX_CLOSEST_POINTS: host points staged in their own type.
 
 constexpr int CQ_THREADS = 128;                        // query block: 96 x 128 x 4 bytes of stack = 48 KiB
@@ -417,13 +418,23 @@ static inline int64_t cq_sort_launches(size_t n) {
   return 2 + 8 * (int64_t)((n + portion - 1) / portion);
 }
 
-template <typename G, typename P>
-int closest_run(ctr_ctx* ctx, const ctr_closest_params* cp, const P* pts, ctr_closest_counts* out) {
+// The tree over the mesh as it stands, shared by ctr_mt3d_closest and ctr_mt3d_raycast: k_cq_box, the queries' own
+// check kernels (`check` enqueues them on the counters and returns their launch count), the one host wait (the id flag,
+// the query flag, the scene box: an error here is `bad_msg`, and nothing has been written), then k_cq_morton, the sort,
+// k_cq_nodes and k_cq_refit.  Fills the root link, the nodes, the device counters and their host copy.
+struct CqTree {
+  int root;
+  CqNode* node;
+  CqCounters* ctr;
+  CqCounters h;
+};
+
+template <typename G, typename Check>
+int cq_build(ctr_ctx* ctx, Check&& check, const char* bad_msg, CqTree* tr) {
   cudaStream_t st = ctx->stream;
-  const size_t nT = (size_t)ctx->last_counts[1], nV = (size_t)ctx->last_counts[0], nP = (size_t)cp->n_points;
+  const size_t nT = (size_t)ctx->last_counts[1], nV = (size_t)ctx->last_counts[0];
   const int* tris = (const int*)ctx->tris.p;
   const G* verts = (const G*)ctx->verts.p;
-  const bool on_device = cp->flags & CTR_FIELD_ON_DEVICE;
   // ---- scratch: counters, leaf boxes, codes and indices (both sort buffers), the sort's temporary storage
   size_t sort_bytes = 0;
   if (nT > 1)
@@ -453,16 +464,13 @@ int closest_run(ctr_ctx* ctx, const ctr_closest_params* cp, const P* pts, ctr_cl
     k_cq_box<G><<<tb, 256, 0, st>>>(verts, tris, (unsigned)nT, (unsigned)nV, box, ctr);
     ctx->launches++;
   }
-  if (on_device && nP) {
-    k_cq_finite<P><<<(unsigned)((nP * 3 + 255) / 256), 256, 0, st>>>(pts, nP * 3, ctr);
-    ctx->launches++;
-  }
+  ctx->launches += check(ctr);
   CTR_CUDA(ctx, cudaGetLastError());
-  CqCounters h;
+  CqCounters& h = tr->h;
   CTR_CUDA(ctx, cudaMemcpyAsync(&h, ctr, sizeof h, cudaMemcpyDeviceToHost, st));
   CTR_CUDA(ctx, cudaStreamSynchronize(st));
   if (h.bad_ids) return fail_shifted_ids(ctx);
-  if (h.bad_points) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "query points must be finite");
+  if (h.bad_points) return ctr_fail(ctx, CTR_ERR_BAD_ARG, bad_msg);
   // ---- the tree
   CqNode* node = nullptr;
   int *node_parent, *leaf_parent;
@@ -474,7 +482,6 @@ int closest_run(ctr_ctx* ctx, const ctr_closest_params* cp, const P* pts, ctr_cl
          c(arrive, nT * 4);
        })))
     return rc;
-  int root = nT == 0 ? CQ_EMPTY : nT == 1 ? ~0 : 0;
   if (nT > 1) {
     double3 lo, scale;
     double l[3], s[3];
@@ -493,6 +500,27 @@ int closest_run(ctr_ctx* ctx, const ctr_closest_params* cp, const P* pts, ctr_cl
     k_cq_refit<<<tb, 256, 0, st>>>((int)nT, box, node, node_parent, leaf_parent, arrive, ctr);
     ctx->launches += 3 + cq_sort_launches(nT);
   }
+  tr->root = nT == 0 ? CQ_EMPTY : nT == 1 ? ~0 : 0;
+  tr->node = node;
+  tr->ctr = ctr;
+  return 0;
+}
+
+template <typename G, typename P>
+int closest_run(ctr_ctx* ctx, const ctr_closest_params* cp, const P* pts, ctr_closest_counts* out) {
+  cudaStream_t st = ctx->stream;
+  const size_t nT = (size_t)ctx->last_counts[1], nP = (size_t)cp->n_points;
+  const int* tris = (const int*)ctx->tris.p;
+  const G* verts = (const G*)ctx->verts.p;
+  const bool on_device = cp->flags & CTR_FIELD_ON_DEVICE;
+  CqTree tr;
+  int rc;
+  if ((rc = cq_build<G>(ctx, [&](CqCounters* ctr) -> int64_t {
+         if (!on_device || !nP) return 0;
+         k_cq_finite<P><<<(unsigned)((nP * 3 + 255) / 256), 256, 0, st>>>(pts, nP * 3, ctr);
+         return 1;
+       }, "query points must be finite", &tr)))
+    return rc;
   // ---- the queries
   double* dist;
   int* tri_out;
@@ -506,11 +534,12 @@ int closest_run(ctr_ctx* ctx, const ctr_closest_params* cp, const P* pts, ctr_cl
   if (nP) {
     const double md = cp->max_distance;
     k_cq_query<G, P><<<(unsigned)((nP + CQ_THREADS - 1) / CQ_THREADS), CQ_THREADS, 0, st>>>(
-        pts, (unsigned)nP, node, root, verts, tris, md * md, dist, tri_out, pt_out, ctr);
+        pts, (unsigned)nP, tr.node, tr.root, verts, tris, md * md, dist, tri_out, pt_out, tr.ctr);
     ctx->launches++;
   }
   CTR_CUDA(ctx, cudaGetLastError());
-  CTR_CUDA(ctx, cudaMemcpyAsync(&h, ctr, sizeof h, cudaMemcpyDeviceToHost, st));
+  CqCounters& h = tr.h;
+  CTR_CUDA(ctx, cudaMemcpyAsync(&h, tr.ctr, sizeof h, cudaMemcpyDeviceToHost, st));
   CTR_CUDA(ctx, cudaStreamSynchronize(st));
   ctx->closest_n = (int64_t)nP;
   out->n_found = h.n_found;

@@ -48,6 +48,8 @@ enum Aux3 : int {
   AUX_CLOSEST_RESULT = 48,   // closest points (ctr_mt3d_closest): distance, triangle, point per query point
   AUX_CLOSEST_TREE = 49,     // ... the tree of the last call (rebuilt by every call)
   AUX_CLOSEST_POINTS = 50,   // ... its host query points, staged
+  AUX_RAY_RESULT = 51,       // ray casting (ctr_mt3d_raycast): t, weights, point, triangle, side per ray (its tree is
+  AUX_RAY_INPUT = 52,        // ... its host rays, staged                      AUX_CLOSEST_TREE, rebuilt by every call)
 };
 
 // ctr_ctx::last3_edited: the passes that have rewritten the device mesh of the last 3D run
@@ -108,6 +110,10 @@ constexpr PassRule PASS_CLIP = {" to clip", false, FULL_ID0, CTR_ERR_STATE,
 // the closest-point query reads the mesh as it stands after any pass
 constexpr PassRule PASS_CLOSEST = {" to query", false, FULL_ID0, CTR_ERR_STATE,
                                    "closest points need a full-volume run with vert_id_base 0 (a slab's halo ids belong to another shard)",
+                                   0u, nullptr};
+// the ray cast reads the mesh as it stands after any pass
+constexpr PassRule PASS_RAYCAST = {" to cast rays at", false, FULL_ID0, CTR_ERR_STATE,
+                                   "ray casting needs a full-volume run with vert_id_base 0 (a slab's halo ids belong to another shard)",
                                    0u, nullptr};
 constexpr PassRule PASS_INTERPOLATE = {" to interpolate on", true, ANY_RUN, 0, nullptr, 0u, nullptr};
 constexpr PassRule PASS_OFFSET_IDS = {"", false, ANY_RUN, 0, nullptr, 0u, nullptr};
@@ -176,9 +182,12 @@ struct ctr_ctx {
   // 3D closest points (ctr_mt3d_closest) in AUX_CLOSEST_RESULT: query points of the last successful call; -1 = none since
   // the last 3D run (or the last call failed)
   int64_t closest_n = -1;
+  // 3D ray casting (ctr_mt3d_raycast) in AUX_RAY_RESULT: rays of the last successful call; -1 = none since the last 3D run
+  // (or the last call failed)
+  int64_t ray_n = -1;
 
   // extra outputs and scratch in generic slots: 3D (Aux3 above); 5-10: 2D; 12-26: 4D; 36-40: 2D polylines
-  DevBuf aux[51];
+  DevBuf aux[53];
 };
 
 static inline int ctr_fail(ctr_ctx* ctx, int code, const char* what, const char* detail = "") {

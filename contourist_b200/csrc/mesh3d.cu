@@ -17,6 +17,7 @@
 // clip3d.cuh (ctr_mt3d_clip) keeps the part of the mesh on one side of a plane or a vertex value, with the section's side
 // test and crossing point, the caps' corner walk and one new vertex per crossed edge, found in the same kind of table.
 // closest3d.cuh (ctr_mt3d_closest) finds the closest point of the mesh to query points through a tree it builds per call.
+// raycast3d.cuh (ctr_mt3d_raycast) finds the first hit of rays on the mesh through the same tree, built the same way.
 #include <math.h>
 #include <string.h>
 
@@ -251,6 +252,7 @@ int orient_typed(ctr_ctx* ctx, int64_t* n_components, int64_t* n_flipped) {
 #include "cap3d.cuh"
 #include "clip3d.cuh"
 #include "closest3d.cuh"
+#include "raycast3d.cuh"
 
 }  // namespace
 
@@ -480,6 +482,69 @@ extern "C" int ctr_mt3d_closest_fetch(ctr_ctx* ctx, double* distance, int32_t* t
   if (distance) CTR_CUDA(ctx, cudaMemcpyAsync(distance, dist, n * 8, cudaMemcpyDefault, st));
   if (triangle) CTR_CUDA(ctx, cudaMemcpyAsync(triangle, tri, n * 4, cudaMemcpyDefault, st));
   if (point) CTR_CUDA(ctx, cudaMemcpyAsync(point, pt, n * 24, cudaMemcpyDefault, st));
+  CTR_CUDA(ctx, cudaStreamSynchronize(st));
+  return 0;
+}
+
+extern "C" int ctr_mt3d_raycast(ctr_ctx* ctx, const ctr_ray_params* rp, ctr_ray_counts* out) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  ctx->ray_n = -1;                                     // a failed call leaves no results
+  if (!rp || !out) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  memset(out, 0, sizeof *out);
+  if (rp->dtype != CTR_F32 && rp->dtype != CTR_F64) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "dtype must be CTR_F32 or CTR_F64");
+  if (rp->flags & ~(uint32_t)CTR_FIELD_ON_DEVICE) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "flags must be 0 or CTR_FIELD_ON_DEVICE");
+  if (rp->n_rays < 0 || rp->n_rays > 0x7fffffffll) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "n_rays must be in [0, 2^31-1]");
+  if (rp->n_rays > 0 && (!rp->origins || !rp->directions)) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "null argument");
+  if (!(rp->t_min <= rp->t_max)) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "t_min and t_max must not be NaN, and t_min <= t_max");
+  const size_t nR = (size_t)rp->n_rays;
+  if (!(rp->flags & CTR_FIELD_ON_DEVICE))              // device rays are checked on the device, at the first host wait
+    for (size_t i = 0; i < nR; ++i) {
+      bool ok = true, moves = false;
+      for (int k = 0; k < 3; ++k) {
+        const size_t j = i * 3 + k;
+        const bool f64 = rp->dtype == CTR_F64;
+        const double o = f64 ? ((const double*)rp->origins)[j] : (double)((const float*)rp->origins)[j];
+        const double d = f64 ? ((const double*)rp->directions)[j] : (double)((const float*)rp->directions)[j];
+        ok = ok && isfinite(o) && isfinite(d);
+        moves = moves || d != 0.0;
+      }
+      if (!(ok && moves)) return ctr_fail(ctx, CTR_ERR_BAD_ARG, "rays must be finite with a non-zero direction");
+    }
+  if (int rc = check_pass(ctx, PASS_RAYCAST)) return rc;
+  if ((rp->flags & CTR_FIELD_ON_DEVICE) && nR)
+    for (const void* p : {rp->origins, rp->directions}) {
+      cudaPointerAttributes at;
+      if (cudaPointerGetAttributes(&at, p) != cudaSuccess || at.device != ctx->device ||
+          (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged)) {
+        cudaGetLastError();
+        return ctr_fail(ctx, CTR_ERR_BAD_ARG, "device rays must be device memory on the context's device");
+      }
+    }
+  return with_geom_type(ctx, [&](auto g) { return raycast_typed<decltype(g)>(ctx, rp, out); });
+}
+
+extern "C" int ctr_mt3d_raycast_fetch(ctr_ctx* ctx, double* t, int32_t* triangle, double* weights, double* point,
+                                      int8_t* side) {
+  if (!ctx) return CTR_ERR_BAD_ARG;
+  if (ctx->last_kind != 3 || ctx->ray_n < 0) return ctr_fail(ctx, CTR_ERR_STATE, "no ctr_mt3d_raycast since the last 3D run");
+  const size_t n = (size_t)ctx->ray_n;
+  if (!n) return 0;
+  CTR_CUDA(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  double *t_d, *wt, *pt;
+  int* tri;
+  signed char* sd;
+  ctr_carve c{(char*)ctx->aux[AUX_RAY_RESULT].p, 0};
+  c(t_d, n * 8);
+  c(wt, n * 24);
+  c(pt, n * 24);
+  c(tri, n * 4);
+  c(sd, n);
+  if (t) CTR_CUDA(ctx, cudaMemcpyAsync(t, t_d, n * 8, cudaMemcpyDefault, st));
+  if (triangle) CTR_CUDA(ctx, cudaMemcpyAsync(triangle, tri, n * 4, cudaMemcpyDefault, st));
+  if (weights) CTR_CUDA(ctx, cudaMemcpyAsync(weights, wt, n * 24, cudaMemcpyDefault, st));
+  if (point) CTR_CUDA(ctx, cudaMemcpyAsync(point, pt, n * 24, cudaMemcpyDefault, st));
+  if (side) CTR_CUDA(ctx, cudaMemcpyAsync(side, sd, n, cudaMemcpyDefault, st));
   CTR_CUDA(ctx, cudaStreamSynchronize(st));
   return 0;
 }

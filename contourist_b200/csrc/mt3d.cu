@@ -1685,6 +1685,7 @@ static int mt3d_dispatch(ctr_ctx* ctx, const ctr_mt3d_params* p, ctr_mt3d_counts
   ctx->comp_count = -1;                                // ... and so are its components
   ctx->sect_count[0] = -1;                             // ... and its plane sections
   ctx->closest_n = -1;                                 // ... and its closest points
+  ctx->ray_n = -1;                                     // ... and its ray hits
   return with_sample_type(ctx, p->dtype, [&](auto t) { return run_typed<decltype(t)>(ctx, p, out, phase); });
 }
 

@@ -719,6 +719,48 @@ class Engine(object):
                     "ctr_mt3d_closest_fetch")
         return out, c
 
+    def mt3d_raycast(self, origins, directions, t_min=0.0, t_max=np.inf, n=None, dtype=None):
+        """First hits of rays on the last 3D run's device mesh as it stands now (ctr_mt3d_raycast;
+        oracle/mt3d_raycast.py is the definition).  origins, directions: numpy [R, 3] in the units of the current
+        positions (one dtype for both: float32 / float64 read as they are, other types widened to float64), or two
+        integer device pointers with n and dtype (float32 or float64) -- e.g. this engine's own vertices and normals
+        from mt3d_device_ptrs() for wall thickness.  Directions need not be unit length: t is in units of |d|.  For
+        each ray: the hit with the smallest t in [t_min, t_max] (the smallest triangle index on a tie), by the
+        watertight test.  The mesh is not edited; a tree over the triangles is built per call, so batch the rays.
+        Returns (dict(t [R] float64, triangle [R] int32, weights [R, 3] float64 (of the triangle's corners a, b, c),
+        point [R, 3] float64, side [R] int8 (+1: the ray arrives from the side the triangle faces, -1: from behind)),
+        RayCounts (n_hit, height)); a ray without a hit has t inf, triangle -1, weights and point NaN and side 0."""
+        from ._bindings import RayCounts, RayParams
+        p = RayParams()
+        if isinstance(origins, np.ndarray) or isinstance(directions, np.ndarray):
+            O, D = np.asarray(origins), np.asarray(directions)
+            if O.ndim != 2 or O.shape[1] != 3 or D.shape != O.shape:
+                raise ValueError("origins and directions of one shape (R, 3) expected, not %r and %r" % (O.shape, D.shape))
+            if O.dtype != D.dtype or O.dtype not in (np.float32, np.float64):
+                O, D = O.astype(np.float64), D.astype(np.float64)
+            O, D = np.ascontiguousarray(O), np.ascontiguousarray(D)
+            p.origins = O.ctypes.data if len(O) else None
+            p.directions = D.ctypes.data if len(D) else None
+            p.dtype = dtype_code(O.dtype)
+            p.flags = 0
+            R = len(O)
+        else:
+            if n is None or dtype is None:
+                raise ValueError("device rays need n and dtype")
+            p.origins, p.directions = int(origins), int(directions)
+            p.dtype = _device_code(dtype, FLOAT_CODES)
+            p.flags = FIELD_ON_DEVICE
+            R = int(n)
+        p.n_rays = R
+        p.t_min, p.t_max = float(t_min), float(t_max)
+        c = RayCounts()
+        self._check(self.lib.ctr_mt3d_raycast(self.h, ctypes.byref(p), ctypes.byref(c)), "ctr_mt3d_raycast")
+        out = dict(t=np.empty(R, np.float64), triangle=np.empty(R, np.int32), weights=np.empty((R, 3), np.float64),
+                   point=np.empty((R, 3), np.float64), side=np.empty(R, np.int8))
+        self._check(self.lib.ctr_mt3d_raycast_fetch(self.h, _ptr(out["t"]), _ptr(out["triangle"]), _ptr(out["weights"]),
+                                                    _ptr(out["point"]), _ptr(out["side"])), "ctr_mt3d_raycast_fetch")
+        return out, c
+
     def mt3d_interpolate(self, field, shape=None, dtype=None):
         """Values of another field at the vertices of the last 3D run's mesh as it stands now (after a selection or
         clean-up too), row for row with mt3d_fetch()'s vertices: a_low + ratio * (a_high - a_low) along each vertex's

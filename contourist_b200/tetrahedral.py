@@ -181,6 +181,12 @@ class GridContour3d(object):
     # closest dict(distance [q], triangle [q] (into the returned triangles), point [q, 3])
     closest_points = None
     closest = None
+    # rays = (O, D), both [r, 3] in world units: get_points_and_triangles() then finds, on the device, the first hit of
+    # each ray o + t d, t in [0, inf), on the returned mesh (ctr_mt3d_raycast), after every other pass, next to
+    # closest_points, and leaves in ray_hits dict(t [r], triangle [r] (into the returned triangles), weights [r, 3],
+    # point [r, 3], side [r])
+    rays = None
+    ray_hits = None
 
     def __init__(self, corner, function, value, segment_endpoints, linear_interpolate=True, callback=None,
                  origin=(0.0, 0.0, 0.0), delta=(1.0, 1.0, 1.0)):
@@ -229,6 +235,7 @@ class GridContour3d(object):
             raise NotImplementedError("flatten / smooth (LP-based decimation, tetrahedral.py:217-351) are out of scope")
         halfspaces = self._halfspaces()
         query = self._closest_points()
+        rays = self._rays()
         eng = E.default_engine()
         flags = (E.GEOM_F64 if np.dtype(self.geometry_dtype) == np.float64 else 0) | (E.WANT_NORMALS if self.want_normals else 0)
         if self.vertex_fields is not None or self.cap is not None:
@@ -309,6 +316,8 @@ class GridContour3d(object):
         if query is not None:
             # after every other pass: the distances are to the mesh returned below
             self.closest = eng.mt3d_closest(query)[0]
+        if rays is not None:
+            self.ray_hits = eng.mt3d_raycast(*rays)[0]
         out = eng.mt3d_fetch()
         self.normals = out["normals"]
         points, triangles = out["verts"], out["tris"]
@@ -344,6 +353,24 @@ class GridContour3d(object):
         if not np.isfinite(Q).all():
             raise ValueError("closest_points must be finite")
         return np.ascontiguousarray(Q)
+
+    def _rays(self):
+        "rays checked: (O [r, 3], D [r, 3]) as finite fp64 arrays with non-zero directions, or None"
+        if self.rays is None:
+            return None
+        try:
+            O, D = self.rays
+        except (TypeError, ValueError):
+            raise ValueError("rays must be a pair (O [r, 3], D [r, 3])")
+        O = np.asarray(O, np.float64)
+        D = np.asarray(D, np.float64)
+        if O.ndim != 2 or O.shape[1] != 3 or D.shape != O.shape:
+            raise ValueError("rays: O and D must both be [r, 3], not %r and %r" % (O.shape, D.shape))
+        if not (np.isfinite(O).all() and np.isfinite(D).all()):
+            raise ValueError("rays: O and D must be finite")
+        if len(D) and not np.any(D != 0.0, axis=1).all():
+            raise ValueError("rays: every direction must be non-zero")
+        return np.ascontiguousarray(O), np.ascontiguousarray(D)
 
     def extract_surface_geometry(self, clean=True):
         points, triangles = self.get_points_and_triangles(clean)
@@ -394,7 +421,7 @@ class Delta3DContour(object):
         for name in ("post_process", "geometry_dtype", "want_normals", "reference_orientation", "quantize_divisions",
                      "tiny_epsilon", "vertex_fields", "measure_components", "keep_components", "smooth_iterations",
                      "smooth_lambda", "smooth_mu", "decimate_cell", "cap", "sections", "clip_halfspaces",
-                     "closest_points"):
+                     "closest_points", "rays"):
             if hasattr(self, name):
                 setattr(maker, name, getattr(self, name))
         maker.field_grid = self.grid
@@ -414,6 +441,7 @@ class Delta3DContour(object):
         self.component_table = maker.component_table
         self.section_polylines = maker.section_polylines
         self.closest = maker.closest
+        self.ray_hits = maker.ray_hits
         return result
 
 

@@ -517,6 +517,54 @@ typedef struct {
 CTR_API int ctr_mt3d_closest(ctr_ctx* ctx, const ctr_closest_params* p, ctr_closest_counts* out);
 CTR_API int ctr_mt3d_closest_fetch(ctr_ctx* ctx, double* distance, int32_t* triangle, double* point);
 
+/* First hits of rays on the LAST 3D run's device mesh as it stands now (after any other pass) (engine extension;
+ * oracle/mt3d_raycast.py:raycast is the definition, and the result equals it bit for bit).  Reads the mesh only;
+ * synchronous on return.  Picking, wall thickness (rays from the vertices along their normals, with t_min > 0),
+ * inside / outside tests (the side of the first hit) and depth images of a camera are all this one query.
+ *   - Positions, origins and directions are widened to fp64 and every operation is rounded on its own.  Ray (o, d)
+ *     against triangle (a, b, c), corners in stored order, is Woop, Benthin and Wald's watertight test (JCGT 2(1),
+ *     2013): the axes kz (the largest |d_k|, the first on a tie), kx, ky from d alone, the shear, the edge functions
+ *     U, V, W, det = (U+V)+W and t = T/det in the definition's order.  A ray through an edge or a vertex cannot pass
+ *     between the triangles around it.  A hit needs t_min <= t <= t_max and the point p = o + t*d inside the
+ *     triangle's box padded by 2^-40 max|coordinate| (this rejects only hits of grazing rays and slivers whose t is
+ *     rounding noise).
+ *   - The winner of a ray is the hit with the smallest t, the smallest triangle index on a tie.  weights = (U, V, W) /
+ *     det are the weights of a, b and c; side = +1 when the ray arrives from the side the triangle faces (det > 0,
+ *     i.e. dot(d, cross(b-a, c-a)) < 0), else -1.  The raw mesh faces the high side of the field, so there +1 means
+ *     the origin is on the high side.  A ray without a hit, and every ray on a mesh without triangles, gets t = +inf,
+ *     triangle -1, weights and point NaN, side 0.
+ *   - ctr_mt3d_closest's linear BVH is built by every call, from the positions and triangles as they are then:
+ *     positions written through ctr_mt3d_device_ptrs are seen by the next call.  Batch the rays in one call.
+ *   - Device rays (CTR_FIELD_ON_DEVICE) may be a context's own vertices and normals (ctr_mt3d_device_ptrs): wall
+ *     thickness with no host round trip.
+ *   - The call edits nothing: the mesh, its generation, component results, vertex values, section results, closest
+ *     results and device pointers are untouched, and every other pass accepts the mesh as before.
+ *   - CTR_ERR_BAD_ARG: a NULL argument (origins and directions may be NULL when n_rays is 0), dtype not CTR_F32 /
+ *     CTR_F64, flags other than CTR_FIELD_ON_DEVICE, n_rays outside [0, 2^31-1], t_min or t_max NaN or t_min > t_max,
+ *     a non-finite origin or direction coordinate or an all-zero direction (checked on the device for device rays,
+ *     read at the first host wait), device rays not in device memory of the context's device.  CTR_ERR_STATE: no 3D
+ *     run or a CTR_NO_GEOMETRY run; a slab run (i_lo != 0 or i_hi != n0) or vert_id_base != 0; a triangle id outside
+ *     [0, n_verts) (e.g. after ctr_mt3d_offset_ids); a _fetch with no successful ctr_mt3d_raycast since the last run.
+ *     All are detected before any result is written; a failed call leaves no results.
+ *   _raycast_fetch: t [n_rays] f64, triangle [n_rays] i32, weights [n_rays][3] f64, point [n_rays][3] f64, side
+ *     [n_rays] i8; any pointer may be NULL.  Copied with cudaMemcpyDefault, so each destination may be host memory or
+ *     device memory on the context's device.  Valid until the next ctr_mt3d_raycast or 3D run.                        */
+typedef struct {
+  const void* origins;     /* [n_rays][3], host or device (CTR_FIELD_ON_DEVICE), in the units of the positions         */
+  const void* directions;  /* [n_rays][3], same dtype and memory; need not be unit length (t is in units of |d|)      */
+  int32_t dtype;           /* CTR_F32 or CTR_F64                                                                       */
+  uint32_t flags;          /* CTR_FIELD_ON_DEVICE                                                                      */
+  int64_t n_rays;          /* 0 .. 2^31-1                                                                              */
+  double t_min, t_max;     /* not NaN, t_min <= t_max; infinities allowed                                              */
+} ctr_ray_params;                            /* 48 bytes */
+typedef struct {
+  int64_t n_hit;                             /* rays with a hit in [t_min, t_max]                                     */
+  int64_t height;                            /* of the tree built by this call (0 for one triangle or none)           */
+} ctr_ray_counts;                            /* 16 bytes */
+CTR_API int ctr_mt3d_raycast(ctr_ctx* ctx, const ctr_ray_params* p, ctr_ray_counts* out);
+CTR_API int ctr_mt3d_raycast_fetch(ctr_ctx* ctx, double* t, int32_t* triangle, double* weights, double* point,
+                                   int8_t* side);
+
 /* Seeded extraction (SURVEY.md 8(f3)): restricts the LAST full-volume run's mesh to what the reference's tracker
  *   tetrahedral.py:443-469  expand_voxels / in_range  (flood fill over the 26-neighbourhood of border voxels)
  * reaches from the given start voxels (the output of find_initial_voxels, tetrahedral.py:396-441, which the binding
