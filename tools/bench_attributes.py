@@ -18,25 +18,15 @@ Prints one JSON line (also written to --out).
 """
 import argparse
 import ctypes
-import json
+import functools
 import os
-import subprocess
 import sys
 import time
 
 import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-
-
-def gpu_info():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
-                             text=True, timeout=30).stdout.strip().splitlines()
-        name, power = (x.strip() for x in out[0].split(","))
-        return dict(name=name, power_limit=power)
-    except Exception as e:                                      # the line still carries torch's device name
-        return dict(name=None, power_limit=None, error=str(e))
+from tools.benchkit import back_to_back, cuda_engine, emit, gpu_info, kernel_table, window  # noqa: E402
 
 
 def main():
@@ -51,7 +41,6 @@ def main():
     from contourist_b200 import engine as E
     from contourist_b200 import synthetic
     from oracle import mt3d_values
-    assert torch.cuda.is_available(), "bench_attributes measures on a CUDA device"
     dev = torch.device("cuda", 0)
     n = args.n
     shape = (n, n, n)
@@ -61,10 +50,7 @@ def main():
     vec3 = torch.stack([s1, synthetic.ct_like(n, device=dev, seed=2), synthetic.ct_like(n, device=dev, seed=3)], -1).contiguous()
     u8 = torch.clamp(torch.round(s1 * 255), 0, 255).to(torch.uint8).contiguous()
     arms = [("scalar_f32", s1, np.float32, 1), ("vec3_f32", vec3, np.float32, 3), ("scalar_u8", u8, np.uint8, 1)]
-    torch.cuda.synchronize()
-    stream = torch.cuda.current_stream()
-    eng = E.Engine(0)
-    eng.set_stream(stream.cuda_stream)
+    eng, stream = cuda_engine()
     flags = E.WANT_NORMALS | E.WANT_KEYS
     c = eng.mt3d_run(field.data_ptr(), value, shape=shape, dtype=np.float32, flags=flags)
     out = eng.mt3d_fetch()
@@ -88,19 +74,8 @@ def main():
     del grid
 
     # pass time per call
-    for name, *_ in arms:
-        for _ in range(20):
-            call(name)
-    pass_ms = {name: [] for name, *_ in arms}
-    for _ in range(args.rounds):
-        for name, *_ in arms:
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record(stream)
-            for _ in range(args.calls):
-                call(name)
-            e1.record(stream)
-            torch.cuda.synchronize()
-            pass_ms[name].append(e0.elapsed_time(e1) / args.calls)
+    interp = {name: functools.partial(call, name) for name, *_ in arms}
+    pass_ms = back_to_back(stream, interp, args.calls, args.rounds, 20)
 
     # reference: k_emit_verts' stage time in the same call
     eng.set_timing(True)
@@ -110,37 +85,19 @@ def main():
         acc += np.array(eng.stage_times(8)) / 10
     eng.set_timing(False)
 
-    # kernel times (a profiled pass of its own)
-    from torch.profiler import ProfilerActivity, profile
-    eng.mt3d_run(field.data_ptr(), value, shape=shape, dtype=np.float32, flags=flags)
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        for _ in range(10):
-            eng.mt3d_run(field.data_ptr(), value, shape=shape, dtype=np.float32, flags=flags)
-            for name, *_ in arms:
-                call(name)
-        torch.cuda.synchronize()
-    kernel_us = {}
-    for ev in prof.key_averages():
-        if "k_interp_attr" in ev.key or "k_emit_verts" in ev.key:
-            tot = getattr(ev, "device_time_total", None)
-            tot = ev.cuda_time_total if tot is None else tot
-            kernel_us[ev.key[:96]] = dict(launches=ev.count, us_per_launch=round(tot / max(ev.count, 1), 2))
+    # kernel times (a profiled pass of its own), keyed by the start of the demangled name, which tells the instantiations
+    # for the sample types apart
+    def run():
+        eng.mt3d_run(field.data_ptr(), value, shape=shape, dtype=np.float32, flags=flags)
+
+    kernel_us = kernel_table(lambda: (run(), [call(name) for name, *_ in arms]), ("k_interp_attr", "k_emit_verts"),
+                             setup=run, reps=10, key=lambda key, tag: key[:96])
     # the two fp32 arms launch the same instantiation: one profiled pass per arm keeps them apart
-    prof_arms = {}
-    for name, *_ in arms:
-        with profile(activities=[ProfilerActivity.CUDA]) as prof:
-            for _ in range(20):
-                call(name)
-            torch.cuda.synchronize()
-        for ev in prof.key_averages():
-            if "k_interp_attr" in ev.key:
-                tot = getattr(ev, "device_time_total", None)
-                tot = ev.cuda_time_total if tot is None else tot
-                prof_arms[name] = round(tot / max(ev.count, 1), 2)
+    prof_arms = {name: kernel_table(lambda: call(name), ("k_interp_attr",), reps=20)["k_interp_attr"]["us_per_launch"]
+                 for name, *_ in arms}
 
     # what the façade option costs the run: WANT_KEYS on and off, alternated
-    engines = (eng, E.Engine(0))
-    engines[1].set_stream(stream.cuda_stream)
+    engines = (eng, cuda_engine()[0])
 
     def run_steps(fl, k):
         pending = None
@@ -159,12 +116,7 @@ def main():
     for _ in range(args.rounds):
         for name, fl in key_arms:
             run_steps(fl, 4)
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record(stream)
-            run_steps(fl, args.steps)
-            e1.record(stream)
-            torch.cuda.synchronize()
-            step_ms[name].append(e0.elapsed_time(e1) / args.steps)
+            step_ms[name].append(window(stream, lambda: run_steps(fl, args.steps)) / args.steps)
 
     # host baseline: the numpy definition on the fetched keys
     hf, ha = field.cpu().numpy(), s1.cpu().numpy()
@@ -189,11 +141,7 @@ def main():
                          step_ms_rounds={k: [round(x, 4) for x in v] for k, v in step_ms.items()}),
                host_oracle_ms=round(float(np.median(ts)), 1),
                oracle_max_abs_diff_scalar_f32=oracle_max_abs_diff, attr_range=scale)
-    line = json.dumps(res)
-    print(line)
-    if args.out:
-        with open(args.out, "w") as fh:
-            fh.write(line + "\n")
+    emit(res, args.out)
 
 
 if __name__ == "__main__":

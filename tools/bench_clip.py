@@ -17,24 +17,13 @@ synchronous: the time includes the launches and the two host waits).  Reported p
 Prints one JSON line (also written to --out).
 """
 import argparse
-import json
 import os
-import subprocess
 import sys
 
 import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-
-
-def gpu_info():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
-                             text=True, timeout=30).stdout.strip().splitlines()
-        name, power = (x.strip() for x in out[0].split(","))
-        return dict(name=name, power_limit=power)
-    except Exception as e:                                      # the line still carries torch's device name
-        return dict(name=None, power_limit=None, error=str(e))
+from tools.benchkit import cuda_engine, emit, gpu_info, kernel_table, per_call  # noqa: E402
 
 
 def main():
@@ -44,20 +33,15 @@ def main():
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     import torch
-    from torch.profiler import ProfilerActivity, profile
     from contourist_b200 import engine as E
     from contourist_b200 import synthetic
     from oracle import mt3d_clip
-    assert torch.cuda.is_available(), "bench_clip measures on a CUDA device"
     dev = torch.device("cuda", 0)
     n = args.n
     shape = (n, n, n)
     field = synthetic.ct_like(n, device=dev)
     second = synthetic.turbulence(n, device=dev).to(torch.float32).contiguous()
-    torch.cuda.synchronize()
-    stream = torch.cuda.current_stream()
-    eng = E.Engine(0)
-    eng.set_stream(stream.cuda_stream)
+    eng, stream = cuda_engine()
     lo, hi = n / 4.0 + 0.25, 3.0 * n / 4.0 + 0.25
     box = [((1.0, 0, 0), lo, "high"), ((1.0, 0, 0), hi, "low"), ((0, 1.0, 0), lo, "high"), ((0, 1.0, 0), hi, "low"),
            ((0, 0, 1.0), lo, "high"), ((0, 0, 1.0), hi, "low")]
@@ -99,45 +83,20 @@ def main():
                 for k in ("tris", "verts", "normals", "keys", "lowmin"):
                     equal = equal and bool(np.array_equal(post[k], np.asarray(want[k]).reshape(post[k].shape)))
                 del pre, post, want
-            ms = []
-            for q in range(args.calls + 1):                           # one untimed call first
-                fresh(value)
-                torch.cuda.synchronize()
-                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                e0.record(stream)
-                for kw in calls:
-                    c = eng.mt3d_clip(**kw)
-                e1.record(stream)
-                torch.cuda.synchronize()
-                if q >= 1:
-                    ms.append(e0.elapsed_time(e1))
-            fresh(value)
-            torch.cuda.synchronize()
-            with profile(activities=[ProfilerActivity.CUDA]) as prof:
+
+            def clip_all():
                 for kw in calls:
                     eng.mt3d_clip(**kw)
-                torch.cuda.synchronize()
-            kernel_us = {}
-            for ev in prof.key_averages():
-                key = ev.key
-                tag = next((t_ for t_ in ("k_clip_", "k_flag_scan", "k_sel_rows", "k_o_init", "Memcpy", "Memset")
-                            if t_ in key), None)
-                if tag is None:
-                    continue
-                short = key[key.index(tag):].split("(")[0].split("<")[0] if tag.startswith("k_") else key
-                tot = getattr(ev, "device_time_total", None)
-                tot = ev.cuda_time_total if tot is None else tot
-                kernel_us[short] = dict(launches=ev.count, us_per_launch=round(tot / max(ev.count, 1), 2))
+
+            ms = per_call(stream, clip_all, args.calls, 1, setup=lambda: fresh(value))
+            kernel_us = kernel_table(clip_all, ("k_clip_", "k_flag_scan", "k_sel_rows", "k_o_init", "Memcpy", "Memset"),
+                                     setup=lambda: fresh(value))
             res["%s_%s" % (gname, cname)] = dict(
                 n_verts_in=int(c0.n_verts), n_tris_in=int(c0.n_tris), n_verts=int(c.n_verts), n_tris=int(c.n_tris),
                 n_new_verts=int(c.n_new_verts), n_cut_tris=int(c.n_cut_tris), n_dropped_tris=int(c.n_dropped_tris),
                 call_ms=round(float(np.median(ms)), 4), calls_ms=[round(x, 4) for x in ms], kernel_us=kernel_us,
                 equal=equal)
-    line = json.dumps(res)
-    print(line)
-    if args.out:
-        with open(args.out, "w") as fh:
-            fh.write(line + "\n")
+    emit(res, args.out)
 
 
 if __name__ == "__main__":

@@ -22,24 +22,13 @@ Reported per geometry and case:
 Prints one JSON line (also written to --out).
 """
 import argparse
-import json
 import os
-import subprocess
 import sys
 
 import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-
-
-def gpu_info():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
-                             text=True, timeout=30).stdout.strip().splitlines()
-        name, power = (x.strip() for x in out[0].split(","))
-        return dict(name=name, power_limit=power)
-    except Exception as e:                                      # the line still carries torch's device name
-        return dict(name=None, power_limit=None, error=str(e))
+from tools.benchkit import cuda_engine, emit, gpu_info, kernel_table, per_call  # noqa: E402
 
 
 def main():
@@ -49,20 +38,15 @@ def main():
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     import torch
-    from torch.profiler import ProfilerActivity, profile
     from contourist_b200 import engine as E
     from contourist_b200 import synthetic
     from oracle import mt3d_closest
-    assert torch.cuda.is_available(), "bench_closest measures on a CUDA device"
     dev = torch.device("cuda", 0)
     n = args.n
     shape = (n, n, n)
     field = synthetic.ct_like(n, device=dev)
-    torch.cuda.synchronize()
-    stream = torch.cuda.current_stream()
-    eng, dec = E.Engine(0), E.Engine(0)
-    for e in (eng, dec):
-        e.set_stream(stream.cuda_stream)
+    eng, stream = cuda_engine()
+    dec, _ = cuda_engine()
     rng = np.random.default_rng(0)
     g = np.linspace(0.0, n - 1.0, 128)
     lattice = np.stack(np.meshgrid(g, g, g, indexing="ij"), axis=-1).reshape(-1, 3)
@@ -108,37 +92,12 @@ def main():
                 equal = all(np.array_equal(got[k][idx], want[k], equal_nan=True) for k in want) and c.n_found == len(pts)
                 extra = dict(n_points=len(pts), n_found=int(c.n_found), height=int(c.height))
             del out
-            ms = []
-            for q in range(args.calls + 1):                           # one untimed call first
-                torch.cuda.synchronize()
-                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                e0.record(stream)
-                call()
-                e1.record(stream)
-                torch.cuda.synchronize()
-                if q >= 1:
-                    ms.append(e0.elapsed_time(e1))
-            with profile(activities=[ProfilerActivity.CUDA]) as prof:
-                call()
-                torch.cuda.synchronize()
-            kernel_us = {}
-            for ev in prof.key_averages():
-                key = ev.key
-                tag = next((t_ for t_ in ("k_cq_", "DeviceRadixSort", "Memcpy", "Memset") if t_ in key), None)
-                if tag is None:
-                    continue
-                short = key[key.index(tag):].split("(")[0].split("<")[0] if tag != "Memcpy" and tag != "Memset" else key
-                tot = getattr(ev, "device_time_total", None)
-                tot = ev.cuda_time_total if tot is None else tot
-                kernel_us[short] = dict(launches=ev.count, us_per_launch=round(tot / max(ev.count, 1), 2))
+            ms = per_call(stream, call, args.calls, 1)
+            kernel_us = kernel_table(call, ("k_cq_", "DeviceRadixSort", "Memcpy", "Memset"))
             res["%s_%s" % (gname, cname)] = dict(n_verts=int(c0.n_verts), n_tris=int(c0.n_tris),
                                                  call_ms=round(float(np.median(ms)), 4), calls_ms=[round(x, 4) for x in ms],
                                                  kernel_us=kernel_us, equal=bool(equal), **extra)
-    line = json.dumps(res)
-    print(line)
-    if args.out:
-        with open(args.out, "w") as fh:
-            fh.write(line + "\n")
+    emit(res, args.out)
 
 
 if __name__ == "__main__":

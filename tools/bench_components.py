@@ -17,25 +17,14 @@ and two 512 MB hash tables.  Prints one JSON line (also written to --out).
 """
 import argparse
 import ctypes
-import json
 import os
-import subprocess
 import sys
 import time
 
 import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-
-
-def gpu_info():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
-                             text=True, timeout=30).stdout.strip().splitlines()
-        name, power = (x.strip() for x in out[0].split(","))
-        return dict(name=name, power_limit=power)
-    except Exception as e:                                      # the line still carries torch's device name
-        return dict(name=None, power_limit=None, error=str(e))
+from tools.benchkit import back_to_back, cuda_engine, emit, gpu_info, kernel_table  # noqa: E402
 
 
 def main():
@@ -49,16 +38,12 @@ def main():
     from contourist_b200 import engine as E
     from contourist_b200 import synthetic
     from oracle import mt3d_components
-    assert torch.cuda.is_available(), "bench_components measures on a CUDA device"
     dev = torch.device("cuda", 0)
     n = args.n
     shape = (n, n, n)
     value = 0.5
     field = synthetic.ct_like(n, device=dev)
-    torch.cuda.synchronize()
-    stream = torch.cuda.current_stream()
-    eng = E.Engine(0)
-    eng.set_stream(stream.cuda_stream)
+    eng, stream = cuda_engine()
     nret, nc, nf = ctypes.c_int64(), ctypes.c_int64(), ctypes.c_int64()
 
     def comp():
@@ -67,23 +52,8 @@ def main():
     def orient():
         eng._check(eng.lib.ctr_mt3d_orient_reference(eng.h, ctypes.byref(nc), ctypes.byref(nf)), "ctr_mt3d_orient_reference")
 
-    def timed(fn):
-        for _ in range(3):
-            fn()
-        ms = []
-        for _ in range(args.rounds):
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record(stream)
-            for _ in range(args.calls):
-                fn()
-            e1.record(stream)
-            torch.cuda.synchronize()
-            ms.append(e0.elapsed_time(e1) / args.calls)
-        return ms
-
     res = dict(tool="bench_components", n=n, calls=args.calls, rounds=args.rounds, gpu=gpu_info(),
                device=torch.cuda.get_device_name(0), isovalue=value, run_flags="WANT_NORMALS")
-    from torch.profiler import ProfilerActivity, profile
     for geom, gflag in (("fp32", 0), ("fp64", E.GEOM_F64)):
         c = eng.mt3d_run(field.data_ptr(), value, shape=shape, dtype=np.float32, flags=E.WANT_NORMALS | gflag)
         out = eng.mt3d_fetch()
@@ -99,22 +69,9 @@ def main():
         rel_area = float(np.max(np.abs(tab["area"] - want["area"]) / want["area"])) if equal else None
         vscale = want["area"] * (want["hi"] - want["lo"]).max(axis=1)
         rel_vol = float(np.max(np.abs(tab["volume"] - want["volume"]) / vscale)) if equal else None
-        pass_ms = timed(comp)
-        orient_ms = timed(orient)
-        with profile(activities=[ProfilerActivity.CUDA]) as prof:
-            for _ in range(10):
-                comp()
-                orient()
-            torch.cuda.synchronize()
-        kernel_us = {}
-        for ev in prof.key_averages():
-            name = ev.key
-            for tag in ("k_m_", "k_o_"):
-                if tag in name:
-                    short = name[name.index(tag):].split("(")[0].split("<")[0]
-                    tot = getattr(ev, "device_time_total", None)
-                    tot = ev.cuda_time_total if tot is None else tot
-                    kernel_us[short] = dict(launches=ev.count, us_per_launch=round(tot / max(ev.count, 1), 2))
+        pass_ms = back_to_back(stream, {"pass": comp}, args.calls, args.rounds, 3)["pass"]
+        orient_ms = back_to_back(stream, {"orient": orient}, args.calls, args.rounds, 3)["orient"]
+        kernel_us = kernel_table(lambda: (comp(), orient()), ("k_m_", "k_o_"), reps=10)
         closed = tab["n_boundary_edges"] == 0
         res[geom] = dict(n_verts=int(c.n_verts), n_tris=int(c.n_tris), n_components=len(tab), closed=int(closed.sum()),
                          largest_component_tris=int(tab["n_tris"].max()) if len(tab) else 0,
@@ -123,11 +80,7 @@ def main():
                          orient_n_components=int(nc.value), kernel_us=kernel_us,
                          host_oracle_ms=round(float(np.median(ts)), 1), oracle_equal=equal,
                          max_rel_area_diff=rel_area, max_rel_volume_diff=rel_vol)
-    line = json.dumps(res)
-    print(line)
-    if args.out:
-        with open(args.out, "w") as fh:
-            fh.write(line + "\n")
+    emit(res, args.out)
 
 
 if __name__ == "__main__":

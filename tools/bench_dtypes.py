@@ -14,25 +14,14 @@ page-locked host array (median of 7 calls after 3 untimed ones) and the bytes st
 checked: the integer mesh equals the float32 mesh bit for bit.  Prints one JSON line (also written to --out).
 """
 import argparse
-import json
 import os
-import subprocess
 import sys
 import time
 
 import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-
-
-def gpu_info():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
-                             text=True, timeout=30).stdout.strip().splitlines()
-        name, power = (x.strip() for x in out[0].split(","))
-        return dict(name=name, power_limit=power)
-    except Exception as e:                                      # the line still carries torch's device name
-        return dict(name=None, power_limit=None, error=str(e))
+from tools.benchkit import cuda_engine, emit, gpu_info, window  # noqa: E402
 
 
 def main():
@@ -46,7 +35,6 @@ def main():
     import torch
     from contourist_b200 import engine as E
     from contourist_b200 import synthetic
-    assert torch.cuda.is_available(), "bench_dtypes measures on a CUDA device"
     dev = torch.device("cuda", 0)
     n = args.n
     q = synthetic.ct_like(n, device=dev)
@@ -64,13 +52,10 @@ def main():
         for v in values:
             arms.append(("%s@%g" % (key, v), t, dt, v, "float32(%s)@%g" % (key, v)))
             arms.append(("float32(%s)@%g" % (key, v), f32, np.float32, v, None))
-    torch.cuda.synchronize()
     shape = (n, n, n)
     flags = E.WANT_NORMALS
-    stream = torch.cuda.current_stream()
-    engines = (E.Engine(0), E.Engine(0))
-    for e in engines:
-        e.set_stream(stream.cuda_stream)
+    eng, stream = cuda_engine()
+    engines = (eng, cuda_engine()[0])
 
     def run_steps(t, dt, v, k):
         pending = None
@@ -121,12 +106,7 @@ def main():
     for _ in range(args.rounds):
         for name, t, dt, v, _ in arms:
             run_steps(t, dt, v, 4)
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record(stream)
-            run_steps(t, dt, v, args.steps)
-            e1.record(stream)
-            torch.cuda.synchronize()
-            per_round[name].append(e0.elapsed_time(e1) / args.steps)
+            per_round[name].append(window(stream, lambda: run_steps(t, dt, v, args.steps)) / args.steps)
 
     # end to end from page-locked host memory (mt3d_extract_host: pipelined upload, extraction, download)
     host = E.Engine(0)
@@ -151,11 +131,7 @@ def main():
         res["arms"][name] = dict(dtype=np.dtype(dt).name, isovalue=v, step_ms=round(float(np.median(ms)), 4),
                                  step_ms_rounds=[round(x, 4) for x in ms], stage1_bytes=n ** 3 * np.dtype(dt).itemsize,
                                  stages=stages[name], e2e=e2e[name], counts=counts[name])
-    line = json.dumps(res)
-    print(line)
-    if args.out:
-        with open(args.out, "w") as fh:
-            fh.write(line + "\n")
+    emit(res, args.out)
 
 
 if __name__ == "__main__":

@@ -19,24 +19,13 @@ Prints one JSON line (also written to --out).
 """
 import argparse
 import ctypes
-import json
 import os
-import subprocess
 import sys
 
 import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-
-
-def gpu_info():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
-                             text=True, timeout=30).stdout.strip().splitlines()
-        name, power = (x.strip() for x in out[0].split(","))
-        return dict(name=name, power_limit=power)
-    except Exception as e:                                      # the line still carries torch's device name
-        return dict(name=None, power_limit=None, error=str(e))
+from tools.benchkit import cuda_engine, emit, gpu_info, kernel_table, per_call  # noqa: E402
 
 
 def bytes_moved(nv, nt, nc, nv2, nt2, nc2, gsz):
@@ -58,20 +47,15 @@ def main():
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     import torch
-    from torch.profiler import ProfilerActivity, profile
     from contourist_b200 import engine as E
     from contourist_b200 import synthetic
     from oracle import mt3d_filter
-    assert torch.cuda.is_available(), "bench_keep_components measures on a CUDA device"
     dev = torch.device("cuda", 0)
     n = args.n
     shape = (n, n, n)
     value = 0.5
     field = synthetic.ct_like(n, device=dev)
-    torch.cuda.synchronize()
-    stream = torch.cuda.current_stream()
-    eng = E.Engine(0)
-    eng.set_stream(stream.cuda_stream)
+    eng, stream = cuda_engine()
     nv_, nt_, nc_ = ctypes.c_int64(), ctypes.c_int64(), ctypes.c_int64()
 
     res = dict(tool="bench_keep_components", n=n, calls=args.calls, gpu=gpu_info(), device=torch.cuda.get_device_name(0),
@@ -107,32 +91,8 @@ def main():
                 eng._check(eng.lib.ctr_mt3d_keep_components(eng.h, mp, len(mask), ctypes.byref(nv_), ctypes.byref(nt_)),
                            "ctr_mt3d_keep_components")
 
-            ms = []
-            for q in range(args.calls + 2):                       # two untimed calls first
-                prepare()
-                torch.cuda.synchronize()
-                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                e0.record(stream)
-                keep()
-                e1.record(stream)
-                torch.cuda.synchronize()
-                if q >= 2:
-                    ms.append(e0.elapsed_time(e1))
-            prepare()
-            torch.cuda.synchronize()
-            with profile(activities=[ProfilerActivity.CUDA]) as prof:
-                keep()
-                torch.cuda.synchronize()
-            kernel_us = {}
-            for ev in prof.key_averages():
-                key = ev.key
-                tag = next((t_ for t_ in ("k_keep_", "k_sel_", "k_flag_scan", "Memcpy", "Memset") if t_ in key), None)
-                if tag is None:
-                    continue
-                short = key[key.index(tag):].split("(")[0].split("<")[0] if tag.startswith("k_") else key
-                tot = getattr(ev, "device_time_total", None)
-                tot = ev.cuda_time_total if tot is None else tot
-                kernel_us[short] = dict(launches=ev.count, us_per_launch=round(tot / max(ev.count, 1), 2))
+            ms = per_call(stream, keep, args.calls, 2, setup=prepare)
+            kernel_us = kernel_table(keep, ("k_keep_", "k_sel_", "k_flag_scan", "Memcpy", "Memset"), setup=prepare)
             gsz = 8 if gflag else 4
             res.setdefault(geom, {})[name] = dict(
                 n_verts=len(pre["verts"]), n_tris=len(pre["tris"]), n_components=len(tab), kept_verts=int(nv_.value),
@@ -141,11 +101,7 @@ def main():
                 bytes_moved=bytes_moved(len(pre["verts"]), len(pre["tris"]), len(tab), int(nv_.value), int(nt_.value),
                                         int(mask.sum()), gsz),
                 equal=equal)
-    line = json.dumps(res)
-    print(line)
-    if args.out:
-        with open(args.out, "w") as fh:
-            fh.write(line + "\n")
+    emit(res, args.out)
 
 
 if __name__ == "__main__":

@@ -16,24 +16,13 @@ Prints one JSON line (also written to --out).
 """
 import argparse
 import ctypes
-import json
 import os
-import subprocess
 import sys
 
 import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-
-
-def gpu_info():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
-                             text=True, timeout=30).stdout.strip().splitlines()
-        name, power = (x.strip() for x in out[0].split(","))
-        return dict(name=name, power_limit=power)
-    except Exception as e:                                      # the line still carries torch's device name
-        return dict(name=None, power_limit=None, error=str(e))
+from tools.benchkit import cuda_engine, emit, gpu_info, kernel_table, per_call  # noqa: E402
 
 
 def same(polys, want):
@@ -58,19 +47,14 @@ def main():
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     import torch
-    from torch.profiler import ProfilerActivity, profile
     from contourist_b200 import engine as E
     from contourist_b200 import synthetic
     from oracle import mt3d_section
-    assert torch.cuda.is_available(), "bench_section measures on a CUDA device"
     dev = torch.device("cuda", 0)
     n = args.n
     shape = (n, n, n)
     field = synthetic.ct_like(n, device=dev)
-    torch.cuda.synchronize()
-    stream = torch.cuda.current_stream()
-    eng = E.Engine(0)
-    eng.set_stream(stream.cuda_stream)
+    eng, stream = cuda_engine()
 
     res = dict(tool="bench_section", n=n, calls=args.calls, gpu=gpu_info(), device=torch.cuda.get_device_name(0))
     for gname, gflag in (("fp32", 0), ("fp64", E.GEOM_F64)):
@@ -85,46 +69,26 @@ def main():
             equal = bool(np.array_equal(seg["plane"], want["plane"]) and np.array_equal(seg["edges"], want["edges"]) and
                          np.array_equal(seg["points"], want["points"]) and same(polys, want["polylines"]))
             del seg, want
-            ms = []
             c, p = E.SectionCounts(), E.SectionParams()
             for a in range(3):
                 p.normal[a] = normal[a]
             off = np.ascontiguousarray(offs, np.float64)
             p.offsets = off.ctypes.data
             p.nplanes = len(off)
-            for q in range(args.calls + 2):                       # two untimed calls first
-                torch.cuda.synchronize()
-                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                e0.record(stream)
+
+            def section():
                 eng._check(eng.lib.ctr_mt3d_section(eng.h, ctypes.byref(p), ctypes.byref(c)), "ctr_mt3d_section")
-                e1.record(stream)
-                torch.cuda.synchronize()
-                if q >= 2:
-                    ms.append(e0.elapsed_time(e1))
-            with profile(activities=[ProfilerActivity.CUDA]) as prof:
-                eng.mt3d_section(normal, offs)
-                torch.cuda.synchronize()
-            kernel_us = {}
-            for ev in prof.key_averages():
-                key = ev.key
-                tag = next((t_ for t_ in ("k_sec_", "k_p_", "k_ps_", "k_m_", "k_o_", "k_s_", "Memcpy", "Memset") if t_ in key), None)
-                if tag is None:
-                    continue
-                short = key[key.index(tag):].split("(")[0].split("<")[0] if tag.startswith("k_") else key
-                tot = getattr(ev, "device_time_total", None)
-                tot = ev.cuda_time_total if tot is None else tot
-                kernel_us[short] = dict(launches=ev.count, us_per_launch=round(tot / max(ev.count, 1), 2))
+
+            ms = per_call(stream, section, args.calls, 2)
+            kernel_us = kernel_table(lambda: eng.mt3d_section(normal, offs),
+                                     ("k_sec_", "k_p_", "k_ps_", "k_m_", "k_o_", "k_s_", "Memcpy", "Memset"))
             res["%s_%s" % (gname, cname)] = dict(
                 n_verts=int(c0.n_verts), n_tris=int(c0.n_tris), n_segments=int(c.n_segments),
                 n_polylines=int(c.n_polylines), n_points=int(c.n_points), n_junction_planes=int(c.n_junction_planes),
                 call_ms=round(float(np.median(ms)), 4), calls_ms=[round(x, 4) for x in ms], kernel_us=kernel_us,
                 equal=equal)
         del mesh
-    line = json.dumps(res)
-    print(line)
-    if args.out:
-        with open(args.out, "w") as fh:
-            fh.write(line + "\n")
+    emit(res, args.out)
 
 
 if __name__ == "__main__":

@@ -20,39 +20,18 @@ waits for the counters).  Reported per mesh:
 Prints one JSON line (also written to --out).
 """
 import argparse
-import json
 import os
-import subprocess
 import sys
 
 import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-
-
-def gpu_info():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
-                             text=True, timeout=30).stdout.strip().splitlines()
-        name, power = (x.strip() for x in out[0].split(","))
-        return dict(name=name, power_limit=power)
-    except Exception as e:                                      # the line still carries torch's device name
-        return dict(name=None, power_limit=None, error=str(e))
+from tools.benchkit import cuda_engine, emit, gpu_info, kernel_table, normals_close, per_call  # noqa: E402
 
 
 def step_bytes(nv, n_free, total_deg):
     "one Jacobi step, neighbour rows assumed in L2: offsets of every vertex, ids and rows of the free vertices"
     return (nv + 1) * 4 + total_deg * 4 + n_free * 24 * 2
-
-
-def normals_close(got, want, verts, tris, geom64):
-    from oracle import mt3d_smooth
-    mag, parts = mt3d_smooth.face_normal_sums(verts, tris)
-    ok = (parts > 0) & (mag >= 1e-6 * parts)
-    g, w = got[ok].astype(np.float64), want[ok].astype(np.float64)
-    if geom64:
-        return bool(np.arctan2(np.linalg.norm(np.cross(g, w), axis=1), (g * w).sum(axis=1)).max(initial=0) < 1e-9)
-    return bool(np.abs(g - w).max(initial=0) <= 2e-6)
 
 
 def main():
@@ -62,20 +41,15 @@ def main():
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     import torch
-    from torch.profiler import ProfilerActivity, profile
     from contourist_b200 import engine as E
     from contourist_b200 import synthetic
     from oracle import mt3d_smooth
-    assert torch.cuda.is_available(), "bench_smooth measures on a CUDA device"
     dev = torch.device("cuda", 0)
     n = args.n
     shape = (n, n, n)
     field = synthetic.ct_like(n, device=dev)
     mask = (field > 0.5).to(torch.uint8)
-    torch.cuda.synchronize()
-    stream = torch.cuda.current_stream()
-    eng = E.Engine(0)
-    eng.set_stream(stream.cuda_stream)
+    eng, stream = cuda_engine()
 
     res = dict(tool="bench_smooth", n=n, calls=args.calls, gpu=gpu_info(), device=torch.cuda.get_device_name(0),
                lam=0.5, mu=-0.53)
@@ -96,35 +70,8 @@ def main():
         off, nbr, fixed, _ = mt3d_smooth.neighbours(len(pre["verts"]), pre["tris"])
         nv, nt, n_free = len(pre["verts"]), len(pre["tris"]), int((~fixed).sum())
         del pre, out, want, off, fixed
-
-        def timed(iterations):
-            ms = []
-            for q in range(args.calls + 2):                       # two untimed calls first
-                torch.cuda.synchronize()
-                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                e0.record(stream)
-                eng.mt3d_smooth(iterations)
-                e1.record(stream)
-                torch.cuda.synchronize()
-                if q >= 2:
-                    ms.append(e0.elapsed_time(e1))
-            return ms
-
-        t0, t10, t20 = timed(0), timed(10), timed(20)
-        torch.cuda.synchronize()
-        with profile(activities=[ProfilerActivity.CUDA]) as prof:
-            eng.mt3d_smooth(10)
-            torch.cuda.synchronize()
-        kernel_us = {}
-        for ev in prof.key_averages():
-            key = ev.key
-            tag = next((t_ for t_ in ("k_s_", "k_m_", "Memcpy", "Memset") if t_ in key), None)
-            if tag is None:
-                continue
-            short = key[key.index(tag):].split("(")[0].split("<")[0] if tag.startswith("k_") else key
-            tot = getattr(ev, "device_time_total", None)
-            tot = ev.cuda_time_total if tot is None else tot
-            kernel_us[short] = dict(launches=ev.count, us_per_launch=round(tot / max(ev.count, 1), 2))
+        t0, t10, t20 = (per_call(stream, lambda: eng.mt3d_smooth(it), args.calls, 2) for it in (0, 10, 20))
+        kernel_us = kernel_table(lambda: eng.mt3d_smooth(10), ("k_s_", "k_m_", "Memcpy", "Memset"))
         step_us = (float(np.median(t20)) - float(np.median(t0))) / 40 * 1000
         sb = step_bytes(nv, n_free, len(nbr))
         res[name] = dict(n_verts=nv, n_tris=nt,
@@ -135,11 +82,7 @@ def main():
                                        it20=[round(x, 4) for x in t20]),
                          step_bytes=sb, step_gbs=round(sb / step_us / 1e3, 1), kernel_us=kernel_us, equal=equal)
         del nbr
-    line = json.dumps(res)
-    print(line)
-    if args.out:
-        with open(args.out, "w") as fh:
-            fh.write(line + "\n")
+    emit(res, args.out)
 
 
 if __name__ == "__main__":

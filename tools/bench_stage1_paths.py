@@ -11,14 +11,13 @@ Per path: the step time (CUDA events over --steps runs after --warmup), stage 1 
 """
 import argparse
 import hashlib
-import json
 import os
 import sys
 
 import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from tools.bench_dtypes import gpu_info  # noqa: E402
+from tools.benchkit import cuda_engine, emit, gpu_info, window  # noqa: E402
 
 
 def digest(out):
@@ -29,20 +28,6 @@ def digest(out):
             h.update(k.encode())
             h.update(np.ascontiguousarray(v).tobytes())
     return h.hexdigest()
-
-
-def timed(run, steps, warmup, stream):
-    import torch
-    for _ in range(warmup):
-        run()
-    torch.cuda.synchronize()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record(stream)
-    for _ in range(steps):
-        run()
-    e1.record(stream)
-    torch.cuda.synchronize()
-    return e0.elapsed_time(e1) / steps
 
 
 def stage1_ms(eng, run, k=10):
@@ -67,11 +52,20 @@ def main():
     import torch
     from contourist_b200 import engine as E
     from contourist_b200 import synthetic
-    assert torch.cuda.is_available(), "bench_stage1_paths measures on a CUDA device"
     dev = torch.device("cuda", 0)
-    eng = E.Engine(0)
-    stream = torch.cuda.current_stream()
-    eng.set_stream(stream.cuda_stream)
+    eng, stream = cuda_engine()
+
+    def timed(run):
+        "ms per step: --steps runs in one window, after --warmup untimed ones"
+        for _ in range(args.warmup):
+            run()
+        torch.cuda.synchronize()
+
+        def steps():
+            for _ in range(args.steps):
+                run()
+        return window(stream, steps) / args.steps
+
     res = dict(tool="bench_stage1_paths", lib=E.LIB_PATH, gpu=gpu_info(), device=torch.cuda.get_device_name(0),
                steps=args.steps, warmup=args.warmup, paths={})
 
@@ -85,7 +79,7 @@ def main():
 
     def run3(flags=E.WANT_NORMALS):
         return eng.mt3d_run(ptr, 0.5, shape=shape3, dtype=np.float32, flags=flags | E.FIELD_ON_DEVICE)
-    ms = timed(run3, args.steps, args.warmup, stream)
+    ms = timed(run3)
     s1 = stage1_ms(eng, run3)
     c = run3(E.WANT_NORMALS | E.WANT_MINMAX)
     res["paths"]["generic"] = dict(shape=list(shape3), ms_per_step=round(ms, 4), stage1_ms=round(s1, 4),
@@ -99,7 +93,7 @@ def main():
 
     def run4(flags=E.MORPH):
         return eng.mp4d_run(f.data_ptr(), 1.2, shape=shape4, dtype=np.float32, flags=flags | E.FIELD_ON_DEVICE)
-    ms = timed(run4, args.steps, args.warmup, stream)
+    ms = timed(run4)
     s1 = stage1_ms(eng, run4)
     c = run4(E.MORPH | E.WANT_MINMAX)
     res["paths"]["4d"] = dict(shape=list(shape4), ms_per_step=round(ms, 4), stage1_ms=round(s1, 4),
@@ -107,11 +101,7 @@ def main():
                                           fmin=c.fmin, fmax=c.fmax),
                               sha256=digest(eng.mp4d_fetch()))
     eng.close()
-    line = json.dumps(res)
-    print(line)
-    if args.out:
-        with open(args.out, "w") as fh:
-            fh.write(line + "\n")
+    emit(res, args.out)
 
 
 if __name__ == "__main__":

@@ -15,20 +15,13 @@ import argparse
 import json
 import os
 import re
-import subprocess
 import sys
 from collections import OrderedDict
 
 import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-
-
-def gpu_info():
-    out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
-                         text=True, timeout=30).stdout.strip().splitlines()
-    name, power = (x.strip() for x in out[0].split(","))
-    return name, power
+from tools.benchkit import gpu_info  # noqa: E402
 
 
 def kernel_times(trace_path):
@@ -83,9 +76,9 @@ def main():
         torch.cuda.synchronize()
     trace = os.path.join(args.out, "trace.json")
     prof.export_chrome_trace(trace)
-    name, power = gpu_info()
+    gpu = gpu_info()
     print("%s%s, power limit %s: %d extractions of %d^3 (%d vertices, %d triangles), mean device time per launch"
-          % (args.label + ": " if args.label else "", name, power, args.iters, n, c.n_verts, c.n_tris))
+          % (args.label + ": " if args.label else "", gpu["name"], gpu["power_limit"], args.iters, n, c.n_verts, c.n_tris))
     per = kernel_times(trace)
     for k, v in per.items():
         print("  %-24s %6d launches %9.2f us" % (k, len(v), sum(v) / len(v)))
